@@ -6,11 +6,16 @@ actor-critic in the loop) -> GAE -> `epochs` x `n_minibatches` fused loss/grad +
 updates, over synthetic env batches of the named shape with random-init weights.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--repeats R] [--impl ours|reference] [--workload c2|c3|c4|c5]
+                  [--dump-outputs DIR]
 
 The default line measures C2 (BASELINE configs[1]) as `value` and carries C4 (65 536 envs/GPU, every N) and C3 (one GPU) under
 `workloads`; --workload c5 runs the rollout-only sweep.
 
-N > 1 is launched by the driver with torch.distributed.run (one rank per GPU): envs shard across
+The timed steps of a workload are exactly K iterations, after a fixed number of untimed ones (the workload's `warmup`, or W if
+larger), so the state every step starts from depends only on the arguments.  --dump-outputs DIR writes what the last timed
+step of the main workload returned (dump_outputs()), to compare two builds output for output.
+
+N > 1 is launched with torch.distributed.run (one rank per GPU): envs shard across
 ranks (weak scaling: per-GPU env count fixed), gradients are allreduced over NVLink peer memory per minibatch
 (NCCL fallback with DRIL_NO_P2P=1).
 Prints ONE JSON line on rank 0.
@@ -27,18 +32,23 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the benchmark leaves the source tree as it found it (it may be read-only)
 
+# warmup: untimed iterations before the timed steps, about 0.3 s of work on one B200 (sustained clocks, steady-state enqueue
+# path).  A fixed count, not a time, because what an iteration costs depends on how far training has come: on a B200 at its
+# 1000 W limit a C2 iteration takes 1.61 ms after 3 iterations and 1.67 ms after 190.
 WORKLOADS = {
     # BASELINE.json configs[1]: the configuration the metric is quoted on (fits one GPU)
     "c2": dict(name="PPO CartPole, 4096 batched envs/GPU, n_steps=128, hidden [64,64], discrete categorical policy",
-               kind="cartpole", n_envs=4096, n_steps=128, hidden=[64, 64], normalize=False),
+               kind="cartpole", n_envs=4096, n_steps=128, hidden=[64, 64], normalize=False, warmup=190),
     "c3": dict(name="PPO Pendulum diag-Gaussian, 16384 envs/GPU, n_steps=128, hidden [128,128,64], NormalizeWrapperEnv obs+reward",
-               kind="pendulum", n_envs=16384, n_steps=128, hidden=[128, 128, 64], normalize=True),
+               kind="pendulum", n_envs=16384, n_steps=128, hidden=[128, 128, 64], normalize=True, warmup=15),
     "c4": dict(name="PPO CartPole, 65536 envs/GPU data-parallel, n_steps=128, hidden [64,64]",
-               kind="cartpole", n_envs=65536, n_steps=128, hidden=[64, 64], normalize=False),
+               kind="cartpole", n_envs=65536, n_steps=128, hidden=[64, 64], normalize=False, warmup=18),
 }
 EPOCHS, N_MINIBATCHES = 4, 4          # BASELINE.json does not fix these (SURVEY §8d); stated with every number
 METRIC, UNIT = "end-to-end PPO env-steps/sec", "env-steps/s"
+DUMP_BYTES = 64 * 10 ** 6             # --dump-outputs: the whole dump stays below this
 
 
 def peaks():
@@ -129,10 +139,33 @@ def dist_setup(n_gpus):
     return rank, world, local, None
 
 
-def measure(D, ctx, dist, rank, world, local, wname, steps, repeats, warmup, p2p_state, clock_sampler=None):
-    """One workload on this rank's GPU: `repeats` timed blocks of `steps` PPO iterations (CUDA events on the library's stream,
-    L2 flushed before every iteration, max over ranks per block, median over blocks), the same through train! (wall clock),
-    and a per-kernel CUDA-event profile.  Returns a dict; every rank must call it with the same arguments."""
+def dump_outputs(out_dir, agent, buf, stats):
+    """Writes what one PPO iteration hands its caller, as out_dir/<name>.npy in float32 or float64: the updated policy
+    parameters (params), the iteration statistics without its two timings (stat_<field>) and every rollout buffer field
+    (buf_<field>, time-major [n_steps, n_envs, ...]).  When the buffer would take the dump above DUMP_BYTES, its fields keep a
+    fixed, seeded sample of env columns; env_index lists the columns kept."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"params": agent.device.get_params()}
+    out.update({"stat_" + k: np.array([v], np.float64) for k, v in stats.as_dict().items() if k not in ("rollout_ms", "update_ms")})
+    fields = {f: buf.download(f) for f in ("obs", "actions", "rewards", "values", "logprobs", "advantages", "returns", "flags",
+                                           "boot", "last_values", "episode_r", "episode_l")}
+    n_envs = buf.n_envs
+    per_env = 8 + sum(4 * a.size // n_envs for a in fields.values())                # float32 columns + their env_index entry
+    fixed = sum(a.nbytes for a in out.values()) + 128 * (len(out) + len(fields) + 1)  # + one .npy header per file
+    keep = min(n_envs, (DUMP_BYTES - fixed) // per_env)
+    idx = np.arange(n_envs) if keep == n_envs else np.sort(np.random.default_rng(0).choice(n_envs, keep, replace=False))
+    out["env_index"] = idx.astype(np.float64)
+    for f, a in fields.items():
+        out["buf_" + f] = (a[idx] if f == "last_values" else a[:, idx]).astype(np.float32)   # flags, actions, lengths: exact
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure(D, ctx, dist, rank, world, local, wname, steps, repeats, warmup, p2p_state, clock_sampler=None, dump_dir=None):
+    """One workload on this rank's GPU: `steps` timed PPO iterations in `repeats` (or fewer) equal blocks (CUDA events on the
+    library's stream, L2 flushed before every iteration, max over ranks per block, median over blocks), the same through
+    train! (wall clock), and a per-kernel CUDA-event profile.  With dump_dir, rank 0 writes what the last timed iteration
+    returned there.  Returns a dict; every rank must call it with the same arguments."""
     import ctypes as C
     from dril_b200 import _lib as L
     w = WORKLOADS[wname]
@@ -201,35 +234,37 @@ def measure(D, ctx, dist, rank, world, local, wname, steps, repeats, warmup, p2p
     # every allocation up front, then all ranks together: no rank sits in a cudaMalloc while a peer's GPU already spins in an exchange
     L.check(lib.dril_iteration_prepare(env.h, agent.device.h, buf.h, int(alg.epochs), int(alg.batch_size)))
     barrier()
-    # ---- warm-up: at least W (>= 3) iterations and at least 0.3 s of work (sustained clocks, steady-state enqueue path) ----
-    t_w = time.perf_counter()
-    n_w = 0
-    while n_w < max(warmup, 3) or time.perf_counter() - t_w < 0.3:
+    # ---- warm-up: max(W, the workload's warm-up) untimed steps, each like a timed one (the first flush allocates its buffer).
+    # A fixed count: the timed steps start from a state that depends on the arguments only ----------------------------------
+    n_w = max(warmup, w["warmup"])
+    for _ in range(n_w):
+        ctx.flush_l2()
         iteration_async()
-        n_w += 1
-        if n_w % 3 == 0:
-            drain()
     drain()
-    # ---- value: `repeats` blocks of K iterations resident on the device, CUDA events on the launching stream -----------
+    # ---- value: K iterations resident on the device in up to `repeats` equal blocks, CUDA events on the launching stream ----
+    n_blocks = max(b for b in range(1, max(repeats, 1) + 1) if steps % b == 0)
+    per_block = steps // n_blocks
     barrier()
     if clock_sampler is not None:
         clock_sampler.start()
     launches0 = ctx.launch_count()
     block_ms = []
-    for _ in range(repeats):
+    for _ in range(n_blocks):
         barrier()
         ctx.event_record(0)
-        for _ in range(steps):
+        for _ in range(per_block):
             ctx.flush_l2()                  # inside the timed region: nothing stays L2-hot from the previous step
             iteration_async()
         ctx.event_record(1)
         barrier()
         block_ms.append(max_over_ranks(ctx.event_elapsed_ms(0, 1)))
     clocks = clock_sampler.stop() if clock_sampler is not None else None
-    launches = (ctx.launch_count() - launches0) // repeats
+    launches = (ctx.launch_count() - launches0) // n_blocks
     st = drain()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, agent, buf, st)
     ms = float(np.median(block_ms))
-    value = steps_per_iter * world * steps / (ms * 1e-3)
+    value = steps_per_iter * world * per_block / (ms * 1e-3)
 
     # ---- e2e: the public API call (train!) with host parameters in and statistics out (no L2 flush on this path) -------
     D.train(agent, env, alg, steps_per_iter * 3)       # warm-up of the public path (its rollout buffer is allocated once per agent)
@@ -262,9 +297,9 @@ def measure(D, ctx, dist, rank, world, local, wname, steps, repeats, warmup, p2p
     for name, (tms, n) in prof.items():
         if n:
             kern[name] = {"ms_per_step": tms / steps, "launches_per_step": n / steps, "share": tms / total_prof_ms}
-    res = dict(workload=w["name"], value=value, ms_per_step=ms / steps, block_ms=block_ms, repeats=repeats, steps=steps,
-               e2e=e2e_value, h2d=h2d, d2h=d2h, launches=int(launches), clocks=clocks, kernels=kern, comm=comm, batch=batch,
-               steps_per_iter=steps_per_iter, warmup_run=n_w, path=agent.device.update_path(),
+    res = dict(workload=w["name"], value=value, ms_per_step=ms / per_block, block_ms=block_ms, repeats=n_blocks, steps=steps,
+               per_block=per_block, e2e=e2e_value, h2d=h2d, d2h=d2h, launches=int(launches), clocks=clocks, kernels=kern, comm=comm,
+               batch=batch, steps_per_iter=steps_per_iter, warmup_run=n_w, path=agent.device.update_path(),
                layer_dims=[layer.layer_dims(0), layer.layer_dims(1)], obs_dim=env.obs_dim,
                last=({k: (v if np.isfinite(v) else None) for k, v in st.as_dict().items()}))
     buf.close(); env.close(); agent.device.close()
@@ -323,9 +358,10 @@ def run_ours(args):
     p2p_state = {}
     sampler = ClockSampler(local) if rank == 0 and not os.environ.get('BENCH_NO_SAMPLER') else None
     main_w = args.workload
-    res = measure(D, ctx, dist, rank, world, local, main_w, args.steps, args.repeats, args.warmup, p2p_state, sampler)
-    # the other BASELINE configs ride along in the same line (the driver only passes --gpus/--steps/--warmup): C4 (65 536
-    # envs/GPU, the data-parallel config) at every N, C3 (Pendulum, wide net, normaliser) on one GPU
+    res = measure(D, ctx, dist, rank, world, local, main_w, args.steps, args.repeats, args.warmup, p2p_state, sampler,
+                  dump_dir=args.dump_outputs)
+    # the other BASELINE configs ride along in the same line (a plain `--gpus/--steps/--warmup` run reports them too): C4
+    # (65 536 envs/GPU, the data-parallel config) at every N, C3 (Pendulum, wide net, normaliser) on one GPU
     extra = {}
     if main_w == "c2" and not args.no_extra:
         extra["c4"] = measure(D, ctx, dist, rank, world, local, "c4", max(2, args.steps // 4), min(args.repeats, 3), 3, p2p_state)
@@ -367,10 +403,11 @@ def run_ours(args):
                         "env_steps_per_step_per_gpu": r["steps_per_iter"], "adam_steps_per_step": EPOCHS * N_MINIBATCHES,
                         "l2": "value: flushed (256 MB memset on the stream before every timed step, inside the timed region); e2e (train!) "
                               "does not pay the flush", "warmup_iterations_run": r["warmup_run"],
-                        "timing": f"median of {r['repeats']} blocks of {r['steps']} steps (CUDA events, max over ranks per block)",
+                        "timing": f"{r['steps']} timed steps: median of {r['repeats']} blocks of {r['per_block']} steps (CUDA events, "
+                                  "max over ranks per block)",
                         "parallelism": f"dp{world} over envs, {r['comm']}" if world > 1 else "single GPU"}
     line = {
-        "metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
+        "metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": res["warmup_run"],
         "repeats": res["repeats"], "block_ms": res["block_ms"],
         "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
         "data": "synthetic (on-device env batches of the named shape, orthogonal random-init weights, seed 0)",
@@ -549,16 +586,24 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=20, help="timed PPO iterations")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed iterations before the timed ones (at least the workload's own)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=None, choices=list(WORKLOADS) + ["c5"])
-    ap.add_argument("--repeats", type=int, default=5, help="timed blocks of --steps iterations; the median block is reported")
+    ap.add_argument("--repeats", type=int, default=5,
+                    help="the --steps iterations run in this many equal blocks (fewer if it does not divide --steps); "
+                         "the median block is reported")
     ap.add_argument("--no-extra", action="store_true", help="C2 only: skip the C4 / C3 blocks under `workloads`")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed iteration of the main workload returned as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     if args.workload is None:
         args.workload = "c2"
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "c5"):
+        ap.error("--dump-outputs needs --impl ours and a PPO workload (c2, c3, c4)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -23,6 +23,45 @@ def test_reference_arm_json_line():
     assert "workload" in d["config"]
 
 
+def test_dump_outputs_sample_below_cap(tmp_path, monkeypatch):
+    """--dump-outputs with a rollout buffer larger than the cap: a seeded sample of env columns, float32 / float64 files only,
+    within the cap, the same columns every time."""
+    import importlib.util
+
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    from dril_b200 import _lib as L
+    T, N = 8, 1000
+
+    class Buf:
+        n_envs = N
+
+        def download(self, f):
+            shape = {"obs": (T, N, 4), "actions": (T, N, 1), "last_values": (N,)}.get(f, (T, N))
+            dt = {"flags": np.uint8, "episode_l": np.int32, "actions": np.int32}.get(f, np.float32)
+            return np.arange(np.prod(shape)).reshape(shape).astype(dt)
+
+    class Agent:
+        class device:
+            get_params = staticmethod(lambda: np.ones(100, np.float32))
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 200_000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), Agent, Buf(), L.IterStats())
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 200_000
+    idx = np.load(tmp_path / "a" / "env_index.npy")
+    assert 0 < idx.size < N and (np.diff(idx) > 0).all()
+    np.testing.assert_array_equal(idx, np.load(tmp_path / "b" / "env_index.npy"))
+    for n in names:
+        assert np.load(tmp_path / "a" / n).dtype in (np.float32, np.float64), n
+    obs = np.load(tmp_path / "a" / "buf_obs.npy")
+    np.testing.assert_array_equal(obs, Buf().download("obs")[:, idx.astype(int)])
+    assert "stat_rollout_ms.npy" not in names and "stat_loss.npy" in names
+
+
 def test_cited_profile_files_exist():
     cited = set()
     for doc in ("README.md", "DESIGN.md", os.path.join("profiles", "README.md")):
