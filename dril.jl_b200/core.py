@@ -9,7 +9,8 @@ import numpy as np
 from . import _lib as L
 from .spaces import Box, Discrete
 
-ENV_KINDS = {"cartpole": 0, "pendulum": 1, "synthetic": 2}
+ENV_KINDS = {"cartpole": 0, "pendulum": 1, "synthetic": 2, "mountaincar": 3, "mountaincar_continuous": 4, "acrobot": 5}
+ENV_STATE_DIMS = {"cartpole": 4, "pendulum": 2, "synthetic": 0, "mountaincar": 2, "mountaincar_continuous": 2, "acrobot": 4}
 
 
 class Context:
@@ -131,6 +132,15 @@ class CudaBatchedEnv:
             self.obs_dim, self.max_steps = 3, max_steps or 200
             hi = np.array([1, 1, 8], dtype=np.float32)
             self._obs_space, self._act_space = Box(-hi, hi), Box(np.array([-2.0], np.float32), np.array([2.0], np.float32))
+        elif self.kind in ("mountaincar", "mountaincar_continuous"):
+            cont = self.kind == "mountaincar_continuous"
+            self.obs_dim, self.max_steps = 2, max_steps or (999 if cont else 200)
+            self._obs_space = Box(np.array([-1.2, -0.07], np.float32), np.array([0.6, 0.07], np.float32))
+            self._act_space = Box(np.array([-1.0], np.float32), np.array([1.0], np.float32)) if cont else Discrete(3, act_start)
+        elif self.kind == "acrobot":
+            self.obs_dim, self.max_steps = 6, max_steps or 500
+            hi = np.array([1, 1, 1, 1, 4 * np.pi, 9 * np.pi], dtype=np.float32)
+            self._obs_space, self._act_space = Box(-hi, hi), Discrete(3, act_start)
         else:
             # multi-dimensional Box observations (test/test_buffers.jl:280-314): the feature extractor of the layer is a
             # parameter-free Flatten (layers/layer_helpers.jl:13-25), so the device works on prod(obs_shape) features and only
@@ -229,7 +239,7 @@ class CudaBatchedEnv:
 
     # ---- wrapper-specific -----------------------------------------------------
     def get_state(self):
-        sd = {"cartpole": 4, "pendulum": 2, "synthetic": 0}[self.kind]
+        sd = ENV_STATE_DIMS[self.kind]
         st = np.empty((max(sd, 1), self.n_envs), np.float32)
         steps = np.empty(self.n_envs, np.int32)
         L.check(self.ctx.lib.dril_env_get_state(self.h, L.ptr(st), L.ptr(steps)))

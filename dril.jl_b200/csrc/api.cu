@@ -78,10 +78,10 @@ extern "C" int32_t dril_set_option(const char* key, int32_t value) {
 // the tensor-core loss/grad kernel covers the reference's default layer: hidden_dims = [64, 64], obs_dim <= 4,
 // Discrete(n <= 2)
 // the general-shape features-on-lanes kernel (update_ftg.cuh): 2 or 3 hidden layers of width 64 / 128 (same in both nets),
-// obs_dim <= 15, Discrete(n <= 2) or Box of dimension <= 2, and everything resident in shared memory
+// obs_dim <= 15, Discrete(n <= 4) or Box of dimension <= 2, and everything resident in shared memory
 static bool ftg_eligible(const PolicyDesc& pd) {
     const int L = pd.n_layers - 1;
-    if (L < 2 || L > 3 || pd.obs_dim > FTG_MAX_OBS || pd.act_n > 2) return false;
+    if (L < 2 || L > 3 || pd.obs_dim > FTG_MAX_OBS || pd.act_n > (pd.act_kind == DRIL_ACT_DISCRETE ? 4 : 2)) return false;
     for (int l = 0; l < L; ++l) {
         if (pd.L[0][l].N != pd.L[1][l].N) return false;
         if (pd.L[0][l].N != 64 && pd.L[0][l].N != 128) return false;
@@ -95,6 +95,23 @@ static bool tc_eligible(const PolicyDesc& pd) {
         if (pd.L[net][2].Np != 4) return false;
     }
     return true;
+}
+
+// rollout kernels by the env kind they step: CartPole, Pendulum and the synthetic env run the instantiations built for those
+// kinds alone (env.cuh), every other kind the one built for all kinds
+static void* rollout_fn(bool ws, int kind) {
+    if (env_kind_set(kind) == ENV_KS_CLASSIC) return ws ? (void*)rollout_kernel<true, ENV_KS_CLASSIC> : (void*)rollout_kernel<false, ENV_KS_CLASSIC>;
+    return ws ? (void*)rollout_kernel<true, ENV_KS_ALL> : (void*)rollout_kernel<false, ENV_KS_ALL>;
+}
+static void* rollout_fast_fn(bool ws, int kind) {
+    if (env_kind_set(kind) == ENV_KS_CLASSIC) return ws ? (void*)rollout_fast_kernel<true, ENV_KS_CLASSIC> : (void*)rollout_fast_kernel<false, ENV_KS_CLASSIC>;
+    return ws ? (void*)rollout_fast_kernel<true, ENV_KS_ALL> : (void*)rollout_fast_kernel<false, ENV_KS_ALL>;
+}
+// tcgen05-actor rollout by hidden-layer count, env kind and action count (2 or 4 staged output columns, gtc_nout)
+static void* rollout_gtc_fn(int L, int kind, int act_n) {
+    if (act_n > 2) return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_ALL, 4> : (void*)rollout_gtc_kernel<3, ENV_KS_ALL, 4>;
+    if (env_kind_set(kind) == ENV_KS_CLASSIC) return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_CLASSIC, 2> : (void*)rollout_gtc_kernel<3, ENV_KS_CLASSIC, 2>;
+    return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_ALL, 2> : (void*)rollout_gtc_kernel<3, ENV_KS_ALL, 2>;
 }
 
 extern "C" int32_t dril_device_count(int32_t* count) {
@@ -335,10 +352,11 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
     c->seed = seed;
     c->sm_count = prop.multiProcessorCount;
     DRIL_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-    DRIL_CUDA(cudaFuncSetAttribute(rollout_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-    DRIL_CUDA(cudaFuncSetAttribute(rollout_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-    DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-    DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+    for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
+        for (int ws = 0; ws < 2; ++ws) {
+            DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, kind), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+            DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, kind), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+        }
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
     DRIL_CUDA(cudaFuncSetAttribute(ppo_loss_grad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
@@ -350,10 +368,14 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
         const void* fns[] = {(const void*)ppo_loss_grad_ftg_kernel<2, 0, 1>, (const void*)ppo_loss_grad_ftg_kernel<2, 0, 2>,
                              (const void*)ppo_loss_grad_ftg_kernel<2, 1, 1>, (const void*)ppo_loss_grad_ftg_kernel<2, 1, 2>,
                              (const void*)ppo_loss_grad_ftg_kernel<3, 0, 1>, (const void*)ppo_loss_grad_ftg_kernel<3, 0, 2>,
-                             (const void*)ppo_loss_grad_ftg_kernel<3, 1, 1>, (const void*)ppo_loss_grad_ftg_kernel<3, 1, 2>};
+                             (const void*)ppo_loss_grad_ftg_kernel<3, 1, 1>, (const void*)ppo_loss_grad_ftg_kernel<3, 1, 2>,
+                             (const void*)ppo_loss_grad_ftg_kernel<2, 0, 3>, (const void*)ppo_loss_grad_ftg_kernel<2, 0, 4>,
+                             (const void*)ppo_loss_grad_ftg_kernel<3, 0, 3>, (const void*)ppo_loss_grad_ftg_kernel<3, 0, 4>};
         for (const void* fn : fns) DRIL_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));   // 1 KB of static shared memory
-        DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
-        DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
+        for (int L = 2; L <= 3; ++L)
+            for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
+                for (int an = 2; an <= 4; an += 2)
+                    DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, kind, an), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
     }
@@ -957,7 +979,7 @@ extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, in
                                    int32_t act_start, int64_t gid_offset, const dril_norm_cfg* norm,
                                    int32_t monitor_window, dril_env** out) {
     DRIL_REQUIRE(c && out && n_envs >= 1, "bad env arguments");
-    DRIL_REQUIRE(kind >= DRIL_ENV_CARTPOLE && kind <= DRIL_ENV_SYNTHETIC, "unknown env kind %d", kind);
+    DRIL_REQUIRE(kind >= DRIL_ENV_CARTPOLE && kind <= DRIL_ENV_ACROBOT, "unknown env kind %d", kind);
     DRIL_REQUIRE(n_envs + gid_offset < (1ll << 32), "global env ids must fit 32 bits");
     DRIL_CUDA(cudaSetDevice(c->device));
     dril_env* e = new dril_env();
@@ -968,6 +990,9 @@ extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, in
     d.kind = kind; d.n_envs = n_envs; d.gid_offset = gid_offset; d.seed = c->seed; d.act_start = act_start;
     if (kind == DRIL_ENV_CARTPOLE) { d.obs_dim = 4; d.state_dim = 4; d.act_dim = 0; d.max_steps = max_steps > 0 ? max_steps : 500; }
     else if (kind == DRIL_ENV_PENDULUM) { d.obs_dim = 3; d.state_dim = 2; d.act_dim = 1; d.max_steps = max_steps > 0 ? max_steps : 200; }
+    else if (kind == DRIL_ENV_MOUNTAINCAR) { d.obs_dim = 2; d.state_dim = 2; d.act_dim = 0; d.max_steps = max_steps > 0 ? max_steps : 200; }
+    else if (kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS) { d.obs_dim = 2; d.state_dim = 2; d.act_dim = 1; d.max_steps = max_steps > 0 ? max_steps : 999; }
+    else if (kind == DRIL_ENV_ACROBOT) { d.obs_dim = 6; d.state_dim = 4; d.act_dim = 0; d.max_steps = max_steps > 0 ? max_steps : 500; }
     else {
         DRIL_REQUIRE(obs_dim >= 1 && obs_dim <= DRIL_MAX_OBS_DIM, "synthetic obs_dim %d out of range", obs_dim);
         d.obs_dim = obs_dim; d.state_dim = 0; d.act_dim = 0; d.max_steps = max_steps > 0 ? max_steps : 500;
@@ -1184,9 +1209,8 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.M4 = M4; a.flags = flags | (ws ? RO_WEIGHTS_SMEM : 0);
             a.n_tiles = (int)((N + M4 - 1) / M4);
             Span sp(c, DRIL_K_ROLLOUT);
-            if (ws) rollout_fast_kernel<true><<<a.n_tiles, threads, tot(M4, threads, ws), c->stream>>>(a);
-            else rollout_fast_kernel<false><<<a.n_tiles, threads, tot(M4, threads, ws), c->stream>>>(a);
-            DRIL_CUDA(cudaGetLastError());
+            void* args[] = {(void*)&a};
+            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, d.kind), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
             return DRIL_OK;
         }
     }
@@ -1223,7 +1247,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.M4 = GTC_ENVS; a.flags = flags;
             a.n_tiles = (int)((N + GTC_ENVS - 1) / GTC_ENVS);
             int grid = a.n_tiles, body_i = (int)body;
-            void* fn = a.pd.n_layers - 1 == 2 ? (void*)rollout_gtc_kernel<2> : (void*)rollout_gtc_kernel<3>;
+            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, d.kind, a.pd.act_n);
             void* args[] = {(void*)&a, (void*)&gl, (void*)&body_i};
             {
                 Span sp(c, DRIL_K_ROLLOUT);
@@ -1285,17 +1309,14 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     Span sp(c, has_policy ? DRIL_K_ROLLOUT : DRIL_K_ENV);
     if (flags & RO_GRID_SYNC) {
         int per_sm = 0;
-        if (ws) DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_kernel<true>, threads, smem));
-        else DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_kernel<false>, threads, smem));
+        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, d.kind), threads, smem));
         DRIL_REQUIRE(per_sm >= 1, "rollout kernel does not fit on an SM");
         grid = std::min(grid, std::min(per_sm * c->sm_count, e->max_blocks));
         void* args[] = {(void*)&a};
-        void* fn = ws ? (void*)rollout_kernel<true> : (void*)rollout_kernel<false>;
-        DRIL_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, d.kind), dim3(grid), dim3(threads), args, smem, c->stream));
     } else {
-        if (ws) rollout_kernel<true><<<grid, threads, smem, c->stream>>>(a);
-        else rollout_kernel<false><<<grid, threads, smem, c->stream>>>(a);
-        DRIL_CUDA(cudaGetLastError());
+        void* args[] = {(void*)&a};
+        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, d.kind), dim3(grid), dim3(threads), args, smem, c->stream));
     }
     if (defer) return launch_critic();
     return DRIL_OK;
@@ -1413,7 +1434,8 @@ extern "C" int32_t dril_env_set_scaling(dril_env* e, int32_t on, const float* ob
     if (!on) { e->d.scaling = 0; return DRIL_OK; }
     DRIL_REQUIRE(obs_low && obs_high && act_low && act_high, "NULL bounds");
     // ScalingWrapperEnv needs Box observation and action spaces (scalingWrapperEnv.jl:22): of the built-in envs that is Pendulum
-    DRIL_REQUIRE(e->d.kind == DRIL_ENV_PENDULUM, "ScalingWrapperEnv: Box observation and action spaces required (pendulum)");
+    DRIL_REQUIRE(e->d.kind == DRIL_ENV_PENDULUM || e->d.kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS,
+                 "ScalingWrapperEnv: Box observation and action spaces required (pendulum, mountaincar_continuous)");
     DRIL_REQUIRE(e->d.obs_dim <= 4 && e->d.act_dim == 1, "ScalingWrapperEnv: obs_dim <= 4, act_dim == 1");
     for (int j = 0; j < e->d.obs_dim; ++j) {
         e->d.sc_obs_f[j] = 2.0f / (obs_high[j] - obs_low[j]);                     // :37-39
@@ -1468,6 +1490,10 @@ static int32_t check_compat(dril_env* e, dril_policy* p, dril_buffer* b) {
     if (p->pd.act_kind == DRIL_ACT_CONTINUOUS) DRIL_REQUIRE(b->d.act_dim == p->pd.act_n, "act_dim mismatch");
     if (e->d.kind == DRIL_ENV_CARTPOLE) DRIL_REQUIRE(p->pd.act_kind == DRIL_ACT_DISCRETE && p->pd.act_n == 2, "CartPole needs Discrete(2)");
     if (e->d.kind == DRIL_ENV_PENDULUM) DRIL_REQUIRE(p->pd.act_kind == DRIL_ACT_CONTINUOUS && p->pd.act_n == 1, "Pendulum needs Box (1,)");
+    if (e->d.kind == DRIL_ENV_MOUNTAINCAR) DRIL_REQUIRE(p->pd.act_kind == DRIL_ACT_DISCRETE && p->pd.act_n == 3, "MountainCar needs Discrete(3)");
+    if (e->d.kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS)
+        DRIL_REQUIRE(p->pd.act_kind == DRIL_ACT_CONTINUOUS && p->pd.act_n == 1, "MountainCarContinuous needs Box (1,)");
+    if (e->d.kind == DRIL_ENV_ACROBOT) DRIL_REQUIRE(p->pd.act_kind == DRIL_ACT_DISCRETE && p->pd.act_n == 3, "Acrobot needs Discrete(3)");
     return DRIL_OK;
 }
 
@@ -1828,9 +1854,11 @@ static const void* ftg_kernel(const PolicyDesc& pd) {
     const int L = pd.n_layers - 1, cont = pd.act_kind == DRIL_ACT_CONTINUOUS ? 1 : 0, n = pd.act_n;
     if (L == 2) {
         if (cont) return n == 1 ? (const void*)ppo_loss_grad_ftg_kernel<2, 1, 1> : (const void*)ppo_loss_grad_ftg_kernel<2, 1, 2>;
+        if (n > 2) return n == 3 ? (const void*)ppo_loss_grad_ftg_kernel<2, 0, 3> : (const void*)ppo_loss_grad_ftg_kernel<2, 0, 4>;
         return n == 1 ? (const void*)ppo_loss_grad_ftg_kernel<2, 0, 1> : (const void*)ppo_loss_grad_ftg_kernel<2, 0, 2>;
     }
     if (cont) return n == 1 ? (const void*)ppo_loss_grad_ftg_kernel<3, 1, 1> : (const void*)ppo_loss_grad_ftg_kernel<3, 1, 2>;
+    if (n > 2) return n == 3 ? (const void*)ppo_loss_grad_ftg_kernel<3, 0, 3> : (const void*)ppo_loss_grad_ftg_kernel<3, 0, 4>;
     return n == 1 ? (const void*)ppo_loss_grad_ftg_kernel<3, 0, 1> : (const void*)ppo_loss_grad_ftg_kernel<3, 0, 2>;
 }
 static int32_t ftg_stage_epoch(dril_policy* p, const BufDev& bd, const FeistelKey& fk, long long n_total, long long batch_size, int identity) {

@@ -2,14 +2,27 @@
 //
 // The reference takes CartPole / Pendulum from the un-vendored ClassicControlEnvironments.jl
 // (call sites README.md:50,76; benchmark/bench_utils.jl:14,20); these follow the Gymnasium
-// CartPole-v1 / Pendulum-v1 equations exactly as restated in oracle/envs.py.  Every fp32
-// operation uses a round-to-nearest intrinsic (never contracted into FMA) and sin/cos are the
-// correctly rounded fp32 values (fp64 evaluation, one rounding), so replayed action sequences
-// reproduce the oracle bit for bit.
+// CartPole-v1 / Pendulum-v1 / MountainCar-v0 / MountainCarContinuous-v0 / Acrobot-v1 equations
+// exactly as restated in oracle/envs.py and oracle/classic_envs.py.  Every fp32 operation uses a round-to-nearest intrinsic
+// (never contracted into FMA) and sin/cos are the correctly rounded fp32 values (fp64 evaluation,
+// one rounding), so replayed action sequences reproduce the oracle bit for bit.
+//
+// This file is the only place that branches on the env kind.  The kernels take the set of kinds
+// they are built for as a template argument (ENV_KS_*): the instantiations for CartPole, Pendulum
+// and the synthetic env contain exactly the code they had before MountainCar and Acrobot existed
+// (Acrobot's RK4 step and 6-wide observation do not enter their register budget).
 #pragma once
 #include "common.cuh"
 
 #define ENV_MAX_STATE 4
+#define ENV_KS_CLASSIC ((1u << DRIL_ENV_CARTPOLE) | (1u << DRIL_ENV_PENDULUM) | (1u << DRIL_ENV_SYNTHETIC))
+#define ENV_KS_ALL (ENV_KS_CLASSIC | (1u << DRIL_ENV_MOUNTAINCAR) | (1u << DRIL_ENV_MOUNTAINCAR_CONTINUOUS) | (1u << DRIL_ENV_ACROBOT))
+
+__host__ __device__ constexpr bool env_in(unsigned ks, int kind) { return (ks >> kind) & 1u; }
+// blocks of four observation components a kernel built for the kinds `ks` handles (Acrobot: 6 components)
+__host__ __device__ constexpr int env_obs_blocks(unsigned ks) { return env_in(ks, DRIL_ENV_ACROBOT) ? 2 : 1; }
+// the kind set whose instantiation serves env kind `kind`
+__host__ __device__ constexpr unsigned env_kind_set(int kind) { return env_in(ENV_KS_CLASSIC, kind) ? ENV_KS_CLASSIC : ENV_KS_ALL; }
 
 __device__ __forceinline__ void sincos_rn(float th, float* s, float* c) {
     double sd, cd;
@@ -18,9 +31,20 @@ __device__ __forceinline__ void sincos_rn(float th, float* s, float* c) {
     *c = (float)cd;
 }
 
-// raw observation d-th component from state (CartPole / Pendulum only)
-__device__ __forceinline__ void env_raw_obs(int kind, const float* st, float* o) {
-    if (kind == DRIL_ENV_CARTPOLE) {
+// observation components 4b .. 4b+3 of a state-based env (zero beyond obs_dim)
+template <unsigned KS>
+__device__ __forceinline__ void env_raw_obs_block(int kind, const float* st, int b, float* o) {
+    if (env_in(KS, DRIL_ENV_ACROBOT) && kind == DRIL_ENV_ACROBOT) {   // (cos th1, sin th1, cos th2, sin th2 | w1, w2)
+        if (b == 0) {
+            sincos_rn(st[0], &o[1], &o[0]);
+            sincos_rn(st[1], &o[3], &o[2]);
+        } else {
+            o[0] = st[2]; o[1] = st[3]; o[2] = 0.f; o[3] = 0.f;
+        }
+    } else if ((env_in(KS, DRIL_ENV_MOUNTAINCAR) && kind == DRIL_ENV_MOUNTAINCAR) ||
+               (env_in(KS, DRIL_ENV_MOUNTAINCAR_CONTINUOUS) && kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS)) {   // (position, velocity)
+        o[0] = st[0]; o[1] = st[1]; o[2] = 0.f; o[3] = 0.f;
+    } else if (kind == DRIL_ENV_CARTPOLE) {
         o[0] = st[0]; o[1] = st[1]; o[2] = st[2]; o[3] = st[3];
     } else {  // pendulum: (cos th, sin th, thdot)
         float s, c;
@@ -29,11 +53,13 @@ __device__ __forceinline__ void env_raw_obs(int kind, const float* st, float* o)
     }
 }
 
-// observation as the wrappers above the env see it: raw, or mapped to [-1, 1] by ScalingWrapperEnv.observe
-// (scalingWrapperEnv.jl:72-75,94-99: `(x - offset) * scale - 1`, three separate fp32 roundings)
-__device__ __forceinline__ void env_obs(const EnvDev& env, const float* st, float* o) {
-    env_raw_obs(env.kind, st, o);
-    if (env.scaling) {
+// observation block b as the wrappers above the env see it: raw, or mapped to [-1, 1] by ScalingWrapperEnv.observe
+// (scalingWrapperEnv.jl:72-75,94-99: `(x - offset) * scale - 1`, three separate fp32 roundings; Box/Box envs of
+// obs_dim <= 4 only, so block 0)
+template <unsigned KS>
+__device__ __forceinline__ void env_obs_block(const EnvDev& env, const float* st, int b, float* o) {
+    env_raw_obs_block<KS>(env.kind, st, b, o);
+    if (env.scaling && b == 0) {
 #pragma unroll
         for (int j = 0; j < 4; ++j)
             if (j < env.obs_dim) o[j] = __fsub_rn(__fmul_rn(__fsub_rn(o[j], env.sc_obs_o[j]), env.sc_obs_f[j]), 1.0f);
@@ -44,6 +70,7 @@ __device__ __forceinline__ float env_unscale_action(const EnvDev& env, float a) 
     return env.scaling ? __fadd_rn(__fdiv_rn(__fadd_rn(a, 1.0f), env.sc_act_f), env.sc_act_o) : a;
 }
 
+template <unsigned KS = ENV_KS_CLASSIC>
 __device__ __forceinline__ void env_reset_state(int kind, uint32_t gid, uint32_t episode, unsigned long long seed,
                                                 float* st) {
     uint32_t x[4];
@@ -55,6 +82,13 @@ __device__ __forceinline__ void env_reset_state(int kind, uint32_t gid, uint32_t
         st[0] = __fadd_rn(-3.14159274101257324f, __fmul_rn(6.28318548202514648f, u01_f32(x[0])));
         st[1] = __fadd_rn(-1.0f, __fmul_rn(2.0f, u01_f32(x[1])));
         st[2] = 0.f; st[3] = 0.f;
+    } else if ((env_in(KS, DRIL_ENV_MOUNTAINCAR) && kind == DRIL_ENV_MOUNTAINCAR) ||
+               (env_in(KS, DRIL_ENV_MOUNTAINCAR_CONTINUOUS) && kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS)) {
+        st[0] = __fadd_rn(-0.6f, __fmul_rn(0.2f, u01_f32(x[0])));
+        st[1] = 0.f; st[2] = 0.f; st[3] = 0.f;
+    } else if (env_in(KS, DRIL_ENV_ACROBOT) && kind == DRIL_ENV_ACROBOT) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) st[k] = __fadd_rn(-0.1f, __fmul_rn(0.2f, u01_f32(x[k])));
     }
 }
 
@@ -104,6 +138,89 @@ __device__ __forceinline__ float pendulum_step(float* st, float u) {
     return -cost;
 }
 
+// MountainCar-v0 / MountainCarContinuous-v0 after the velocity increment dv: clip, move, clip, left wall, goal test
+__device__ __forceinline__ void mountaincar_move(float* st, float dv, float goal, bool* terminated) {
+    const float MAX_SPEED = 0.07f, MIN_POS = -1.2f, MAX_POS = 0.6f;
+    float vel = fminf(fmaxf(__fadd_rn(st[1], dv), -MAX_SPEED), MAX_SPEED);
+    const float pos = fminf(fmaxf(__fadd_rn(st[0], vel), MIN_POS), MAX_POS);
+    if (pos == MIN_POS && vel < 0.f) vel = 0.f;
+    st[0] = pos; st[1] = vel;
+    *terminated = pos >= goal && vel >= 0.f;
+}
+// MountainCar-v0: idx 0 = push left, 1 = none, 2 = push right.  Returns reward -1.
+__device__ __forceinline__ float mountaincar_step(float* st, int idx, bool* terminated) {
+    float s, c;
+    sincos_rn(__fmul_rn(3.0f, st[0]), &s, &c);
+    mountaincar_move(st, __fadd_rn(__fmul_rn((float)(idx - 1), 0.001f), __fmul_rn(c, -0.0025f)), 0.5f, terminated);
+    return -1.0f;
+}
+// MountainCarContinuous-v0: a = env-space force (clipped to [-1, 1] for the dynamics, not for the reward)
+__device__ __forceinline__ float mountaincar_continuous_step(float* st, float a, bool* terminated) {
+    const float f = fminf(fmaxf(a, -1.0f), 1.0f);
+    float s, c;
+    sincos_rn(__fmul_rn(3.0f, st[0]), &s, &c);
+    mountaincar_move(st, __fsub_rn(__fmul_rn(f, 0.0015f), __fmul_rn(0.0025f, c)), 0.45f, terminated);
+    return __fsub_rn(*terminated ? 100.0f : 0.0f, __fmul_rn(__fmul_rn(a, a), 0.1f));
+}
+
+// Acrobot-v1 "book" dynamics f(s) for torque a (m1 = m2 = l1 = I1 = I2 = 1, lc1 = lc2 = 0.5, g = 9.8 folded into exact
+// fp32 constants; (m1 lc1 + m2 l1) g = 1.5 * 9.8f rounded once)
+__device__ __forceinline__ void acrobot_dsdt(const float* s, float a, float* ds) {
+    const float HALF_PI = 1.57079637050628662f, G_LC2 = 4.90000009536743164f, G_12 = 14.7000007629394531f;
+    const float th1 = s[0], th2 = s[1], w1 = s[2], w2 = s[3];
+    float s2, c2, sp, cp2, cp1;
+    sincos_rn(th2, &s2, &c2);
+    const float d1 = __fadd_rn(__fadd_rn(__fadd_rn(0.25f, __fadd_rn(1.25f, c2)), 1.0f), 1.0f);
+    const float d2 = __fadd_rn(__fadd_rn(0.25f, __fmul_rn(0.5f, c2)), 1.0f);
+    sincos_rn(__fsub_rn(__fadd_rn(th1, th2), HALF_PI), &sp, &cp2);
+    const float phi2 = __fmul_rn(G_LC2, cp2);
+    sincos_rn(__fsub_rn(th1, HALF_PI), &sp, &cp1);
+    const float phi1 = __fadd_rn(__fadd_rn(__fsub_rn(__fmul_rn(__fmul_rn(-0.5f, __fmul_rn(w2, w2)), s2), __fmul_rn(__fmul_rn(w2, w1), s2)),
+                                           __fmul_rn(G_12, cp1)), phi2);
+    const float num = __fsub_rn(__fsub_rn(__fadd_rn(a, __fmul_rn(__fdiv_rn(d2, d1), phi1)), __fmul_rn(__fmul_rn(0.5f, __fmul_rn(w1, w1)), s2)), phi2);
+    const float al2 = __fdiv_rn(num, __fsub_rn(1.25f, __fdiv_rn(__fmul_rn(d2, d2), d1)));
+    const float al1 = __fdiv_rn(-__fadd_rn(__fmul_rn(d2, al2), phi1), d1);
+    ds[0] = w1; ds[1] = w2; ds[2] = al1; ds[3] = al2;
+}
+// Gymnasium's wrap(x, -pi, pi): subtract / add 2 pi until inside (a non-finite angle, only reachable through set_state, is
+// left as it is instead of looping forever)
+__device__ __forceinline__ float acrobot_wrap(float x) {
+    const float PI = 3.14159274101257324f, TWO_PI = 6.28318548202514648f;
+    if (!isfinite(x)) return x;
+    while (x > PI) x = __fsub_rn(x, TWO_PI);
+    while (x < -PI) x = __fadd_rn(x, TWO_PI);
+    return x;
+}
+// Acrobot-v1: idx 0 / 1 / 2 = torque -1 / 0 / +1 held over one RK4 step of dt = 0.2.  Returns reward 0 on termination, else -1.
+__device__ __forceinline__ float acrobot_step(float* st, int idx, bool* terminated) {
+    const float DT = 0.2f, DT2 = 0.1f, DT6 = 0.0333333350718021393f;
+    const float MAX_VEL_1 = 12.5663709640502930f, MAX_VEL_2 = 28.2743339538574219f;
+    const float a = (float)(idx - 1);
+    float k1[4], k2[4], k3[4], k4[4], y[4];
+    acrobot_dsdt(st, a, k1);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) y[i] = __fadd_rn(st[i], __fmul_rn(DT2, k1[i]));
+    acrobot_dsdt(y, a, k2);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) y[i] = __fadd_rn(st[i], __fmul_rn(DT2, k2[i]));
+    acrobot_dsdt(y, a, k3);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) y[i] = __fadd_rn(st[i], __fmul_rn(DT, k3[i]));
+    acrobot_dsdt(y, a, k4);
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        y[i] = __fadd_rn(st[i], __fmul_rn(DT6, __fadd_rn(__fadd_rn(__fadd_rn(k1[i], __fmul_rn(2.0f, k2[i])), __fmul_rn(2.0f, k3[i])), k4[i])));
+    st[0] = acrobot_wrap(y[0]);
+    st[1] = acrobot_wrap(y[1]);
+    st[2] = fminf(fmaxf(y[2], -MAX_VEL_1), MAX_VEL_1);
+    st[3] = fminf(fmaxf(y[3], -MAX_VEL_2), MAX_VEL_2);
+    float s, c1, c12;
+    sincos_rn(st[0], &s, &c1);
+    sincos_rn(__fadd_rn(st[1], st[0]), &s, &c12);
+    *terminated = __fsub_rn(-c1, c12) > 1.0f;
+    return *terminated ? 0.0f : -1.0f;
+}
+
 // Synthetic env (SURVEY §8d C5): obs block b of lifetime step `life`
 __device__ __forceinline__ void synthetic_obs_block(uint32_t gid, uint32_t life, int b, unsigned long long seed, float o[4]) {
     uint32_t x[4];
@@ -116,4 +233,35 @@ __device__ __forceinline__ float synthetic_step(uint32_t gid, uint32_t life, uns
     philox4x32(gid, life, 0u, DRIL_TAG_SYN_DYN, seed, x);
     *terminated = u01_f32(x[1]) < 0.005f;
     return u01_f32(x[0]);
+}
+
+// env_step tests the kinds of KS in the order CartPole, Pendulum, MountainCar, MountainCarContinuous, Acrobot, synthetic; the
+// last kind of KS in that order is taken without a test
+__host__ __device__ constexpr int env_last_kind(unsigned ks) {
+    return env_in(ks, DRIL_ENV_SYNTHETIC) ? DRIL_ENV_SYNTHETIC
+         : env_in(ks, DRIL_ENV_ACROBOT) ? DRIL_ENV_ACROBOT
+         : env_in(ks, DRIL_ENV_MOUNTAINCAR_CONTINUOUS) ? DRIL_ENV_MOUNTAINCAR_CONTINUOUS
+         : env_in(ks, DRIL_ENV_MOUNTAINCAR) ? DRIL_ENV_MOUNTAINCAR
+         : env_in(ks, DRIL_ENV_PENDULUM) ? DRIL_ENV_PENDULUM : DRIL_ENV_CARTPOLE;
+}
+template <unsigned KS, int K>
+__device__ __forceinline__ bool env_is(int kind) { return env_in(KS, K) && (K == env_last_kind(KS) || kind == K); }
+
+// one step of env n: a_disc = env-space action of a Discrete env, a_cont = the Box env's action as the wrappers above it hand it
+// over (read only for Box envs), life = the synthetic env's lifetime step counter (read and advanced for that kind only).
+// Returns the reward; sets terminated.
+template <unsigned KS>
+__device__ __forceinline__ float env_step(const EnvDev& env, float* st, long long n, int a_disc, const float* a_cont, uint32_t* life,
+                                          bool* terminated) {
+    if (env_is<KS, DRIL_ENV_CARTPOLE>(env.kind)) return cartpole_step(st, a_disc - env.act_start, terminated);
+    if (env_is<KS, DRIL_ENV_PENDULUM>(env.kind)) return pendulum_step(st, env_unscale_action(env, *a_cont));
+    if (env_is<KS, DRIL_ENV_MOUNTAINCAR>(env.kind)) return mountaincar_step(st, a_disc - env.act_start, terminated);
+    if (env_is<KS, DRIL_ENV_MOUNTAINCAR_CONTINUOUS>(env.kind))
+        return mountaincar_continuous_step(st, env_unscale_action(env, *a_cont), terminated);
+    if (env_is<KS, DRIL_ENV_ACROBOT>(env.kind)) return acrobot_step(st, a_disc - env.act_start, terminated);
+    *life = env.life[n];
+    const float r = synthetic_step((uint32_t)(env.gid_offset + n), *life, env.seed, terminated);
+    *life += 1;
+    env.life[n] = *life;
+    return r;
 }

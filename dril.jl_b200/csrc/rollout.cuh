@@ -184,7 +184,8 @@ struct MlpForward {
     }
 };
 
-template <bool WS, bool TCA, class Fwd>
+// KS: the env kinds this instantiation serves (env.cuh)
+template <bool WS, bool TCA, unsigned KS, class Fwd>
 __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, Fwd& fwd) {
     const EnvDev& env = a.env;
     const BufDev& buf = a.buf;
@@ -310,15 +311,18 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
             }
         } else {
             if (tid < M4) {
-                float o[4] = {0.f, 0.f, 0.f, 0.f};
-                if (tid < nvalid) {
-                    float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-                    for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * N + n0 + tid];
-                    env_obs(env, st, o);
+                for (int b = 0; b < env_obs_blocks(KS); ++b) {
+                    float o[4] = {0.f, 0.f, 0.f, 0.f};
+                    if (tid < nvalid) {
+                        float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+                        for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * N + n0 + tid];
+                        env_obs_block<KS>(env, st, b, o);
+                    }
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) if (4 * b + j < Dp) sRaw[(size_t)(4 * b + j) * ld + tid] = o[j];
                 }
-#pragma unroll
-                for (int j = 0; j < 4; ++j) if (j < Dp) sRaw[(size_t)j * ld + tid] = o[j];
             }
         }
         __syncthreads();
@@ -440,9 +444,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                 bool term = false;
                 float r;
                 uint32_t life = 0;
-                if (env.kind == DRIL_ENV_CARTPOLE) r = cartpole_step(st, a_disc - env.act_start, &term);
-                else if (env.kind == DRIL_ENV_PENDULUM) r = pendulum_step(st, env_unscale_action(env, sEnvAct[tid]));
-                else { life = env.life[n]; r = synthetic_step(gid, life, env.seed, &term); life += 1; env.life[n] = life; }
+                r = env_step<KS>(env, st, n, a_disc, sEnvAct + tid, &life, &term);
                 steps += 1;
                 const bool trunc = steps >= env.max_steps;
                 const bool done = term || trunc;
@@ -472,15 +474,18 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                             for (int j = 0; j < 4; ++j) if (4 * b + j < D) env.tobs[(size_t)n * D + 4 * b + j] = o[j];
                         }
                     } else {
-                        float o[4];
-                        env_obs(env, st, o);
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) if (j < D) env.tobs[(size_t)n * D + j] = o[j];
+                        for (int b = 0; b < env_obs_blocks(KS); ++b) {
+                            float o[4];
+                            env_obs_block<KS>(env, st, b, o);
+#pragma unroll
+                            for (int j = 0; j < 4; ++j) if (4 * b + j < D) env.tobs[(size_t)n * D + 4 * b + j] = o[j];
+                        }
                     }
                 }
                 if (done) {                                     // reset!(env_i)
                     uint32_t ep = env.episode[n];
-                    env_reset_state(env.kind, gid, ep, env.seed, st);
+                    env_reset_state<KS>(env.kind, gid, ep, env.seed, st);
                     env.episode[n] = ep + 1;
                     steps = 0;
                 }
@@ -584,15 +589,15 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
     }
 }
 
-template <bool WS>
+template <bool WS, unsigned KS>
 __global__ void __launch_bounds__(DRIL_THREADS) rollout_kernel(const __grid_constant__ RolloutArgs a) {
     extern __shared__ float4 smem4[];
     MlpForward fwd;
-    rollout_body<WS, false>(a, reinterpret_cast<float*>(smem4), fwd);
+    rollout_body<WS, false, KS>(a, reinterpret_cast<float*>(smem4), fwd);
 }
 
 // ---------------------------------------------------------------------------------------
-// Fast path of the fused rollout (the common case): CartPole / Pendulum, no running-statistics
+// Fast path of the fused rollout (the common case): every state-based env, no running-statistics
 // update (no NormalizeWrapperEnv, or one in eval mode), one tile of envs per CTA.
 //   * env state, step counters and monitor accumulators stay in registers for all n_steps
 //     (no global round trip on the per-step critical path);
@@ -624,8 +629,9 @@ __host__ __device__ inline RolloutFastSmem rollout_fast_smem_layout(const Policy
     return s;
 }
 
-template <bool WS>
+template <bool WS, unsigned KS>
 __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid_constant__ RolloutArgs a) {
+    constexpr int OW = 4 * env_obs_blocks(KS);   // observation components held per env
     extern __shared__ float4 smem4[];
     float* smem = reinterpret_cast<float*>(smem4);
     const EnvDev& env = a.env;
@@ -684,23 +690,24 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
     // write the (normalised) observation of the register state into sX and optionally the buffer
     auto stage_obs = [&](float* obs_row /* nullable global [D] */) {
         if (tid < M4) {
-            float o[4] = {0.f, 0.f, 0.f, 0.f};
+            float o[OW] = {};
             if (mine) {
-                env_obs(env, st, o);
+#pragma unroll
+                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, o + 4 * b);
                 if (norm_obs) {
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) if (j < D) o[j] = normalize_obs_val(o[j], sMean[j], sVar[j], env.eps, env.clip_obs);
+                    for (int j = 0; j < OW; ++j) if (j < D) o[j] = normalize_obs_val(o[j], sMean[j], sVar[j], env.eps, env.clip_obs);
                 }
                 if (obs_row) {
                     if (D == 4) *reinterpret_cast<float4*>(obs_row) = make_float4(o[0], o[1], o[2], o[3]);
                     else {
 #pragma unroll
-                        for (int j = 0; j < 4; ++j) if (j < D) obs_row[j] = o[j];
+                        for (int j = 0; j < OW; ++j) if (j < D) obs_row[j] = o[j];
                     }
                 }
             }
 #pragma unroll
-            for (int j = 0; j < 4; ++j) if (j < Dp) sX[(size_t)j * ld + tid] = o[j];
+            for (int j = 0; j < OW; ++j) if (j < Dp) sX[(size_t)j * ld + tid] = o[j];
         }
         __syncthreads();
     };
@@ -769,7 +776,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         const int par = hidden_forward(3);
         output_partials(par, 3);
         int trunc_i = 0;
-        float tobs[4] = {0.f, 0.f, 0.f, 0.f};
+        float tobs[OW] = {};
         if (mine) {
             const float value = reduce_out(0, 1);
             float z[RF_MAX_OUT - 1];
@@ -834,8 +841,8 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             // env step + monitor + auto-reset
             bool term = false;
             float r;
-            if (env.kind == DRIL_ENV_CARTPOLE) r = cartpole_step(st, a_disc - env.act_start, &term);
-            else r = pendulum_step(st, env_unscale_action(env, a_cont));
+            uint32_t life = 0;
+            r = env_step<KS & ~(1u << DRIL_ENV_SYNTHETIC)>(env, st, n, a_disc, &a_cont, &life, &term);   // (no synthetic env here)
             steps += 1;
             const bool trunc = steps >= env.max_steps;
             const bool done = term || trunc;
@@ -861,14 +868,15 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             }
             if (trunc) {
                 trunc_i = 1;
-                env_obs(env, st, tobs);
+#pragma unroll
+                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, tobs + 4 * b);
                 if (norm_obs) {
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) if (j < D) tobs[j] = normalize_obs_val(tobs[j], sMean[j], sVar[j], env.eps, env.clip_obs);
+                    for (int j = 0; j < OW; ++j) if (j < D) tobs[j] = normalize_obs_val(tobs[j], sMean[j], sVar[j], env.eps, env.clip_obs);
                 }
             }
             if (done) {
-                env_reset_state(env.kind, gid, episode, env.seed, st);
+                env_reset_state<KS>(env.kind, gid, episode, env.seed, st);
                 episode += 1;
                 steps = 0;
                 if (env.normalize) env.ret[n] = 0.f;             // normalizeWrapperEnv.jl:153-156
@@ -878,7 +886,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         if (__syncthreads_or(trunc_i)) {
             if (tid < M4) {
 #pragma unroll
-                for (int j = 0; j < 4; ++j) if (j < Dp) sX[(size_t)j * ld + tid] = trunc_i ? tobs[j] : 0.f;
+                for (int j = 0; j < OW; ++j) if (j < Dp) sX[(size_t)j * ld + tid] = trunc_i ? tobs[j] : 0.f;
             }
             __syncthreads();
             const int p2 = hidden_forward(2);
@@ -1001,7 +1009,7 @@ __global__ void env_reset_kernel(EnvDev env) {
     if (n >= env.n_envs) return;
     float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
     uint32_t ep = env.episode[n];
-    env_reset_state(env.kind, (uint32_t)(env.gid_offset + n), ep, env.seed, st);
+    env_reset_state<ENV_KS_ALL>(env.kind, (uint32_t)(env.gid_offset + n), ep, env.seed, st);
     env.episode[n] = ep + 1;
 #pragma unroll
     for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) env.state[(size_t)k * env.n_envs + n] = st[k];

@@ -7,7 +7,7 @@
 // included (x image with a ones row carries the bias), tanh's 2·log2(e) folded into the weight images.  Weight images of the
 // actor (W_1.., [W_0; b_0]) stay resident in shared memory for the whole rollout; ONE activation image buffer is reused by all
 // layers (a layer's MMAs have completed before its epilogue overwrites their B operand) and ends as the fp32 tile of the last
-// hidden layer, from which the thin output layer (<= 2 outputs) is evaluated on CUDA cores.
+// hidden layer, from which the thin output layer (<= 4 outputs) is evaluated on CUDA cores.
 // Replaces the mma.sync tiles of mlp.cuh in the step loop for the shapes update_ftg.cuh covers (2-3 hidden layers of 64 / 128).
 // Reference: the layer call of collect_trajectories (layers/layer_forward.jl:3-39, layer_helpers.jl:27-57).
 #pragma once
@@ -22,10 +22,12 @@ struct GtcLayout {             // byte offsets from the 1024-aligned start of th
     int w0a;                   // images (hi, lo) of C2 * [W_0; b_0; 0]^T: rows = features of layer 0, 16 columns
     int h;                     // activation images (hi, lo) [width][128 envs] of the current layer / fp32 [width L-1][132] at the end
     int ximg;                  // x images (hi, lo): 16 rows x 128 envs
-    int wout;                  // output layer [width L-1][2] floats + bias [2]
-    int part;                  // output-layer partials [2 halves][2 outputs][128]
+    int wout;                  // output layer [width L-1][NO] floats + bias [NO]
+    int part;                  // output-layer partials [2 halves][NO outputs][128]
     int total;
 };
+// output columns the kernel stages: 2, or 4 for Discrete(3 | 4)
+__host__ __device__ inline int gtc_nout(const PolicyDesc& pd) { return pd.act_n > 2 ? 4 : 2; }
 __host__ __device__ inline GtcLayout gtc_layout(const PolicyDesc& pd) {
     GtcLayout s;
     const int L = pd.n_layers - 1;
@@ -39,8 +41,9 @@ __host__ __device__ inline GtcLayout gtc_layout(const PolicyDesc& pd) {
     const int last = pd.L[0][L - 1].N * GTC_HS_LD * 4;
     s.h = take(hb > last ? hb : last);
     s.ximg = take(2 * 16 * GTC_ENVS * 2);
-    s.wout = take((pd.L[0][L - 1].N * 2 + 4) * 4);
-    s.part = take(2 * 2 * GTC_ENVS * 4);
+    const int no = gtc_nout(pd);
+    s.wout = take((pd.L[0][L - 1].N * no + 4) * 4);
+    s.part = take(2 * no * GTC_ENVS * 4);
     s.total = o + 1024;
     return s;
 }
@@ -48,7 +51,7 @@ __host__ __device__ inline GtcLayout gtc_layout(const PolicyDesc& pd) {
 // 16-byte row (8 consecutive envs starting at c, c % 8 == 0) of feature row r of a [rows][128] fp16 image, no-swizzle core layout
 __device__ __forceinline__ uint32_t gtc_row_off(int r, int c) { return (uint32_t)((((r >> 3) * 16 + (c >> 3)) << 7) + ((r & 7) << 4)); }
 
-template <int L>
+template <int L, int NO>
 struct GtcForward {
     unsigned char* sm;         // image region (generic pointer)
     uint32_t sm_base;          // its shared-space address
@@ -140,27 +143,40 @@ struct GtcForward {
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             __syncthreads();
         }
-        // ---- output layer (<= 2 outputs) on CUDA cores: the feature range is split over the two halves of the block ------------
+        // ---- output layer (<= NO outputs) on CUDA cores: the feature range is split over the two halves of the block ------------
         {
             const float* sWout = reinterpret_cast<const float*>(sm + ly.wout);
             float* sPart = reinterpret_cast<float*>(sm + ly.part);
             const int m = tid & (GTC_ENVS - 1), half = (tid >> 7) & 1, per = wd[L - 1] >> 1;
             if (tid < 2 * GTC_ENVS) {
-                float p0 = 0.f, p1 = 0.f;
                 const float* hp = Hs + (half * per) * GTC_HS_LD + m;
-                for (int n = 0; n < per; ++n) {
-                    const float hv = hp[n * GTC_HS_LD];
-                    const float2 w = *reinterpret_cast<const float2*>(sWout + 2 * (half * per + n));
-                    p0 = fmaf(hv, w.x, p0); p1 = fmaf(hv, w.y, p1);
+                if constexpr (NO == 2) {
+                    float p0 = 0.f, p1 = 0.f;
+                    for (int n = 0; n < per; ++n) {
+                        const float hv = hp[n * GTC_HS_LD];
+                        const float2 w = *reinterpret_cast<const float2*>(sWout + 2 * (half * per + n));
+                        p0 = fmaf(hv, w.x, p0); p1 = fmaf(hv, w.y, p1);
+                    }
+                    sPart[(half * 2 + 0) * GTC_ENVS + m] = p0;
+                    sPart[(half * 2 + 1) * GTC_ENVS + m] = p1;
+                } else {
+                    float p0 = 0.f, p1 = 0.f, p2 = 0.f, p3 = 0.f;
+                    for (int n = 0; n < per; ++n) {
+                        const float hv = hp[n * GTC_HS_LD];
+                        const float4 w = *reinterpret_cast<const float4*>(sWout + 4 * (half * per + n));
+                        p0 = fmaf(hv, w.x, p0); p1 = fmaf(hv, w.y, p1); p2 = fmaf(hv, w.z, p2); p3 = fmaf(hv, w.w, p3);
+                    }
+                    sPart[(half * 4 + 0) * GTC_ENVS + m] = p0;
+                    sPart[(half * 4 + 1) * GTC_ENVS + m] = p1;
+                    sPart[(half * 4 + 2) * GTC_ENVS + m] = p2;
+                    sPart[(half * 4 + 3) * GTC_ENVS + m] = p3;
                 }
-                sPart[(half * 2 + 0) * GTC_ENVS + m] = p0;
-                sPart[(half * 2 + 1) * GTC_ENVS + m] = p1;
             }
             __syncthreads();
             if (tid < GTC_ENVS) {
 #pragma unroll
-                for (int j = 0; j < 2; ++j)
-                    if (j < A) sActA[(size_t)j * ld + tid] = sWout[2 * wd[L - 1] + j] + (sPart[j * GTC_ENVS + tid] + sPart[(2 + j) * GTC_ENVS + tid]);
+                for (int j = 0; j < NO; ++j)
+                    if (j < A) sActA[(size_t)j * ld + tid] = sWout[NO * wd[L - 1] + j] + (sPart[j * GTC_ENVS + tid] + sPart[(NO + j) * GTC_ENVS + tid]);
             }
             __syncthreads();
         }
@@ -168,7 +184,8 @@ struct GtcForward {
     }
 };
 
-template <int L>
+// KS: env kinds served (env.cuh); NO: output columns staged (gtc_nout)
+template <int L, unsigned KS, int NO>
 __global__ void __launch_bounds__(DRIL_THREADS, 1) rollout_gtc_kernel(const __grid_constant__ RolloutArgs a, const __grid_constant__ GtcLayout ly,
                                                                       const int body_bytes) {
     extern __shared__ __align__(1024) unsigned char gtc_smem_raw[];
@@ -190,7 +207,7 @@ __global__ void __launch_bounds__(DRIL_THREADS, 1) rollout_gtc_kernel(const __gr
         asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(tc_smem_u32(&barM)));
         asm volatile("fence.mbarrier_init.release.cluster;");
     }
-    GtcForward<L> fwd;
+    GtcForward<L, NO> fwd;
     fwd.sm = sm; fwd.sm_base = sm_base; fwd.ly = ly; fwd.barM = &barM; fwd.n_mma = 0; fwd.D = pd.obs_dim; fwd.A = pd.act_n;
 #pragma unroll
     for (int l = 0; l < L; ++l) {
@@ -237,10 +254,14 @@ __global__ void __launch_bounds__(DRIL_THREADS, 1) rollout_gtc_kernel(const __gr
         const LayerDesc& Lout = pd.L[net][L];
         float* sWout = reinterpret_cast<float*>(sm + ly.wout);
         for (int i = tid; i < fwd.wd[L - 1]; i += blockDim.x) {
-            sWout[2 * i] = a.pack[Lout.pw_off + i * Lout.Np];
-            sWout[2 * i + 1] = fwd.A > 1 ? a.pack[Lout.pw_off + i * Lout.Np + 1] : 0.f;
+            sWout[NO * i] = a.pack[Lout.pw_off + i * Lout.Np];
+            sWout[NO * i + 1] = fwd.A > 1 ? a.pack[Lout.pw_off + i * Lout.Np + 1] : 0.f;
+            if (NO == 4) {
+                sWout[NO * i + 2] = fwd.A > 2 ? a.pack[Lout.pw_off + i * Lout.Np + 2] : 0.f;
+                sWout[NO * i + 3] = fwd.A > 3 ? a.pack[Lout.pw_off + i * Lout.Np + 3] : 0.f;
+            }
         }
-        if (tid < 2) sWout[2 * fwd.wd[L - 1] + tid] = tid < fwd.A ? a.pack[Lout.pb_off + tid] : 0.f;
+        if (tid < NO) sWout[NO * fwd.wd[L - 1] + tid] = tid < fwd.A ? a.pack[Lout.pb_off + tid] : 0.f;
     }
     {
         __half* sXimg = reinterpret_cast<__half*>(sm + ly.ximg);
@@ -258,7 +279,7 @@ __global__ void __launch_bounds__(DRIL_THREADS, 1) rollout_gtc_kernel(const __gr
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     fwd.tb = __shfl_sync(0xffffffffu, tmem_base_s, 0);
 
-    rollout_body<false, true>(a, reinterpret_cast<float*>(gtc_smem_raw), fwd);
+    rollout_body<false, true, KS>(a, reinterpret_cast<float*>(gtc_smem_raw), fwd);
 
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();

@@ -1,5 +1,5 @@
 // General-shape features-on-lanes tcgen05 loss/grad kernel: two or three tanh hidden layers of width 64 or 128 per net,
-// obs_dim <= 15, Discrete(n <= 2) or Box actions of dimension <= 2 — e.g. BASELINE config C3, Pendulum with
+// obs_dim <= 15, Discrete(n <= 4) or Box actions of dimension <= 2 — e.g. BASELINE config C3, Pendulum with
 // hidden_dims = [128, 128, 64] and a diagonal Gaussian (layers/layer_helpers.jl:27-57, DRiLDistributions/diagGaussian.jl:13-47,
 // loss functor algorithms/ppo.jl:365-407).  Same formulation as update_ft.cuh (features on TMEM lanes, samples on columns,
 // fp16 hi/lo operands on kind::f16, one no-swizzle image per matrix for both GEMM orientations), generalised:
@@ -38,8 +38,8 @@ struct FtgLayout {             // byte offsets inside the dynamic shared memory 
     int rec;                   // two tile records
     int ximg;                  // x images (hi, lo) of the next tile: 16 rows x 64 samples
     int part;                  // [8 feature slices][64 samples] float4 output-layer partials
-    int dout;                  // [64 samples] float4: dL/dout (<= 2) per sample
-    int small;                 // output-layer weights [width L-1][2] float2, bias, reduction scratch
+    int dout;                  // [64 samples] float4: dL/dout (<= 4) per sample
+    int small;                 // output-layer weights [width L-1] float2 (float4 for Discrete(3 | 4)), bias, reduction scratch
     int total;
     int rec_floats;
 };
@@ -68,7 +68,10 @@ __host__ inline FtgLayout ftg_layout(const PolicyDesc& pd) {
     s.ximg = take(2 * 2048);
     s.part = take(8 * 64 * 16);
     s.dout = take(64 * 16);
-    s.small = take(128 * 8 + 64 + 4 * 8 * 128 * 4);     // W_out [128] float2 | bias, bounds | thin-sum scratch [4 sample quarters][8][128]
+    // W_out [128] float2 | bias, bounds | thin-sum scratch [4 sample quarters][8][128]; Discrete(3 | 4): W_out [128] float4 and the
+    // four output biases behind the bound / dmax / head-sum slots (ftg_pass)
+    const bool wide = pd.act_kind == DRIL_ACT_DISCRETE && pd.act_n > 2;
+    s.small = take((wide ? 128 * 16 + 128 : 128 * 8 + 64) + 4 * 8 * 128 * 4);
     s.total = o + 1024;
     return s;
 }
@@ -170,10 +173,14 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
     uint64_t* barG0 = bars + 2;     // G0 of the next tile
     uint64_t* barM = bars + 3;      // the GEMM(s) a phase waits for
     uint64_t* barW = bars + 4;      // dW GEMMs (image buffers may be overwritten)
+    constexpr bool W4 = NOUT > 2;                             // Discrete(3 | 4): four output columns
     float* sSmall = reinterpret_cast<float*>(sm + ly.small);
     float2* sWout = reinterpret_cast<float2*>(sSmall);        // [width L-1] output-layer weights (columns 0, 1)
-    float* sMisc = sSmall + 256;                              // [0..1] output bias, [2] |W_out| bound, [4..7] per-warp dmax of the head warps
-    float* sThin = sSmall + 272;                              // [4 sample quarters][8 sums][128] end-of-pass scratch
+    float4* sWout4 = reinterpret_cast<float4*>(sSmall);       // W4: [width L-1] output-layer weights (columns 0 .. 3)
+    float* sMisc = sSmall + (W4 ? 512 : 256);                 // [0..1] output bias (W4: [16..19]), [2] |W_out| bound, [4..7] per-warp
+                                                              // dmax of the head warps, [8..15] end-of-pass head sums
+    float* sBout = W4 ? sMisc + 16 : sMisc;
+    float* sThin = sSmall + (W4 ? 544 : 272);                 // [4 sample quarters][8 sums][128] end-of-pass scratch
     float* Hs = reinterpret_cast<float*>(sm + ly.last);
     float4* sPart = reinterpret_cast<float4*>(sm + ly.part);
     float4* sDout = reinterpret_cast<float4*>(sm + ly.dout);
@@ -216,9 +223,17 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
             lo[idx] = __float2half_rn(w - __half2float(h));
         }
     }
-    for (int i = tid; i < wd[L - 1]; i += FTG_THREADS)
-        sWout[i] = make_float2(a.pack[Lout.pw_off + i * Lout.Np], NOUT > 1 ? a.pack[Lout.pw_off + i * Lout.Np + 1] : 0.f);
-    if (tid < 2) sMisc[tid] = tid < NOUT ? a.pack[Lout.pb_off + tid] : 0.f;
+    if (W4) {
+        for (int i = tid; i < wd[L - 1]; i += FTG_THREADS) {
+            const float* w = a.pack + Lout.pw_off + i * Lout.Np;
+            sWout4[i] = make_float4(w[0], w[1], w[2], NOUT > 3 ? w[3] : 0.f);
+        }
+        if (tid < 4) sBout[tid] = tid < NOUT ? a.pack[Lout.pb_off + tid] : 0.f;
+    } else {
+        for (int i = tid; i < wd[L - 1]; i += FTG_THREADS)
+            sWout[i] = make_float2(a.pack[Lout.pw_off + i * Lout.Np], NOUT > 1 ? a.pack[Lout.pw_off + i * Lout.Np + 1] : 0.f);
+        if (tid < 2) sMisc[tid] = tid < NOUT ? a.pack[Lout.pb_off + tid] : 0.f;
+    }
     for (int i = tid; i < 2 * 1024; i += FTG_THREADS) {       // x images: rows > obs_dim zero, row obs_dim of the hi image = 1 (bias)
         const int e = i & 1023, d = ((e >> 9) << 3) + ((e >> 3) & 7);
         sXimg[i] = __float2half_rn((i < 1024 && d == D) ? 1.0f : 0.f);
@@ -231,10 +246,15 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
     const int flast = fl[L - 1];
     const float wo0 = flast >= 0 ? a.pack[Lout.pw_off + flast * Lout.Np] : 0.f;
     const float wo1 = (flast >= 0 && NOUT > 1) ? a.pack[Lout.pw_off + flast * Lout.Np + 1] : 0.f;
+    const float wo2 = (flast >= 0 && NOUT > 2) ? a.pack[Lout.pw_off + flast * Lout.Np + 2] : 0.f;
+    const float wo3 = (flast >= 0 && NOUT > 3) ? a.pack[Lout.pw_off + flast * Lout.Np + 3] : 0.f;
     __syncthreads();
     if (tid < 32) {                                                // bound of the output-layer weight row sums
         float wb = 0.f;
-        for (int i = tid; i < wd[L - 1]; i += 32) wb = fmaxf(wb, fabsf(sWout[i].x) + fabsf(sWout[i].y));
+        for (int i = tid; i < wd[L - 1]; i += 32) {
+            if (W4) { const float4 w = sWout4[i]; wb = fmaxf(wb, ((fabsf(w.x) + fabsf(w.y)) + fabsf(w.z)) + fabsf(w.w)); }
+            else wb = fmaxf(wb, fabsf(sWout[i].x) + fabsf(sWout[i].y));
+        }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) wb = fmaxf(wb, __shfl_xor_sync(0xffffffffu, wb, o));
         if (tid == 0) sMisc[2] = wb;
@@ -250,8 +270,9 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
     float accW0[FTG_MAX_OBS + 1];
 #pragma unroll
     for (int d = 0; d < FTG_MAX_OBS + 1; ++d) accW0[d] = 0.f;
-    float accWo0 = 0.f, accWo1 = 0.f;                              // dW_out[flast][0..1] (unscaled)
+    float accWo0 = 0.f, accWo1 = 0.f, accWo2 = 0.f, accWo3 = 0.f;  // dW_out[flast][0..3] (unscaled)
     float accbo0 = 0.f, accbo1 = 0.f, accls0 = 0.f, accls1 = 0.f;  // head threads: output bias / log_std gradient sums
+    float accbo2 = 0.f, accbo3 = 0.f;
     float S = 1.0f, invS = 1.0f;
     bool s_fixed = false;
 
@@ -383,25 +404,39 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
         // ---- output layer partials: thread <-> (sample ms, feature slice) -------------------------------------------------
         {
             const int per = wd[L - 1] >> 3;
-            float p0 = 0.f, p1 = 0.f;
+            float p0 = 0.f, p1 = 0.f, p2 = 0.f, p3 = 0.f;
             const float* hp = Hs + (slice * per) * FT_HS_LD + ms;
             for (int n = 0; n < per; ++n) {
-                const float2 w = sWout[slice * per + n];
                 const float hv = hp[n * FT_HS_LD];
-                p0 = fmaf(hv, w.x, p0);
-                if (NOUT > 1) p1 = fmaf(hv, w.y, p1);
+                if (W4) {
+                    const float4 w = sWout4[slice * per + n];
+                    p0 = fmaf(hv, w.x, p0); p1 = fmaf(hv, w.y, p1); p2 = fmaf(hv, w.z, p2); p3 = fmaf(hv, w.w, p3);
+                } else {
+                    const float2 w = sWout[slice * per + n];
+                    p0 = fmaf(hv, w.x, p0);
+                    if (NOUT > 1) p1 = fmaf(hv, w.y, p1);
+                }
             }
-            sPart[slice * 64 + ms] = make_float4(p0, p1, 0.f, 0.f);
+            sPart[slice * 64 + ms] = make_float4(p0, p1, p2, p3);
         }
         __syncthreads();
         // ---- loss head: one thread per sample (warps 0 and 1) ----------------------------------------------------------------
         if (tid < 64) {
-            float out[2] = {sMisc[0], sMisc[1]};
+            constexpr int NA = W4 ? 4 : 2;
+            float out[NA];
 #pragma unroll
-            for (int sl = 0; sl < 8; ++sl) { const float4 p = sPart[sl * 64 + ms]; out[0] += p.x; out[1] += p.y; }
+            for (int j = 0; j < NA; ++j) out[j] = sBout[j];
+#pragma unroll
+            for (int sl = 0; sl < 8; ++sl) {
+                const float4 p = sPart[sl * 64 + ms];
+                out[0] += p.x; out[1] += p.y;
+                if (W4) { out[2] += p.z; out[3] += p.w; }
+            }
             const long long tile = (long long)blockIdx.x + (long long)it * gridDim.x;
             const bool valid = tile * 64 + ms < a.mb.count;
-            float dout[2] = {0.f, 0.f};
+            float dout[NA];
+#pragma unroll
+            for (int j = 0; j < NA; ++j) dout[j] = 0.f;
             if (HEAD == 2) {
                 const float ret = sc[128 + ms], ov = sc[192 + ms];
                 const float v_raw = out[0];
@@ -420,14 +455,18 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
                 if (valid && a.hp.normalize_advantage) adv = (adv - adv_mean) / adv_den;
                 const float olp = sc[64 + ms];
                 float logp = 0.f, ent = 0.f;
-                float pj[2] = {0.f, 0.f}, lpj[2] = {0.f, 0.f}, diff[2] = {0.f, 0.f}, vi[2] = {0.f, 0.f};
+                float pj[NA], lpj[NA], diff[NA], vi[NA];
+#pragma unroll
+                for (int j = 0; j < NA; ++j) { pj[j] = 0.f; lpj[j] = 0.f; diff[j] = 0.f; vi[j] = 0.f; }
                 int aidx = 0;
                 if (HEAD == 0) {
                     aidx = reinterpret_cast<const int*>(sc)[256 + ms];
                     int jmax = 0;
                     float mx = out[0];
                     if (NOUT > 1 && out[1] > mx) { mx = out[1]; jmax = 1; }
-                    float ex[2], s = 0.f;
+                    if (NOUT > 2 && out[2] > mx) { mx = out[2]; jmax = 2; }
+                    if (NOUT > 3 && out[3] > mx) { mx = out[3]; jmax = 3; }
+                    float ex[NA], s = 0.f;
 #pragma unroll
                     for (int j = 0; j < NOUT; ++j) { ex[j] = j == jmax ? 1.0f : expf(out[j] - mx); s += ex[j]; }
                     float hsum = 0.f;
@@ -474,8 +513,10 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
                 }
             }
             accbo0 += dout[0]; accbo1 += dout[1];
-            sDout[ms] = make_float4(dout[0], dout[1], 0.f, 0.f);
+            if (W4) { accbo2 += dout[2]; accbo3 += dout[3]; }
+            sDout[ms] = make_float4(dout[0], dout[1], W4 ? dout[2] : 0.f, W4 ? dout[3] : 0.f);
             float dmax = fmaxf(fabsf(dout[0]), fabsf(dout[1]));
+            if (W4) dmax = fmaxf(dmax, fmaxf(fabsf(dout[2]), fabsf(dout[3])));
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) dmax = fmaxf(dmax, __shfl_xor_sync(0xffffffffu, dmax, o));
             if (lane == 0) sMisc[4 + warp] = dmax;
@@ -497,21 +538,26 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
             float z[16];
             ft_ld16(my + FTG_COL_D + m0, z);
             asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            const float ws0 = wo0 * S, ws1 = wo1 * S;
-            float sb = 0.f, sw0 = 0.f, sw1 = 0.f;
+            const float ws0 = wo0 * S, ws1 = wo1 * S, ws2 = wo2 * S, ws3 = wo3 * S;
+            float sb = 0.f, sw0 = 0.f, sw1 = 0.f, sw2 = 0.f, sw3 = 0.f;
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
                 const float4 d = sDout[m0 + j];
                 const float h = z[j];
                 sw0 = fmaf(h, d.x, sw0);
                 if (NOUT > 1) sw1 = fmaf(h, d.y, sw1);
+                if (NOUT > 2) sw2 = fmaf(h, d.z, sw2);
+                if (NOUT > 3) sw3 = fmaf(h, d.w, sw3);
                 float u = d.x * ws0;
                 if (NOUT > 1) u = fmaf(d.y, ws1, u);
+                if (NOUT > 2) u = fmaf(d.z, ws2, u);
+                if (NOUT > 3) u = fmaf(d.w, ws3, u);
                 z[j] = u * fmaf(-h, h, 1.0f);
                 sb += z[j];
             }
             if (flast >= 0) {
                 accb[L - 1] += sb; accWo0 += sw0; accWo1 += sw1;
+                if (W4) { accWo2 += sw2; accWo3 += sw3; }
                 unsigned char* pz = sm + ly.last;
 #pragma unroll
                 for (int c = 0; c < 2; ++c) {
@@ -661,8 +707,16 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
         quarter_sum(accWo1, 0);
         reduce_write(0, wd[L - 1], L - 1, [&](int f, float s) { gp[Lout.pw_off + f * Lout.Np + 1] = s; });
     }
+    if (NOUT > 2) {
+        quarter_sum(accWo2, 0);
+        reduce_write(0, wd[L - 1], L - 1, [&](int f, float s) { gp[Lout.pw_off + f * Lout.Np + 2] = s; });
+    }
+    if (NOUT > 3) {
+        quarter_sum(accWo3, 0);
+        reduce_write(0, wd[L - 1], L - 1, [&](int f, float s) { gp[Lout.pw_off + f * Lout.Np + 3] = s; });
+    }
     if (tid < 64) {
-        float hv[4] = {accbo0, accbo1, accls0, accls1};
+        float hv[4] = {accbo0, accbo1, W4 ? accbo2 : accls0, W4 ? accbo3 : accls1};   // W4: discrete head, no log_std
 #pragma unroll
         for (int i = 0; i < 4; ++i) hv[i] = warp_sum(hv[i]);
         if (lane == 0) {
@@ -673,7 +727,8 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
     __syncthreads();
     if (tid < 4) {
         const float s = sMisc[8 + tid] + sMisc[12 + tid];
-        if (tid < 2) { if (tid < NOUT) gp[Lout.pb_off + tid] = s; }
+        if (W4) { if (tid < NOUT) gp[Lout.pb_off + tid] = s; }
+        else if (tid < 2) { if (tid < NOUT) gp[Lout.pb_off + tid] = s; }
         else if (HEAD == 1 && tid - 2 < NOUT) gp[pd.pack_fwd + (tid - 2)] = s;
     }
     __syncthreads();

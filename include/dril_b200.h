@@ -40,8 +40,10 @@ typedef struct dril_policy dril_policy;
 typedef struct dril_buffer dril_buffer;
 
 /* env kinds (dynamics live in ClassicControlEnvironments.jl for the reference; SYNTHETIC is
- * the rollout-sweep env of SURVEY.md §8d C5) */
-enum { DRIL_ENV_CARTPOLE = 0, DRIL_ENV_PENDULUM = 1, DRIL_ENV_SYNTHETIC = 2 };
+ * the rollout-sweep env of SURVEY.md §8d C5).  MOUNTAINCAR and ACROBOT: Discrete(3) actions (Discrete.start = act_start),
+ * MOUNTAINCAR_CONTINUOUS: Box(1) force on [-1, 1] */
+enum { DRIL_ENV_CARTPOLE = 0, DRIL_ENV_PENDULUM = 1, DRIL_ENV_SYNTHETIC = 2, DRIL_ENV_MOUNTAINCAR = 3,
+       DRIL_ENV_MOUNTAINCAR_CONTINUOUS = 4, DRIL_ENV_ACROBOT = 5 };
 /* action-space kinds: Discrete / Box (src/spaces.jl:28-44,157-164) */
 enum { DRIL_ACT_DISCRETE = 0, DRIL_ACT_CONTINUOUS = 1 };
 #define DRIL_MAX_HIDDEN_LAYERS 5
@@ -127,8 +129,8 @@ int32_t dril_device_count(int32_t* count);
  * test_gpu_parity.py::test_kernel_paths_vs_oracle).  Unknown keys are an error.
  *   "ft"          features-on-lanes tcgen05 loss/grad kernel (fp16 hi/lo split, actor + critic merged) for hidden_dims = [64, 64],
  *                 obs_dim <= 4, Discrete(<= 2): the default for such policies
- *   "ftg"         general-shape features-on-lanes tcgen05 loss/grad kernel (1-3 hidden layers of width <= 128, discrete or
- *                 Gaussian head); 2 = also prefer it where "ft" applies
+ *   "ftg"         general-shape features-on-lanes tcgen05 loss/grad kernel (2-3 hidden layers of width 64 / 128, Discrete(<= 4) or
+ *                 Box(<= 2) head); 2 = also prefer it where "ft" applies
  *   "tc"          round-1 samples-on-lanes tcgen05 (3xTF32) loss/grad kernel for the "ft" shapes (used when "ft" is 0)
  *   "defer_critic" general rollout kernel: actor-only step loop, values from one batched tcgen05 critic pass afterwards
  *   "persistent"  "ft" kernel with the fused tail: all minibatch steps of an update (epochs x minibatches, tile records of all
@@ -196,7 +198,8 @@ int32_t dril_env_observe(dril_env* env, float* obs_out);
 int32_t dril_env_step(dril_env* env, const void* actions, float* rewards, uint8_t* terminated,
                       uint8_t* truncated, float* terminal_obs, float* episode_r, int64_t* episode_l);
 int32_t dril_env_num_envs(dril_env* env, int64_t* n);
-/* raw internal state, for replay tests: float[state_dim][n] + int32 steps[n]. state_dim: cartpole 4, pendulum 2, synthetic 0 */
+/* raw internal state, for replay tests: float[state_dim][n] + int32 steps[n]. state_dim: cartpole 4, pendulum 2, synthetic 0,
+ * mountaincar 2, mountaincar_continuous 2, acrobot 4 */
 int32_t dril_env_get_state(dril_env* env, float* state, int32_t* steps);
 int32_t dril_env_set_state(dril_env* env, const float* state, const int32_t* steps);
 /* normaliser statistics (save/load/sync_normalization_stats, normalizeWrapperEnv.jl:261-309) */
@@ -207,7 +210,8 @@ int32_t dril_env_set_norm_stats(dril_env* env, const float* obs_mean, const floa
 int32_t dril_env_set_training(dril_env* env, int32_t training);
 /* ScalingWrapperEnv(env) around every env of the batch (environment_wrappers/scalingWrapperEnv.jl:14-49): observations are
  * mapped from the ORIGINAL Box [obs_low, obs_high] to [-1, 1] (observe, :94-99), actions arrive in [-1, 1] and are mapped back
- * to [act_low, act_high] before act! (:112-115).  The wrapper sits below Monitor / Normalize.  Box/Box envs only (pendulum). */
+ * to [act_low, act_high] before act! (:112-115).  The wrapper sits below Monitor / Normalize.  Box/Box envs only (pendulum,
+ * mountaincar_continuous). */
 int32_t dril_env_set_scaling(dril_env* env, int32_t on, const float* obs_low, const float* obs_high,
                              const float* act_low, const float* act_high);
 /* original (un-normalised) obs / rewards of the last observe/act (old_obs, old_rewards) */
@@ -225,8 +229,9 @@ int32_t dril_policy_create(dril_ctx* ctx, int32_t obs_dim, int32_t n_hidden, con
                            const float* act_low, const float* act_high, dril_policy** out);
 int32_t dril_policy_destroy(dril_policy* p);
 int32_t dril_policy_num_params(dril_policy* p, int64_t* n);
-/* which loss/grad kernel the update uses for this policy: 1 = tensor cores (tcgen05, 3xTF32; hidden_dims = [64, 64],
- * obs_dim <= 4, Discrete(n <= 2), option "tc" on), 2 = general-shape kernel with the layers whose padded dims are
+/* which loss/grad kernel the update uses for this policy: 1 = tensor cores (tcgen05: hidden_dims = [64, 64], obs_dim <= 4,
+ * Discrete(n <= 2), option "tc" on; or 2-3 hidden layers of width 64 / 128, obs_dim <= 15, Discrete(n <= 4) or Box(n <= 2), option
+ * "ftg" on), 2 = general-shape kernel with the layers whose padded dims are
  * multiples of 16 on warp-level tensor-core tiles (mma.sync TF32, 3xTF32; option "mma"), 0 = general-shape kernel on
  * fp32 FMA tiles only.  All replace the same reference code (src/algorithms/ppo.jl:188-254 loss functor + Zygote
  * pullback) and meet the same 1e-4 parity bound. */

@@ -67,13 +67,13 @@ const DEFAULT_CTX = Ref{Union{Nothing, Context}}(nothing)
 default_ctx() = (isnothing(DEFAULT_CTX[]) && (DEFAULT_CTX[] = Context()); DEFAULT_CTX[])
 
 # ---- batched env -------------------------------------------------------------------------------
-const ENV_KINDS = Dict(:cartpole => 0, :pendulum => 1, :synthetic => 2)
+const ENV_KINDS = Dict(:cartpole => 0, :pendulum => 1, :synthetic => 2, :mountaincar => 3, :mountaincar_continuous => 4, :acrobot => 5)
 
 """
     CudaBatchedEnv(kind, n_envs; max_steps, act_start, monitor_window, normalize)
 
 Device-resident replacement of `NormalizeWrapperEnv(MonitorWrapperEnv(MultiThreadedParallelEnv(envs)))`
-for `kind in (:cartpole, :pendulum, :synthetic)`.
+for `kind in (:cartpole, :pendulum, :synthetic, :mountaincar, :mountaincar_continuous, :acrobot)`.
 """
 mutable struct CudaBatchedEnv <: AbstractParallelEnv
     ctx::Context
@@ -95,6 +95,13 @@ function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_
         Box(-hi, hi), Discrete(2, act_start)
     elseif kind == :pendulum
         Box(Float32[-1, -1, -8], Float32[1, 1, 8]), Box(Float32[-2], Float32[2])
+    elseif kind == :mountaincar
+        Box(Float32[-1.2, -0.07], Float32[0.6, 0.07]), Discrete(3, act_start)
+    elseif kind == :mountaincar_continuous
+        Box(Float32[-1.2, -0.07], Float32[0.6, 0.07]), Box(Float32[-1], Float32[1])
+    elseif kind == :acrobot
+        hi = Float32[1, 1, 1, 1, 4pi, 9pi]
+        Box(-hi, hi), Discrete(3, act_start)
     else
         Box(-ones(Float32, obs_dim), ones(Float32, obs_dim)), Discrete(2, act_start)
     end

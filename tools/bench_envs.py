@@ -1,0 +1,110 @@
+"""PPO throughput on MountainCar, MountainCarContinuous and Acrobot: one JSON line per env and env count.
+
+    python tools/bench_envs.py [--envs mountaincar,mountaincar_continuous,acrobot] [--n-envs 4096,65536] [--steps 20] [--normalize]
+
+Each run: [64, 64] policy, n_steps 128, 4 epochs x 4 minibatches; warm-up iterations, then --steps iterations timed with CUDA events
+on the library's stream, L2 overwritten before every iteration (as bench.py does), then the same iterations again with the
+per-kernel profile on for the rollout / update split.  Reports env-steps/s, ms per iteration, the loss/grad kernel path, the rollout
+kernel the library's dispatch rule picks for the configuration, and the card name and power limit read in the same run."""
+import argparse
+import ctypes as C
+import json
+import os
+import subprocess
+import sys
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
+
+
+def card():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                             text=True, timeout=30).stdout.strip().splitlines()[0]
+        name, power = [x.strip() for x in out.split(",")]
+        return name, power
+    except Exception as e:                  # the numbers still stand; say that the card could not be read
+        return f"unknown ({e})", "unknown"
+
+
+def rollout_kernel(n, sms, normalize, act_n):
+    """launch_rollout's choice (csrc/api.cu) for a [64, 64] policy: without a training normaliser the fast kernel; with one the
+    cooperative general kernel, its actor on tcgen05 (rollout_gtc.cuh) from 64 envs per SM on"""
+    if not normalize:
+        return "fast"
+    return "gtc" if n >= 64 * sms else "general"
+
+
+def run(D, kind, n, steps, warmup, normalize):
+    from dril_b200 import _lib as L
+    T = 128
+    env = D.CudaBatchedEnv(kind, n, seed=0, monitor_window=100, normalize=D.NormalizeConfig() if normalize else None)
+    layer = D.ActorCriticLayer(env.observation_space(), env.action_space(), hidden_dims=[64, 64])
+    alg = D.PPO(n_steps=T, batch_size=T * n // 4, epochs=4)
+    agent = D.Agent(layer, alg, rng=np.random.default_rng(0))
+    ctx = agent.ctx
+    lib = ctx.lib
+    buf = D.RolloutBuffer(env.observation_space(), env.action_space(), alg.gae_lambda, alg.gamma, T, n)
+    hyper = alg.hyper()
+    L.check(lib.dril_iteration_prepare(env.h, agent.device.h, buf.h, int(alg.epochs), int(alg.batch_size)))
+
+    def iterate(k):
+        for _ in range(k):
+            ctx.flush_l2()
+            L.check(lib.dril_ppo_iteration_async(env.h, agent.device.h, buf.h, C.byref(hyper), alg.epochs, alg.batch_size,
+                                                 agent.shuffle_seed, agent.epoch_counter))
+            agent.epoch_counter += alg.epochs
+            st = L.IterStats()
+            L.check(lib.dril_iteration_result(agent.device.h, C.byref(st)))
+
+    iterate(warmup)
+    ctx.synchronize()
+    ctx.event_record(0)
+    iterate(steps)
+    ctx.event_record(1)
+    ctx.synchronize()
+    ms = ctx.event_elapsed_ms(0, 1) / steps
+    ctx.set_profiling(True)
+    ctx.reset_profile()
+    iterate(steps)
+    ctx.synchronize()
+    prof = ctx.profile()
+    ctx.set_profiling(False)
+    upd = sum(prof.get(k, (0.0, 0))[0] for k in ("loss_grad", "grad_reduce", "adam", "permute", "adv_stats")) / steps
+    sms = ctx.sm_count()
+    act = env.action_space()
+    res = dict(env=kind, n_envs=n, n_steps=T, hidden=[64, 64], epochs=4, minibatches=4, normalize=bool(normalize),
+               env_steps_per_s=n * T / (ms * 1e-3), ms_per_iter=ms,
+               rollout_ms=prof.get("rollout", (0.0, 0))[0] / steps, update_ms=upd,
+               update_path=agent.device.update_path(),
+               rollout_kernel=rollout_kernel(n, sms, normalize, getattr(act, "n", 1)),
+               ep_rew_mean=env.monitor_stats()["ep_rew_mean"], timed_iters=steps, warmup_iters=warmup)
+    buf.close()
+    env.close()
+    return res
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--envs", default="mountaincar,mountaincar_continuous,acrobot")
+    ap.add_argument("--n-envs", default="4096,65536")
+    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--normalize", action="store_true")
+    args = ap.parse_args()
+    import __graft_entry__
+    __graft_entry__.build()
+    import dril_b200 as D
+    name, power = card()
+    for kind in args.envs.split(","):
+        for n in (int(x) for x in args.n_envs.split(",")):
+            r = run(D, kind, n, args.steps, args.warmup, args.normalize)
+            r.update(card=name, power_limit=power)
+            print(json.dumps(r), flush=True)
+
+
+if __name__ == "__main__":
+    main()
