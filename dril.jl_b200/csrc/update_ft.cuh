@@ -17,8 +17,10 @@
 // hi*lo, fp32 accumulation): 22 significant bits like 3xTF32 at half the instructions and half the operand bytes.
 // H0/H1 are tanh outputs and W1 is a weight matrix (bounded); the deltas dZ1 are not, so every group scales them by a
 // power of two S chosen from a tile's max |dL/dout| and the net's max |W2| row sum such that |S dZ1|
-// is below 2^4 on the tile that fixes it (the first tile of a group with a non-zero gradient; later tiles may be 2^12 times
-// larger before fp16 overflows), so dW1 stays in TMEM over all tiles of a group and everything is unscaled exactly at the end.
+// is below 2^4 on the tile that fixes it (the first tile of a group with a non-zero gradient).  dW1 stays in TMEM over all
+// tiles of a group and everything is unscaled exactly at the end.  A later tile whose scaled bound would pass fp16's
+// 65504 lowers S to sit where the first tile sat, and the group's dW1 columns and scaled sums are multiplied by the
+// exact ratio; tiles inside that headroom compute what a fixed S computes.
 //
 // M = 64 accumulators use 16 lanes of every TMEM lane quadrant; the actor's sit at lane offset 0 and the critic's at
 // lane offset 16 of the same columns, so warp q, lane l is feature 16 q + l % 16 of net l / 16 and both nets run in ONE
@@ -203,6 +205,25 @@ __device__ __forceinline__ void ft_ld16(uint32_t taddr, float* r) {
 #pragma unroll
     for (int j = 0; j < 16; ++j) r[j] = __uint_as_float(u[j]);
 }
+// TMEM columns taddr .. taddr + n - 1 (n a multiple of 16) of this warp's lanes multiplied by r1 r2 (powers of two), after the
+// MMAs that wrote them completed; out of line: it runs only when a tile lowers the delta scale
+__device__ __noinline__ void ft_rescale_tmem(uint32_t taddr, int n, float r1, float r2) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+#pragma unroll 1
+    for (int c = 0; c < n; c += 16) {
+        float v[16];
+        ft_ld16(taddr + c, v);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+        for (int j = 0; j < 16; ++j) v[j] = (v[j] * r1) * r2;
+        asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr + c),
+                     "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])),
+                     "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7])),
+                     "r"(__float_as_uint(v[8])), "r"(__float_as_uint(v[9])), "r"(__float_as_uint(v[10])), "r"(__float_as_uint(v[11])),
+                     "r"(__float_as_uint(v[12])), "r"(__float_as_uint(v[13])), "r"(__float_as_uint(v[14])), "r"(__float_as_uint(v[15])) : "memory");
+    }
+    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+}
 __device__ __forceinline__ float ft_tanh_scaled(float xs) {       // tanh(x) from xs = C2 * x
     float e, r;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(xs));
@@ -385,8 +406,9 @@ __global__ void __launch_bounds__(FT_THREADS, 1) ppo_loss_grad_ft_kernel(const _
     const float invB = (float)(1.0 / gcount);
     float stats[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     float accb2_0 = 0.f, accb2_1 = 0.f;                               // head threads: sums of dL/dout (output-layer bias gradients)
-    // delta scale of this thread's net in this group: a power of two fixed at the group's first tile with a non-zero gradient, so
-    // that dW1 can stay in TMEM over all the group's tiles; the scaled sums below are unscaled once at the end
+    // delta scale of this thread's net in this group: a power of two fixed at the group's first tile with a non-zero gradient
+    // and lowered only when a later tile would leave fp16's range, so that dW1 can stay in TMEM over all the group's tiles;
+    // the scaled sums below are unscaled once at the end
     float S = 1.0f, invS = 1.0f;
     bool s_fixed = false;
     float accb1 = 0.f, accW2_0 = 0.f, accb0 = 0.f, accW0_0 = 0.f, accW0_1 = 0.f, accW0_2 = 0.f, accW0_3 = 0.f;
@@ -614,15 +636,26 @@ __global__ void __launch_bounds__(FT_THREADS, 1) ppo_loss_grad_ft_kernel(const _
         FT_MARK(10);
         // ---- B2: dZ1 = (W2 dout) .* (1 - H1^2), scaled by the tile's power of two -> dZ1 images; db1, dW2 sums -------------------
         {
-            if (!s_fixed) {
-                const float bound = fmaxf(sMax[net * 2], sMax[net * 2 + 1]) * w2bound;
-                if (bound > 0.f && bound < 3.0e38f) {
-                    int E = ((__float_as_int(bound) >> 23) & 255) - 127;          // bound < 2^(E + 1)
-                    E = E < -100 ? -100 : (E > 100 ? 100 : E);
-                    S = __int_as_float((3 - E + 127) << 23);                      // |S dZ1| < 2^4 on this tile: later tiles may grow 2^12-fold
-                    invS = __int_as_float((E - 3 + 127) << 23);
-                    s_fixed = true;
-                }
+            // the scale is fixed at the first tile with a non-zero gradient; a later tile whose bound would pass fp16's 65504
+            // moves it down to sit where the first tile sat, and the group's dW1 in TMEM and the scaled register sums
+            // are multiplied by the exact ratio of the two powers of two (dW1: the previous tile's G3 completed at bar3, this
+            // tile's is issued after the group barrier below)
+            const float bound = fmaxf(sMax[net * 2], sMax[net * 2 + 1]) * w2bound;
+            const bool fix = bound > 0.f && bound < 3.0e38f && (!s_fixed || bound * S > 65504.0f);
+            int E = ((__float_as_int(bound) >> 23) & 255) - 127;                  // bound < 2^(E + 1)
+            E = E < -100 ? -100 : (E > 100 ? 100 : E);
+            if (__any_sync(0xffffffffu, fix && s_fixed)) {                        // warp-uniform: both nets share the warp
+                const int sE = 130 - (__float_as_int(S) >> 23);                   // S = 2^(3 - sE)
+                const int d = (fix && s_fixed) ? sE - E : 0;                      // S_new / S_old = 2^d, -200 <= d <= 0
+                const float r1 = __int_as_float((d / 2 + 127) << 23), r2 = __int_as_float((d - d / 2 + 127) << 23);
+                ft_rescale_tmem(my + FT_COL_D3 + m0, 32, r1, r2);
+                accb1 = (accb1 * r1) * r2; accb0 = (accb0 * r1) * r2;
+                accW0_0 = (accW0_0 * r1) * r2; accW0_1 = (accW0_1 * r1) * r2; accW0_2 = (accW0_2 * r1) * r2; accW0_3 = (accW0_3 * r1) * r2;
+            }
+            if (fix) {
+                S = __int_as_float((3 - E + 127) << 23);                          // |S dZ1| < 2^4 on this tile
+                invS = __int_as_float((E - 3 + 127) << 23);
+                s_fixed = true;
             }
             const float wsd = (w2_0 - w2_1) * S;                                  // actor, two logits: W2[f][0] - W2[f][1]; else W2[f][0] (w2_1 = 0)
             float z[32];

@@ -11,9 +11,10 @@
 //                                                          dH_{l-1} = W_l dZ_l              (A = the same image, MN-major),
 //                                                          dW_l     = H_{l-1} dZ_l^T        (A = H_{l-1} image, K-major);
 //   * the dW_l accumulators stay in TMEM over all tiles of the pass.  The deltas are scaled by ONE power of two per CTA and
-//     pass, fixed at the first tile with a non-zero gradient such that its largest |dZ_last| bound sits at 2^2 (later
-//     tiles may grow 2^13-fold before fp16 saturates; conversions saturate instead of overflowing); everything is
-//     unscaled exactly when the partial plane is written;
+//     pass, fixed at the first tile with a non-zero gradient such that its largest |dZ_last| bound sits at 2^2; a later
+//     tile whose scaled bound would reach 2^14 lowers the scale to sit where the first tile sat and multiplies the dW
+//     accumulators and scaled sums by the exact ratio (fp16 ends at 65504); everything is unscaled exactly when the
+//     partial plane is written;
 //   * shared memory: weight images of the pass (W_1.., W_0 with the bias row), one image buffer per hidden layer but
 //     the last (H_l, later reused for dZ_l), one buffer for the last layer's fp32 tile / delta image, two tile records.
 // The kernel ends with the cooperative tail of update_tc.cuh.  Tile records of all epochs are written by one launch of
@@ -273,7 +274,7 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
     float accWo0 = 0.f, accWo1 = 0.f, accWo2 = 0.f, accWo3 = 0.f;  // dW_out[flast][0..3] (unscaled)
     float accbo0 = 0.f, accbo1 = 0.f, accls0 = 0.f, accls1 = 0.f;  // head threads: output bias / log_std gradient sums
     float accbo2 = 0.f, accbo3 = 0.f;
-    float S = 1.0f, invS = 1.0f;
+    float S = 1.0f, invS = 1.0f;                                   // delta scale of the pass
     bool s_fixed = false;
 
     const long long n_tiles = (a.mb.count + 63) / 64;
@@ -522,22 +523,34 @@ __device__ __forceinline__ void ftg_pass(const LossArgs& a, const FtgArgs& fa, u
             if (lane == 0) sMisc[4 + warp] = dmax;
         }
         __syncthreads();
-        // ---- the pass's delta scale: fixed at the first tile with a non-zero gradient -----------------------------------------
-        if (!s_fixed) {
+        // ---- dZ_{L-1} = (W_out dout) .* (1 - H^2), scaled -> delta images (over the fp32 tile); bias / W_out sums -------------
+        {
             const float bound = fmaxf(sMisc[4], sMisc[5]) * wbound * (float)NOUT;
-            if (bound > 0.f && bound < 3.0e38f) {
+            float z[16];
+            ft_ld16(my + FTG_COL_D + m0, z);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            // the pass's delta scale: fixed at the first tile with a non-zero gradient; a later tile whose bound would reach 2^14
+            // moves it down to sit where the first tile sat, and the dW accumulators in TMEM and the scaled register sums are
+            // multiplied by the exact ratio of the two powers of two (the previous tile's dW GEMMs completed at barW, this
+            // tile's are issued after the barrier that follows the delta images).  The decision is CTA-uniform; its shared
+            // memory loads were issued before the TMEM load above.
+            if (bound > 0.f && bound < 3.0e38f && (!s_fixed || bound * S >= 16384.0f)) {
                 int E = ((__float_as_int(bound) >> 23) & 255) - 127;              // bound < 2^(E + 1)
                 E = E < -100 ? -100 : (E > 100 ? 100 : E);
+                if (s_fixed) {
+                    const int d = (128 - (__float_as_int(S) >> 23)) - E;          // S = 2^(1 - E_old): S_new / S_old = 2^d, -200 <= d <= 0
+                    const float r1 = __int_as_float((d / 2 + 127) << 23), r2 = __int_as_float((d - d / 2 + 127) << 23);
+#pragma unroll
+                    for (int l = 1; l < L; ++l) ft_rescale_tmem(my + FTG_COL_DW + (l - 1) * 128 + sg * (wd[l] >> 2), wd[l] >> 2, r1, r2);
+#pragma unroll
+                    for (int l = 0; l < L; ++l) accb[l] = (accb[l] * r1) * r2;
+#pragma unroll
+                    for (int k = 0; k < FTG_MAX_OBS + 1; ++k) accW0[k] = (accW0[k] * r1) * r2;
+                }
                 S = __int_as_float((1 - E + 127) << 23);                          // S * bound < 2^2
                 invS = __int_as_float((E - 1 + 127) << 23);
                 s_fixed = true;
             }
-        }
-        // ---- dZ_{L-1} = (W_out dout) .* (1 - H^2), scaled -> delta images (over the fp32 tile); bias / W_out sums -------------
-        {
-            float z[16];
-            ft_ld16(my + FTG_COL_D + m0, z);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
             const float ws0 = wo0 * S, ws1 = wo1 * S, ws2 = wo2 * S, ws3 = wo3 * S;
             float sb = 0.f, sw0 = 0.f, sw1 = 0.f, sw2 = 0.f, sw3 = 0.f;
 #pragma unroll

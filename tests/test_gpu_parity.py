@@ -836,8 +836,10 @@ def test_c2_shape_update_vs_oracle(D, tc, ft):
 @pytest.mark.parametrize("B", [1, 63, 64, 65, 1000, 148 * 64 * 2 + 31])
 def test_tcgen05_kernels_vs_oracle(D, ft, B):
     """Both tcgen05 loss/grad kernels for the default [64,64] layer (features-on-lanes fp16 hi/lo, option "ft" = 1, and
-    samples-on-lanes 3xTF32, "ft" = 0) on ragged tile counts, with large and tiny advantage / return scales (the fp16
-    kernel rescales its deltas per tile) and with one action (Discrete(1): zero actor gradient)."""
+    samples-on-lanes 3xTF32, "ft" = 0) on ragged tile counts, with large and tiny advantage / return scales applied to the
+    whole minibatch (the fp16 kernel scales its deltas by a power of two fixed at a warp group's first tile with a non-zero
+    gradient; tiles of different scales: tests/test_gpu_grad_scale.py) and with one action (Discrete(1): zero actor
+    gradient)."""
     D.set_option("ft", ft)
     try:
         for name, scale in (("cartpole", 1.0), ("cartpole", 3e4), ("cartpole", 1e-6), ("one_action", 1.0)):

@@ -311,8 +311,8 @@ def test_reference_order_matches_timemajor():
 
 @pytest.mark.parametrize("kind", ["discrete", "continuous"])
 def test_analytic_gradients_vs_torch_autograd(kind):
-    """ppo.jl:365-407 restated in torch fp64 with autograd vs the oracle's hand-written backward."""
-    import torch
+    """ppo.jl:365-407 restated in torch fp64 with autograd (oracle/ppo64.py) vs the oracle's hand-written backward."""
+    from oracle.ppo64 import loss64
     rng = np.random.default_rng(5)
     if kind == "discrete":
         spec = P.PolicySpec(4, [16, 8], "discrete", 3, act_start=0)
@@ -329,61 +329,11 @@ def test_analytic_gradients_vs_torch_autograd(kind):
     old_v = (v0 + rng.normal(size=40).astype(f32) * 0.3).astype(f32)
     for cfg in (O.PPOConfig(ent_coef=0.01), O.PPOConfig(ent_coef=0.02, clip_range_vf=0.2, normalize_advantage=False)):
         loss, stats, g = O.ppo_loss_and_grads(spec, flat, obs, actions, adv, ret, old_lp, old_v, cfg)
-        tl, tg, tstats = _torch_loss(spec, flat, obs, actions, adv, ret, old_lp, old_v, cfg)
+        tl, tg, tstats = loss64(spec, flat, obs, actions, adv, ret, old_lp, old_v, cfg)
         assert abs(loss - tl) < 1e-5 * max(1, abs(tl))
         np.testing.assert_allclose(g, tg, rtol=2e-4, atol=2e-6)
         for k in ("clip_fraction", "approx_kl_div", "entropy", "ratio"):
             assert abs(stats[k] - tstats[k]) < 1e-5, k
-
-
-def _torch_loss(spec, flat, obs, actions, adv, ret, old_lp, old_v, cfg):
-    import torch
-    t = torch.tensor(flat.astype(np.float64), requires_grad=True)
-    p = 0
-    nets = []
-    for net in (0, 1):
-        layers = []
-        for (i, o) in spec.layer_dims(net):
-            W = t[p:p + i * o].reshape(i, o); p += i * o
-            b = t[p:p + o]; p += o
-            layers.append((W, b))
-        nets.append(layers)
-
-    def mlp(layers, x):
-        for li, (W, b) in enumerate(layers):
-            x = x @ W + b
-            if li < len(layers) - 1:
-                x = torch.tanh(x)
-        return x
-    x = torch.tensor(obs.astype(np.float64))
-    out = mlp(nets[0], x)
-    values = mlp(nets[1], x).reshape(-1)
-    A = torch.tensor(adv.astype(np.float64))
-    if cfg.normalize_advantage:
-        A = (A - A.mean()) / (A.std(unbiased=True) + 1e-8)
-    if spec.act_kind == "discrete":
-        probs = torch.softmax(out, dim=1)
-        idx = torch.tensor(actions.reshape(-1) - spec.act_start)
-        logp = torch.log(probs[torch.arange(len(idx)), idx])
-        ent = -(probs * torch.log(probs)).sum(1)
-    else:
-        ls = t[p:p + spec.act_n]
-        a = torch.tensor(actions.astype(np.float64))
-        k = spec.act_n
-        logp = -0.5 * (2 * ls.sum() + ((a - out) ** 2 * torch.exp(-2 * ls)).sum(1) + k * np.log(2 * np.pi))
-        ent = (0.5 * k * (1 + np.log(2 * np.pi)) + ls.sum()) * torch.ones(len(a), dtype=torch.float64)
-    ov = torch.tensor(old_v.astype(np.float64))
-    if cfg.clip_range_vf is not None:
-        values = ov + torch.clamp(values - ov, -cfg.clip_range_vf, cfg.clip_range_vf)
-    lr = logp - torch.tensor(old_lp.astype(np.float64))
-    r = torch.exp(lr)
-    rc = torch.clamp(r, 1 - cfg.clip_range, 1 + cfg.clip_range)
-    p_loss = -torch.minimum(r * A, rc * A).mean()
-    loss = p_loss + cfg.ent_coef * (-ent.mean()) + cfg.vf_coef * ((values - torch.tensor(ret.astype(np.float64))) ** 2).mean()
-    loss.backward()
-    st = dict(clip_fraction=float((r != rc).double().mean()), approx_kl_div=float((torch.exp(lr) - 1 - lr).mean()),
-              entropy=float(ent.mean()), ratio=float(r.mean()))
-    return float(loss), t.grad.numpy(), st
 
 
 def test_feistel_is_permutation():
