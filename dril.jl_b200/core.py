@@ -11,6 +11,16 @@ from .spaces import Box, Discrete
 
 ENV_KINDS = {"cartpole": 0, "pendulum": 1, "synthetic": 2, "mountaincar": 3, "mountaincar_continuous": 4, "acrobot": 5}
 ENV_STATE_DIMS = {"cartpole": 4, "pendulum": 2, "synthetic": 0, "mountaincar": 2, "mountaincar_continuous": 2, "acrobot": 4}
+# per-env physical parameters (dril_b200.h): (name, default) in the order of the C arrays; names are Gymnasium's attributes
+ENV_PARAMS = {
+    "cartpole": (("gravity", 9.8), ("masscart", 1.0), ("masspole", 0.1), ("length", 0.5), ("force_mag", 10.0), ("tau", 0.02)),
+    "pendulum": (("g", 10.0), ("m", 1.0), ("l", 1.0), ("dt", 0.05)),
+    "synthetic": (),
+    "mountaincar": (("force", 0.001), ("gravity", 0.0025)),
+    "mountaincar_continuous": (("power", 0.0015), ("gravity", 0.0025)),
+    "acrobot": (("link_length_1", 1.0), ("link_mass_1", 1.0), ("link_mass_2", 1.0), ("link_com_pos_1", 0.5),
+                ("link_com_pos_2", 0.5), ("link_moi", 1.0)),
+}
 
 
 class Context:
@@ -117,7 +127,7 @@ class CudaBatchedEnv:
     path used by evaluate_agent and callbacks; training uses the fused device rollout."""
 
     def __init__(self, kind, n_envs, max_steps=0, obs_dim=0, act_start=1, seed=None, ctx=None,
-                 monitor_window=0, normalize=None, gid_offset=0, obs_shape=None, scaling=False):
+                 monitor_window=0, normalize=None, gid_offset=0, obs_shape=None, scaling=False, env_params=None):
         self.kind = kind.lower()
         assert self.kind in ENV_KINDS, f"unknown env kind {kind}"
         self.ctx = ctx or Context.default()
@@ -172,6 +182,9 @@ class CudaBatchedEnv:
             self._act_space = Box(-np.ones_like(al), np.ones_like(ah))
         self._term = np.zeros(self.n_envs, dtype=bool)
         self._trunc = np.zeros(self.n_envs, dtype=bool)
+        self._param_ranges = None
+        if env_params:
+            self.set_env_params(**env_params)
         if seed is not None:
             self.seed(seed)
             self.reset()
@@ -249,6 +262,42 @@ class CudaBatchedEnv:
         st = None if state is None else L.f32(state)
         sp = None if steps is None else np.ascontiguousarray(steps, dtype=np.int32)
         L.check(self.ctx.lib.dril_env_set_state(self.h, L.ptr(st), L.ptr(sp)))
+
+    # ---- per-env physical parameters ----
+    def set_env_params(self, **kw):
+        """Per-env parameter ranges, e.g. set_env_params(length=(0.25, 1.0), masspole=0.2).  Each value is a scalar, an
+        (n_envs,) array, or a tuple (lo, hi) of either; every reset draws a value per env from [lo, hi] (a scalar or array is
+        a fixed value).  Unnamed parameters keep their defaults (ENV_PARAMS).  With no keyword the env returns to the
+        built-in constants."""
+        names = [nm for nm, _ in ENV_PARAMS[self.kind]]
+        unknown = set(kw) - set(names)
+        assert not unknown, f"{self.kind} has no parameter(s) {sorted(unknown)}; it has {names}"
+        lib, n = self.ctx.lib, self.n_envs
+        if not kw:
+            if names:
+                L.check(lib.dril_env_set_params(self.h, len(names), None, None))
+            self._param_ranges = None
+            return
+        lo = np.empty((len(names), n), np.float32)
+        hi = np.empty((len(names), n), np.float32)
+        for k, (nm, default) in enumerate(ENV_PARAMS[self.kind]):
+            v = kw.get(nm, default)
+            a, b = v if isinstance(v, tuple) else (v, v)
+            lo[k], hi[k] = np.broadcast_to(np.asarray(a, np.float32), (n,)), np.broadcast_to(np.asarray(b, np.float32), (n,))
+        L.check(lib.dril_env_set_params(self.h, len(names), L.ptr(lo), L.ptr(hi)))
+        self._param_ranges = {nm: (lo[k].copy(), hi[k].copy()) for k, nm in enumerate(names)}
+
+    def env_param_ranges(self):
+        """{name: (lo, hi)} as set by set_env_params, or None for the built-in constants."""
+        return None if self._param_ranges is None else dict(self._param_ranges)
+
+    def env_params(self):
+        """{name: (n_envs,) float32 array}: each env's parameter values for its running episode."""
+        names = [nm for nm, _ in ENV_PARAMS[self.kind]]
+        out = np.empty((len(names), self.n_envs), np.float32)
+        if names:
+            L.check(self.ctx.lib.dril_env_get_params(self.h, len(names), L.ptr(out)))
+        return {nm: out[k].copy() for k, nm in enumerate(names)}
 
     def set_training(self, training):
         L.check(self.ctx.lib.dril_env_set_training(self.h, int(bool(training))))

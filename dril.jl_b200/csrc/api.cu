@@ -2,6 +2,7 @@
 // host<->device staging.  All compute is in the kernels of rollout.cuh / gae.cuh / update.cuh.
 #include <dlfcn.h>
 #include <math.h>
+#include <cmath>
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
@@ -98,20 +99,33 @@ static bool tc_eligible(const PolicyDesc& pd) {
 }
 
 // rollout kernels by the env kind they step: CartPole, Pendulum and the synthetic env run the instantiations built for those
-// kinds alone (env.cuh), every other kind the one built for all kinds
-static void* rollout_fn(bool ws, int kind) {
-    if (env_kind_set(kind) == ENV_KS_CLASSIC) return ws ? (void*)rollout_kernel<true, ENV_KS_CLASSIC> : (void*)rollout_kernel<false, ENV_KS_CLASSIC>;
-    return ws ? (void*)rollout_kernel<true, ENV_KS_ALL> : (void*)rollout_kernel<false, ENV_KS_ALL>;
+// kinds alone (env.cuh), every other kind the one built for all kinds; an env with per-env parameters (dril_env_set_params)
+// runs the ENV_KS_PARAMS instantiation of its kind set
+#define KS_CP_ ENV_KS_CLASSIC
+#define KS_ALL_ ENV_KS_ALL
+#define KS_CP_P_ env_param_kind_set(DRIL_ENV_CARTPOLE)
+#define KS_ALL_P_ env_param_kind_set(DRIL_ENV_ACROBOT)
+#define DRIL_KS_PICK(K_, kind, params) \
+    (env_kind_set(kind) == ENV_KS_CLASSIC ? ((params) ? K_(KS_CP_P_) : K_(KS_CP_)) : ((params) ? K_(KS_ALL_P_) : K_(KS_ALL_)))
+static void* rollout_fn(bool ws, int kind, bool params) {
+#define K_(ks) (ws ? (void*)rollout_kernel<true, ks> : (void*)rollout_kernel<false, ks>)
+    return DRIL_KS_PICK(K_, kind, params);
+#undef K_
 }
-static void* rollout_fast_fn(bool ws, int kind) {
-    if (env_kind_set(kind) == ENV_KS_CLASSIC) return ws ? (void*)rollout_fast_kernel<true, ENV_KS_CLASSIC> : (void*)rollout_fast_kernel<false, ENV_KS_CLASSIC>;
-    return ws ? (void*)rollout_fast_kernel<true, ENV_KS_ALL> : (void*)rollout_fast_kernel<false, ENV_KS_ALL>;
+static void* rollout_fast_fn(bool ws, int kind, bool params) {
+#define K_(ks) (ws ? (void*)rollout_fast_kernel<true, ks> : (void*)rollout_fast_kernel<false, ks>)
+    return DRIL_KS_PICK(K_, kind, params);
+#undef K_
 }
 // tcgen05-actor rollout by hidden-layer count, env kind and action count (2 or 4 staged output columns, gtc_nout)
-static void* rollout_gtc_fn(int L, int kind, int act_n) {
-    if (act_n > 2) return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_ALL, 4> : (void*)rollout_gtc_kernel<3, ENV_KS_ALL, 4>;
-    if (env_kind_set(kind) == ENV_KS_CLASSIC) return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_CLASSIC, 2> : (void*)rollout_gtc_kernel<3, ENV_KS_CLASSIC, 2>;
-    return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_ALL, 2> : (void*)rollout_gtc_kernel<3, ENV_KS_ALL, 2>;
+static void* rollout_gtc_fn(int L, int kind, int act_n, bool params) {
+    if (act_n > 2) {
+        if (params) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_P_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_P_, 4>;
+        return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_ALL, 4> : (void*)rollout_gtc_kernel<3, ENV_KS_ALL, 4>;
+    }
+#define K_(ks) (L == 2 ? (void*)rollout_gtc_kernel<2, ks, 2> : (void*)rollout_gtc_kernel<3, ks, 2>)
+    return DRIL_KS_PICK(K_, kind, params);
+#undef K_
 }
 
 extern "C" int32_t dril_device_count(int32_t* count) {
@@ -353,10 +367,11 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
     c->sm_count = prop.multiProcessorCount;
     DRIL_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
-        for (int ws = 0; ws < 2; ++ws) {
-            DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, kind), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-            DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, kind), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-        }
+        for (int ws = 0; ws < 2; ++ws)
+            for (int params = 0; params < 2; ++params) {
+                DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, kind, params), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+                DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, kind, params), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+            }
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
     DRIL_CUDA(cudaFuncSetAttribute(ppo_loss_grad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
@@ -375,7 +390,8 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
         for (int L = 2; L <= 3; ++L)
             for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
                 for (int an = 2; an <= 4; an += 2)
-                    DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, kind, an), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
+                    for (int params = 0; params < 2; ++params)
+                        DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, kind, an, params), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
     }
@@ -1055,7 +1071,8 @@ extern "C" int32_t dril_env_destroy(dril_env* e) {
     EnvDev& d = e->d;
     void* ps[] = {d.state, d.steps, d.episode, d.life, d.tobs, d.old_obs, d.old_rewards, d.ep_ret, d.ep_len, d.roll_sums,
                   d.roll_eps, d.ret, d.obs_mean, d.obs_var, d.ret_stats, d.counts, d.partials, e->ring.ret, e->ring.len,
-                  e->ring.head, e->compat_actions, e->compat_obs, e->roll_moments, e->xr, e->norm_snap, e->norm_snap_cnt};
+                  e->ring.head, e->compat_actions, e->compat_obs, e->roll_moments, e->xr, e->norm_snap, e->norm_snap_cnt,
+                  d.pval, d.plo, d.phi};
     for (void* p : ps) if (p) cudaFree(p);
     dril_buffer_destroy(e->compat);
     delete e;
@@ -1076,12 +1093,84 @@ extern "C" int32_t dril_env_reset(dril_env* e) {
     DRIL_CUDA(cudaSetDevice(c->device));
     {
         Span sp(c, DRIL_K_ENV);
-        env_reset_kernel<<<(unsigned)((e->d.n_envs + 255) / 256), 256, 0, c->stream>>>(e->d);
+        const unsigned grid = (unsigned)((e->d.n_envs + 255) / 256);
+        if (e->d.has_params) env_reset_kernel<ENV_KS_ALL | ENV_KS_PARAMS><<<grid, 256, 0, c->stream>>>(e->d);
+        else env_reset_kernel<ENV_KS_ALL><<<grid, 256, 0, c->stream>>>(e->d);
         DRIL_CUDA(cudaGetLastError());
     }
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
     return DRIL_OK;
 }
+// per-env physical parameters (dril_b200.h): the defaults of the table, and whether a value must be > 0 (1) or >= 0 (0)
+static const float k_env_param_default[6][DRIL_ENV_MAX_PARAMS] = {
+    {9.8f, 1.0f, 0.1f, 0.5f, 10.0f, 0.02f},          // cartpole: gravity masscart masspole length force_mag tau
+    {10.0f, 1.0f, 1.0f, 0.05f},                       // pendulum: g m l dt
+    {},                                               // synthetic
+    {0.001f, 0.0025f},                                // mountaincar: force gravity
+    {0.0015f, 0.0025f},                               // mountaincar_continuous: power gravity
+    {1.0f, 1.0f, 1.0f, 0.5f, 0.5f, 1.0f}};            // acrobot: link_length_1 link_mass_1 link_mass_2 link_com_pos_1 link_com_pos_2 link_moi
+static const int k_env_param_positive[6][DRIL_ENV_MAX_PARAMS] = {
+    {0, 1, 1, 1, 0, 1}, {0, 1, 1, 1}, {}, {0, 0}, {0, 0}, {1, 1, 1, 1, 1, 1}};
+
+extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const float* lo, const float* hi) {
+    DRIL_REQUIRE(e, "NULL argument");
+    EnvDev& d = e->d;
+    const int np = env_n_params(d.kind);
+    DRIL_REQUIRE(np > 0, "env kind %d has no physical parameters", d.kind);
+    DRIL_REQUIRE(n_params == np, "env kind %d has %d parameters, got %d", d.kind, np, n_params);
+    dril_ctx* c = e->ctx;
+    DRIL_CUDA(cudaSetDevice(c->device));
+    const size_t n = (size_t)d.n_envs;
+    if (!lo) {   // back to the built-in constants and the default instantiations
+        DRIL_CUDA(cudaStreamSynchronize(c->stream));
+        for (float* p : {d.pval, d.plo, d.phi}) if (p) cudaFree(p);
+        d.pval = d.plo = d.phi = nullptr;
+        d.has_params = 0;
+        return DRIL_OK;
+    }
+    if (!hi) hi = lo;
+    for (int k = 0; k < np; ++k) {
+        const bool pos = k_env_param_positive[d.kind][k] != 0;
+        for (size_t i = 0; i < n; ++i) {
+            const float l = lo[(size_t)k * n + i], h = hi[(size_t)k * n + i];
+            DRIL_REQUIRE(std::isfinite(l) && std::isfinite(h) && l <= h, "parameter %d of env %zu: range [%g, %g] is not finite with lo <= hi",
+                         k, i, (double)l, (double)h);
+            DRIL_REQUIRE(pos ? l > 0.f : l >= 0.f, "parameter %d of env %zu: lo %g must be %s 0", k, i, (double)l, pos ? ">" : ">=");
+        }
+    }
+    if (!d.pval) {
+        DRIL_TRY(dmalloc(&d.pval, n * DRIL_ENV_MAX_PARAMS));
+        DRIL_TRY(dmalloc(&d.plo, n * DRIL_ENV_MAX_PARAMS));
+        DRIL_TRY(dmalloc(&d.phi, n * DRIL_ENV_MAX_PARAMS));
+    }
+    DRIL_CUDA(cudaMemcpyAsync(d.plo, lo, n * np * 4, cudaMemcpyHostToDevice, c->stream));
+    DRIL_CUDA(cudaMemcpyAsync(d.phi, hi, n * np * 4, cudaMemcpyHostToDevice, c->stream));
+    d.has_params = 1;
+    {
+        Span sp(c, DRIL_K_ENV);
+        env_params_draw_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(d);
+        DRIL_CUDA(cudaGetLastError());
+    }
+    DRIL_CUDA(cudaStreamSynchronize(c->stream));
+    return DRIL_OK;
+}
+extern "C" int32_t dril_env_get_params(dril_env* e, int32_t n_params, float* values) {
+    DRIL_REQUIRE(e && values, "NULL argument");
+    const EnvDev& d = e->d;
+    const int np = env_n_params(d.kind);
+    DRIL_REQUIRE(n_params == np, "env kind %d has %d parameters, got %d", d.kind, np, n_params);
+    const size_t n = (size_t)d.n_envs;
+    if (!d.has_params) {
+        for (int k = 0; k < np; ++k) std::fill(values + (size_t)k * n, values + (size_t)(k + 1) * n, k_env_param_default[d.kind][k]);
+        return DRIL_OK;
+    }
+    dril_ctx* c = e->ctx;
+    DRIL_CUDA(cudaSetDevice(c->device));
+    DRIL_CUDA(cudaMemcpyAsync(values, d.pval, n * np * 4, cudaMemcpyDeviceToHost, c->stream));
+    DRIL_CUDA(cudaStreamSynchronize(c->stream));
+    return DRIL_OK;
+}
+
 extern "C" int32_t dril_env_num_envs(dril_env* e, int64_t* n) {
     DRIL_REQUIRE(e && n, "NULL argument");
     *n = e->d.n_envs;
@@ -1134,7 +1223,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     if (upd) flags |= RO_GRID_SYNC;
     const long long N = d.n_envs;
     const bool general_only = (base_flags & RO_DETERMINISTIC) != 0 || b->is_view;   // evaluation / chunked collection
-    if (has_policy && !general_only && g_opt_tc_rollout && !d.normalize && d.kind == DRIL_ENV_CARTPOLE && d.obs_dim == 4 && T > 0 && tc_eligible(a.pd) &&
+    if (has_policy && !general_only && g_opt_tc_rollout && !d.normalize && !d.has_params && d.kind == DRIL_ENV_CARTPOLE && d.obs_dim == 4 && T > 0 && tc_eligible(a.pd) &&
         T == b->d.T) {
         // tensor-core path: actor-only step loop (64 envs per CTA) + one batched critic pass for values / bootstrap values
         DRIL_TRY(ensure_tcs(b));
@@ -1210,7 +1299,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.n_tiles = (int)((N + M4 - 1) / M4);
             Span sp(c, DRIL_K_ROLLOUT);
             void* args[] = {(void*)&a};
-            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, d.kind), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
+            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, d.kind, d.has_params), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
             return DRIL_OK;
         }
     }
@@ -1247,7 +1336,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.M4 = GTC_ENVS; a.flags = flags;
             a.n_tiles = (int)((N + GTC_ENVS - 1) / GTC_ENVS);
             int grid = a.n_tiles, body_i = (int)body;
-            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, d.kind, a.pd.act_n);
+            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, d.kind, a.pd.act_n, d.has_params);
             void* args[] = {(void*)&a, (void*)&gl, (void*)&body_i};
             {
                 Span sp(c, DRIL_K_ROLLOUT);
@@ -1309,14 +1398,14 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     Span sp(c, has_policy ? DRIL_K_ROLLOUT : DRIL_K_ENV);
     if (flags & RO_GRID_SYNC) {
         int per_sm = 0;
-        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, d.kind), threads, smem));
+        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, d.kind, d.has_params), threads, smem));
         DRIL_REQUIRE(per_sm >= 1, "rollout kernel does not fit on an SM");
         grid = std::min(grid, std::min(per_sm * c->sm_count, e->max_blocks));
         void* args[] = {(void*)&a};
-        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, d.kind), dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, d.kind, d.has_params), dim3(grid), dim3(threads), args, smem, c->stream));
     } else {
         void* args[] = {(void*)&a};
-        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, d.kind), dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, d.kind, d.has_params), dim3(grid), dim3(threads), args, smem, c->stream));
     }
     if (defer) return launch_critic();
     return DRIL_OK;

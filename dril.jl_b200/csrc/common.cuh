@@ -97,6 +97,11 @@ struct EnvDev {
     float* tobs;                // [n][obs_dim] raw terminal observations scratch
     float* old_obs;             // [n][obs_dim] raw obs of the last observe (compat path)
     float* old_rewards;         // [n]
+    // per-env physical parameters (env.cuh); null unless dril_env_set_params gave ranges
+    int has_params;
+    float* pval;                // [DRIL_ENV_MAX_PARAMS][n] values of the running episode
+    float* plo;                 // [DRIL_ENV_MAX_PARAMS][n] ranges
+    float* phi;
 };
 
 struct BufDev {
@@ -118,6 +123,7 @@ struct BufDev {
 #define DRIL_TAG_SYN_OBS 3u
 #define DRIL_TAG_SHUFFLE 4u
 #define DRIL_TAG_SYN_DYN 5u
+#define DRIL_TAG_ENV_PARAMS 6u
 
 __host__ __device__ __forceinline__ void philox4x32(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                      unsigned long long seed, uint32_t out[4]) {

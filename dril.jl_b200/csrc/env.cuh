@@ -191,22 +191,24 @@ __device__ __forceinline__ float acrobot_wrap(float x) {
     while (x < -PI) x = __fadd_rn(x, TWO_PI);
     return x;
 }
-// Acrobot-v1: idx 0 / 1 / 2 = torque -1 / 0 / +1 held over one RK4 step of dt = 0.2.  Returns reward 0 on termination, else -1.
-__device__ __forceinline__ float acrobot_step(float* st, int idx, bool* terminated) {
+// Acrobot-v1: idx 0 / 1 / 2 = torque -1 / 0 / +1 held over one RK4 step of dt = 0.2 of the dynamics dsdt(s, a, ds).  Returns
+// reward 0 on termination, else -1.
+template <class Dsdt>
+__device__ __forceinline__ float acrobot_rk4_step(float* st, int idx, const Dsdt& dsdt, bool* terminated) {
     const float DT = 0.2f, DT2 = 0.1f, DT6 = 0.0333333350718021393f;
     const float MAX_VEL_1 = 12.5663709640502930f, MAX_VEL_2 = 28.2743339538574219f;
     const float a = (float)(idx - 1);
     float k1[4], k2[4], k3[4], k4[4], y[4];
-    acrobot_dsdt(st, a, k1);
+    dsdt(st, a, k1);
 #pragma unroll
     for (int i = 0; i < 4; ++i) y[i] = __fadd_rn(st[i], __fmul_rn(DT2, k1[i]));
-    acrobot_dsdt(y, a, k2);
+    dsdt(y, a, k2);
 #pragma unroll
     for (int i = 0; i < 4; ++i) y[i] = __fadd_rn(st[i], __fmul_rn(DT2, k2[i]));
-    acrobot_dsdt(y, a, k3);
+    dsdt(y, a, k3);
 #pragma unroll
     for (int i = 0; i < 4; ++i) y[i] = __fadd_rn(st[i], __fmul_rn(DT, k3[i]));
-    acrobot_dsdt(y, a, k4);
+    dsdt(y, a, k4);
 #pragma unroll
     for (int i = 0; i < 4; ++i)
         y[i] = __fadd_rn(st[i], __fmul_rn(DT6, __fadd_rn(__fadd_rn(__fadd_rn(k1[i], __fmul_rn(2.0f, k2[i])), __fmul_rn(2.0f, k3[i])), k4[i])));
@@ -219,6 +221,159 @@ __device__ __forceinline__ float acrobot_step(float* st, int idx, bool* terminat
     sincos_rn(__fadd_rn(st[1], st[0]), &s, &c12);
     *terminated = __fsub_rn(-c1, c12) > 1.0f;
     return *terminated ? 0.0f : -1.0f;
+}
+__device__ __forceinline__ float acrobot_step(float* st, int idx, bool* terminated) {
+    return acrobot_rk4_step(st, idx, [](const float* s, float a, float* ds) { acrobot_dsdt(s, a, ds); }, terminated);
+}
+
+// ---------------------------------------------------------------------------------------
+// Per-env physical parameters (dril_b200.h has the table).  The kernels built for ENV_KS_PARAMS take every constant of the
+// table from `p` (the env's values for the running episode, in table order); the default instantiations keep the folded
+// constants above and their exact code.  Each derived coefficient below is one fixed fp32 sequence, restated in
+// oracle/env_params.py, that gives the folded constant bit for bit at the default values.
+// ---------------------------------------------------------------------------------------
+#define ENV_KS_PARAMS (1u << 16)
+__host__ __device__ constexpr bool env_has_params(unsigned ks) { return (ks & ENV_KS_PARAMS) != 0; }
+__host__ __device__ constexpr int env_n_params(int kind) {
+    return kind == DRIL_ENV_CARTPOLE || kind == DRIL_ENV_ACROBOT ? 6
+         : kind == DRIL_ENV_PENDULUM ? 4
+         : kind == DRIL_ENV_MOUNTAINCAR || kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS ? 2 : 0;
+}
+// the parametrised kind set whose instantiation serves env kind `kind` (the synthetic env has no parameters)
+__host__ __device__ constexpr unsigned env_param_kind_set(int kind) {
+    return (env_kind_set(kind) & ~(1u << DRIL_ENV_SYNTHETIC)) | ENV_KS_PARAMS;
+}
+
+// the values of env n's episode `episode`: lo + (hi - lo) * u, u from Philox (gid, episode, k / 4, DRIL_TAG_ENV_PARAMS) word
+// k % 4; written to par and env.pval
+__device__ __forceinline__ void env_draw_params(const EnvDev& env, long long n, uint32_t gid, uint32_t episode, float* par) {
+    const int np = env_n_params(env.kind);
+    const long long N = env.n_envs;
+    uint32_t x[4];
+#pragma unroll
+    for (int k = 0; k < DRIL_ENV_MAX_PARAMS; ++k) {
+        if (k < np) {
+            if ((k & 3) == 0) philox4x32(gid, episode, (uint32_t)(k >> 2), DRIL_TAG_ENV_PARAMS, env.seed, x);
+            const float lo = env.plo[(size_t)k * N + n], hi = env.phi[(size_t)k * N + n];
+            par[k] = __fadd_rn(lo, __fmul_rn(__fsub_rn(hi, lo), u01_f32(x[k & 3])));
+            env.pval[(size_t)k * N + n] = par[k];
+        }
+    }
+}
+__device__ __forceinline__ void env_load_params(const EnvDev& env, long long n, float* par) {
+    const int np = env_n_params(env.kind);
+#pragma unroll
+    for (int k = 0; k < DRIL_ENV_MAX_PARAMS; ++k) par[k] = k < np ? env.pval[(size_t)k * env.n_envs + n] : 0.f;
+}
+
+// CartPole: p = (gravity, masscart, masspole, length, force_mag, tau); total_mass = masspole + masscart,
+// polemass_length = masspole * length
+__device__ __forceinline__ float cartpole_step_p(float* st, int a01, const float* p, bool* terminated) {
+    const float gravity = p[0], masscart = p[1], masspole = p[2], length = p[3], force_mag = p[4], tau = p[5];
+    const float total_mass = __fadd_rn(masspole, masscart);
+    const float pml = __fmul_rn(masspole, length);
+    const float THETA_THR = 0.20943951023931953f, X_THR = 2.4f, FOUR_THIRDS = 1.3333333333333333f;
+    float sinth, costh;
+    sincos_rn(st[2], &sinth, &costh);
+    float x = st[0], x_dot = st[1], th = st[2], th_dot = st[3];
+    float force = (a01 == 1) ? force_mag : -force_mag;
+    float temp = __fdiv_rn(__fadd_rn(force, __fmul_rn(__fmul_rn(pml, __fmul_rn(th_dot, th_dot)), sinth)), total_mass);
+    float den = __fmul_rn(length, __fsub_rn(FOUR_THIRDS, __fdiv_rn(__fmul_rn(masspole, __fmul_rn(costh, costh)), total_mass)));
+    float thetaacc = __fdiv_rn(__fsub_rn(__fmul_rn(gravity, sinth), __fmul_rn(costh, temp)), den);
+    float xacc = __fsub_rn(temp, __fdiv_rn(__fmul_rn(__fmul_rn(pml, thetaacc), costh), total_mass));
+    float xn = __fadd_rn(x, __fmul_rn(tau, x_dot));
+    float xdn = __fadd_rn(x_dot, __fmul_rn(tau, xacc));
+    float thn = __fadd_rn(th, __fmul_rn(tau, th_dot));
+    float thdn = __fadd_rn(th_dot, __fmul_rn(tau, thetaacc));
+    st[0] = xn; st[1] = xdn; st[2] = thn; st[3] = thdn;
+    *terminated = (xn < -X_THR) || (xn > X_THR) || (thn < -THETA_THR) || (thn > THETA_THR);
+    return 1.0f;
+}
+
+// Pendulum: p = (g, m, l, dt); thdot += (3 g / (2 l) * sin th + 3 / (m l^2) * u) * dt with 3 g / (2 l) = (3 g) / (2 l) and
+// 3 / (m l^2) = 3 / (m (l l))  (15 and 3 at the defaults)
+__device__ __forceinline__ float pendulum_step_p(float* st, float u, const float* p) {
+    const float g = p[0], m = p[1], l = p[2], dt = p[3];
+    const float c_sin = __fdiv_rn(__fmul_rn(3.0f, g), __fmul_rn(2.0f, l));
+    const float c_u = __fdiv_rn(3.0f, __fmul_rn(m, __fmul_rn(l, l)));
+    const float MAX_SPEED = 8.0f, MAX_TORQUE = 2.0f;
+    const float PI = 3.14159274101257324f, TWO_PI = 6.28318548202514648f;
+    u = fminf(fmaxf(u, -MAX_TORQUE), MAX_TORQUE);
+    float th = st[0], thdot = st[1];
+    float xp = __fadd_rn(th, PI);
+    float an = __fsub_rn(__fsub_rn(xp, __fmul_rn(TWO_PI, floorf(__fdiv_rn(xp, TWO_PI)))), PI);
+    float cost = __fadd_rn(__fadd_rn(__fmul_rn(an, an), __fmul_rn(0.1f, __fmul_rn(thdot, thdot))),
+                           __fmul_rn(0.001f, __fmul_rn(u, u)));
+    float sinth, costh;
+    sincos_rn(th, &sinth, &costh);
+    float nthdot = __fadd_rn(thdot, __fmul_rn(__fadd_rn(__fmul_rn(c_sin, sinth), __fmul_rn(c_u, u)), dt));
+    nthdot = fminf(fmaxf(nthdot, -MAX_SPEED), MAX_SPEED);
+    float nth = __fadd_rn(th, __fmul_rn(nthdot, dt));
+    st[0] = nth; st[1] = nthdot;
+    return -cost;
+}
+
+// MountainCar: p = (force, gravity); MountainCarContinuous: p = (power, gravity)
+__device__ __forceinline__ float mountaincar_step_p(float* st, int idx, const float* p, bool* terminated) {
+    float s, c;
+    sincos_rn(__fmul_rn(3.0f, st[0]), &s, &c);
+    mountaincar_move(st, __fadd_rn(__fmul_rn((float)(idx - 1), p[0]), __fmul_rn(c, -p[1])), 0.5f, terminated);
+    return -1.0f;
+}
+__device__ __forceinline__ float mountaincar_continuous_step_p(float* st, float a, const float* p, bool* terminated) {
+    const float f = fminf(fmaxf(a, -1.0f), 1.0f);
+    float s, c;
+    sincos_rn(__fmul_rn(3.0f, st[0]), &s, &c);
+    mountaincar_move(st, __fsub_rn(__fmul_rn(f, p[0]), __fmul_rn(p[1], c)), 0.45f, terminated);
+    return __fsub_rn(*terminated ? 100.0f : 0.0f, __fmul_rn(__fmul_rn(a, a), 0.1f));
+}
+
+// Acrobot: p = (l1, m1, m2, lc1, lc2, I) with I1 = I2 = I (link_moi) and g = 9.8.  The book dynamics as
+//   d1 = ((m1 lc1^2 + m2 ((l1^2 + lc2^2) + (2 l1) lc2 c2)) + I) + I       d2 = m2 (lc2^2 + (l1 lc2) c2) + I
+//   phi2 = ((m2 lc2) g) cos(th1 + th2 - pi/2)
+//   phi1 = (((-h w2^2) s2 - ((2 h) (w2 w1)) s2) + ((m1 lc1 + m2 l1) g) cos(th1 - pi/2)) + phi2,   h = m2 (l1 lc2)
+//   al2 = (((a + (d2 / d1) phi1) - (h w1^2) s2) - phi2) / ((m2 lc2^2 + I) - d2^2 / d1)      al1 = -(d2 al2 + phi1) / d1
+// with every coefficient rounded once in the order written (at the defaults: 0.25, 1.25, 1, 0.25, 0.5, 0.5, 1, 4.9f, 14.7f,
+// 1.25 -- the folded constants of acrobot_dsdt, where the two products by 1 are exact)
+struct AcrobotCoef { float a1, p, k, m2, i, l2, q, h, h2, g_lc2, g_12, j; };
+__device__ __forceinline__ AcrobotCoef acrobot_coef(const float* p) {
+    const float l1 = p[0], m1 = p[1], m2 = p[2], lc1 = p[3], lc2 = p[4], moi = p[5];
+    AcrobotCoef c;
+    c.a1 = __fmul_rn(m1, __fmul_rn(lc1, lc1));
+    c.p = __fadd_rn(__fmul_rn(l1, l1), __fmul_rn(lc2, lc2));
+    c.k = __fmul_rn(__fmul_rn(2.0f, l1), lc2);
+    c.m2 = m2;
+    c.i = moi;
+    c.l2 = __fmul_rn(lc2, lc2);
+    c.q = __fmul_rn(l1, lc2);
+    c.h = __fmul_rn(m2, c.q);
+    c.h2 = __fmul_rn(2.0f, c.h);
+    c.g_lc2 = __fmul_rn(__fmul_rn(m2, lc2), 9.8f);
+    c.g_12 = __fmul_rn(__fadd_rn(__fmul_rn(m1, lc1), __fmul_rn(m2, l1)), 9.8f);
+    c.j = __fadd_rn(__fmul_rn(m2, c.l2), moi);
+    return c;
+}
+__device__ __forceinline__ void acrobot_dsdt_p(const float* s, float a, const AcrobotCoef& C, float* ds) {
+    const float HALF_PI = 1.57079637050628662f;
+    const float th1 = s[0], th2 = s[1], w1 = s[2], w2 = s[3];
+    float s2, c2, sp, cp2, cp1;
+    sincos_rn(th2, &s2, &c2);
+    const float d1 = __fadd_rn(__fadd_rn(__fadd_rn(C.a1, __fmul_rn(C.m2, __fadd_rn(C.p, __fmul_rn(C.k, c2)))), C.i), C.i);
+    const float d2 = __fadd_rn(__fmul_rn(C.m2, __fadd_rn(C.l2, __fmul_rn(C.q, c2))), C.i);
+    sincos_rn(__fsub_rn(__fadd_rn(th1, th2), HALF_PI), &sp, &cp2);
+    const float phi2 = __fmul_rn(C.g_lc2, cp2);
+    sincos_rn(__fsub_rn(th1, HALF_PI), &sp, &cp1);
+    const float phi1 = __fadd_rn(__fadd_rn(__fsub_rn(__fmul_rn(__fmul_rn(-C.h, __fmul_rn(w2, w2)), s2),
+                                                     __fmul_rn(__fmul_rn(C.h2, __fmul_rn(w2, w1)), s2)),
+                                           __fmul_rn(C.g_12, cp1)), phi2);
+    const float num = __fsub_rn(__fsub_rn(__fadd_rn(a, __fmul_rn(__fdiv_rn(d2, d1), phi1)), __fmul_rn(__fmul_rn(C.h, __fmul_rn(w1, w1)), s2)), phi2);
+    const float al2 = __fdiv_rn(num, __fsub_rn(C.j, __fdiv_rn(__fmul_rn(d2, d2), d1)));
+    const float al1 = __fdiv_rn(-__fadd_rn(__fmul_rn(d2, al2), phi1), d1);
+    ds[0] = w1; ds[1] = w2; ds[2] = al1; ds[3] = al2;
+}
+__device__ __forceinline__ float acrobot_step_p(float* st, int idx, const float* p, bool* terminated) {
+    const AcrobotCoef C = acrobot_coef(p);
+    return acrobot_rk4_step(st, idx, [&C](const float* s, float a, float* ds) { acrobot_dsdt_p(s, a, C, ds); }, terminated);
 }
 
 // Synthetic env (SURVEY §8d C5): obs block b of lifetime step `life`
@@ -249,10 +404,18 @@ __device__ __forceinline__ bool env_is(int kind) { return env_in(KS, K) && (K ==
 
 // one step of env n: a_disc = env-space action of a Discrete env, a_cont = the Box env's action as the wrappers above it hand it
 // over (read only for Box envs), life = the synthetic env's lifetime step counter (read and advanced for that kind only).
-// Returns the reward; sets terminated.
+// par: the env's parameter values (read only by the ENV_KS_PARAMS instantiations).  Returns the reward; sets terminated.
 template <unsigned KS>
 __device__ __forceinline__ float env_step(const EnvDev& env, float* st, long long n, int a_disc, const float* a_cont, uint32_t* life,
-                                          bool* terminated) {
+                                          bool* terminated, const float* par = nullptr) {
+    if (env_has_params(KS)) {
+        if (env_is<KS, DRIL_ENV_CARTPOLE>(env.kind)) return cartpole_step_p(st, a_disc - env.act_start, par, terminated);
+        if (env_is<KS, DRIL_ENV_PENDULUM>(env.kind)) return pendulum_step_p(st, env_unscale_action(env, *a_cont), par);
+        if (env_is<KS, DRIL_ENV_MOUNTAINCAR>(env.kind)) return mountaincar_step_p(st, a_disc - env.act_start, par, terminated);
+        if (env_is<KS, DRIL_ENV_MOUNTAINCAR_CONTINUOUS>(env.kind))
+            return mountaincar_continuous_step_p(st, env_unscale_action(env, *a_cont), par, terminated);
+        return acrobot_step_p(st, a_disc - env.act_start, par, terminated);
+    }
     if (env_is<KS, DRIL_ENV_CARTPOLE>(env.kind)) return cartpole_step(st, a_disc - env.act_start, terminated);
     if (env_is<KS, DRIL_ENV_PENDULUM>(env.kind)) return pendulum_step(st, env_unscale_action(env, *a_cont));
     if (env_is<KS, DRIL_ENV_MOUNTAINCAR>(env.kind)) return mountaincar_step(st, a_disc - env.act_start, terminated);

@@ -444,7 +444,9 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                 bool term = false;
                 float r;
                 uint32_t life = 0;
-                r = env_step<KS>(env, st, n, a_disc, sEnvAct + tid, &life, &term);
+                float par[DRIL_ENV_MAX_PARAMS];
+                if (env_has_params(KS)) env_load_params(env, n, par);
+                r = env_step<KS>(env, st, n, a_disc, sEnvAct + tid, &life, &term, par);
                 steps += 1;
                 const bool trunc = steps >= env.max_steps;
                 const bool done = term || trunc;
@@ -486,6 +488,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                 if (done) {                                     // reset!(env_i)
                     uint32_t ep = env.episode[n];
                     env_reset_state<KS>(env.kind, gid, ep, env.seed, st);
+                    if (env_has_params(KS)) env_draw_params(env, n, gid, ep, par);
                     env.episode[n] = ep + 1;
                     steps = 0;
                 }
@@ -671,11 +674,13 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
     int steps = 0, ep_len = 0;
     float ep_ret = 0.f;
     uint32_t episode = 0;
+    float eparam[DRIL_ENV_MAX_PARAMS] = {};   // parameter values of the running episode (ENV_KS_PARAMS)
     if (mine) {
 #pragma unroll
         for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * N + n];
         steps = env.steps[n];
         episode = env.episode[n];
+        if (env_has_params(KS)) env_load_params(env, n, eparam);
         if (env.monitor) { ep_ret = env.ep_ret[n]; ep_len = env.ep_len[n]; }
     }
     // output-layer split: thread (e = tid % M4, ks = tid / M4) covers k in [ks*Kc, ks*Kc + Kc)
@@ -842,7 +847,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             bool term = false;
             float r;
             uint32_t life = 0;
-            r = env_step<KS & ~(1u << DRIL_ENV_SYNTHETIC)>(env, st, n, a_disc, &a_cont, &life, &term);   // (no synthetic env here)
+            r = env_step<KS & ~(1u << DRIL_ENV_SYNTHETIC)>(env, st, n, a_disc, &a_cont, &life, &term, eparam);   // (no synthetic env here)
             steps += 1;
             const bool trunc = steps >= env.max_steps;
             const bool done = term || trunc;
@@ -877,6 +882,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             }
             if (done) {
                 env_reset_state<KS>(env.kind, gid, episode, env.seed, st);
+                if (env_has_params(KS)) env_draw_params(env, n, gid, episode, eparam);
                 episode += 1;
                 steps = 0;
                 if (env.normalize) env.ret[n] = 0.f;             // normalizeWrapperEnv.jl:153-156
@@ -1003,17 +1009,31 @@ __global__ void __launch_bounds__(DRIL_THREADS) policy_apply_kernel(const __grid
     }
 }
 
-// env reset (reset!(env)): new episode for every env, monitor/normaliser accumulators zeroed.
+// env reset (reset!(env)): new episode for every env, monitor/normaliser accumulators zeroed (and, for KS with ENV_KS_PARAMS,
+// the new episode's parameter values drawn).
+template <unsigned KS>
 __global__ void env_reset_kernel(EnvDev env) {
     long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= env.n_envs) return;
     float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
     uint32_t ep = env.episode[n];
     env_reset_state<ENV_KS_ALL>(env.kind, (uint32_t)(env.gid_offset + n), ep, env.seed, st);
+    if (env_has_params(KS)) {
+        float par[DRIL_ENV_MAX_PARAMS];
+        env_draw_params(env, n, (uint32_t)(env.gid_offset + n), ep, par);
+    }
     env.episode[n] = ep + 1;
 #pragma unroll
     for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) env.state[(size_t)k * env.n_envs + n] = st[k];
     env.steps[n] = 0;
     if (env.monitor) { env.ep_ret[n] = 0.f; env.ep_len[n] = 0; }
     if (env.normalize) env.ret[n] = 0.f;
+}
+
+// new ranges (dril_env_set_params): the running episode takes the values its own (gid, episode) draws from them
+__global__ void env_params_draw_kernel(EnvDev env) {
+    long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= env.n_envs) return;
+    float par[DRIL_ENV_MAX_PARAMS];
+    env_draw_params(env, n, (uint32_t)(env.gid_offset + n), env.episode[n] - 1u, par);
 }

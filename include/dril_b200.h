@@ -222,6 +222,27 @@ int32_t dril_env_zero_returns(dril_env* env);
 int32_t dril_env_monitor_stats(dril_env* env, float* ep_rew_mean, float* ep_len_mean,
                                int64_t* n_in_window, int64_t* total_episodes);
 
+/* Per-env physical parameters, in this order (names are Gymnasium's attributes; the defaults are the built-in constants):
+ *   cartpole                6: gravity 9.8, masscart 1.0, masspole 0.1, length 0.5, force_mag 10.0, tau 0.02
+ *   pendulum                4: g 10.0, m 1.0, l 1.0, dt 0.05
+ *   mountaincar             2: force 0.001, gravity 0.0025
+ *   mountaincar_continuous  2: power 0.0015, gravity 0.0025
+ *   acrobot                 6: link_length_1 1, link_mass_1 1, link_mass_2 1, link_com_pos_1 0.5, link_com_pos_2 0.5, link_moi 1
+ *   synthetic               0:
+ * Env n holds a range [lo[k][n], hi[k][n]] per parameter.  During env n's episode e (the reset counter of the RESET stream) the
+ * value of parameter k is lo + (hi - lo) * u, three fp32 roundings, u = u01_f32 of Philox block (gid, e, k / 4, tag 6) word
+ * k % 4: a pure function of the seed, the global env id, e and the range, so lo == hi is a fixed value and draws do not depend
+ * on sharding.  Every reset draws anew (auto-reset, act!, reset!).
+ * dril_env_set_params: lo, hi float[n_params][n_envs], n_params = the kind's count; hi == NULL: hi = lo (fixed values);
+ * lo == NULL: back to the built-in constants.  Values must be finite with lo <= hi; masses, lengths, link_moi, tau and dt > 0;
+ * gravity, g, force, force_mag and power >= 0 (else DRIL_ERR_INVALID).  The running episode takes the value its own (gid, e)
+ * draws from the new ranges.  Thresholds, speed clips, max_torque and the spaces stay fixed.  Envs with parameters do not use
+ * the CartPole tensor-core rollout.
+ * dril_env_get_params: the current per-env values, float[n_params][n_envs] (the defaults for an env without parameters). */
+#define DRIL_ENV_MAX_PARAMS 8
+int32_t dril_env_set_params(dril_env* env, int32_t n_params, const float* lo, const float* hi);
+int32_t dril_env_get_params(dril_env* env, int32_t n_params, float* values);
+
 /* ---- actor-critic layer + optimiser state: replaces Discrete/ContinuousActorCriticLayer
  *      (layers/) and the Lux TrainState held by Agent (agents/agent_types.jl) ------------ */
 int32_t dril_policy_create(dril_ctx* ctx, int32_t obs_dim, int32_t n_hidden, const int32_t* hidden_dims,

@@ -68,12 +68,22 @@ default_ctx() = (isnothing(DEFAULT_CTX[]) && (DEFAULT_CTX[] = Context()); DEFAUL
 
 # ---- batched env -------------------------------------------------------------------------------
 const ENV_KINDS = Dict(:cartpole => 0, :pendulum => 1, :synthetic => 2, :mountaincar => 3, :mountaincar_continuous => 4, :acrobot => 5)
+# per-env physical parameters (dril_b200.h): name => default, in the order of the C arrays
+const ENV_PARAMS = Dict(
+    :cartpole => (:gravity => 9.8, :masscart => 1.0, :masspole => 0.1, :length => 0.5, :force_mag => 10.0, :tau => 0.02),
+    :pendulum => (:g => 10.0, :m => 1.0, :l => 1.0, :dt => 0.05),
+    :synthetic => (),
+    :mountaincar => (:force => 0.001, :gravity => 0.0025),
+    :mountaincar_continuous => (:power => 0.0015, :gravity => 0.0025),
+    :acrobot => (:link_length_1 => 1.0, :link_mass_1 => 1.0, :link_mass_2 => 1.0, :link_com_pos_1 => 0.5, :link_com_pos_2 => 0.5, :link_moi => 1.0),
+)
 
 """
-    CudaBatchedEnv(kind, n_envs; max_steps, act_start, monitor_window, normalize)
+    CudaBatchedEnv(kind, n_envs; max_steps, act_start, monitor_window, normalize, env_params)
 
 Device-resident replacement of `NormalizeWrapperEnv(MonitorWrapperEnv(MultiThreadedParallelEnv(envs)))`
 for `kind in (:cartpole, :pendulum, :synthetic, :mountaincar, :mountaincar_continuous, :acrobot)`.
+`env_params = Dict(:length => (0.25, 1.0), ...)`: per-env physical parameters, see `set_env_params!`.
 """
 mutable struct CudaBatchedEnv <: AbstractParallelEnv
     ctx::Context
@@ -89,7 +99,8 @@ mutable struct CudaBatchedEnv <: AbstractParallelEnv
 end
 
 function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_steps = 0, obs_dim = 0, act_start = 1,
-        monitor_window = 0, normalize::Union{Nothing, NormCfg} = nothing, gid_offset = 0, scaling::Bool = false)
+        monitor_window = 0, normalize::Union{Nothing, NormCfg} = nothing, gid_offset = 0, scaling::Bool = false,
+        env_params = nothing)
     obs_space, act_space = if kind == :cartpole
         hi = Float32[4.8, Inf32, 0.41887903, Inf32]
         Box(-hi, hi), Discrete(2, act_start)
@@ -123,6 +134,51 @@ function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_
     env = CudaBatchedEnv(ctx, out[], kind, n_envs, obs_space, act_space, monitor_window, normalize,
         falses(n_envs), falses(n_envs))
     finalizer(e -> ccall((:dril_env_destroy, LIB), Int32, (Ptr{Cvoid},), e.h), env)
+    isnothing(env_params) || isempty(env_params) || set_env_params!(env; env_params...)
+    env
+end
+
+"""
+    set_env_params!(env; length = (0.25, 1.0), masspole = 0.2, ...)
+
+Per-env physical parameters (names and defaults: `ENV_PARAMS[kind]`).  Each value is a number, a vector of `n_envs`, or a
+tuple `(lo, hi)` of either: every reset draws a value per env from `[lo, hi]`.  Unnamed parameters keep their defaults; with
+no keyword the env returns to the built-in constants.
+"""
+function set_env_params!(env::CudaBatchedEnv; kw...)
+    spec = ENV_PARAMS[env.kind]
+    names = Symbol[first(p) for p in spec]
+    for k in keys(kw)
+        k in names || error("$(env.kind) has no parameter $k; it has $names")
+    end
+    if isempty(kw)
+        isempty(names) || check(ccall((:dril_env_set_params, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{Float32}, Ptr{Float32}),
+            env.h, length(names), C_NULL, C_NULL))
+        return env
+    end
+    n = env.n_envs
+    lo = Matrix{Float32}(undef, n, length(names))   # column k = parameter k: the C layout [n_params][n_envs]
+    hi = similar(lo)
+    for (k, (name, default)) in enumerate(spec)
+        v = get(kw, name, default)
+        a, b = v isa Tuple ? v : (v, v)
+        lo[:, k] .= Float32.(a)
+        hi[:, k] .= Float32.(b)
+    end
+    check(ccall((:dril_env_set_params, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{Float32}, Ptr{Float32}), env.h, length(names), lo, hi))
+    env
+end
+
+"""
+    env_params(env) -> Dict(name => Vector{Float32}(n_envs))
+
+Each env's parameter values for its running episode.
+"""
+function env_params(env::CudaBatchedEnv)
+    spec = ENV_PARAMS[env.kind]
+    v = Matrix{Float32}(undef, env.n_envs, length(spec))
+    isempty(spec) || check(ccall((:dril_env_get_params, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{Float32}), env.h, length(spec), v))
+    Dict(first(p) => v[:, k] for (k, p) in enumerate(spec))
 end
 
 DRiL.number_of_envs(env::CudaBatchedEnv) = env.n_envs

@@ -1,6 +1,10 @@
-"""PPO throughput on MountainCar, MountainCarContinuous and Acrobot: one JSON line per env and env count.
+"""PPO throughput per classic-control env: one JSON line per env, env count and (with --randomize) parameter setting.
 
-    python tools/bench_envs.py [--envs mountaincar,mountaincar_continuous,acrobot] [--n-envs 4096,65536] [--steps 20] [--normalize]
+    python tools/bench_envs.py [--envs cartpole,pendulum,mountaincar,mountaincar_continuous,acrobot] [--n-envs 4096,65536]
+                               [--steps 20] [--normalize] [--randomize] [--repeats 1]
+
+--randomize runs every configuration twice, alternating: with the built-in constants and with per-env parameters drawn at every
+reset from +-50 % of each default (set_env_params), --repeats times.
 
 Each run: [64, 64] policy, n_steps 128, 4 epochs x 4 minibatches; warm-up iterations, then --steps iterations timed with CUDA events
 on the library's stream, L2 overwritten before every iteration (as bench.py does), then the same iterations again with the
@@ -30,18 +34,22 @@ def card():
         return f"unknown ({e})", "unknown"
 
 
-def rollout_kernel(n, sms, normalize, act_n):
-    """launch_rollout's choice (csrc/api.cu) for a [64, 64] policy: without a training normaliser the fast kernel; with one the
-    cooperative general kernel, its actor on tcgen05 (rollout_gtc.cuh) from 64 envs per SM on"""
+def rollout_kernel(kind, n, sms, normalize, act_n, randomize):
+    """launch_rollout's choice (csrc/api.cu) for a [64, 64] policy: CartPole without normaliser or per-env parameters the
+    tensor-core rollout; otherwise without a training normaliser the fast kernel; with one the cooperative general kernel, its
+    actor on tcgen05 (rollout_gtc.cuh) from 64 envs per SM on"""
     if not normalize:
-        return "fast"
+        return "tc" if kind == "cartpole" and not randomize else "fast"
     return "gtc" if n >= 64 * sms else "general"
 
 
-def run(D, kind, n, steps, warmup, normalize):
+def run(D, kind, n, steps, warmup, normalize, randomize):
     from dril_b200 import _lib as L
+    from dril_b200.core import ENV_PARAMS
     T = 128
-    env = D.CudaBatchedEnv(kind, n, seed=0, monitor_window=100, normalize=D.NormalizeConfig() if normalize else None)
+    params = {nm: (0.5 * d, 1.5 * d) for nm, d in ENV_PARAMS[kind]} if randomize else None
+    env = D.CudaBatchedEnv(kind, n, seed=0, monitor_window=100, normalize=D.NormalizeConfig() if normalize else None,
+                           env_params=params)
     layer = D.ActorCriticLayer(env.observation_space(), env.action_space(), hidden_dims=[64, 64])
     alg = D.PPO(n_steps=T, batch_size=T * n // 4, epochs=4)
     agent = D.Agent(layer, alg, rng=np.random.default_rng(0))
@@ -77,10 +85,11 @@ def run(D, kind, n, steps, warmup, normalize):
     sms = ctx.sm_count()
     act = env.action_space()
     res = dict(env=kind, n_envs=n, n_steps=T, hidden=[64, 64], epochs=4, minibatches=4, normalize=bool(normalize),
+               randomize=bool(randomize),
                env_steps_per_s=n * T / (ms * 1e-3), ms_per_iter=ms,
                rollout_ms=prof.get("rollout", (0.0, 0))[0] / steps, update_ms=upd,
                update_path=agent.device.update_path(),
-               rollout_kernel=rollout_kernel(n, sms, normalize, getattr(act, "n", 1)),
+               rollout_kernel=rollout_kernel(kind, n, sms, normalize, getattr(act, "n", 1), randomize),
                ep_rew_mean=env.monitor_stats()["ep_rew_mean"], timed_iters=steps, warmup_iters=warmup)
     buf.close()
     env.close()
@@ -94,6 +103,8 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--normalize", action="store_true")
+    ap.add_argument("--randomize", action="store_true", help="alternate built-in constants and +-50 %% per-env parameters")
+    ap.add_argument("--repeats", type=int, default=1)
     args = ap.parse_args()
     import __graft_entry__
     __graft_entry__.build()
@@ -101,9 +112,11 @@ def main():
     name, power = card()
     for kind in args.envs.split(","):
         for n in (int(x) for x in args.n_envs.split(",")):
-            r = run(D, kind, n, args.steps, args.warmup, args.normalize)
-            r.update(card=name, power_limit=power)
-            print(json.dumps(r), flush=True)
+            for _ in range(args.repeats):
+                for randomize in ((False, True) if args.randomize else (False,)):
+                    r = run(D, kind, n, args.steps, args.warmup, args.normalize, randomize)
+                    r.update(card=name, power_limit=power)
+                    print(json.dumps(r), flush=True)
 
 
 if __name__ == "__main__":
