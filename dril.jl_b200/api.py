@@ -26,7 +26,8 @@ def _rewrap(env, **over):
     args = dict(kind=env.kind, n_envs=env.n_envs, max_steps=env.max_steps, obs_dim=env.obs_dim,
                 act_start=env.act_start, ctx=env.ctx, monitor_window=env.monitor_window,
                 normalize=env.normalize, gid_offset=env.gid_offset, scaling=env.scaling,
-                obs_shape=env.obs_shape if len(env.obs_shape) > 1 else None, env_params=env.env_param_ranges())
+                obs_shape=env.obs_shape if len(env.obs_shape) > 1 else None, env_params=env.env_param_ranges(),
+                observe_params=env.observes_params())
     args.update(over)
     kind, n = args.pop("kind"), args.pop("n_envs")
     st, steps = env.get_state()

@@ -23,6 +23,15 @@ ENV_PARAMS = {
 }
 
 
+def observation_space_with_params(space, kind):
+    """The observation space of an env with observe_params=True: the base space's bounds (scaled or not), then [0, inf) per
+    parameter -- the components are raw values, validated >= 0, so the space does not change when the ranges do."""
+    P = len(ENV_PARAMS[kind])
+    low = np.concatenate([np.asarray(space.low, np.float32).ravel(), np.zeros(P, np.float32)])
+    high = np.concatenate([np.asarray(space.high, np.float32).ravel(), np.full(P, np.inf, np.float32)])
+    return Box(low, high)
+
+
 class Context:
     """One CUDA device + stream; not thread-safe (one per GPU)."""
     _default = {}
@@ -127,7 +136,8 @@ class CudaBatchedEnv:
     path used by evaluate_agent and callbacks; training uses the fused device rollout."""
 
     def __init__(self, kind, n_envs, max_steps=0, obs_dim=0, act_start=1, seed=None, ctx=None,
-                 monitor_window=0, normalize=None, gid_offset=0, obs_shape=None, scaling=False, env_params=None):
+                 monitor_window=0, normalize=None, gid_offset=0, obs_shape=None, scaling=False, env_params=None,
+                 observe_params=False):
         self.kind = kind.lower()
         assert self.kind in ENV_KINDS, f"unknown env kind {kind}"
         self.ctx = ctx or Context.default()
@@ -170,6 +180,10 @@ class CudaBatchedEnv:
                                     self.act_start, self.gid_offset, C.byref(cfg) if cfg is not None else None,
                                     self.monitor_window, C.byref(h)))
         self.h = h
+        self._observe_params = bool(observe_params)
+        if self._observe_params:
+            # [base observation | the running episode's parameter values]: set before the first observation
+            L.check(lib.dril_env_set_observe_params(self.h, 1))
         self.scaling = bool(scaling)
         if self.scaling:
             # ScalingWrapperEnv around every env (scalingWrapperEnv.jl:14-49): spaces become [-1, 1] boxes, the originals are kept
@@ -180,6 +194,13 @@ class CudaBatchedEnv:
             L.check(lib.dril_env_set_scaling(self.h, 1, L.ptr(ol), L.ptr(oh), L.ptr(al), L.ptr(ah)))
             self._obs_space = Box(-np.ones_like(ol).reshape(self._obs_space.low.shape), np.ones_like(oh).reshape(self._obs_space.low.shape))
             self._act_space = Box(-np.ones_like(al), np.ones_like(ah))
+        if self._observe_params:
+            self._obs_space = observation_space_with_params(self._obs_space, self.kind)
+            self.obs_dim = int(self._obs_space.size()[0])
+            self.obs_shape = (self.obs_dim,)
+            d = L.c_i32(0)
+            L.check(lib.dril_env_obs_dim(self.h, C.byref(d)))
+            assert d.value == self.obs_dim, (d.value, self.obs_dim)
         self._term = np.zeros(self.n_envs, dtype=bool)
         self._trunc = np.zeros(self.n_envs, dtype=bool)
         self._param_ranges = None
@@ -264,11 +285,15 @@ class CudaBatchedEnv:
         L.check(self.ctx.lib.dril_env_set_state(self.h, L.ptr(st), L.ptr(sp)))
 
     # ---- per-env physical parameters ----
+    def observes_params(self):
+        """True if every observation ends in the running episode's parameter values (observe_params=True)."""
+        return self._observe_params
+
     def set_env_params(self, **kw):
         """Per-env parameter ranges, e.g. set_env_params(length=(0.25, 1.0), masspole=0.2).  Each value is a scalar, an
         (n_envs,) array, or a tuple (lo, hi) of either; every reset draws a value per env from [lo, hi] (a scalar or array is
         a fixed value).  Unnamed parameters keep their defaults (ENV_PARAMS).  With no keyword the env returns to the
-        built-in constants."""
+        built-in constants (which an env with observe_params=True keeps observing)."""
         names = [nm for nm, _ in ENV_PARAMS[self.kind]]
         unknown = set(kw) - set(names)
         assert not unknown, f"{self.kind} has no parameter(s) {sorted(unknown)}; it has {names}"

@@ -100,31 +100,36 @@ static bool tc_eligible(const PolicyDesc& pd) {
 
 // rollout kernels by the env kind they step: CartPole, Pendulum and the synthetic env run the instantiations built for those
 // kinds alone (env.cuh), every other kind the one built for all kinds; an env with per-env parameters (dril_env_set_params)
-// runs the ENV_KS_PARAMS instantiation of its kind set
+// runs the ENV_KS_PARAMS instantiation of its kind set, and one that observes its parameters (dril_env_set_observe_params) the
+// ENV_KS_OBS_PARAMS instantiation
 #define KS_CP_ ENV_KS_CLASSIC
 #define KS_ALL_ ENV_KS_ALL
 #define KS_CP_P_ env_param_kind_set(DRIL_ENV_CARTPOLE)
 #define KS_ALL_P_ env_param_kind_set(DRIL_ENV_ACROBOT)
-#define DRIL_KS_PICK(K_, kind, params) \
-    (env_kind_set(kind) == ENV_KS_CLASSIC ? ((params) ? K_(KS_CP_P_) : K_(KS_CP_)) : ((params) ? K_(KS_ALL_P_) : K_(KS_ALL_)))
-static void* rollout_fn(bool ws, int kind, bool params) {
+#define KS_CP_OP_ env_obs_param_kind_set(DRIL_ENV_CARTPOLE)
+#define KS_ALL_OP_ env_obs_param_kind_set(DRIL_ENV_ACROBOT)
+#define DRIL_KS_PICK(K_, kind, params, obsp)                                                               \
+    (env_kind_set(kind) == ENV_KS_CLASSIC ? ((obsp) ? K_(KS_CP_OP_) : (params) ? K_(KS_CP_P_) : K_(KS_CP_)) \
+                                          : ((obsp) ? K_(KS_ALL_OP_) : (params) ? K_(KS_ALL_P_) : K_(KS_ALL_)))
+static void* rollout_fn(bool ws, int kind, bool params, bool obsp) {
 #define K_(ks) (ws ? (void*)rollout_kernel<true, ks> : (void*)rollout_kernel<false, ks>)
-    return DRIL_KS_PICK(K_, kind, params);
+    return DRIL_KS_PICK(K_, kind, params, obsp);
 #undef K_
 }
-static void* rollout_fast_fn(bool ws, int kind, bool params) {
+static void* rollout_fast_fn(bool ws, int kind, bool params, bool obsp) {
 #define K_(ks) (ws ? (void*)rollout_fast_kernel<true, ks> : (void*)rollout_fast_kernel<false, ks>)
-    return DRIL_KS_PICK(K_, kind, params);
+    return DRIL_KS_PICK(K_, kind, params, obsp);
 #undef K_
 }
 // tcgen05-actor rollout by hidden-layer count, env kind and action count (2 or 4 staged output columns, gtc_nout)
-static void* rollout_gtc_fn(int L, int kind, int act_n, bool params) {
+static void* rollout_gtc_fn(int L, int kind, int act_n, bool params, bool obsp) {
     if (act_n > 2) {
+        if (obsp) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_OP_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_OP_, 4>;
         if (params) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_P_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_P_, 4>;
         return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_ALL, 4> : (void*)rollout_gtc_kernel<3, ENV_KS_ALL, 4>;
     }
 #define K_(ks) (L == 2 ? (void*)rollout_gtc_kernel<2, ks, 2> : (void*)rollout_gtc_kernel<3, ks, 2>)
-    return DRIL_KS_PICK(K_, kind, params);
+    return DRIL_KS_PICK(K_, kind, params, obsp);
 #undef K_
 }
 
@@ -241,6 +246,9 @@ struct dril_env {
     double* xr = nullptr;
     float* norm_snap = nullptr;
     long long* norm_snap_cnt = nullptr;
+    bool observe_params = false;     // dril_env_set_observe_params: the ENV_KS_OBS_PARAMS instantiations, obs_dim = D + P
+    bool default_params = false;     // parameters held at lo = hi = the defaults only because observe_params is on
+    bool observed = false;           // an observation was made (observe, step, rollout, evaluate): the width is fixed
 };
 
 struct dril_policy {
@@ -368,9 +376,9 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
     DRIL_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
         for (int ws = 0; ws < 2; ++ws)
-            for (int params = 0; params < 2; ++params) {
-                DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, kind, params), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-                DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, kind, params), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+            for (int params = 0; params < 3; ++params) {   // 2: observed parameters
+                DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, kind, params > 0, params == 2), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+                DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, kind, params > 0, params == 2), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
             }
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
@@ -390,8 +398,8 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
         for (int L = 2; L <= 3; ++L)
             for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
                 for (int an = 2; an <= 4; an += 2)
-                    for (int params = 0; params < 2; ++params)
-                        DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, kind, an, params), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
+                    for (int params = 0; params < 3; ++params)
+                        DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, kind, an, params > 0, params == 2), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
     }
@@ -991,6 +999,7 @@ extern "C" int32_t dril_policy_predict_values(dril_policy* p, const float* obs, 
 // ---------------------------------------------------------------------------------------
 // env
 // ---------------------------------------------------------------------------------------
+static int32_t env_alloc_obs_arrays(dril_env* e);
 extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, int32_t max_steps, int32_t obs_dim,
                                    int32_t act_start, int64_t gid_offset, const dril_norm_cfg* norm,
                                    int32_t monitor_window, dril_env** out) {
@@ -1016,10 +1025,9 @@ extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, in
     size_t n = (size_t)n_envs;
     DRIL_TRY(dmalloc(&d.state, n * std::max(d.state_dim, 1))); DRIL_TRY(dmalloc(&d.steps, n));
     DRIL_TRY(dmalloc(&d.episode, n)); DRIL_TRY(dmalloc(&d.life, n));
-    DRIL_TRY(dmalloc(&d.tobs, n * d.obs_dim)); DRIL_TRY(dmalloc(&d.old_obs, n * d.obs_dim)); DRIL_TRY(dmalloc(&d.old_rewards, n));
+    DRIL_TRY(dmalloc(&d.old_rewards, n));
     DRIL_CUDA(cudaMemset(d.state, 0, n * std::max(d.state_dim, 1) * 4)); DRIL_CUDA(cudaMemset(d.steps, 0, n * 4));
     DRIL_CUDA(cudaMemset(d.episode, 0, n * 4)); DRIL_CUDA(cudaMemset(d.life, 0, n * 4));
-    DRIL_CUDA(cudaMemset(d.tobs, 0, n * d.obs_dim * 4)); DRIL_CUDA(cudaMemset(d.old_obs, 0, n * d.obs_dim * 4));
     DRIL_CUDA(cudaMemset(d.old_rewards, 0, n * 4));
     d.monitor = monitor_window > 0 ? monitor_window : 0;
     DRIL_TRY(dmalloc(&d.ep_ret, n)); DRIL_TRY(dmalloc(&d.ep_len, n)); DRIL_TRY(dmalloc(&d.roll_sums, 2)); DRIL_TRY(dmalloc(&d.roll_eps, 1));
@@ -1035,28 +1043,46 @@ extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, in
         d.clip_obs = norm->clip_obs; d.clip_reward = norm->clip_reward; d.ngamma = norm->gamma; d.eps = norm->epsilon;
     }
     e->max_blocks = c->sm_count * 8;
-    DRIL_TRY(dmalloc(&d.ret, n)); DRIL_TRY(dmalloc(&d.obs_mean, (size_t)d.obs_dim)); DRIL_TRY(dmalloc(&d.obs_var, (size_t)d.obs_dim));
+    DRIL_TRY(dmalloc(&d.ret, n));
     DRIL_TRY(dmalloc(&d.ret_stats, 2)); DRIL_TRY(dmalloc(&d.counts, 2));
-    DRIL_TRY(dmalloc(&d.partials, (size_t)2 * e->max_blocks * (2 * d.obs_dim + 2)));
-    DRIL_TRY(dmalloc(&e->roll_moments, (size_t)2 * (d.obs_dim + 1) + 2));     // handed to the kernels only in data-parallel runs
-    DRIL_TRY(dmalloc(&e->xr, (size_t)4 + 3 + 2 * (d.obs_dim + 1) + 2));
-    DRIL_TRY(dmalloc(&e->norm_snap, (size_t)2 * d.obs_dim + 2)); DRIL_TRY(dmalloc(&e->norm_snap_cnt, 2));
+    DRIL_TRY(dmalloc(&e->norm_snap_cnt, 2));
     d.roll_moments = nullptr;
     DRIL_CUDA(cudaMemset(d.ret, 0, n * 4));
-    {   // RunningMeanStd init: mean 0, var 1, count 0 (normalizeWrapperEnv.jl:13-15)
-        std::vector<float> ones((size_t)d.obs_dim, 1.0f);
+    {   // RunningMeanStd init: mean 0, var 1, count 0 (normalizeWrapperEnv.jl:13-15); the obs columns in env_alloc_obs_arrays
         float rs[2] = {0.f, 1.f};
-        DRIL_CUDA(cudaMemset(d.obs_mean, 0, d.obs_dim * 4));
-        DRIL_CUDA(cudaMemcpy(d.obs_var, ones.data(), d.obs_dim * 4, cudaMemcpyHostToDevice));
         DRIL_CUDA(cudaMemcpy(d.ret_stats, rs, 8, cudaMemcpyHostToDevice));
         DRIL_CUDA(cudaMemset(d.counts, 0, 16));
     }
-    DRIL_TRY(dril_buffer_create(c, 1, n_envs, d.obs_dim, d.act_dim == 0 ? DRIL_ACT_DISCRETE : DRIL_ACT_CONTINUOUS,
-                                std::max(d.act_dim, 1), &e->compat));
     DRIL_CUDA(cudaMalloc(&e->compat_actions, n * std::max(d.act_dim, 1) * 4));
-    DRIL_TRY(dmalloc(&e->compat_obs, n * d.obs_dim));
+    DRIL_TRY(env_alloc_obs_arrays(e));
     *out = e;
     DRIL_TRY(dril_env_reset(e));
+    return DRIL_OK;
+}
+// the arrays sized by obs_dim, (re)allocated for the env's current width: terminal and old observations, the normaliser's
+// obs mean / var (mean 0, var 1), its per-CTA partials, the data-parallel moments and exchange buffers, the compat buffer
+static int32_t env_alloc_obs_arrays(dril_env* e) {
+    dril_ctx* c = e->ctx;
+    EnvDev& d = e->d;
+    const size_t n = (size_t)d.n_envs, D = (size_t)d.obs_dim;
+    for (float** p : {&d.tobs, &d.old_obs, &d.obs_mean, &d.obs_var, &e->norm_snap, &e->compat_obs}) { if (*p) cudaFree(*p); *p = nullptr; }
+    for (double** p : {&d.partials, &e->roll_moments, &e->xr}) { if (*p) cudaFree(*p); *p = nullptr; }
+    if (e->compat) { dril_buffer_destroy(e->compat); e->compat = nullptr; }
+    DRIL_TRY(dmalloc(&d.tobs, n * D)); DRIL_TRY(dmalloc(&d.old_obs, n * D));
+    DRIL_CUDA(cudaMemset(d.tobs, 0, n * D * 4)); DRIL_CUDA(cudaMemset(d.old_obs, 0, n * D * 4));
+    DRIL_TRY(dmalloc(&d.obs_mean, D)); DRIL_TRY(dmalloc(&d.obs_var, D));
+    DRIL_TRY(dmalloc(&d.partials, (size_t)2 * e->max_blocks * (2 * D + 2)));
+    DRIL_TRY(dmalloc(&e->roll_moments, (size_t)2 * (D + 1) + 2));     // handed to the kernels only in data-parallel runs
+    DRIL_TRY(dmalloc(&e->xr, (size_t)4 + 3 + 2 * (D + 1) + 2));
+    DRIL_TRY(dmalloc(&e->norm_snap, (size_t)2 * D + 2));
+    {
+        std::vector<float> ones(D, 1.0f);
+        DRIL_CUDA(cudaMemset(d.obs_mean, 0, D * 4));
+        DRIL_CUDA(cudaMemcpy(d.obs_var, ones.data(), D * 4, cudaMemcpyHostToDevice));
+    }
+    DRIL_TRY(dril_buffer_create(c, 1, d.n_envs, d.obs_dim, d.act_dim == 0 ? DRIL_ACT_DISCRETE : DRIL_ACT_CONTINUOUS,
+                                std::max(d.act_dim, 1), &e->compat));
+    DRIL_TRY(dmalloc(&e->compat_obs, n * D));
     return DRIL_OK;
 }
 extern "C" int32_t dril_env_destroy(dril_env* e) {
@@ -1121,8 +1147,15 @@ extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const floa
     dril_ctx* c = e->ctx;
     DRIL_CUDA(cudaSetDevice(c->device));
     const size_t n = (size_t)d.n_envs;
+    std::vector<float> dflt;
+    if (!lo && e->observe_params) {   // observed parameters stay: back to lo = hi = the built-in constants
+        dflt.resize(n * np);
+        for (int k = 0; k < np; ++k) std::fill(dflt.begin() + (size_t)k * n, dflt.begin() + (size_t)(k + 1) * n, k_env_param_default[d.kind][k]);
+        lo = hi = dflt.data();
+    }
     if (!lo) {   // back to the built-in constants and the default instantiations
         DRIL_CUDA(cudaStreamSynchronize(c->stream));
+        e->default_params = false;
         for (float* p : {d.pval, d.plo, d.phi}) if (p) cudaFree(p);
         d.pval = d.plo = d.phi = nullptr;
         d.has_params = 0;
@@ -1146,6 +1179,7 @@ extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const floa
     DRIL_CUDA(cudaMemcpyAsync(d.plo, lo, n * np * 4, cudaMemcpyHostToDevice, c->stream));
     DRIL_CUDA(cudaMemcpyAsync(d.phi, hi, n * np * 4, cudaMemcpyHostToDevice, c->stream));
     d.has_params = 1;
+    e->default_params = !dflt.empty();
     {
         Span sp(c, DRIL_K_ENV);
         env_params_draw_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(d);
@@ -1168,6 +1202,30 @@ extern "C" int32_t dril_env_get_params(dril_env* e, int32_t n_params, float* val
     DRIL_CUDA(cudaSetDevice(c->device));
     DRIL_CUDA(cudaMemcpyAsync(values, d.pval, n * np * 4, cudaMemcpyDeviceToHost, c->stream));
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
+    return DRIL_OK;
+}
+
+extern "C" int32_t dril_env_set_observe_params(dril_env* e, int32_t on) {
+    DRIL_REQUIRE(e, "NULL argument");
+    EnvDev& d = e->d;
+    const int np = env_n_params(d.kind);
+    if (np == 0) { dril_set_error("env kind %d has no physical parameters to observe", d.kind); return DRIL_ERR_UNSUPPORTED; }
+    DRIL_REQUIRE(!e->observed, "observe_params can only change before the env's first observation");
+    if ((on != 0) == e->observe_params) return DRIL_OK;
+    DRIL_CUDA(cudaSetDevice(e->ctx->device));
+    DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
+    e->observe_params = on != 0;
+    d.obs_dim = env_base_obs_dim(d.kind) + (e->observe_params ? np : 0);
+    if (e->observe_params && !d.has_params) {            // the parametrised kernels with lo = hi = the defaults
+        DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
+    } else if (!e->observe_params && e->default_params) {   // parameters that were only held for observing: dropped
+        DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
+    }
+    return env_alloc_obs_arrays(e);
+}
+extern "C" int32_t dril_env_obs_dim(dril_env* e, int32_t* obs_dim) {
+    DRIL_REQUIRE(e && obs_dim, "NULL argument");
+    *obs_dim = e->d.obs_dim;
     return DRIL_OK;
 }
 
@@ -1219,6 +1277,8 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     a.T = T;
     int flags = base_flags | (has_policy ? RO_HAS_POLICY : 0);
     const EnvDev& d = e->d;
+    const bool obsp = e->observe_params;
+    e->observed = true;
     const bool upd = d.normalize && d.training && (d.norm_obs || d.norm_reward);
     if (upd) flags |= RO_GRID_SYNC;
     const long long N = d.n_envs;
@@ -1299,7 +1359,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.n_tiles = (int)((N + M4 - 1) / M4);
             Span sp(c, DRIL_K_ROLLOUT);
             void* args[] = {(void*)&a};
-            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, d.kind, d.has_params), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
+            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, d.kind, d.has_params, obsp), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
             return DRIL_OK;
         }
     }
@@ -1336,7 +1396,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.M4 = GTC_ENVS; a.flags = flags;
             a.n_tiles = (int)((N + GTC_ENVS - 1) / GTC_ENVS);
             int grid = a.n_tiles, body_i = (int)body;
-            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, d.kind, a.pd.act_n, d.has_params);
+            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, d.kind, a.pd.act_n, d.has_params, obsp);
             void* args[] = {(void*)&a, (void*)&gl, (void*)&body_i};
             {
                 Span sp(c, DRIL_K_ROLLOUT);
@@ -1398,14 +1458,14 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     Span sp(c, has_policy ? DRIL_K_ROLLOUT : DRIL_K_ENV);
     if (flags & RO_GRID_SYNC) {
         int per_sm = 0;
-        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, d.kind, d.has_params), threads, smem));
+        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, d.kind, d.has_params, obsp), threads, smem));
         DRIL_REQUIRE(per_sm >= 1, "rollout kernel does not fit on an SM");
         grid = std::min(grid, std::min(per_sm * c->sm_count, e->max_blocks));
         void* args[] = {(void*)&a};
-        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, d.kind, d.has_params), dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, d.kind, d.has_params, obsp), dim3(grid), dim3(threads), args, smem, c->stream));
     } else {
         void* args[] = {(void*)&a};
-        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, d.kind, d.has_params), dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, d.kind, d.has_params, obsp), dim3(grid), dim3(threads), args, smem, c->stream));
     }
     if (defer) return launch_critic();
     return DRIL_OK;
@@ -1525,8 +1585,10 @@ extern "C" int32_t dril_env_set_scaling(dril_env* e, int32_t on, const float* ob
     // ScalingWrapperEnv needs Box observation and action spaces (scalingWrapperEnv.jl:22): of the built-in envs that is Pendulum
     DRIL_REQUIRE(e->d.kind == DRIL_ENV_PENDULUM || e->d.kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS,
                  "ScalingWrapperEnv: Box observation and action spaces required (pendulum, mountaincar_continuous)");
-    DRIL_REQUIRE(e->d.obs_dim <= 4 && e->d.act_dim == 1, "ScalingWrapperEnv: obs_dim <= 4, act_dim == 1");
-    for (int j = 0; j < e->d.obs_dim; ++j) {
+    // observed parameters (dril_env_set_observe_params) pass through raw: the bounds cover the base observation only
+    const int D0 = env_base_obs_dim(e->d.kind);
+    DRIL_REQUIRE(D0 <= 4 && e->d.act_dim == 1, "ScalingWrapperEnv: obs_dim <= 4, act_dim == 1");
+    for (int j = 0; j < D0; ++j) {
         e->d.sc_obs_f[j] = 2.0f / (obs_high[j] - obs_low[j]);                     // :37-39
         e->d.sc_obs_o[j] = obs_low[j];
     }

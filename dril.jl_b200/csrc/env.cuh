@@ -18,9 +18,27 @@
 #define ENV_KS_CLASSIC ((1u << DRIL_ENV_CARTPOLE) | (1u << DRIL_ENV_PENDULUM) | (1u << DRIL_ENV_SYNTHETIC))
 #define ENV_KS_ALL (ENV_KS_CLASSIC | (1u << DRIL_ENV_MOUNTAINCAR) | (1u << DRIL_ENV_MOUNTAINCAR_CONTINUOUS) | (1u << DRIL_ENV_ACROBOT))
 
+// kind-set bits beyond the kinds: ENV_KS_PARAMS = per-env physical parameters (below); ENV_KS_OBS_PARAMS (only together with
+// ENV_KS_PARAMS) = observations [base observation | the running episode's parameter values in table order]
+#define ENV_KS_PARAMS (1u << 16)
+#define ENV_KS_OBS_PARAMS (1u << 17)
+
 __host__ __device__ constexpr bool env_in(unsigned ks, int kind) { return (ks >> kind) & 1u; }
-// blocks of four observation components a kernel built for the kinds `ks` handles (Acrobot: 6 components)
-__host__ __device__ constexpr int env_obs_blocks(unsigned ks) { return env_in(ks, DRIL_ENV_ACROBOT) ? 2 : 1; }
+__host__ __device__ constexpr bool env_obs_params(unsigned ks) { return (ks & ENV_KS_OBS_PARAMS) != 0; }
+__host__ __device__ constexpr int env_n_params(int kind) {
+    return kind == DRIL_ENV_CARTPOLE || kind == DRIL_ENV_ACROBOT ? 6
+         : kind == DRIL_ENV_PENDULUM ? 4
+         : kind == DRIL_ENV_MOUNTAINCAR || kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS ? 2 : 0;
+}
+// observation components of a state-based kind without its parameters
+__host__ __device__ constexpr int env_base_obs_dim(int kind) {
+    return kind == DRIL_ENV_CARTPOLE ? 4 : kind == DRIL_ENV_PENDULUM ? 3 : kind == DRIL_ENV_ACROBOT ? 6 : 2;
+}
+// blocks of four observation components a kernel built for the kinds `ks` handles (Acrobot: 6 components; with
+// ENV_KS_OBS_PARAMS both parametrised kind sets hold a kind of base + parameter width > 8: CartPole 10, Acrobot 12)
+__host__ __device__ constexpr int env_obs_blocks(unsigned ks) {
+    return env_obs_params(ks) ? 3 : (env_in(ks, DRIL_ENV_ACROBOT) ? 2 : 1);
+}
 // the kind set whose instantiation serves env kind `kind`
 __host__ __device__ constexpr unsigned env_kind_set(int kind) { return env_in(ENV_KS_CLASSIC, kind) ? ENV_KS_CLASSIC : ENV_KS_ALL; }
 
@@ -55,9 +73,32 @@ __device__ __forceinline__ void env_raw_obs_block(int kind, const float* st, int
 
 // observation block b as the wrappers above the env see it: raw, or mapped to [-1, 1] by ScalingWrapperEnv.observe
 // (scalingWrapperEnv.jl:72-75,94-99: `(x - offset) * scale - 1`, three separate fp32 roundings; Box/Box envs of
-// obs_dim <= 4 only, so block 0)
+// obs_dim <= 4 only, so block 0).
+// ENV_KS_OBS_PARAMS: components D0 .. D0+P-1 (D0 = env_base_obs_dim, P = env_n_params) are par[0 .. P-1], raw; the blocks
+// straddle the boundary (Acrobot's block 1 is (w1, w2, p0, p1)), and Scaling maps only the D0 base components.
 template <unsigned KS>
-__device__ __forceinline__ void env_obs_block(const EnvDev& env, const float* st, int b, float* o) {
+__device__ __forceinline__ void env_obs_block(const EnvDev& env, const float* st, int b, float* o, const float* par = nullptr) {
+    if (env_obs_params(KS)) {
+        const int D0 = env_base_obs_dim(env.kind), P = env_n_params(env.kind);
+        if (4 * b < D0) {
+            env_raw_obs_block<KS>(env.kind, st, b, o);
+            if (env.scaling && b == 0) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                    if (j < D0) o[j] = __fsub_rn(__fmul_rn(__fsub_rn(o[j], env.sc_obs_o[j]), env.sc_obs_f[j]), 1.0f);
+            }
+        } else {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) o[j] = 0.f;
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+#pragma unroll
+            for (int k = 0; k < DRIL_ENV_MAX_PARAMS; ++k)   // a select per (j, k): no dynamic index into the register array
+                if (k < P && 4 * b + j == D0 + k) o[j] = par[k];
+        }
+        return;
+    }
     env_raw_obs_block<KS>(env.kind, st, b, o);
     if (env.scaling && b == 0) {
 #pragma unroll
@@ -232,17 +273,13 @@ __device__ __forceinline__ float acrobot_step(float* st, int idx, bool* terminat
 // constants above and their exact code.  Each derived coefficient below is one fixed fp32 sequence, restated in
 // oracle/env_params.py, that gives the folded constant bit for bit at the default values.
 // ---------------------------------------------------------------------------------------
-#define ENV_KS_PARAMS (1u << 16)
 __host__ __device__ constexpr bool env_has_params(unsigned ks) { return (ks & ENV_KS_PARAMS) != 0; }
-__host__ __device__ constexpr int env_n_params(int kind) {
-    return kind == DRIL_ENV_CARTPOLE || kind == DRIL_ENV_ACROBOT ? 6
-         : kind == DRIL_ENV_PENDULUM ? 4
-         : kind == DRIL_ENV_MOUNTAINCAR || kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS ? 2 : 0;
-}
 // the parametrised kind set whose instantiation serves env kind `kind` (the synthetic env has no parameters)
 __host__ __device__ constexpr unsigned env_param_kind_set(int kind) {
     return (env_kind_set(kind) & ~(1u << DRIL_ENV_SYNTHETIC)) | ENV_KS_PARAMS;
 }
+// ... and the one that also observes the parameters
+__host__ __device__ constexpr unsigned env_obs_param_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_OBS_PARAMS; }
 
 // the values of env n's episode `episode`: lo + (hi - lo) * u, u from Philox (gid, episode, k / 4, DRIL_TAG_ENV_PARAMS) word
 // k % 4; written to par and env.pval

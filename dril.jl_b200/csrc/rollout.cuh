@@ -318,7 +318,13 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                         float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
                         for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * N + n0 + tid];
-                        env_obs_block<KS>(env, st, b, o);
+                        if (env_obs_params(KS)) {   // the running episode's values (after an auto-reset: the new draw)
+                            float par[DRIL_ENV_MAX_PARAMS];
+                            env_load_params(env, n0 + tid, par);
+                            env_obs_block<KS>(env, st, b, o, par);
+                        } else {
+                            env_obs_block<KS>(env, st, b, o);
+                        }
                     }
 #pragma unroll
                     for (int j = 0; j < 4; ++j) if (4 * b + j < Dp) sRaw[(size_t)(4 * b + j) * ld + tid] = o[j];
@@ -479,7 +485,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
 #pragma unroll
                         for (int b = 0; b < env_obs_blocks(KS); ++b) {
                             float o[4];
-                            env_obs_block<KS>(env, st, b, o);
+                            env_obs_block<KS>(env, st, b, o, par);   // the ended episode's values: drawn anew below
 #pragma unroll
                             for (int j = 0; j < 4; ++j) if (4 * b + j < D) env.tobs[(size_t)n * D + 4 * b + j] = o[j];
                         }
@@ -698,7 +704,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             float o[OW] = {};
             if (mine) {
 #pragma unroll
-                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, o + 4 * b);
+                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, o + 4 * b, eparam);
                 if (norm_obs) {
 #pragma unroll
                     for (int j = 0; j < OW; ++j) if (j < D) o[j] = normalize_obs_val(o[j], sMean[j], sVar[j], env.eps, env.clip_obs);
@@ -874,10 +880,14 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             if (trunc) {
                 trunc_i = 1;
 #pragma unroll
-                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, tobs + 4 * b);
+                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, tobs + 4 * b, eparam);   // before the redraw below
                 if (norm_obs) {
 #pragma unroll
                     for (int j = 0; j < OW; ++j) if (j < D) tobs[j] = normalize_obs_val(tobs[j], sMean[j], sVar[j], env.eps, env.clip_obs);
+                }
+                if (env_obs_params(KS)) {   // staged now (this step's forward has read sX): 12 components live across the redraw
+#pragma unroll                             // and the barrier would spill
+                    for (int j = 0; j < OW; ++j) if (j < Dp) sX[(size_t)j * ld + tid] = tobs[j];
                 }
             }
             if (done) {
@@ -892,7 +902,8 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         if (__syncthreads_or(trunc_i)) {
             if (tid < M4) {
 #pragma unroll
-                for (int j = 0; j < OW; ++j) if (j < Dp) sX[(size_t)j * ld + tid] = trunc_i ? tobs[j] : 0.f;
+                for (int j = 0; j < OW; ++j)
+                    if (j < Dp && !(env_obs_params(KS) && trunc_i)) sX[(size_t)j * ld + tid] = trunc_i ? tobs[j] : 0.f;
             }
             __syncthreads();
             const int p2 = hidden_forward(2);

@@ -243,6 +243,25 @@ int32_t dril_env_monitor_stats(dril_env* env, float* ep_rew_mean, float* ep_len_
 int32_t dril_env_set_params(dril_env* env, int32_t n_params, const float* lo, const float* hi);
 int32_t dril_env_get_params(dril_env* env, int32_t n_params, float* values);
 
+/* Parameter-augmented observations.  observe_params = 1: every observation of env n is
+ *   [base observation (D components) | p_0 ... p_{P-1}],  obs_dim = D + P,
+ * p_k = the value of parameter k in the running episode, in the table order above: exactly what dril_env_get_params returns,
+ * raw fp32.  (cartpole 4 + 6, pendulum 3 + 4, mountaincar 2 + 2, mountaincar_continuous 2 + 2, acrobot 6 + 6.)
+ *   - ScalingWrapperEnv maps the D base components only; the parameter components pass through raw.
+ *   - NormalizeWrapperEnv normalises all D + P columns like any other (running statistics, clip, terminal observations), so
+ *     a column that is constant over the batch (lo == hi everywhere) normalises to exactly 0 after the first update.
+ *   - The terminal observation of a truncated step (and V(terminal_obs)) carries the values of the episode that ended; the
+ *     observation after a reset carries the values just drawn for the new episode.
+ *   - An env without ranges observes the defaults (it runs with lo = hi = the defaults); dril_env_set_params(lo = NULL)
+ *     returns to that instead of dropping the parameters.  New ranges show as the running episode's own (gid, e) draw.
+ * dril_env_set_observe_params is allowed only before the env's first observation (observe, step, rollout, evaluate;
+ * reset and set_state do not count), else DRIL_ERR_INVALID: it resizes the obs-sized arrays (normaliser statistics, old and
+ * terminal observations).  The synthetic env has no parameters: DRIL_ERR_UNSUPPORTED.  A policy or buffer built for the
+ * other width fails the obs_dim check of the rollout.
+ * dril_env_obs_dim: the env's current observation width, for hosts that build the policy from the env. */
+int32_t dril_env_set_observe_params(dril_env* env, int32_t on);
+int32_t dril_env_obs_dim(dril_env* env, int32_t* obs_dim);
+
 /* ---- actor-critic layer + optimiser state: replaces Discrete/ContinuousActorCriticLayer
  *      (layers/) and the Lux TrainState held by Agent (agents/agent_types.jl) ------------ */
 int32_t dril_policy_create(dril_ctx* ctx, int32_t obs_dim, int32_t n_hidden, const int32_t* hidden_dims,

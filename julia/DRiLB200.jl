@@ -79,11 +79,13 @@ const ENV_PARAMS = Dict(
 )
 
 """
-    CudaBatchedEnv(kind, n_envs; max_steps, act_start, monitor_window, normalize, env_params)
+    CudaBatchedEnv(kind, n_envs; max_steps, act_start, monitor_window, normalize, env_params, observe_params)
 
 Device-resident replacement of `NormalizeWrapperEnv(MonitorWrapperEnv(MultiThreadedParallelEnv(envs)))`
 for `kind in (:cartpole, :pendulum, :synthetic, :mountaincar, :mountaincar_continuous, :acrobot)`.
 `env_params = Dict(:length => (0.25, 1.0), ...)`: per-env physical parameters, see `set_env_params!`.
+`observe_params = true`: every observation is `[base observation | the running episode's parameter values]` in the order of
+`ENV_PARAMS[kind]`, raw (Scaling maps the base components only); `observation_space` is widened by `[0, Inf)` per parameter.
 """
 mutable struct CudaBatchedEnv <: AbstractParallelEnv
     ctx::Context
@@ -100,7 +102,7 @@ end
 
 function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_steps = 0, obs_dim = 0, act_start = 1,
         monitor_window = 0, normalize::Union{Nothing, NormCfg} = nothing, gid_offset = 0, scaling::Bool = false,
-        env_params = nothing)
+        env_params = nothing, observe_params::Bool = false)
     obs_space, act_space = if kind == :cartpole
         hi = Float32[4.8, Inf32, 0.41887903, Inf32]
         Box(-hi, hi), Discrete(2, act_start)
@@ -122,6 +124,7 @@ function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_
         (Ptr{Cvoid}, Int32, Int64, Int32, Int32, Int32, Int64, Ptr{NormCfg}, Int32, Ref{Ptr{Cvoid}}),
         ctx.h, ENV_KINDS[kind], n_envs, max_steps, size(obs_space)[1], act_start, gid_offset,
         isnothing(normalize) ? C_NULL : Base.unsafe_convert(Ptr{NormCfg}, normptr), monitor_window, out))
+    observe_params && check(ccall((:dril_env_set_observe_params, LIB), Int32, (Ptr{Cvoid}, Int32), out[], 1))
     if scaling
         # ScalingWrapperEnv around every env of the batch (scalingWrapperEnv.jl:14-49): Box/Box envs only; the device maps
         # observations to [-1, 1] and actions back from [-1, 1], so the spaces the agent sees are the scaled ones
@@ -130,6 +133,13 @@ function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_
             out[], 1, vec(obs_space.low), vec(obs_space.high), vec(act_space.low), vec(act_space.high)))
         obs_space = Box(-ones(Float32, size(obs_space.low)), ones(Float32, size(obs_space.high)))
         act_space = Box(-ones(Float32, size(act_space.low)), ones(Float32, size(act_space.high)))
+    end
+    if observe_params
+        P = length(ENV_PARAMS[kind])
+        obs_space = Box(vcat(vec(obs_space.low), zeros(Float32, P)), vcat(vec(obs_space.high), fill(Inf32, P)))
+        d = Ref{Int32}(0)
+        check(ccall((:dril_env_obs_dim, LIB), Int32, (Ptr{Cvoid}, Ref{Int32}), out[], d))
+        d[] == size(obs_space)[1] || error("observation width $(d[]) != $(size(obs_space)[1])")
     end
     env = CudaBatchedEnv(ctx, out[], kind, n_envs, obs_space, act_space, monitor_window, normalize,
         falses(n_envs), falses(n_envs))

@@ -1,10 +1,11 @@
 """PPO throughput per classic-control env: one JSON line per env, env count and (with --randomize) parameter setting.
 
     python tools/bench_envs.py [--envs cartpole,pendulum,mountaincar,mountaincar_continuous,acrobot] [--n-envs 4096,65536]
-                               [--steps 20] [--normalize] [--randomize] [--repeats 1]
+                               [--steps 20] [--normalize] [--randomize] [--observe-params] [--repeats 1]
 
 --randomize runs every configuration twice, alternating: with the built-in constants and with per-env parameters drawn at every
-reset from +-50 % of each default (set_env_params), --repeats times.
+reset from +-50 % of each default (set_env_params), --repeats times.  --observe-params adds a third run in the alternation: the
+same randomised parameters, observed by the policy (observe_params=True: obs_dim = base + parameter count).
 
 Each run: [64, 64] policy, n_steps 128, 4 epochs x 4 minibatches; warm-up iterations, then --steps iterations timed with CUDA events
 on the library's stream, L2 overwritten before every iteration (as bench.py does), then the same iterations again with the
@@ -43,13 +44,13 @@ def rollout_kernel(kind, n, sms, normalize, act_n, randomize):
     return "gtc" if n >= 64 * sms else "general"
 
 
-def run(D, kind, n, steps, warmup, normalize, randomize):
+def run(D, kind, n, steps, warmup, normalize, randomize, observe_params=False):
     from dril_b200 import _lib as L
     from dril_b200.core import ENV_PARAMS
     T = 128
     params = {nm: (0.5 * d, 1.5 * d) for nm, d in ENV_PARAMS[kind]} if randomize else None
     env = D.CudaBatchedEnv(kind, n, seed=0, monitor_window=100, normalize=D.NormalizeConfig() if normalize else None,
-                           env_params=params)
+                           env_params=params, observe_params=observe_params)
     layer = D.ActorCriticLayer(env.observation_space(), env.action_space(), hidden_dims=[64, 64])
     alg = D.PPO(n_steps=T, batch_size=T * n // 4, epochs=4)
     agent = D.Agent(layer, alg, rng=np.random.default_rng(0))
@@ -85,7 +86,7 @@ def run(D, kind, n, steps, warmup, normalize, randomize):
     sms = ctx.sm_count()
     act = env.action_space()
     res = dict(env=kind, n_envs=n, n_steps=T, hidden=[64, 64], epochs=4, minibatches=4, normalize=bool(normalize),
-               randomize=bool(randomize),
+               randomize=bool(randomize), observe_params=bool(observe_params), obs_dim=env.obs_dim,
                env_steps_per_s=n * T / (ms * 1e-3), ms_per_iter=ms,
                rollout_ms=prof.get("rollout", (0.0, 0))[0] / steps, update_ms=upd,
                update_path=agent.device.update_path(),
@@ -104,6 +105,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--normalize", action="store_true")
     ap.add_argument("--randomize", action="store_true", help="alternate built-in constants and +-50 %% per-env parameters")
+    ap.add_argument("--observe-params", action="store_true", help="also randomised parameters observed by the policy")
     ap.add_argument("--repeats", type=int, default=1)
     args = ap.parse_args()
     import __graft_entry__
@@ -113,8 +115,9 @@ def main():
     for kind in args.envs.split(","):
         for n in (int(x) for x in args.n_envs.split(",")):
             for _ in range(args.repeats):
-                for randomize in ((False, True) if args.randomize else (False,)):
-                    r = run(D, kind, n, args.steps, args.warmup, args.normalize, randomize)
+                variants = [(False, False)] + ([(True, False)] if args.randomize else []) + ([(True, True)] if args.observe_params else [])
+                for randomize, observe in variants:
+                    r = run(D, kind, n, args.steps, args.warmup, args.normalize, randomize, observe)
                     r.update(card=name, power_limit=power)
                     print(json.dumps(r), flush=True)
 
