@@ -23,11 +23,14 @@ BroadcastedParallelEnv = MultiThreadedParallelEnv
 
 
 def _rewrap(env, **over):
+    """The env re-created with `over` switched on: state and step counters are carried over through set_state, which, like
+    dril_env_set_state, restarts an observation history from each env's current frame."""
     args = dict(kind=env.kind, n_envs=env.n_envs, max_steps=env.max_steps, obs_dim=env.obs_dim,
                 act_start=env.act_start, ctx=env.ctx, monitor_window=env.monitor_window,
                 normalize=env.normalize, gid_offset=env.gid_offset, scaling=env.scaling,
                 obs_shape=env.obs_shape if len(env.obs_shape) > 1 else None, env_params=env.env_param_ranges(),
-                observe_params=env.observes_params())
+                observe_params=env.observes_params(), history_len=env.history_len(),
+                mask_velocities=env.masks_velocities())
     args.update(over)
     kind, n = args.pop("kind"), args.pop("n_envs")
     st, steps = env.get_state()

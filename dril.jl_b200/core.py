@@ -32,6 +32,22 @@ def observation_space_with_params(space, kind):
     return Box(low, high)
 
 
+# the non-velocity components of each kind's observation: the frame of an env with mask_velocities=True
+VELOCITY_FREE = {"cartpole": (0, 2), "pendulum": (0, 1), "mountaincar": (0,), "mountaincar_continuous": (0,),
+                 "acrobot": (0, 1, 2, 3)}
+MAX_HISTORY = 4
+
+
+def observation_space_with_history(space, kind, history_len, mask_velocities):
+    """The observation space of an env with an observation history: the bounds (scaled or not) of the frame's components
+    (the kept ones with mask_velocities), tiled history_len times, oldest frame first."""
+    low, high = np.asarray(space.low, np.float32).ravel(), np.asarray(space.high, np.float32).ravel()
+    if mask_velocities:
+        idx = list(VELOCITY_FREE[kind])
+        low, high = low[idx], high[idx]
+    return Box(np.tile(low, history_len), np.tile(high, history_len))
+
+
 class Context:
     """One CUDA device + stream; not thread-safe (one per GPU)."""
     _default = {}
@@ -137,7 +153,7 @@ class CudaBatchedEnv:
 
     def __init__(self, kind, n_envs, max_steps=0, obs_dim=0, act_start=1, seed=None, ctx=None,
                  monitor_window=0, normalize=None, gid_offset=0, obs_shape=None, scaling=False, env_params=None,
-                 observe_params=False):
+                 observe_params=False, history_len=1, mask_velocities=False):
         self.kind = kind.lower()
         assert self.kind in ENV_KINDS, f"unknown env kind {kind}"
         self.ctx = ctx or Context.default()
@@ -194,8 +210,14 @@ class CudaBatchedEnv:
             L.check(lib.dril_env_set_scaling(self.h, 1, L.ptr(ol), L.ptr(oh), L.ptr(al), L.ptr(ah)))
             self._obs_space = Box(-np.ones_like(ol).reshape(self._obs_space.low.shape), np.ones_like(oh).reshape(self._obs_space.low.shape))
             self._act_space = Box(-np.ones_like(al), np.ones_like(ah))
+        self._history_len, self._mask_velocities = int(history_len), bool(mask_velocities)
+        if self._history_len != 1 or self._mask_velocities:
+            # [f_{t-k+1} | ... | f_t], frames without velocities if masked: after Scaling (given the full base bounds above)
+            L.check(lib.dril_env_set_obs_history(self.h, self._history_len, int(self._mask_velocities)))
+            self._obs_space = observation_space_with_history(self._obs_space, self.kind, self._history_len, self._mask_velocities)
         if self._observe_params:
             self._obs_space = observation_space_with_params(self._obs_space, self.kind)
+        if self._observe_params or self._history_len != 1 or self._mask_velocities:
             self.obs_dim = int(self._obs_space.size()[0])
             self.obs_shape = (self.obs_dim,)
             d = L.c_i32(0)
@@ -283,6 +305,15 @@ class CudaBatchedEnv:
         st = None if state is None else L.f32(state)
         sp = None if steps is None else np.ascontiguousarray(steps, dtype=np.int32)
         L.check(self.ctx.lib.dril_env_set_state(self.h, L.ptr(st), L.ptr(sp)))
+
+    # ---- observation history ----
+    def history_len(self):
+        """k of the frame-stacked observation [f_{t-k+1} | ... | f_t] (1: the plain observation)."""
+        return self._history_len
+
+    def masks_velocities(self):
+        """True if every frame keeps only the non-velocity components (VELOCITY_FREE)."""
+        return self._mask_velocities
 
     # ---- per-env physical parameters ----
     def observes_params(self):

@@ -100,36 +100,39 @@ static bool tc_eligible(const PolicyDesc& pd) {
 
 // rollout kernels by the env kind they step: CartPole, Pendulum and the synthetic env run the instantiations built for those
 // kinds alone (env.cuh), every other kind the one built for all kinds; an env with per-env parameters (dril_env_set_params)
-// runs the ENV_KS_PARAMS instantiation of its kind set, and one that observes its parameters (dril_env_set_observe_params) the
-// ENV_KS_OBS_PARAMS instantiation
+// runs the ENV_KS_PARAMS instantiation of its kind set, one that observes its parameters (dril_env_set_observe_params) the
+// ENV_KS_OBS_PARAMS instantiation, and one with an observation history (dril_env_set_obs_history) the ENV_KS_HISTORY one
 #define KS_CP_ ENV_KS_CLASSIC
 #define KS_ALL_ ENV_KS_ALL
 #define KS_CP_P_ env_param_kind_set(DRIL_ENV_CARTPOLE)
 #define KS_ALL_P_ env_param_kind_set(DRIL_ENV_ACROBOT)
 #define KS_CP_OP_ env_obs_param_kind_set(DRIL_ENV_CARTPOLE)
 #define KS_ALL_OP_ env_obs_param_kind_set(DRIL_ENV_ACROBOT)
-#define DRIL_KS_PICK(K_, kind, params, obsp)                                                               \
-    (env_kind_set(kind) == ENV_KS_CLASSIC ? ((obsp) ? K_(KS_CP_OP_) : (params) ? K_(KS_CP_P_) : K_(KS_CP_)) \
-                                          : ((obsp) ? K_(KS_ALL_OP_) : (params) ? K_(KS_ALL_P_) : K_(KS_ALL_)))
-static void* rollout_fn(bool ws, int kind, bool params, bool obsp) {
+#define KS_CP_H_ env_hist_kind_set(DRIL_ENV_CARTPOLE)
+#define KS_ALL_H_ env_hist_kind_set(DRIL_ENV_ACROBOT)
+#define DRIL_KS_PICK(K_, kind, params, obsp, hist)                                                                             \
+    (env_kind_set(kind) == ENV_KS_CLASSIC ? ((hist) ? K_(KS_CP_H_) : (obsp) ? K_(KS_CP_OP_) : (params) ? K_(KS_CP_P_) : K_(KS_CP_)) \
+                                          : ((hist) ? K_(KS_ALL_H_) : (obsp) ? K_(KS_ALL_OP_) : (params) ? K_(KS_ALL_P_) : K_(KS_ALL_)))
+static void* rollout_fn(bool ws, int kind, bool params, bool obsp, bool hist) {
 #define K_(ks) (ws ? (void*)rollout_kernel<true, ks> : (void*)rollout_kernel<false, ks>)
-    return DRIL_KS_PICK(K_, kind, params, obsp);
+    return DRIL_KS_PICK(K_, kind, params, obsp, hist);
 #undef K_
 }
-static void* rollout_fast_fn(bool ws, int kind, bool params, bool obsp) {
+static void* rollout_fast_fn(bool ws, int kind, bool params, bool obsp, bool hist) {
 #define K_(ks) (ws ? (void*)rollout_fast_kernel<true, ks> : (void*)rollout_fast_kernel<false, ks>)
-    return DRIL_KS_PICK(K_, kind, params, obsp);
+    return DRIL_KS_PICK(K_, kind, params, obsp, hist);
 #undef K_
 }
 // tcgen05-actor rollout by hidden-layer count, env kind and action count (2 or 4 staged output columns, gtc_nout)
-static void* rollout_gtc_fn(int L, int kind, int act_n, bool params, bool obsp) {
+static void* rollout_gtc_fn(int L, int kind, int act_n, bool params, bool obsp, bool hist) {
     if (act_n > 2) {
+        if (hist) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_H_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_H_, 4>;
         if (obsp) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_OP_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_OP_, 4>;
         if (params) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_P_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_P_, 4>;
         return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_ALL, 4> : (void*)rollout_gtc_kernel<3, ENV_KS_ALL, 4>;
     }
 #define K_(ks) (L == 2 ? (void*)rollout_gtc_kernel<2, ks, 2> : (void*)rollout_gtc_kernel<3, ks, 2>)
-    return DRIL_KS_PICK(K_, kind, params, obsp);
+    return DRIL_KS_PICK(K_, kind, params, obsp, hist);
 #undef K_
 }
 
@@ -247,8 +250,9 @@ struct dril_env {
     float* norm_snap = nullptr;
     long long* norm_snap_cnt = nullptr;
     bool observe_params = false;     // dril_env_set_observe_params: the ENV_KS_OBS_PARAMS instantiations, obs_dim = D + P
-    bool default_params = false;     // parameters held at lo = hi = the defaults only because observe_params is on
+    bool default_params = false;     // parameters held at lo = hi = the defaults only because observe_params or history is on
     bool observed = false;           // an observation was made (observe, step, rollout, evaluate): the width is fixed
+    bool history = false;            // dril_env_set_obs_history (k > 1 or velocities masked): the ENV_KS_HISTORY instantiations
 };
 
 struct dril_policy {
@@ -376,9 +380,9 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
     DRIL_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
         for (int ws = 0; ws < 2; ++ws)
-            for (int params = 0; params < 3; ++params) {   // 2: observed parameters
-                DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, kind, params > 0, params == 2), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-                DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, kind, params > 0, params == 2), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+            for (int params = 0; params < 4; ++params) {   // 2: observed parameters, 3: observation history
+                DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, kind, params > 0, params == 2, params == 3), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+                DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, kind, params > 0, params == 2, params == 3), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
             }
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
@@ -398,8 +402,8 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
         for (int L = 2; L <= 3; ++L)
             for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
                 for (int an = 2; an <= 4; an += 2)
-                    for (int params = 0; params < 3; ++params)
-                        DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, kind, an, params > 0, params == 2), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
+                    for (int params = 0; params < 4; ++params)
+                        DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, kind, an, params > 0, params == 2, params == 3), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
     }
@@ -1000,6 +1004,7 @@ extern "C" int32_t dril_policy_predict_values(dril_policy* p, const float* obs, 
 // env
 // ---------------------------------------------------------------------------------------
 static int32_t env_alloc_obs_arrays(dril_env* e);
+static int32_t env_hist_refill(dril_env* e);
 extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, int32_t max_steps, int32_t obs_dim,
                                    int32_t act_start, int64_t gid_offset, const dril_norm_cfg* norm,
                                    int32_t monitor_window, dril_env** out) {
@@ -1022,6 +1027,7 @@ extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, in
         DRIL_REQUIRE(obs_dim >= 1 && obs_dim <= DRIL_MAX_OBS_DIM, "synthetic obs_dim %d out of range", obs_dim);
         d.obs_dim = obs_dim; d.state_dim = 0; d.act_dim = 0; d.max_steps = max_steps > 0 ? max_steps : 500;
     }
+    d.hist_len = 1; d.frame_dim = d.obs_dim;
     size_t n = (size_t)n_envs;
     DRIL_TRY(dmalloc(&d.state, n * std::max(d.state_dim, 1))); DRIL_TRY(dmalloc(&d.steps, n));
     DRIL_TRY(dmalloc(&d.episode, n)); DRIL_TRY(dmalloc(&d.life, n));
@@ -1060,12 +1066,13 @@ extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, in
     return DRIL_OK;
 }
 // the arrays sized by obs_dim, (re)allocated for the env's current width: terminal and old observations, the normaliser's
-// obs mean / var (mean 0, var 1), its per-CTA partials, the data-parallel moments and exchange buffers, the compat buffer
+// obs mean / var (mean 0, var 1), its per-CTA partials, the data-parallel moments and exchange buffers, the compat buffer, and
+// the observation-history store (filled from the current state)
 static int32_t env_alloc_obs_arrays(dril_env* e) {
     dril_ctx* c = e->ctx;
     EnvDev& d = e->d;
     const size_t n = (size_t)d.n_envs, D = (size_t)d.obs_dim;
-    for (float** p : {&d.tobs, &d.old_obs, &d.obs_mean, &d.obs_var, &e->norm_snap, &e->compat_obs}) { if (*p) cudaFree(*p); *p = nullptr; }
+    for (float** p : {&d.tobs, &d.old_obs, &d.obs_mean, &d.obs_var, &e->norm_snap, &e->compat_obs, &d.hist}) { if (*p) cudaFree(*p); *p = nullptr; }
     for (double** p : {&d.partials, &e->roll_moments, &e->xr}) { if (*p) cudaFree(*p); *p = nullptr; }
     if (e->compat) { dril_buffer_destroy(e->compat); e->compat = nullptr; }
     DRIL_TRY(dmalloc(&d.tobs, n * D)); DRIL_TRY(dmalloc(&d.old_obs, n * D));
@@ -1083,6 +1090,20 @@ static int32_t env_alloc_obs_arrays(dril_env* e) {
     DRIL_TRY(dril_buffer_create(c, 1, d.n_envs, d.obs_dim, d.act_dim == 0 ? DRIL_ACT_DISCRETE : DRIL_ACT_CONTINUOUS,
                                 std::max(d.act_dim, 1), &e->compat));
     DRIL_TRY(dmalloc(&e->compat_obs, n * D));
+    if (d.hist_len > 1) {
+        DRIL_TRY(dmalloc(&d.hist, n * (size_t)(d.hist_len - 1) * d.frame_dim));
+        DRIL_TRY(env_hist_refill(e));
+    }
+    return DRIL_OK;
+}
+// every env's observation history restarted from its current frame (no-op without a history store)
+static int32_t env_hist_refill(dril_env* e) {
+    if (!e->d.hist) return DRIL_OK;
+    dril_ctx* c = e->ctx;
+    Span sp(c, DRIL_K_ENV);
+    env_hist_fill_kernel<<<(unsigned)((e->d.n_envs + 255) / 256), 256, 0, c->stream>>>(e->d);
+    DRIL_CUDA(cudaGetLastError());
+    DRIL_CUDA(cudaStreamSynchronize(c->stream));
     return DRIL_OK;
 }
 extern "C" int32_t dril_env_destroy(dril_env* e) {
@@ -1098,7 +1119,7 @@ extern "C" int32_t dril_env_destroy(dril_env* e) {
     void* ps[] = {d.state, d.steps, d.episode, d.life, d.tobs, d.old_obs, d.old_rewards, d.ep_ret, d.ep_len, d.roll_sums,
                   d.roll_eps, d.ret, d.obs_mean, d.obs_var, d.ret_stats, d.counts, d.partials, e->ring.ret, e->ring.len,
                   e->ring.head, e->compat_actions, e->compat_obs, e->roll_moments, e->xr, e->norm_snap, e->norm_snap_cnt,
-                  d.pval, d.plo, d.phi};
+                  d.pval, d.plo, d.phi, d.hist};
     for (void* p : ps) if (p) cudaFree(p);
     dril_buffer_destroy(e->compat);
     delete e;
@@ -1125,7 +1146,7 @@ extern "C" int32_t dril_env_reset(dril_env* e) {
         DRIL_CUDA(cudaGetLastError());
     }
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
-    return DRIL_OK;
+    return env_hist_refill(e);
 }
 // per-env physical parameters (dril_b200.h): the defaults of the table, and whether a value must be > 0 (1) or >= 0 (0)
 static const float k_env_param_default[6][DRIL_ENV_MAX_PARAMS] = {
@@ -1148,7 +1169,7 @@ extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const floa
     DRIL_CUDA(cudaSetDevice(c->device));
     const size_t n = (size_t)d.n_envs;
     std::vector<float> dflt;
-    if (!lo && e->observe_params) {   // observed parameters stay: back to lo = hi = the built-in constants
+    if (!lo && (e->observe_params || e->history)) {   // observed parameters / history stay: back to lo = hi = the built-in constants
         dflt.resize(n * np);
         for (int k = 0; k < np; ++k) std::fill(dflt.begin() + (size_t)k * n, dflt.begin() + (size_t)(k + 1) * n, k_env_param_default[d.kind][k]);
         lo = hi = dflt.data();
@@ -1210,6 +1231,7 @@ extern "C" int32_t dril_env_set_observe_params(dril_env* e, int32_t on) {
     EnvDev& d = e->d;
     const int np = env_n_params(d.kind);
     if (np == 0) { dril_set_error("env kind %d has no physical parameters to observe", d.kind); return DRIL_ERR_UNSUPPORTED; }
+    if (on && e->history) { dril_set_error("observe_params cannot be combined with an observation history"); return DRIL_ERR_UNSUPPORTED; }
     DRIL_REQUIRE(!e->observed, "observe_params can only change before the env's first observation");
     if ((on != 0) == e->observe_params) return DRIL_OK;
     DRIL_CUDA(cudaSetDevice(e->ctx->device));
@@ -1219,6 +1241,30 @@ extern "C" int32_t dril_env_set_observe_params(dril_env* e, int32_t on) {
     if (e->observe_params && !d.has_params) {            // the parametrised kernels with lo = hi = the defaults
         DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
     } else if (!e->observe_params && e->default_params) {   // parameters that were only held for observing: dropped
+        DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
+    }
+    return env_alloc_obs_arrays(e);
+}
+extern "C" int32_t dril_env_set_obs_history(dril_env* e, int32_t history_len, int32_t mask_velocities) {
+    DRIL_REQUIRE(e, "NULL argument");
+    EnvDev& d = e->d;
+    const int np = env_n_params(d.kind);
+    const bool on = history_len != 1 || mask_velocities != 0;
+    if (np == 0) { dril_set_error("env kind %d has no observation history", d.kind); return DRIL_ERR_UNSUPPORTED; }
+    if (on && e->observe_params) { dril_set_error("an observation history cannot be combined with observe_params"); return DRIL_ERR_UNSUPPORTED; }
+    DRIL_REQUIRE(history_len >= 1 && history_len <= DRIL_ENV_MAX_HISTORY, "history_len %d outside [1, %d]", history_len, DRIL_ENV_MAX_HISTORY);
+    const bool mask = mask_velocities != 0;
+    if (history_len == d.hist_len && env_frame_dim(d.kind, mask) == d.frame_dim) return DRIL_OK;
+    DRIL_REQUIRE(!e->observed, "the observation history can only change before the env's first observation");
+    DRIL_CUDA(cudaSetDevice(e->ctx->device));
+    DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
+    e->history = on;
+    d.hist_len = history_len;
+    d.frame_dim = env_frame_dim(d.kind, mask);
+    d.obs_dim = d.frame_dim * history_len;
+    if (e->history && !d.has_params) {                    // the parametrised kernels with lo = hi = the defaults
+        DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
+    } else if (!e->history && e->default_params) {        // parameters that were only held for the history: dropped
         DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
     }
     return env_alloc_obs_arrays(e);
@@ -1277,7 +1323,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     a.T = T;
     int flags = base_flags | (has_policy ? RO_HAS_POLICY : 0);
     const EnvDev& d = e->d;
-    const bool obsp = e->observe_params;
+    const bool obsp = e->observe_params, hist = e->history;
     e->observed = true;
     const bool upd = d.normalize && d.training && (d.norm_obs || d.norm_reward);
     if (upd) flags |= RO_GRID_SYNC;
@@ -1351,7 +1397,8 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
         static const int f_threads = getenv("DRIL_FAST_THREADS") ? atoi(getenv("DRIL_FAST_THREADS")) : 0;
         if (f_threads >= tq && f_threads <= DRIL_THREADS && f_threads % tq == 0) threads = f_threads;
         bool ws = true;
-        auto tot = [&](int m4, int th, bool w) { return rollout_fast_smem_layout(a.pd, m4, th, w).total; };
+        const int hist_rows = hist ? d.obs_dim - d.frame_dim : 0;
+        auto tot = [&](int m4, int th, bool w) { return rollout_fast_smem_layout(a.pd, m4, th, w, hist_rows).total; };
         if (tot(M4, threads, true) > DRIL_SMEM_MAX) ws = false;
         while (M4 > 8 && tot(M4, threads, ws) > DRIL_SMEM_MAX) M4 >>= 1;
         if (tot(M4, threads, ws) <= DRIL_SMEM_MAX) {
@@ -1359,7 +1406,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.n_tiles = (int)((N + M4 - 1) / M4);
             Span sp(c, DRIL_K_ROLLOUT);
             void* args[] = {(void*)&a};
-            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, d.kind, d.has_params, obsp), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
+            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, d.kind, d.has_params, obsp, hist), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
             return DRIL_OK;
         }
     }
@@ -1396,7 +1443,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.M4 = GTC_ENVS; a.flags = flags;
             a.n_tiles = (int)((N + GTC_ENVS - 1) / GTC_ENVS);
             int grid = a.n_tiles, body_i = (int)body;
-            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, d.kind, a.pd.act_n, d.has_params, obsp);
+            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, d.kind, a.pd.act_n, d.has_params, obsp, hist);
             void* args[] = {(void*)&a, (void*)&gl, (void*)&body_i};
             {
                 Span sp(c, DRIL_K_ROLLOUT);
@@ -1458,14 +1505,14 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     Span sp(c, has_policy ? DRIL_K_ROLLOUT : DRIL_K_ENV);
     if (flags & RO_GRID_SYNC) {
         int per_sm = 0;
-        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, d.kind, d.has_params, obsp), threads, smem));
+        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, d.kind, d.has_params, obsp, hist), threads, smem));
         DRIL_REQUIRE(per_sm >= 1, "rollout kernel does not fit on an SM");
         grid = std::min(grid, std::min(per_sm * c->sm_count, e->max_blocks));
         void* args[] = {(void*)&a};
-        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, d.kind, d.has_params, obsp), dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, d.kind, d.has_params, obsp, hist), dim3(grid), dim3(threads), args, smem, c->stream));
     } else {
         void* args[] = {(void*)&a};
-        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, d.kind, d.has_params, obsp), dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, d.kind, d.has_params, obsp, hist), dim3(grid), dim3(threads), args, smem, c->stream));
     }
     if (defer) return launch_critic();
     return DRIL_OK;
@@ -1538,7 +1585,7 @@ extern "C" int32_t dril_env_set_state(dril_env* e, const float* state, const int
     if (state && e->d.state_dim) DRIL_CUDA(cudaMemcpyAsync(e->d.state, state, (size_t)e->d.n_envs * e->d.state_dim * 4, cudaMemcpyHostToDevice, c->stream));
     if (steps) DRIL_CUDA(cudaMemcpyAsync(e->d.steps, steps, (size_t)e->d.n_envs * 4, cudaMemcpyHostToDevice, c->stream));
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
-    return DRIL_OK;
+    return env_hist_refill(e);
 }
 extern "C" int32_t dril_env_get_norm_stats(dril_env* e, float* obs_mean, float* obs_var, int64_t* obs_count,
                                            float* ret_mean, float* ret_var, int64_t* ret_count) {
@@ -1580,12 +1627,14 @@ extern "C" int32_t dril_env_set_training(dril_env* e, int32_t training) {
 extern "C" int32_t dril_env_set_scaling(dril_env* e, int32_t on, const float* obs_low, const float* obs_high, const float* act_low,
                                         const float* act_high) {
     DRIL_REQUIRE(e, "NULL argument");
-    if (!on) { e->d.scaling = 0; return DRIL_OK; }
+    // frames change with the mapping: an observation history restarts from the mapped frame
+    if (!on) { e->d.scaling = 0; return env_hist_refill(e); }
     DRIL_REQUIRE(obs_low && obs_high && act_low && act_high, "NULL bounds");
     // ScalingWrapperEnv needs Box observation and action spaces (scalingWrapperEnv.jl:22): of the built-in envs that is Pendulum
     DRIL_REQUIRE(e->d.kind == DRIL_ENV_PENDULUM || e->d.kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS,
                  "ScalingWrapperEnv: Box observation and action spaces required (pendulum, mountaincar_continuous)");
-    // observed parameters (dril_env_set_observe_params) pass through raw: the bounds cover the base observation only
+    // observed parameters (dril_env_set_observe_params) pass through raw: the bounds cover the base observation only (with
+    // masked velocities (dril_env_set_obs_history) too: the kept components use their own bounds)
     const int D0 = env_base_obs_dim(e->d.kind);
     DRIL_REQUIRE(D0 <= 4 && e->d.act_dim == 1, "ScalingWrapperEnv: obs_dim <= 4, act_dim == 1");
     for (int j = 0; j < D0; ++j) {
@@ -1595,7 +1644,7 @@ extern "C" int32_t dril_env_set_scaling(dril_env* e, int32_t on, const float* ob
     e->d.sc_act_f = 2.0f / (act_high[0] - act_low[0]);                            // :42-44
     e->d.sc_act_o = act_low[0];
     e->d.scaling = 1;
-    return DRIL_OK;
+    return env_hist_refill(e);
 }
 extern "C" int32_t dril_env_get_original(dril_env* e, float* obs_out, float* rewards_out) {
     DRIL_REQUIRE(e, "NULL argument");

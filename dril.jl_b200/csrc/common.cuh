@@ -102,6 +102,11 @@ struct EnvDev {
     float* pval;                // [DRIL_ENV_MAX_PARAMS][n] values of the running episode
     float* plo;                 // [DRIL_ENV_MAX_PARAMS][n] ranges
     float* phi;
+    // observation history (env.cuh, ENV_KS_HISTORY); hist_len 1 and hist null unless dril_env_set_obs_history turned it on.
+    // frame_dim < the kind's base width means velocity-free frames.  (16 bytes: the offsets behind EnvDev in RolloutArgs keep
+    // their 16-byte alignment, and with it the existing kernels' code.)
+    int hist_len, frame_dim;
+    float* hist;                // [(hist_len - 1) * frame_dim][n] the older frames of the stack, oldest first
 };
 
 struct BufDev {

@@ -19,12 +19,15 @@
 #define ENV_KS_ALL (ENV_KS_CLASSIC | (1u << DRIL_ENV_MOUNTAINCAR) | (1u << DRIL_ENV_MOUNTAINCAR_CONTINUOUS) | (1u << DRIL_ENV_ACROBOT))
 
 // kind-set bits beyond the kinds: ENV_KS_PARAMS = per-env physical parameters (below); ENV_KS_OBS_PARAMS (only together with
-// ENV_KS_PARAMS) = observations [base observation | the running episode's parameter values in table order]
+// ENV_KS_PARAMS) = observations [base observation | the running episode's parameter values in table order]; ENV_KS_HISTORY
+// (only together with ENV_KS_PARAMS) = observations [f_{t-k+1} | ... | f_t], the last k frames (env_frame), k = hist_len
 #define ENV_KS_PARAMS (1u << 16)
 #define ENV_KS_OBS_PARAMS (1u << 17)
+#define ENV_KS_HISTORY (1u << 18)
 
 __host__ __device__ constexpr bool env_in(unsigned ks, int kind) { return (ks >> kind) & 1u; }
 __host__ __device__ constexpr bool env_obs_params(unsigned ks) { return (ks & ENV_KS_OBS_PARAMS) != 0; }
+__host__ __device__ constexpr bool env_history(unsigned ks) { return (ks & ENV_KS_HISTORY) != 0; }
 __host__ __device__ constexpr int env_n_params(int kind) {
     return kind == DRIL_ENV_CARTPOLE || kind == DRIL_ENV_ACROBOT ? 6
          : kind == DRIL_ENV_PENDULUM ? 4
@@ -35,9 +38,17 @@ __host__ __device__ constexpr int env_base_obs_dim(int kind) {
     return kind == DRIL_ENV_CARTPOLE ? 4 : kind == DRIL_ENV_PENDULUM ? 3 : kind == DRIL_ENV_ACROBOT ? 6 : 2;
 }
 // blocks of four observation components a kernel built for the kinds `ks` handles (Acrobot: 6 components; with
-// ENV_KS_OBS_PARAMS both parametrised kind sets hold a kind of base + parameter width > 8: CartPole 10, Acrobot 12)
+// ENV_KS_OBS_PARAMS both parametrised kind sets hold a kind of base + parameter width > 8: CartPole 10, Acrobot 12; with
+// ENV_KS_HISTORY the blocks of one frame, at most 6 components, which the kernels assemble into the k-frame stack)
 __host__ __device__ constexpr int env_obs_blocks(unsigned ks) {
-    return env_obs_params(ks) ? 3 : (env_in(ks, DRIL_ENV_ACROBOT) ? 2 : 1);
+    return env_obs_params(ks) ? 3 : (env_in(ks, DRIL_ENV_ACROBOT) || env_history(ks) ? 2 : 1);
+}
+// components of one frame of an env with an observation history: the base observation, or with mask_velocities its
+// non-velocity components (CartPole (x, theta), Pendulum (cos, sin), MountainCar(Continuous) (position), Acrobot
+// (cos th1, sin th1, cos th2, sin th2))
+__host__ __device__ constexpr int env_frame_dim(int kind, bool mask_velocities) {
+    return !mask_velocities ? env_base_obs_dim(kind)
+         : kind == DRIL_ENV_ACROBOT ? 4 : kind == DRIL_ENV_CARTPOLE || kind == DRIL_ENV_PENDULUM ? 2 : 1;
 }
 // the kind set whose instantiation serves env kind `kind`
 __host__ __device__ constexpr unsigned env_kind_set(int kind) { return env_in(ENV_KS_CLASSIC, kind) ? ENV_KS_CLASSIC : ENV_KS_ALL; }
@@ -106,6 +117,48 @@ __device__ __forceinline__ void env_obs_block(const EnvDev& env, const float* st
             if (j < env.obs_dim) o[j] = __fsub_rn(__fmul_rn(__fsub_rn(o[j], env.sc_obs_o[j]), env.sc_obs_f[j]), 1.0f);
     }
 }
+// ---------------------------------------------------------------------------------------
+// Observation history (ENV_KS_HISTORY).  The observation of env n at step t is the stack [f_{t-k+1} | ... | f_t], oldest
+// first; a frame is env_frame of the state.  The k-1 older frames live in a history store of H = (k-1) * F rows (component j
+// of the stack in row j, one column per env): env.hist in global memory, or a shared-memory copy in the fast kernel.  It
+// moves once per env step (env_hist_push, before the reset) and is refilled with the new frame after every reset
+// (env_hist_fill); every observation only reads it.
+// ---------------------------------------------------------------------------------------
+#define ENV_MAX_FRAME 6
+// f[0 .. frame_dim-1]: the base observation as the wrappers below Normalize see it (raw, or mapped by Scaling), without its
+// velocity components when frame_dim says so (env_frame_dim); the components beyond frame_dim are unspecified
+template <unsigned KS>
+__device__ __forceinline__ void env_frame(const EnvDev& env, const float* st, float* f) {
+    env_raw_obs_block<KS>(env.kind, st, 0, f);
+    if (env.scaling) {
+        const int D0 = env_base_obs_dim(env.kind);
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+            if (j < D0) f[j] = __fsub_rn(__fmul_rn(__fsub_rn(f[j], env.sc_obs_o[j]), env.sc_obs_f[j]), 1.0f);
+    }
+    if (env_in(KS, DRIL_ENV_ACROBOT) && env.kind == DRIL_ENV_ACROBOT) {
+        f[4] = st[2]; f[5] = st[3];
+    } else if (env.kind == DRIL_ENV_CARTPOLE && env.frame_dim < 4) {
+        f[1] = f[2];   // (x, theta)
+    }
+}
+// stack component rows [0, H) of one env in a history store with row stride `stride`: f (the frame an action was chosen on)
+// enters as the newest of the older frames, the oldest leaves
+__device__ __forceinline__ void env_hist_push(float* h, size_t stride, int H, int F, const float* f) {
+    for (int j = 0; j + F < H; ++j) h[(size_t)j * stride] = h[(size_t)(j + F) * stride];
+#pragma unroll
+    for (int j = 0; j < ENV_MAX_FRAME; ++j)
+        if (j < F && H > 0) h[(size_t)(H - F + j) * stride] = f[j];
+}
+// ... every older frame = f (reset padding: before an episode's first observation the frames are that observation)
+__device__ __forceinline__ void env_hist_fill(float* h, size_t stride, int H, int F, const float* f) {
+    for (int j0 = 0; j0 < H; j0 += F) {
+#pragma unroll
+        for (int j = 0; j < ENV_MAX_FRAME; ++j)
+            if (j < F) h[(size_t)(j0 + j) * stride] = f[j];
+    }
+}
+
 // ScalingWrapperEnv.act! (scalingWrapperEnv.jl:77-80,112-115): `(a + 1) / scale + offset` before the wrapped env's act!
 __device__ __forceinline__ float env_unscale_action(const EnvDev& env, float a) {
     return env.scaling ? __fadd_rn(__fdiv_rn(__fadd_rn(a, 1.0f), env.sc_act_f), env.sc_act_o) : a;
@@ -280,6 +333,9 @@ __host__ __device__ constexpr unsigned env_param_kind_set(int kind) {
 }
 // ... and the one that also observes the parameters
 __host__ __device__ constexpr unsigned env_obs_param_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_OBS_PARAMS; }
+// ... and the one with an observation history (an env with history always runs with parameters: lo = hi = the defaults
+// without ranges)
+__host__ __device__ constexpr unsigned env_hist_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_HISTORY; }
 
 // the values of env n's episode `episode`: lo + (hi - lo) * u, u from Philox (gid, episode, k / 4, DRIL_TAG_ENV_PARAMS) word
 // k % 4; written to par and env.pval

@@ -309,6 +309,22 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
 #pragma unroll
                 for (int j = 0; j < 4; ++j) sRaw[(size_t)(4 * b + j) * ld + e] = (4 * b + j < D) ? o[j] : 0.f;
             }
+        } else if (env_history(KS)) {   // [older frames from the history store | the frame of the current state]
+            if (tid < M4) {
+                const int F = env.frame_dim, H = D - F;
+                const bool v = tid < nvalid;
+                float f[ENV_MAX_FRAME] = {};
+                if (v) {
+                    float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+                    for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * N + n0 + tid];
+                    env_frame<KS>(env, st, f);
+                }
+                for (int j = 0; j < H; ++j) sRaw[(size_t)j * ld + tid] = v ? env.hist[(size_t)j * N + n0 + tid] : 0.f;
+#pragma unroll
+                for (int j = 0; j < ENV_MAX_FRAME; ++j) if (j < F) sRaw[(size_t)(H + j) * ld + tid] = f[j];
+                for (int j = D; j < Dp; ++j) sRaw[(size_t)j * ld + tid] = 0.f;
+            }
         } else {
             if (tid < M4) {
 #pragma unroll
@@ -452,6 +468,11 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                 uint32_t life = 0;
                 float par[DRIL_ENV_MAX_PARAMS];
                 if (env_has_params(KS)) env_load_params(env, n, par);
+                if (env_history(KS)) {                          // the frame the action was chosen on enters the history
+                    float f[ENV_MAX_FRAME];
+                    env_frame<KS>(env, st, f);
+                    env_hist_push(env.hist + n, (size_t)N, D - env.frame_dim, env.frame_dim, f);
+                }
                 r = env_step<KS>(env, st, n, a_disc, sEnvAct + tid, &life, &term, par);
                 steps += 1;
                 const bool trunc = steps >= env.max_steps;
@@ -481,6 +502,13 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
 #pragma unroll
                             for (int j = 0; j < 4; ++j) if (4 * b + j < D) env.tobs[(size_t)n * D + 4 * b + j] = o[j];
                         }
+                    } else if (env_history(KS)) {             // the stack that ends in the ended episode's final frame
+                        const int F = env.frame_dim, H = D - F;
+                        float f[ENV_MAX_FRAME];
+                        env_frame<KS>(env, st, f);
+                        for (int j = 0; j < H; ++j) env.tobs[(size_t)n * D + j] = env.hist[(size_t)j * N + n];
+#pragma unroll
+                        for (int j = 0; j < ENV_MAX_FRAME; ++j) if (j < F) env.tobs[(size_t)n * D + H + j] = f[j];
                     } else {
 #pragma unroll
                         for (int b = 0; b < env_obs_blocks(KS); ++b) {
@@ -495,6 +523,11 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                     uint32_t ep = env.episode[n];
                     env_reset_state<KS>(env.kind, gid, ep, env.seed, st);
                     if (env_has_params(KS)) env_draw_params(env, n, gid, ep, par);
+                    if (env_history(KS)) {
+                        float f[ENV_MAX_FRAME];
+                        env_frame<KS>(env, st, f);
+                        env_hist_fill(env.hist + n, (size_t)N, D - env.frame_dim, env.frame_dim, f);
+                    }
                     env.episode[n] = ep + 1;
                     steps = 0;
                 }
@@ -620,10 +653,12 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_kernel(const __grid_cons
 
 struct RolloutFastSmem {
     int ld, slices;
-    size_t w, x, acta, actc, part, stat, total;   // float offsets; total in bytes
+    size_t w, x, acta, actc, part, stat, hist, total;   // float offsets; total in bytes
 };
 
-__host__ __device__ inline RolloutFastSmem rollout_fast_smem_layout(const PolicyDesc& pd, int M4, int threads, bool weights_smem) {
+// hist_rows: rows of the tile's observation-history store (ENV_KS_HISTORY), 0 otherwise
+__host__ __device__ inline RolloutFastSmem rollout_fast_smem_layout(const PolicyDesc& pd, int M4, int threads, bool weights_smem,
+                                                                   int hist_rows = 0) {
     RolloutFastSmem s;
     s.ld = M4 + 4;
     s.slices = threads / M4;
@@ -634,6 +669,7 @@ __host__ __device__ inline RolloutFastSmem rollout_fast_smem_layout(const Policy
     s.actc = o; o += (size_t)2 * pd.max_np * s.ld;
     s.part = o; o += (size_t)s.slices * RF_MAX_OUT * s.ld;
     s.stat = o; o += (size_t)2 * pd.obs_dim_p + 4;
+    s.hist = o; o += (size_t)hist_rows * s.ld;
     s.total = ((o + 3) & ~(size_t)3) * sizeof(float);
     return s;
 }
@@ -648,7 +684,9 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
     const PolicyDesc& pd = a.pd;
     const int D = env.obs_dim, Dp = pd.obs_dim_p, M4 = a.M4, NL = pd.n_layers;
     const long long N = env.n_envs;
-    const RolloutFastSmem L = rollout_fast_smem_layout(pd, M4, blockDim.x, WS);
+    // ENV_KS_HISTORY: the tile's history store in shared memory for the whole rollout, rows [0, H), written back at the end
+    const int F = env_history(KS) ? env.frame_dim : 0, H = env_history(KS) ? D - F : 0;
+    const RolloutFastSmem L = rollout_fast_smem_layout(pd, M4, blockDim.x, WS, H);
     const int ld = L.ld, S = L.slices;
     float* sX = smem + L.x;
     float* sActA = smem + L.acta;
@@ -656,6 +694,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
     float* sPart = smem + L.part;
     float* sMean = smem + L.stat;
     float* sVar = sMean + Dp;
+    float* sHist = smem + L.hist;
     const int tid = threadIdx.x;
     const float* __restrict__ Wbase = WS ? smem : a.pack;
     if (WS) {
@@ -688,6 +727,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         episode = env.episode[n];
         if (env_has_params(KS)) env_load_params(env, n, eparam);
         if (env.monitor) { ep_ret = env.ep_ret[n]; ep_len = env.ep_len[n]; }
+        for (int j = 0; j < H; ++j) sHist[(size_t)j * ld + tid] = env.hist[(size_t)j * N + n];
     }
     // output-layer split: thread (e = tid % M4, ks = tid / M4) covers k in [ks*Kc, ks*Kc + Kc)
     const LayerDesc& Lao = pd.L[0][NL - 1];
@@ -700,6 +740,30 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
 
     // write the (normalised) observation of the register state into sX and optionally the buffer
     auto stage_obs = [&](float* obs_row /* nullable global [D] */) {
+        if (env_history(KS)) {   // older frames straight from sHist, the newest from the registers: no D-wide register array
+            if (tid < M4) {
+                float f[ENV_MAX_FRAME] = {};
+                if (mine) env_frame<KS>(env, st, f);
+                for (int j = 0; j < H; ++j) {
+                    float x = mine ? sHist[(size_t)j * ld + tid] : 0.f;
+                    if (mine && norm_obs) x = normalize_obs_val(x, sMean[j], sVar[j], env.eps, env.clip_obs);
+                    if (obs_row) obs_row[j] = x;
+                    sX[(size_t)j * ld + tid] = x;
+                }
+#pragma unroll
+                for (int j = 0; j < ENV_MAX_FRAME; ++j) {
+                    if (j < F) {
+                        float x = f[j];
+                        if (mine && norm_obs) x = normalize_obs_val(x, sMean[H + j], sVar[H + j], env.eps, env.clip_obs);
+                        if (obs_row) obs_row[H + j] = x;
+                        sX[(size_t)(H + j) * ld + tid] = x;
+                    }
+                }
+                for (int j = D; j < Dp; ++j) sX[(size_t)j * ld + tid] = 0.f;
+            }
+            __syncthreads();
+            return;
+        }
         if (tid < M4) {
             float o[OW] = {};
             if (mine) {
@@ -853,6 +917,11 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             bool term = false;
             float r;
             uint32_t life = 0;
+            if (env_history(KS)) {                               // the frame the action was chosen on enters the history
+                float f[ENV_MAX_FRAME];
+                env_frame<KS>(env, st, f);
+                env_hist_push(sHist + tid, (size_t)ld, H, F, f);
+            }
             r = env_step<KS & ~(1u << DRIL_ENV_SYNTHETIC)>(env, st, n, a_disc, &a_cont, &life, &term, eparam);   // (no synthetic env here)
             steps += 1;
             const bool trunc = steps >= env.max_steps;
@@ -877,7 +946,24 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
                     ep_ret = 0.f; ep_len = 0;
                 }
             }
-            if (trunc) {
+            if (trunc && env_history(KS)) {   // the stack ending in the ended episode's final frame, staged like ENV_KS_OBS_PARAMS
+                trunc_i = 1;
+                float f[ENV_MAX_FRAME];
+                env_frame<KS>(env, st, f);
+                for (int j = 0; j < H; ++j) {
+                    float x = sHist[(size_t)j * ld + tid];
+                    if (norm_obs) x = normalize_obs_val(x, sMean[j], sVar[j], env.eps, env.clip_obs);
+                    sX[(size_t)j * ld + tid] = x;
+                }
+#pragma unroll
+                for (int j = 0; j < ENV_MAX_FRAME; ++j) {
+                    if (j < F) {
+                        float x = f[j];
+                        if (norm_obs) x = normalize_obs_val(x, sMean[H + j], sVar[H + j], env.eps, env.clip_obs);
+                        sX[(size_t)(H + j) * ld + tid] = x;
+                    }
+                }
+            } else if (trunc) {
                 trunc_i = 1;
 #pragma unroll
                 for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, tobs + 4 * b, eparam);   // before the redraw below
@@ -893,6 +979,11 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             if (done) {
                 env_reset_state<KS>(env.kind, gid, episode, env.seed, st);
                 if (env_has_params(KS)) env_draw_params(env, n, gid, episode, eparam);
+                if (env_history(KS)) {
+                    float f[ENV_MAX_FRAME];
+                    env_frame<KS>(env, st, f);
+                    env_hist_fill(sHist + tid, (size_t)ld, H, F, f);
+                }
                 episode += 1;
                 steps = 0;
                 if (env.normalize) env.ret[n] = 0.f;             // normalizeWrapperEnv.jl:153-156
@@ -900,7 +991,9 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         }
         // V(terminal_obs) for truncated envs (trajectory.jl:57-61): rare, CTA-uniform branch
         if (__syncthreads_or(trunc_i)) {
-            if (tid < M4) {
+            if (tid < M4 && env_history(KS)) {
+                if (!trunc_i) for (int j = 0; j < Dp; ++j) sX[(size_t)j * ld + tid] = 0.f;
+            } else if (tid < M4) {
 #pragma unroll
                 for (int j = 0; j < OW; ++j)
                     if (j < Dp && !(env_obs_params(KS) && trunc_i)) sX[(size_t)j * ld + tid] = trunc_i ? tobs[j] : 0.f;
@@ -925,7 +1018,21 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         env.steps[n] = steps;
         env.episode[n] = episode;
         if (env.monitor) { env.ep_ret[n] = ep_ret; env.ep_len[n] = ep_len; }
+        for (int j = 0; j < H; ++j) env.hist[(size_t)j * N + n] = sHist[(size_t)j * ld + tid];
     }
+}
+
+// the observation history of every env restarted from its current state (ENV_KS_HISTORY): reset, set_state, Scaling turned
+// on, or the history turned on
+__global__ void env_hist_fill_kernel(EnvDev env) {
+    long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= env.n_envs) return;
+    float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * env.n_envs + n];
+    float f[ENV_MAX_FRAME];
+    env_frame<ENV_KS_ALL>(env, st, f);
+    env_hist_fill(env.hist + n, (size_t)env.n_envs, (env.hist_len - 1) * env.frame_dim, env.frame_dim, f);
 }
 
 // ---------------------------------------------------------------------------------------

@@ -262,6 +262,32 @@ int32_t dril_env_get_params(dril_env* env, int32_t n_params, float* values);
 int32_t dril_env_set_observe_params(dril_env* env, int32_t on);
 int32_t dril_env_obs_dim(dril_env* env, int32_t* obs_dim);
 
+/* Observation history (frame stacking) and velocity-free observations.  history_len = k in [1, DRIL_ENV_MAX_HISTORY]: the
+ * observation of env n at step t is
+ *   [f_{t-k+1} | ... | f_{t-1} | f_t],  oldest first,  obs_dim = F * k,
+ * f_j = the frame at step j: the base observation as the wrappers below NormalizeWrapperEnv see it (raw, or mapped to
+ * [-1, 1] by ScalingWrapperEnv).  mask_velocities = 1 keeps only the non-velocity components of every frame:
+ *   cartpole (x, theta), pendulum (cos theta, sin theta), mountaincar(_continuous) (position),
+ *   acrobot (cos th1, sin th1, cos th2, sin th2);
+ * F = 4 / 2, 3 / 2, 2 / 1, 2 / 1, 6 / 4 (full / masked).  Scaling maps the kept components with their own bounds.
+ *   - Frames from before the episode's first observation are that observation (padding "reset"): after a reset all k frames
+ *     are the reset frame.
+ *   - On act!, the frame the action was chosen on enters the history, then the env steps.  A truncated step's terminal
+ *     observation (and V(terminal_obs)) is the stack ending in the ended episode's final frame; after the auto-reset the
+ *     stack is k copies of the reset frame.  observe() never moves the history.
+ *   - dril_env_reset, dril_env_set_state, dril_env_set_scaling and dril_evaluate's initial reset restart every env's history
+ *     from its current frame.  Chunked collection, compat act! and successive rollouts continue it.
+ *   - NormalizeWrapperEnv normalises all F * k columns; Monitor is unaffected; parameter ranges work as without history.
+ *   - No RNG is involved: observations do not depend on gid_offset sharding.
+ * (k = 1, mask_velocities = 0) is the plain env.  Otherwise the env runs the parametrised kernels (lo = hi = the defaults
+ * without ranges; dril_env_set_params(lo = NULL) returns to that), so CartPole leaves the tensor-core rollout.
+ * Allowed only before the env's first observation, else DRIL_ERR_INVALID, as is k outside [1, DRIL_ENV_MAX_HISTORY].  The
+ * synthetic env, and an env with observe_params (in either call order): DRIL_ERR_UNSUPPORTED.  A policy or buffer built for
+ * another width fails the obs_dim check of the rollout.  A policy deployed outside this library expects the stacked
+ * observation. */
+#define DRIL_ENV_MAX_HISTORY 4
+int32_t dril_env_set_obs_history(dril_env* env, int32_t history_len, int32_t mask_velocities);
+
 /* ---- actor-critic layer + optimiser state: replaces Discrete/ContinuousActorCriticLayer
  *      (layers/) and the Lux TrainState held by Agent (agents/agent_types.jl) ------------ */
 int32_t dril_policy_create(dril_ctx* ctx, int32_t obs_dim, int32_t n_hidden, const int32_t* hidden_dims,

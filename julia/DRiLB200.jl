@@ -78,14 +78,22 @@ const ENV_PARAMS = Dict(
     :acrobot => (:link_length_1 => 1.0, :link_mass_1 => 1.0, :link_mass_2 => 1.0, :link_com_pos_1 => 0.5, :link_com_pos_2 => 0.5, :link_moi => 1.0),
 )
 
+# the non-velocity components (1-based) of each kind's observation: the frame of an env with mask_velocities = true
+const VELOCITY_FREE = Dict(:cartpole => [1, 3], :pendulum => [1, 2], :mountaincar => [1], :mountaincar_continuous => [1],
+                           :acrobot => [1, 2, 3, 4])
+
 """
-    CudaBatchedEnv(kind, n_envs; max_steps, act_start, monitor_window, normalize, env_params, observe_params)
+    CudaBatchedEnv(kind, n_envs; max_steps, act_start, monitor_window, normalize, env_params, observe_params, history_len,
+                   mask_velocities)
 
 Device-resident replacement of `NormalizeWrapperEnv(MonitorWrapperEnv(MultiThreadedParallelEnv(envs)))`
 for `kind in (:cartpole, :pendulum, :synthetic, :mountaincar, :mountaincar_continuous, :acrobot)`.
 `env_params = Dict(:length => (0.25, 1.0), ...)`: per-env physical parameters, see `set_env_params!`.
 `observe_params = true`: every observation is `[base observation | the running episode's parameter values]` in the order of
 `ENV_PARAMS[kind]`, raw (Scaling maps the base components only); `observation_space` is widened by `[0, Inf)` per parameter.
+`history_len = k` (1 to 4): every observation is the last k frames `[f_{t-k+1} | ... | f_t]`, oldest first;
+`mask_velocities = true` keeps only each frame's non-velocity components (`VELOCITY_FREE[kind]`); `observation_space` is the
+(scaled) bounds of the kept components tiled k times.  `reset!` restarts the history from the current frame.
 """
 mutable struct CudaBatchedEnv <: AbstractParallelEnv
     ctx::Context
@@ -102,7 +110,7 @@ end
 
 function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_steps = 0, obs_dim = 0, act_start = 1,
         monitor_window = 0, normalize::Union{Nothing, NormCfg} = nothing, gid_offset = 0, scaling::Bool = false,
-        env_params = nothing, observe_params::Bool = false)
+        env_params = nothing, observe_params::Bool = false, history_len::Integer = 1, mask_velocities::Bool = false)
     obs_space, act_space = if kind == :cartpole
         hi = Float32[4.8, Inf32, 0.41887903, Inf32]
         Box(-hi, hi), Discrete(2, act_start)
@@ -134,9 +142,16 @@ function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_
         obs_space = Box(-ones(Float32, size(obs_space.low)), ones(Float32, size(obs_space.high)))
         act_space = Box(-ones(Float32, size(act_space.low)), ones(Float32, size(act_space.high)))
     end
+    if history_len != 1 || mask_velocities
+        check(ccall((:dril_env_set_obs_history, LIB), Int32, (Ptr{Cvoid}, Int32, Int32), out[], history_len, mask_velocities))
+        keep = mask_velocities ? VELOCITY_FREE[kind] : collect(1:length(obs_space.low))
+        obs_space = Box(repeat(vec(obs_space.low)[keep], history_len), repeat(vec(obs_space.high)[keep], history_len))
+    end
     if observe_params
         P = length(ENV_PARAMS[kind])
         obs_space = Box(vcat(vec(obs_space.low), zeros(Float32, P)), vcat(vec(obs_space.high), fill(Inf32, P)))
+    end
+    if observe_params || history_len != 1 || mask_velocities
         d = Ref{Int32}(0)
         check(ccall((:dril_env_obs_dim, LIB), Int32, (Ptr{Cvoid}, Ref{Int32}), out[], d))
         d[] == size(obs_space)[1] || error("observation width $(d[]) != $(size(obs_space)[1])")
