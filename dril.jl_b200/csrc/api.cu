@@ -8,6 +8,8 @@
 #include <string.h>
 
 #include <algorithm>
+#include <type_traits>
+#include <utility>
 
 #include "common.cuh"
 #include "gae.cuh"
@@ -98,42 +100,48 @@ static bool tc_eligible(const PolicyDesc& pd) {
     return true;
 }
 
-// rollout kernels by the env kind they step: CartPole, Pendulum and the synthetic env run the instantiations built for those
-// kinds alone (env.cuh), every other kind the one built for all kinds; an env with per-env parameters (dril_env_set_params)
-// runs the ENV_KS_PARAMS instantiation of its kind set, one that observes its parameters (dril_env_set_observe_params) the
-// ENV_KS_OBS_PARAMS instantiation, and one with an observation history (dril_env_set_obs_history) the ENV_KS_HISTORY one
-#define KS_CP_ ENV_KS_CLASSIC
-#define KS_ALL_ ENV_KS_ALL
-#define KS_CP_P_ env_param_kind_set(DRIL_ENV_CARTPOLE)
-#define KS_ALL_P_ env_param_kind_set(DRIL_ENV_ACROBOT)
-#define KS_CP_OP_ env_obs_param_kind_set(DRIL_ENV_CARTPOLE)
-#define KS_ALL_OP_ env_obs_param_kind_set(DRIL_ENV_ACROBOT)
-#define KS_CP_H_ env_hist_kind_set(DRIL_ENV_CARTPOLE)
-#define KS_ALL_H_ env_hist_kind_set(DRIL_ENV_ACROBOT)
-#define DRIL_KS_PICK(K_, kind, params, obsp, hist)                                                                             \
-    (env_kind_set(kind) == ENV_KS_CLASSIC ? ((hist) ? K_(KS_CP_H_) : (obsp) ? K_(KS_CP_OP_) : (params) ? K_(KS_CP_P_) : K_(KS_CP_)) \
-                                          : ((hist) ? K_(KS_ALL_H_) : (obsp) ? K_(KS_ALL_OP_) : (params) ? K_(KS_ALL_P_) : K_(KS_ALL_)))
-static void* rollout_fn(bool ws, int kind, bool params, bool obsp, bool hist) {
-#define K_(ks) (ws ? (void*)rollout_kernel<true, ks> : (void*)rollout_kernel<false, ks>)
-    return DRIL_KS_PICK(K_, kind, params, obsp, hist);
-#undef K_
+// the kind sets the rollout kernels are instantiated for (env.cuh): CartPole, Pendulum and the synthetic env run the ones built
+// for those kinds alone, every other kind the ones built for all kinds, each plain, with per-env parameters (dril_env_set_params),
+// observing its parameters (dril_env_set_observe_params) or with an observation history (dril_env_set_obs_history)
+static constexpr unsigned k_kind_sets[] = {
+    ENV_KS_CLASSIC, env_param_kind_set(DRIL_ENV_CARTPOLE), env_obs_param_kind_set(DRIL_ENV_CARTPOLE), env_hist_kind_set(DRIL_ENV_CARTPOLE),
+    ENV_KS_ALL, env_param_kind_set(DRIL_ENV_ACROBOT), env_obs_param_kind_set(DRIL_ENV_ACROBOT), env_hist_kind_set(DRIL_ENV_ACROBOT)};
+// f(std::integral_constant<unsigned, KS>) for the entry KS == ks of k_kind_sets (nullptr for a kind set not in the list)
+template <class F, size_t... I>
+static void* ks_pick(unsigned ks, F f, std::index_sequence<I...>) {
+    void* fn = nullptr;
+    ((ks == k_kind_sets[I] ? (void)(fn = f(std::integral_constant<unsigned, k_kind_sets[I]>{})) : (void)0), ...);
+    return fn;
 }
-static void* rollout_fast_fn(bool ws, int kind, bool params, bool obsp, bool hist) {
-#define K_(ks) (ws ? (void*)rollout_fast_kernel<true, ks> : (void*)rollout_fast_kernel<false, ks>)
-    return DRIL_KS_PICK(K_, kind, params, obsp, hist);
-#undef K_
+template <class F>
+static void* ks_pick(unsigned ks, F f) { return ks_pick(ks, f, std::make_index_sequence<sizeof(k_kind_sets) / sizeof(unsigned)>{}); }
+static void* rollout_fn(bool ws, unsigned ks) {
+    return ks_pick(ks, [ws](auto k) {
+        constexpr unsigned KS = decltype(k)::value;
+        return ws ? (void*)rollout_kernel<true, KS> : (void*)rollout_kernel<false, KS>;
+    });
 }
-// tcgen05-actor rollout by hidden-layer count, env kind and action count (2 or 4 staged output columns, gtc_nout)
-static void* rollout_gtc_fn(int L, int kind, int act_n, bool params, bool obsp, bool hist) {
+static void* rollout_fast_fn(bool ws, unsigned ks) {
+    return ks_pick(ks, [ws](auto k) {
+        constexpr unsigned KS = decltype(k)::value;
+        return ws ? (void*)rollout_fast_kernel<true, KS> : (void*)rollout_fast_kernel<false, KS>;
+    });
+}
+// tcgen05-actor rollout by hidden-layer count, kind set and action count (2 or 4 staged output columns, gtc_nout); the 4-column
+// variant exists for the all-kinds sets only, which also serve the other kinds
+static void* rollout_gtc_fn(int L, unsigned ks, int act_n) {
     if (act_n > 2) {
-        if (hist) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_H_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_H_, 4>;
-        if (obsp) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_OP_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_OP_, 4>;
-        if (params) return L == 2 ? (void*)rollout_gtc_kernel<2, KS_ALL_P_, 4> : (void*)rollout_gtc_kernel<3, KS_ALL_P_, 4>;
-        return L == 2 ? (void*)rollout_gtc_kernel<2, ENV_KS_ALL, 4> : (void*)rollout_gtc_kernel<3, ENV_KS_ALL, 4>;
+        ks |= env_has_params(ks) ? env_param_kind_set(DRIL_ENV_ACROBOT) : ENV_KS_ALL;
+        return ks_pick(ks, [L](auto k) -> void* {
+            constexpr unsigned KS = decltype(k)::value;
+            if constexpr (env_in(KS, DRIL_ENV_ACROBOT)) return L == 2 ? (void*)rollout_gtc_kernel<2, KS, 4> : (void*)rollout_gtc_kernel<3, KS, 4>;
+            else return nullptr;
+        });
     }
-#define K_(ks) (L == 2 ? (void*)rollout_gtc_kernel<2, ks, 2> : (void*)rollout_gtc_kernel<3, ks, 2>)
-    return DRIL_KS_PICK(K_, kind, params, obsp, hist);
-#undef K_
+    return ks_pick(ks, [L](auto k) {
+        constexpr unsigned KS = decltype(k)::value;
+        return L == 2 ? (void*)rollout_gtc_kernel<2, KS, 2> : (void*)rollout_gtc_kernel<3, KS, 2>;
+    });
 }
 
 extern "C" int32_t dril_device_count(int32_t* count) {
@@ -249,11 +257,16 @@ struct dril_env {
     double* xr = nullptr;
     float* norm_snap = nullptr;
     long long* norm_snap_cnt = nullptr;
-    bool observe_params = false;     // dril_env_set_observe_params: the ENV_KS_OBS_PARAMS instantiations, obs_dim = D + P
-    bool default_params = false;     // parameters held at lo = hi = the defaults only because observe_params or history is on
+    unsigned obs_ks = 0;             // ENV_KS_OBS_PARAMS (dril_env_set_observe_params), ENV_KS_HISTORY (dril_env_set_obs_history:
+                                     // k > 1 or velocities masked) or 0: the observation layout, as a kind-set bit
+    bool default_params = false;     // parameters held at lo = hi = the defaults only because obs_ks is set
     bool observed = false;           // an observation was made (observe, step, rollout, evaluate): the width is fixed
-    bool history = false;            // dril_env_set_obs_history (k > 1 or velocities masked): the ENV_KS_HISTORY instantiations
 };
+// the kind set whose kernels run env e (one of k_kind_sets)
+static unsigned env_ks(const dril_env* e) {
+    const int kind = e->d.kind;
+    return e->obs_ks ? env_param_kind_set(kind) | e->obs_ks : e->d.has_params ? env_param_kind_set(kind) : env_kind_set(kind);
+}
 
 struct dril_policy {
     dril_ctx* ctx;
@@ -378,12 +391,11 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
     c->seed = seed;
     c->sm_count = prop.multiProcessorCount;
     DRIL_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-    for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
-        for (int ws = 0; ws < 2; ++ws)
-            for (int params = 0; params < 4; ++params) {   // 2: observed parameters, 3: observation history
-                DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, kind, params > 0, params == 2, params == 3), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-                DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, kind, params > 0, params == 2, params == 3), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
-            }
+    for (unsigned ks : k_kind_sets)
+        for (int ws = 0; ws < 2; ++ws) {
+            DRIL_CUDA(cudaFuncSetAttribute(rollout_fn(ws, ks), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+            DRIL_CUDA(cudaFuncSetAttribute(rollout_fast_fn(ws, ks), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
+        }
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
     DRIL_CUDA(cudaFuncSetAttribute(policy_apply_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
     DRIL_CUDA(cudaFuncSetAttribute(ppo_loss_grad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX));
@@ -400,10 +412,9 @@ extern "C" int32_t dril_ctx_create(int32_t device, uint64_t seed, dril_ctx** out
                              (const void*)ppo_loss_grad_ftg_kernel<3, 0, 3>, (const void*)ppo_loss_grad_ftg_kernel<3, 0, 4>};
         for (const void* fn : fns) DRIL_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));   // 1 KB of static shared memory
         for (int L = 2; L <= 3; ++L)
-            for (int kind : {DRIL_ENV_CARTPOLE, DRIL_ENV_ACROBOT})
+            for (unsigned ks : k_kind_sets)
                 for (int an = 2; an <= 4; an += 2)
-                    for (int params = 0; params < 4; ++params)
-                        DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, kind, an, params > 0, params == 2, params == 3), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
+                    DRIL_CUDA(cudaFuncSetAttribute(rollout_gtc_fn(L, ks, an), cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
         DRIL_CUDA(cudaFuncSetAttribute(critic_values_ftg_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DRIL_SMEM_MAX - 2048));
     }
@@ -1141,24 +1152,13 @@ extern "C" int32_t dril_env_reset(dril_env* e) {
     {
         Span sp(c, DRIL_K_ENV);
         const unsigned grid = (unsigned)((e->d.n_envs + 255) / 256);
-        if (e->d.has_params) env_reset_kernel<ENV_KS_ALL | ENV_KS_PARAMS><<<grid, 256, 0, c->stream>>>(e->d);
+        if (env_has_params(env_ks(e))) env_reset_kernel<ENV_KS_ALL | ENV_KS_PARAMS><<<grid, 256, 0, c->stream>>>(e->d);
         else env_reset_kernel<ENV_KS_ALL><<<grid, 256, 0, c->stream>>>(e->d);
         DRIL_CUDA(cudaGetLastError());
     }
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
     return env_hist_refill(e);
 }
-// per-env physical parameters (dril_b200.h): the defaults of the table, and whether a value must be > 0 (1) or >= 0 (0)
-static const float k_env_param_default[6][DRIL_ENV_MAX_PARAMS] = {
-    {9.8f, 1.0f, 0.1f, 0.5f, 10.0f, 0.02f},          // cartpole: gravity masscart masspole length force_mag tau
-    {10.0f, 1.0f, 1.0f, 0.05f},                       // pendulum: g m l dt
-    {},                                               // synthetic
-    {0.001f, 0.0025f},                                // mountaincar: force gravity
-    {0.0015f, 0.0025f},                               // mountaincar_continuous: power gravity
-    {1.0f, 1.0f, 1.0f, 0.5f, 0.5f, 1.0f}};            // acrobot: link_length_1 link_mass_1 link_mass_2 link_com_pos_1 link_com_pos_2 link_moi
-static const int k_env_param_positive[6][DRIL_ENV_MAX_PARAMS] = {
-    {0, 1, 1, 1, 0, 1}, {0, 1, 1, 1}, {}, {0, 0}, {0, 0}, {1, 1, 1, 1, 1, 1}};
-
 extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const float* lo, const float* hi) {
     DRIL_REQUIRE(e, "NULL argument");
     EnvDev& d = e->d;
@@ -1169,9 +1169,9 @@ extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const floa
     DRIL_CUDA(cudaSetDevice(c->device));
     const size_t n = (size_t)d.n_envs;
     std::vector<float> dflt;
-    if (!lo && (e->observe_params || e->history)) {   // observed parameters / history stay: back to lo = hi = the built-in constants
+    if (!lo && e->obs_ks) {   // observed parameters / history stay: back to lo = hi = the built-in constants
         dflt.resize(n * np);
-        for (int k = 0; k < np; ++k) std::fill(dflt.begin() + (size_t)k * n, dflt.begin() + (size_t)(k + 1) * n, k_env_param_default[d.kind][k]);
+        for (int k = 0; k < np; ++k) std::fill(dflt.begin() + (size_t)k * n, dflt.begin() + (size_t)(k + 1) * n, env_param_default(d.kind).v[k]);
         lo = hi = dflt.data();
     }
     if (!lo) {   // back to the built-in constants and the default instantiations
@@ -1216,7 +1216,7 @@ extern "C" int32_t dril_env_get_params(dril_env* e, int32_t n_params, float* val
     DRIL_REQUIRE(n_params == np, "env kind %d has %d parameters, got %d", d.kind, np, n_params);
     const size_t n = (size_t)d.n_envs;
     if (!d.has_params) {
-        for (int k = 0; k < np; ++k) std::fill(values + (size_t)k * n, values + (size_t)(k + 1) * n, k_env_param_default[d.kind][k]);
+        for (int k = 0; k < np; ++k) std::fill(values + (size_t)k * n, values + (size_t)(k + 1) * n, env_param_default(d.kind).v[k]);
         return DRIL_OK;
     }
     dril_ctx* c = e->ctx;
@@ -1226,48 +1226,41 @@ extern "C" int32_t dril_env_get_params(dril_env* e, int32_t n_params, float* val
     return DRIL_OK;
 }
 
+// the observation layout: obs_ks (0, ENV_KS_OBS_PARAMS or ENV_KS_HISTORY), the history's k and frame width, the observation width
+// and the obs-sized arrays.  An env with either option runs the parametrised kernels: without ranges it holds lo = hi = the
+// defaults, which it drops again with the option.
+static int32_t env_set_obs_layout(dril_env* e, unsigned obs_ks, int hist_len, int frame_dim) {
+    EnvDev& d = e->d;
+    const int np = env_n_params(d.kind);
+    DRIL_CUDA(cudaSetDevice(e->ctx->device));
+    DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
+    e->obs_ks = obs_ks;
+    d.hist_len = hist_len;
+    d.frame_dim = frame_dim;
+    d.obs_dim = frame_dim * hist_len + (obs_ks == ENV_KS_OBS_PARAMS ? np : 0);
+    if ((obs_ks && !d.has_params) || (!obs_ks && e->default_params)) DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
+    return env_alloc_obs_arrays(e);
+}
 extern "C" int32_t dril_env_set_observe_params(dril_env* e, int32_t on) {
     DRIL_REQUIRE(e, "NULL argument");
     EnvDev& d = e->d;
-    const int np = env_n_params(d.kind);
-    if (np == 0) { dril_set_error("env kind %d has no physical parameters to observe", d.kind); return DRIL_ERR_UNSUPPORTED; }
-    if (on && e->history) { dril_set_error("observe_params cannot be combined with an observation history"); return DRIL_ERR_UNSUPPORTED; }
+    if (env_n_params(d.kind) == 0) { dril_set_error("env kind %d has no physical parameters to observe", d.kind); return DRIL_ERR_UNSUPPORTED; }
+    if (on && e->obs_ks == ENV_KS_HISTORY) { dril_set_error("observe_params cannot be combined with an observation history"); return DRIL_ERR_UNSUPPORTED; }
     DRIL_REQUIRE(!e->observed, "observe_params can only change before the env's first observation");
-    if ((on != 0) == e->observe_params) return DRIL_OK;
-    DRIL_CUDA(cudaSetDevice(e->ctx->device));
-    DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
-    e->observe_params = on != 0;
-    d.obs_dim = env_base_obs_dim(d.kind) + (e->observe_params ? np : 0);
-    if (e->observe_params && !d.has_params) {            // the parametrised kernels with lo = hi = the defaults
-        DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
-    } else if (!e->observe_params && e->default_params) {   // parameters that were only held for observing: dropped
-        DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
-    }
-    return env_alloc_obs_arrays(e);
+    if ((on != 0) == (e->obs_ks == ENV_KS_OBS_PARAMS)) return DRIL_OK;
+    return env_set_obs_layout(e, on ? ENV_KS_OBS_PARAMS : 0u, 1, env_base_obs_dim(d.kind));
 }
 extern "C" int32_t dril_env_set_obs_history(dril_env* e, int32_t history_len, int32_t mask_velocities) {
     DRIL_REQUIRE(e, "NULL argument");
     EnvDev& d = e->d;
-    const int np = env_n_params(d.kind);
     const bool on = history_len != 1 || mask_velocities != 0;
-    if (np == 0) { dril_set_error("env kind %d has no observation history", d.kind); return DRIL_ERR_UNSUPPORTED; }
-    if (on && e->observe_params) { dril_set_error("an observation history cannot be combined with observe_params"); return DRIL_ERR_UNSUPPORTED; }
+    if (env_n_params(d.kind) == 0) { dril_set_error("env kind %d has no observation history", d.kind); return DRIL_ERR_UNSUPPORTED; }
+    if (on && e->obs_ks == ENV_KS_OBS_PARAMS) { dril_set_error("an observation history cannot be combined with observe_params"); return DRIL_ERR_UNSUPPORTED; }
     DRIL_REQUIRE(history_len >= 1 && history_len <= DRIL_ENV_MAX_HISTORY, "history_len %d outside [1, %d]", history_len, DRIL_ENV_MAX_HISTORY);
-    const bool mask = mask_velocities != 0;
-    if (history_len == d.hist_len && env_frame_dim(d.kind, mask) == d.frame_dim) return DRIL_OK;
+    const int frame_dim = env_frame_dim(d.kind, mask_velocities != 0);
+    if (history_len == d.hist_len && frame_dim == d.frame_dim) return DRIL_OK;
     DRIL_REQUIRE(!e->observed, "the observation history can only change before the env's first observation");
-    DRIL_CUDA(cudaSetDevice(e->ctx->device));
-    DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
-    e->history = on;
-    d.hist_len = history_len;
-    d.frame_dim = env_frame_dim(d.kind, mask);
-    d.obs_dim = d.frame_dim * history_len;
-    if (e->history && !d.has_params) {                    // the parametrised kernels with lo = hi = the defaults
-        DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
-    } else if (!e->history && e->default_params) {        // parameters that were only held for the history: dropped
-        DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
-    }
-    return env_alloc_obs_arrays(e);
+    return env_set_obs_layout(e, on ? ENV_KS_HISTORY : 0u, history_len, frame_dim);
 }
 extern "C" int32_t dril_env_obs_dim(dril_env* e, int32_t* obs_dim) {
     DRIL_REQUIRE(e && obs_dim, "NULL argument");
@@ -1323,7 +1316,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     a.T = T;
     int flags = base_flags | (has_policy ? RO_HAS_POLICY : 0);
     const EnvDev& d = e->d;
-    const bool obsp = e->observe_params, hist = e->history;
+    const unsigned ks = env_ks(e);
     e->observed = true;
     const bool upd = d.normalize && d.training && (d.norm_obs || d.norm_reward);
     if (upd) flags |= RO_GRID_SYNC;
@@ -1397,7 +1390,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
         static const int f_threads = getenv("DRIL_FAST_THREADS") ? atoi(getenv("DRIL_FAST_THREADS")) : 0;
         if (f_threads >= tq && f_threads <= DRIL_THREADS && f_threads % tq == 0) threads = f_threads;
         bool ws = true;
-        const int hist_rows = hist ? d.obs_dim - d.frame_dim : 0;
+        const int hist_rows = env_history(ks) ? d.obs_dim - d.frame_dim : 0;
         auto tot = [&](int m4, int th, bool w) { return rollout_fast_smem_layout(a.pd, m4, th, w, hist_rows).total; };
         if (tot(M4, threads, true) > DRIL_SMEM_MAX) ws = false;
         while (M4 > 8 && tot(M4, threads, ws) > DRIL_SMEM_MAX) M4 >>= 1;
@@ -1406,7 +1399,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.n_tiles = (int)((N + M4 - 1) / M4);
             Span sp(c, DRIL_K_ROLLOUT);
             void* args[] = {(void*)&a};
-            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, d.kind, d.has_params, obsp, hist), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
+            DRIL_CUDA(cudaLaunchKernel(rollout_fast_fn(ws, ks), dim3(a.n_tiles), dim3(threads), args, tot(M4, threads, ws), c->stream));
             return DRIL_OK;
         }
     }
@@ -1443,7 +1436,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
             a.M4 = GTC_ENVS; a.flags = flags;
             a.n_tiles = (int)((N + GTC_ENVS - 1) / GTC_ENVS);
             int grid = a.n_tiles, body_i = (int)body;
-            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, d.kind, a.pd.act_n, d.has_params, obsp, hist);
+            void* fn = rollout_gtc_fn(a.pd.n_layers - 1, ks, a.pd.act_n);
             void* args[] = {(void*)&a, (void*)&gl, (void*)&body_i};
             {
                 Span sp(c, DRIL_K_ROLLOUT);
@@ -1505,14 +1498,14 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
     Span sp(c, has_policy ? DRIL_K_ROLLOUT : DRIL_K_ENV);
     if (flags & RO_GRID_SYNC) {
         int per_sm = 0;
-        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, d.kind, d.has_params, obsp, hist), threads, smem));
+        DRIL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rollout_fn(ws, ks), threads, smem));
         DRIL_REQUIRE(per_sm >= 1, "rollout kernel does not fit on an SM");
         grid = std::min(grid, std::min(per_sm * c->sm_count, e->max_blocks));
         void* args[] = {(void*)&a};
-        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, d.kind, d.has_params, obsp, hist), dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchCooperativeKernel(rollout_fn(ws, ks), dim3(grid), dim3(threads), args, smem, c->stream));
     } else {
         void* args[] = {(void*)&a};
-        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, d.kind, d.has_params, obsp, hist), dim3(grid), dim3(threads), args, smem, c->stream));
+        DRIL_CUDA(cudaLaunchKernel(rollout_fn(ws, ks), dim3(grid), dim3(threads), args, smem, c->stream));
     }
     if (defer) return launch_critic();
     return DRIL_OK;

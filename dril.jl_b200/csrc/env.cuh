@@ -186,36 +186,109 @@ __device__ __forceinline__ void env_reset_state(int kind, uint32_t gid, uint32_t
     }
 }
 
-// CartPole-v1 Euler step with the (correctly rounded) sin/cos of the pole angle supplied by the caller.
+// ---------------------------------------------------------------------------------------
+// Per-env physical parameters (dril_b200.h has the table).  Every step below takes the constants of the table from `p`, in table
+// order: the kernels built for ENV_KS_PARAMS pass the env's values for the running episode, the default instantiations pass
+// env_param_default as compile-time constants, which the compiler folds into the code of a step with the constants written in.
+// Each derived coefficient is one fixed fp32 sequence, restated in oracle/env_params.py, that gives Gymnasium's constant bit
+// for bit at the default values.
+// ---------------------------------------------------------------------------------------
+__host__ __device__ constexpr bool env_has_params(unsigned ks) { return (ks & ENV_KS_PARAMS) != 0; }
+// the parametrised kind set whose instantiation serves env kind `kind` (the synthetic env has no parameters)
+__host__ __device__ constexpr unsigned env_param_kind_set(int kind) {
+    return (env_kind_set(kind) & ~(1u << DRIL_ENV_SYNTHETIC)) | ENV_KS_PARAMS;
+}
+// ... and the one that also observes the parameters
+__host__ __device__ constexpr unsigned env_obs_param_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_OBS_PARAMS; }
+// ... and the one with an observation history (an env with history always runs with parameters: lo = hi = the defaults
+// without ranges)
+__host__ __device__ constexpr unsigned env_hist_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_HISTORY; }
+
+// the defaults of the table (Gymnasium's constants), by kind
+struct EnvParams { float v[DRIL_ENV_MAX_PARAMS]; };
+__host__ __device__ constexpr EnvParams env_param_default(int kind) {
+    constexpr EnvParams k_env_param_default[6] = {
+        {{9.8f, 1.0f, 0.1f, 0.5f, 10.0f, 0.02f}},        // cartpole: gravity masscart masspole length force_mag tau
+        {{10.0f, 1.0f, 1.0f, 0.05f}},                     // pendulum: g m l dt
+        {},                                               // synthetic
+        {{0.001f, 0.0025f}},                              // mountaincar: force gravity
+        {{0.0015f, 0.0025f}},                             // mountaincar_continuous: power gravity
+        {{1.0f, 1.0f, 1.0f, 0.5f, 0.5f, 1.0f}}};          // acrobot: link_length_1 link_mass_1 link_mass_2 link_com_pos_1 link_com_pos_2 link_moi
+    return k_env_param_default[kind];
+}
+// whether a value must be > 0 (1) or >= 0 (0)
+static const int k_env_param_positive[6][DRIL_ENV_MAX_PARAMS] = {
+    {0, 1, 1, 1, 0, 1}, {0, 1, 1, 1}, {}, {0, 0}, {0, 0}, {1, 1, 1, 1, 1, 1}};
+
+// the values of env n's episode `episode`: lo + (hi - lo) * u, u from Philox (gid, episode, k / 4, DRIL_TAG_ENV_PARAMS) word
+// k % 4; written to par and env.pval
+__device__ __forceinline__ void env_draw_params(const EnvDev& env, long long n, uint32_t gid, uint32_t episode, float* par) {
+    const int np = env_n_params(env.kind);
+    const long long N = env.n_envs;
+    uint32_t x[4];
+#pragma unroll
+    for (int k = 0; k < DRIL_ENV_MAX_PARAMS; ++k) {
+        if (k < np) {
+            if ((k & 3) == 0) philox4x32(gid, episode, (uint32_t)(k >> 2), DRIL_TAG_ENV_PARAMS, env.seed, x);
+            const float lo = env.plo[(size_t)k * N + n], hi = env.phi[(size_t)k * N + n];
+            par[k] = __fadd_rn(lo, __fmul_rn(__fsub_rn(hi, lo), u01_f32(x[k & 3])));
+            env.pval[(size_t)k * N + n] = par[k];
+        }
+    }
+}
+__device__ __forceinline__ void env_load_params(const EnvDev& env, long long n, float* par) {
+    const int np = env_n_params(env.kind);
+#pragma unroll
+    for (int k = 0; k < DRIL_ENV_MAX_PARAMS; ++k) par[k] = k < np ? env.pval[(size_t)k * env.n_envs + n] : 0.f;
+}
+
+// CartPole-v1: p = (gravity, masscart, masspole, length, force_mag, tau); total_mass = masspole + masscart,
+// polemass_length = masspole * length
+struct CartPoleCoef { float gravity, masspole, length, force_mag, tau, total_mass, pml; };
+__device__ __forceinline__ CartPoleCoef cartpole_coef(const float* p) {
+    const float gravity = p[0], masscart = p[1], masspole = p[2], length = p[3], force_mag = p[4], tau = p[5];
+    return {gravity, masspole, length, force_mag, tau, __fadd_rn(masspole, masscart), __fmul_rn(masspole, length)};
+}
+// Euler step with the (correctly rounded) sin/cos of the pole angle supplied by the caller.
 // a01: 0 = push left, 1 = push right. Returns reward; sets terminated.
-__device__ __forceinline__ float cartpole_step_sc(float* st, int a01, float sinth, float costh, bool* terminated) {
-    const float GRAVITY = 9.8f, MASSPOLE = 0.1f, LENGTH = 0.5f, FORCE_MAG = 10.0f, TAU = 0.02f;
-    const float TOTAL_MASS = __fadd_rn(0.1f, 1.0f);
-    const float PML = __fmul_rn(0.1f, 0.5f);
+__device__ __forceinline__ float cartpole_step_sc(float* st, int a01, float sinth, float costh, const CartPoleCoef& C, bool* terminated) {
     const float THETA_THR = 0.20943951023931953f, X_THR = 2.4f, FOUR_THIRDS = 1.3333333333333333f;
     float x = st[0], x_dot = st[1], th = st[2], th_dot = st[3];
-    float force = (a01 == 1) ? FORCE_MAG : -FORCE_MAG;
-    float temp = __fdiv_rn(__fadd_rn(force, __fmul_rn(__fmul_rn(PML, __fmul_rn(th_dot, th_dot)), sinth)), TOTAL_MASS);
-    float den = __fmul_rn(LENGTH, __fsub_rn(FOUR_THIRDS, __fdiv_rn(__fmul_rn(MASSPOLE, __fmul_rn(costh, costh)), TOTAL_MASS)));
-    float thetaacc = __fdiv_rn(__fsub_rn(__fmul_rn(GRAVITY, sinth), __fmul_rn(costh, temp)), den);
-    float xacc = __fsub_rn(temp, __fdiv_rn(__fmul_rn(__fmul_rn(PML, thetaacc), costh), TOTAL_MASS));
-    float xn = __fadd_rn(x, __fmul_rn(TAU, x_dot));
-    float xdn = __fadd_rn(x_dot, __fmul_rn(TAU, xacc));
-    float thn = __fadd_rn(th, __fmul_rn(TAU, th_dot));
-    float thdn = __fadd_rn(th_dot, __fmul_rn(TAU, thetaacc));
+    float force = (a01 == 1) ? C.force_mag : -C.force_mag;
+    float temp = __fdiv_rn(__fadd_rn(force, __fmul_rn(__fmul_rn(C.pml, __fmul_rn(th_dot, th_dot)), sinth)), C.total_mass);
+    float den = __fmul_rn(C.length, __fsub_rn(FOUR_THIRDS, __fdiv_rn(__fmul_rn(C.masspole, __fmul_rn(costh, costh)), C.total_mass)));
+    float thetaacc = __fdiv_rn(__fsub_rn(__fmul_rn(C.gravity, sinth), __fmul_rn(costh, temp)), den);
+    float xacc = __fsub_rn(temp, __fdiv_rn(__fmul_rn(__fmul_rn(C.pml, thetaacc), costh), C.total_mass));
+    float xn = __fadd_rn(x, __fmul_rn(C.tau, x_dot));
+    float xdn = __fadd_rn(x_dot, __fmul_rn(C.tau, xacc));
+    float thn = __fadd_rn(th, __fmul_rn(C.tau, th_dot));
+    float thdn = __fadd_rn(th_dot, __fmul_rn(C.tau, thetaacc));
     st[0] = xn; st[1] = xdn; st[2] = thn; st[3] = thdn;
     *terminated = (xn < -X_THR) || (xn > X_THR) || (thn < -THETA_THR) || (thn > THETA_THR);
     return 1.0f;
 }
-__device__ __forceinline__ float cartpole_step(float* st, int a01, bool* terminated) {
+__device__ __forceinline__ float cartpole_step(float* st, int a01, const CartPoleCoef& C, bool* terminated) {
     float sinth, costh;
     sincos_rn(st[2], &sinth, &costh);
-    return cartpole_step_sc(st, a01, sinth, costh, terminated);
+    return cartpole_step_sc(st, a01, sinth, costh, C, terminated);
 }
 
-// Pendulum-v1 step (g = 10, m = l = 1). u: env-space torque (clipped again like Gymnasium).
-__device__ __forceinline__ float pendulum_step(float* st, float u) {
-    const float MAX_SPEED = 8.0f, MAX_TORQUE = 2.0f, DT = 0.05f;
+// Pendulum-v1: p = (g, m, l, dt); thdot += (3 g / (2 l) * sin th + 3 / (m l^2) * u) * dt with the coefficients
+// c_sin = (3 g) / (2 l) and c_u = 3 / (m (l l))
+struct PendulumCoef { float c_sin, c_u, dt; };
+__device__ __forceinline__ PendulumCoef pendulum_coef(const float* p) {
+    const float g = p[0], m = p[1], l = p[2], dt = p[3];
+    return {__fdiv_rn(__fmul_rn(3.0f, g), __fmul_rn(2.0f, l)), __fdiv_rn(3.0f, __fmul_rn(m, __fmul_rn(l, l))), dt};
+}
+// ... at the defaults, as compile-time constants (15, 3, 0.05: every product and quotient is exact there).  The compiler does
+// not fold __fdiv_rn of constants, so the default instantiations take these instead of pendulum_coef of the defaults.
+__host__ __device__ constexpr PendulumCoef pendulum_default_coef() {
+    constexpr EnvParams d = env_param_default(DRIL_ENV_PENDULUM);
+    return {(3.0f * d.v[0]) / (2.0f * d.v[2]), 3.0f / (d.v[1] * (d.v[2] * d.v[2])), d.v[3]};
+}
+// u: env-space torque (clipped again like Gymnasium)
+__device__ __forceinline__ float pendulum_step(float* st, float u, const PendulumCoef& C) {
+    const float MAX_SPEED = 8.0f, MAX_TORQUE = 2.0f;
     const float PI = 3.14159274101257324f, TWO_PI = 6.28318548202514648f;
     u = fminf(fmaxf(u, -MAX_TORQUE), MAX_TORQUE);
     float th = st[0], thdot = st[1];
@@ -225,9 +298,9 @@ __device__ __forceinline__ float pendulum_step(float* st, float u) {
                            __fmul_rn(0.001f, __fmul_rn(u, u)));
     float sinth, costh;
     sincos_rn(th, &sinth, &costh);
-    float nthdot = __fadd_rn(thdot, __fmul_rn(__fadd_rn(__fmul_rn(15.0f, sinth), __fmul_rn(3.0f, u)), DT));
+    float nthdot = __fadd_rn(thdot, __fmul_rn(__fadd_rn(__fmul_rn(C.c_sin, sinth), __fmul_rn(C.c_u, u)), C.dt));
     nthdot = fminf(fmaxf(nthdot, -MAX_SPEED), MAX_SPEED);
-    float nth = __fadd_rn(th, __fmul_rn(nthdot, DT));
+    float nth = __fadd_rn(th, __fmul_rn(nthdot, C.dt));
     st[0] = nth; st[1] = nthdot;
     return -cost;
 }
@@ -241,25 +314,70 @@ __device__ __forceinline__ void mountaincar_move(float* st, float dv, float goal
     st[0] = pos; st[1] = vel;
     *terminated = pos >= goal && vel >= 0.f;
 }
-// MountainCar-v0: idx 0 = push left, 1 = none, 2 = push right.  Returns reward -1.
-__device__ __forceinline__ float mountaincar_step(float* st, int idx, bool* terminated) {
+// MountainCar-v0: p = (force, gravity); idx 0 = push left, 1 = none, 2 = push right.  Returns reward -1.
+__device__ __forceinline__ float mountaincar_step(float* st, int idx, const float* p, bool* terminated) {
     float s, c;
     sincos_rn(__fmul_rn(3.0f, st[0]), &s, &c);
-    mountaincar_move(st, __fadd_rn(__fmul_rn((float)(idx - 1), 0.001f), __fmul_rn(c, -0.0025f)), 0.5f, terminated);
+    mountaincar_move(st, __fadd_rn(__fmul_rn((float)(idx - 1), p[0]), __fmul_rn(c, -p[1])), 0.5f, terminated);
     return -1.0f;
 }
-// MountainCarContinuous-v0: a = env-space force (clipped to [-1, 1] for the dynamics, not for the reward)
-__device__ __forceinline__ float mountaincar_continuous_step(float* st, float a, bool* terminated) {
+// MountainCarContinuous-v0: p = (power, gravity); a = env-space force (clipped to [-1, 1] for the dynamics, not for the reward)
+__device__ __forceinline__ float mountaincar_continuous_step(float* st, float a, const float* p, bool* terminated) {
     const float f = fminf(fmaxf(a, -1.0f), 1.0f);
     float s, c;
     sincos_rn(__fmul_rn(3.0f, st[0]), &s, &c);
-    mountaincar_move(st, __fsub_rn(__fmul_rn(f, 0.0015f), __fmul_rn(0.0025f, c)), 0.45f, terminated);
+    mountaincar_move(st, __fsub_rn(__fmul_rn(f, p[0]), __fmul_rn(p[1], c)), 0.45f, terminated);
     return __fsub_rn(*terminated ? 100.0f : 0.0f, __fmul_rn(__fmul_rn(a, a), 0.1f));
 }
 
-// Acrobot-v1 "book" dynamics f(s) for torque a (m1 = m2 = l1 = I1 = I2 = 1, lc1 = lc2 = 0.5, g = 9.8 folded into exact
-// fp32 constants; (m1 lc1 + m2 l1) g = 1.5 * 9.8f rounded once)
-__device__ __forceinline__ void acrobot_dsdt(const float* s, float a, float* ds) {
+// Acrobot-v1: p = (l1, m1, m2, lc1, lc2, I) with I1 = I2 = I (link_moi) and g = 9.8.  The book dynamics f(s) for torque a as
+//   d1 = ((m1 lc1^2 + m2 ((l1^2 + lc2^2) + (2 l1) lc2 c2)) + I) + I       d2 = m2 (lc2^2 + (l1 lc2) c2) + I
+//   phi2 = ((m2 lc2) g) cos(th1 + th2 - pi/2)
+//   phi1 = (((-h w2^2) s2 - ((2 h) (w2 w1)) s2) + ((m1 lc1 + m2 l1) g) cos(th1 - pi/2)) + phi2,   h = m2 (l1 lc2)
+//   al2 = (((a + (d2 / d1) phi1) - (h w1^2) s2) - phi2) / ((m2 lc2^2 + I) - d2^2 / d1)      al1 = -(d2 al2 + phi1) / d1
+// with every coefficient rounded once in the order written (at the defaults: 0.25, 1.25, 1, 1, 1, 0.25, 0.5, 0.5, 1, 4.9f, 14.7f,
+// 1.25; (m1 lc1 + m2 l1) g = 1.5 * 9.8f rounded once)
+struct AcrobotCoef { float a1, p, k, m2, i, l2, q, h, h2, g_lc2, g_12, j; };
+__device__ __forceinline__ AcrobotCoef acrobot_coef(const float* p) {
+    const float l1 = p[0], m1 = p[1], m2 = p[2], lc1 = p[3], lc2 = p[4], moi = p[5];
+    AcrobotCoef c;
+    c.a1 = __fmul_rn(m1, __fmul_rn(lc1, lc1));
+    c.p = __fadd_rn(__fmul_rn(l1, l1), __fmul_rn(lc2, lc2));
+    c.k = __fmul_rn(__fmul_rn(2.0f, l1), lc2);
+    c.m2 = m2;
+    c.i = moi;
+    c.l2 = __fmul_rn(lc2, lc2);
+    c.q = __fmul_rn(l1, lc2);
+    c.h = __fmul_rn(m2, c.q);
+    c.h2 = __fmul_rn(2.0f, c.h);
+    c.g_lc2 = __fmul_rn(__fmul_rn(m2, lc2), 9.8f);
+    c.g_12 = __fmul_rn(__fadd_rn(__fmul_rn(m1, lc1), __fmul_rn(m2, l1)), 9.8f);
+    c.j = __fadd_rn(__fmul_rn(m2, c.l2), moi);
+    return c;
+}
+__device__ __forceinline__ void acrobot_dsdt(const float* s, float a, const AcrobotCoef& C, float* ds) {
+    const float HALF_PI = 1.57079637050628662f;
+    const float th1 = s[0], th2 = s[1], w1 = s[2], w2 = s[3];
+    float s2, c2, sp, cp2, cp1;
+    sincos_rn(th2, &s2, &c2);
+    const float d1 = __fadd_rn(__fadd_rn(__fadd_rn(C.a1, __fmul_rn(C.m2, __fadd_rn(C.p, __fmul_rn(C.k, c2)))), C.i), C.i);
+    const float d2 = __fadd_rn(__fmul_rn(C.m2, __fadd_rn(C.l2, __fmul_rn(C.q, c2))), C.i);
+    sincos_rn(__fsub_rn(__fadd_rn(th1, th2), HALF_PI), &sp, &cp2);
+    const float phi2 = __fmul_rn(C.g_lc2, cp2);
+    sincos_rn(__fsub_rn(th1, HALF_PI), &sp, &cp1);
+    const float phi1 = __fadd_rn(__fadd_rn(__fsub_rn(__fmul_rn(__fmul_rn(-C.h, __fmul_rn(w2, w2)), s2),
+                                                     __fmul_rn(__fmul_rn(C.h2, __fmul_rn(w2, w1)), s2)),
+                                           __fmul_rn(C.g_12, cp1)), phi2);
+    const float num = __fsub_rn(__fsub_rn(__fadd_rn(a, __fmul_rn(__fdiv_rn(d2, d1), phi1)), __fmul_rn(__fmul_rn(C.h, __fmul_rn(w1, w1)), s2)), phi2);
+    const float al2 = __fdiv_rn(num, __fsub_rn(C.j, __fdiv_rn(__fmul_rn(d2, d2), d1)));
+    const float al1 = __fdiv_rn(-__fadd_rn(__fmul_rn(d2, al2), phi1), d1);
+    ds[0] = w1; ds[1] = w2; ds[2] = al1; ds[3] = al2;
+}
+// ... at the defaults, for the default instantiations: acrobot_dsdt with the products by m2 = 1, 2 l1 lc2 = 1 and 2 h = 1 left
+// out (they are exact).  This is the one step kept twice: the compiler does not remove __fmul_rn(1, x), so acrobot_dsdt with the
+// defaults as constants is not the code of these dynamics (16 more instructions per RK4 step), and turning those three products
+// into plain ones changes the code of the parametrised instantiations.
+__device__ __forceinline__ void acrobot_dsdt_default(const float* s, float a, float* ds) {
     const float HALF_PI = 1.57079637050628662f, G_LC2 = 4.90000009536743164f, G_12 = 14.7000007629394531f;
     const float th1 = s[0], th2 = s[1], w1 = s[2], w2 = s[3];
     float s2, c2, sp, cp2, cp1;
@@ -288,7 +406,7 @@ __device__ __forceinline__ float acrobot_wrap(float x) {
 // Acrobot-v1: idx 0 / 1 / 2 = torque -1 / 0 / +1 held over one RK4 step of dt = 0.2 of the dynamics dsdt(s, a, ds).  Returns
 // reward 0 on termination, else -1.
 template <class Dsdt>
-__device__ __forceinline__ float acrobot_rk4_step(float* st, int idx, const Dsdt& dsdt, bool* terminated) {
+__device__ __forceinline__ float acrobot_step(float* st, int idx, const Dsdt& dsdt, bool* terminated) {
     const float DT = 0.2f, DT2 = 0.1f, DT6 = 0.0333333350718021393f;
     const float MAX_VEL_1 = 12.5663709640502930f, MAX_VEL_2 = 28.2743339538574219f;
     const float a = (float)(idx - 1);
@@ -315,158 +433,6 @@ __device__ __forceinline__ float acrobot_rk4_step(float* st, int idx, const Dsdt
     sincos_rn(__fadd_rn(st[1], st[0]), &s, &c12);
     *terminated = __fsub_rn(-c1, c12) > 1.0f;
     return *terminated ? 0.0f : -1.0f;
-}
-__device__ __forceinline__ float acrobot_step(float* st, int idx, bool* terminated) {
-    return acrobot_rk4_step(st, idx, [](const float* s, float a, float* ds) { acrobot_dsdt(s, a, ds); }, terminated);
-}
-
-// ---------------------------------------------------------------------------------------
-// Per-env physical parameters (dril_b200.h has the table).  The kernels built for ENV_KS_PARAMS take every constant of the
-// table from `p` (the env's values for the running episode, in table order); the default instantiations keep the folded
-// constants above and their exact code.  Each derived coefficient below is one fixed fp32 sequence, restated in
-// oracle/env_params.py, that gives the folded constant bit for bit at the default values.
-// ---------------------------------------------------------------------------------------
-__host__ __device__ constexpr bool env_has_params(unsigned ks) { return (ks & ENV_KS_PARAMS) != 0; }
-// the parametrised kind set whose instantiation serves env kind `kind` (the synthetic env has no parameters)
-__host__ __device__ constexpr unsigned env_param_kind_set(int kind) {
-    return (env_kind_set(kind) & ~(1u << DRIL_ENV_SYNTHETIC)) | ENV_KS_PARAMS;
-}
-// ... and the one that also observes the parameters
-__host__ __device__ constexpr unsigned env_obs_param_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_OBS_PARAMS; }
-// ... and the one with an observation history (an env with history always runs with parameters: lo = hi = the defaults
-// without ranges)
-__host__ __device__ constexpr unsigned env_hist_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_HISTORY; }
-
-// the values of env n's episode `episode`: lo + (hi - lo) * u, u from Philox (gid, episode, k / 4, DRIL_TAG_ENV_PARAMS) word
-// k % 4; written to par and env.pval
-__device__ __forceinline__ void env_draw_params(const EnvDev& env, long long n, uint32_t gid, uint32_t episode, float* par) {
-    const int np = env_n_params(env.kind);
-    const long long N = env.n_envs;
-    uint32_t x[4];
-#pragma unroll
-    for (int k = 0; k < DRIL_ENV_MAX_PARAMS; ++k) {
-        if (k < np) {
-            if ((k & 3) == 0) philox4x32(gid, episode, (uint32_t)(k >> 2), DRIL_TAG_ENV_PARAMS, env.seed, x);
-            const float lo = env.plo[(size_t)k * N + n], hi = env.phi[(size_t)k * N + n];
-            par[k] = __fadd_rn(lo, __fmul_rn(__fsub_rn(hi, lo), u01_f32(x[k & 3])));
-            env.pval[(size_t)k * N + n] = par[k];
-        }
-    }
-}
-__device__ __forceinline__ void env_load_params(const EnvDev& env, long long n, float* par) {
-    const int np = env_n_params(env.kind);
-#pragma unroll
-    for (int k = 0; k < DRIL_ENV_MAX_PARAMS; ++k) par[k] = k < np ? env.pval[(size_t)k * env.n_envs + n] : 0.f;
-}
-
-// CartPole: p = (gravity, masscart, masspole, length, force_mag, tau); total_mass = masspole + masscart,
-// polemass_length = masspole * length
-__device__ __forceinline__ float cartpole_step_p(float* st, int a01, const float* p, bool* terminated) {
-    const float gravity = p[0], masscart = p[1], masspole = p[2], length = p[3], force_mag = p[4], tau = p[5];
-    const float total_mass = __fadd_rn(masspole, masscart);
-    const float pml = __fmul_rn(masspole, length);
-    const float THETA_THR = 0.20943951023931953f, X_THR = 2.4f, FOUR_THIRDS = 1.3333333333333333f;
-    float sinth, costh;
-    sincos_rn(st[2], &sinth, &costh);
-    float x = st[0], x_dot = st[1], th = st[2], th_dot = st[3];
-    float force = (a01 == 1) ? force_mag : -force_mag;
-    float temp = __fdiv_rn(__fadd_rn(force, __fmul_rn(__fmul_rn(pml, __fmul_rn(th_dot, th_dot)), sinth)), total_mass);
-    float den = __fmul_rn(length, __fsub_rn(FOUR_THIRDS, __fdiv_rn(__fmul_rn(masspole, __fmul_rn(costh, costh)), total_mass)));
-    float thetaacc = __fdiv_rn(__fsub_rn(__fmul_rn(gravity, sinth), __fmul_rn(costh, temp)), den);
-    float xacc = __fsub_rn(temp, __fdiv_rn(__fmul_rn(__fmul_rn(pml, thetaacc), costh), total_mass));
-    float xn = __fadd_rn(x, __fmul_rn(tau, x_dot));
-    float xdn = __fadd_rn(x_dot, __fmul_rn(tau, xacc));
-    float thn = __fadd_rn(th, __fmul_rn(tau, th_dot));
-    float thdn = __fadd_rn(th_dot, __fmul_rn(tau, thetaacc));
-    st[0] = xn; st[1] = xdn; st[2] = thn; st[3] = thdn;
-    *terminated = (xn < -X_THR) || (xn > X_THR) || (thn < -THETA_THR) || (thn > THETA_THR);
-    return 1.0f;
-}
-
-// Pendulum: p = (g, m, l, dt); thdot += (3 g / (2 l) * sin th + 3 / (m l^2) * u) * dt with 3 g / (2 l) = (3 g) / (2 l) and
-// 3 / (m l^2) = 3 / (m (l l))  (15 and 3 at the defaults)
-__device__ __forceinline__ float pendulum_step_p(float* st, float u, const float* p) {
-    const float g = p[0], m = p[1], l = p[2], dt = p[3];
-    const float c_sin = __fdiv_rn(__fmul_rn(3.0f, g), __fmul_rn(2.0f, l));
-    const float c_u = __fdiv_rn(3.0f, __fmul_rn(m, __fmul_rn(l, l)));
-    const float MAX_SPEED = 8.0f, MAX_TORQUE = 2.0f;
-    const float PI = 3.14159274101257324f, TWO_PI = 6.28318548202514648f;
-    u = fminf(fmaxf(u, -MAX_TORQUE), MAX_TORQUE);
-    float th = st[0], thdot = st[1];
-    float xp = __fadd_rn(th, PI);
-    float an = __fsub_rn(__fsub_rn(xp, __fmul_rn(TWO_PI, floorf(__fdiv_rn(xp, TWO_PI)))), PI);
-    float cost = __fadd_rn(__fadd_rn(__fmul_rn(an, an), __fmul_rn(0.1f, __fmul_rn(thdot, thdot))),
-                           __fmul_rn(0.001f, __fmul_rn(u, u)));
-    float sinth, costh;
-    sincos_rn(th, &sinth, &costh);
-    float nthdot = __fadd_rn(thdot, __fmul_rn(__fadd_rn(__fmul_rn(c_sin, sinth), __fmul_rn(c_u, u)), dt));
-    nthdot = fminf(fmaxf(nthdot, -MAX_SPEED), MAX_SPEED);
-    float nth = __fadd_rn(th, __fmul_rn(nthdot, dt));
-    st[0] = nth; st[1] = nthdot;
-    return -cost;
-}
-
-// MountainCar: p = (force, gravity); MountainCarContinuous: p = (power, gravity)
-__device__ __forceinline__ float mountaincar_step_p(float* st, int idx, const float* p, bool* terminated) {
-    float s, c;
-    sincos_rn(__fmul_rn(3.0f, st[0]), &s, &c);
-    mountaincar_move(st, __fadd_rn(__fmul_rn((float)(idx - 1), p[0]), __fmul_rn(c, -p[1])), 0.5f, terminated);
-    return -1.0f;
-}
-__device__ __forceinline__ float mountaincar_continuous_step_p(float* st, float a, const float* p, bool* terminated) {
-    const float f = fminf(fmaxf(a, -1.0f), 1.0f);
-    float s, c;
-    sincos_rn(__fmul_rn(3.0f, st[0]), &s, &c);
-    mountaincar_move(st, __fsub_rn(__fmul_rn(f, p[0]), __fmul_rn(p[1], c)), 0.45f, terminated);
-    return __fsub_rn(*terminated ? 100.0f : 0.0f, __fmul_rn(__fmul_rn(a, a), 0.1f));
-}
-
-// Acrobot: p = (l1, m1, m2, lc1, lc2, I) with I1 = I2 = I (link_moi) and g = 9.8.  The book dynamics as
-//   d1 = ((m1 lc1^2 + m2 ((l1^2 + lc2^2) + (2 l1) lc2 c2)) + I) + I       d2 = m2 (lc2^2 + (l1 lc2) c2) + I
-//   phi2 = ((m2 lc2) g) cos(th1 + th2 - pi/2)
-//   phi1 = (((-h w2^2) s2 - ((2 h) (w2 w1)) s2) + ((m1 lc1 + m2 l1) g) cos(th1 - pi/2)) + phi2,   h = m2 (l1 lc2)
-//   al2 = (((a + (d2 / d1) phi1) - (h w1^2) s2) - phi2) / ((m2 lc2^2 + I) - d2^2 / d1)      al1 = -(d2 al2 + phi1) / d1
-// with every coefficient rounded once in the order written (at the defaults: 0.25, 1.25, 1, 0.25, 0.5, 0.5, 1, 4.9f, 14.7f,
-// 1.25 -- the folded constants of acrobot_dsdt, where the two products by 1 are exact)
-struct AcrobotCoef { float a1, p, k, m2, i, l2, q, h, h2, g_lc2, g_12, j; };
-__device__ __forceinline__ AcrobotCoef acrobot_coef(const float* p) {
-    const float l1 = p[0], m1 = p[1], m2 = p[2], lc1 = p[3], lc2 = p[4], moi = p[5];
-    AcrobotCoef c;
-    c.a1 = __fmul_rn(m1, __fmul_rn(lc1, lc1));
-    c.p = __fadd_rn(__fmul_rn(l1, l1), __fmul_rn(lc2, lc2));
-    c.k = __fmul_rn(__fmul_rn(2.0f, l1), lc2);
-    c.m2 = m2;
-    c.i = moi;
-    c.l2 = __fmul_rn(lc2, lc2);
-    c.q = __fmul_rn(l1, lc2);
-    c.h = __fmul_rn(m2, c.q);
-    c.h2 = __fmul_rn(2.0f, c.h);
-    c.g_lc2 = __fmul_rn(__fmul_rn(m2, lc2), 9.8f);
-    c.g_12 = __fmul_rn(__fadd_rn(__fmul_rn(m1, lc1), __fmul_rn(m2, l1)), 9.8f);
-    c.j = __fadd_rn(__fmul_rn(m2, c.l2), moi);
-    return c;
-}
-__device__ __forceinline__ void acrobot_dsdt_p(const float* s, float a, const AcrobotCoef& C, float* ds) {
-    const float HALF_PI = 1.57079637050628662f;
-    const float th1 = s[0], th2 = s[1], w1 = s[2], w2 = s[3];
-    float s2, c2, sp, cp2, cp1;
-    sincos_rn(th2, &s2, &c2);
-    const float d1 = __fadd_rn(__fadd_rn(__fadd_rn(C.a1, __fmul_rn(C.m2, __fadd_rn(C.p, __fmul_rn(C.k, c2)))), C.i), C.i);
-    const float d2 = __fadd_rn(__fmul_rn(C.m2, __fadd_rn(C.l2, __fmul_rn(C.q, c2))), C.i);
-    sincos_rn(__fsub_rn(__fadd_rn(th1, th2), HALF_PI), &sp, &cp2);
-    const float phi2 = __fmul_rn(C.g_lc2, cp2);
-    sincos_rn(__fsub_rn(th1, HALF_PI), &sp, &cp1);
-    const float phi1 = __fadd_rn(__fadd_rn(__fsub_rn(__fmul_rn(__fmul_rn(-C.h, __fmul_rn(w2, w2)), s2),
-                                                     __fmul_rn(__fmul_rn(C.h2, __fmul_rn(w2, w1)), s2)),
-                                           __fmul_rn(C.g_12, cp1)), phi2);
-    const float num = __fsub_rn(__fsub_rn(__fadd_rn(a, __fmul_rn(__fdiv_rn(d2, d1), phi1)), __fmul_rn(__fmul_rn(C.h, __fmul_rn(w1, w1)), s2)), phi2);
-    const float al2 = __fdiv_rn(num, __fsub_rn(C.j, __fdiv_rn(__fmul_rn(d2, d2), d1)));
-    const float al1 = __fdiv_rn(-__fadd_rn(__fmul_rn(d2, al2), phi1), d1);
-    ds[0] = w1; ds[1] = w2; ds[2] = al1; ds[3] = al2;
-}
-__device__ __forceinline__ float acrobot_step_p(float* st, int idx, const float* p, bool* terminated) {
-    const AcrobotCoef C = acrobot_coef(p);
-    return acrobot_rk4_step(st, idx, [&C](const float* s, float a, float* ds) { acrobot_dsdt_p(s, a, C, ds); }, terminated);
 }
 
 // Synthetic env (SURVEY §8d C5): obs block b of lifetime step `life`
@@ -497,24 +463,34 @@ __device__ __forceinline__ bool env_is(int kind) { return env_in(KS, K) && (K ==
 
 // one step of env n: a_disc = env-space action of a Discrete env, a_cont = the Box env's action as the wrappers above it hand it
 // over (read only for Box envs), life = the synthetic env's lifetime step counter (read and advanced for that kind only).
-// par: the env's parameter values (read only by the ENV_KS_PARAMS instantiations).  Returns the reward; sets terminated.
+// par: the env's parameter values, which the ENV_KS_PARAMS instantiations step with; the others step with the defaults.
+// Returns the reward; sets terminated.
 template <unsigned KS>
 __device__ __forceinline__ float env_step(const EnvDev& env, float* st, long long n, int a_disc, const float* a_cont, uint32_t* life,
                                           bool* terminated, const float* par = nullptr) {
-    if (env_has_params(KS)) {
-        if (env_is<KS, DRIL_ENV_CARTPOLE>(env.kind)) return cartpole_step_p(st, a_disc - env.act_start, par, terminated);
-        if (env_is<KS, DRIL_ENV_PENDULUM>(env.kind)) return pendulum_step_p(st, env_unscale_action(env, *a_cont), par);
-        if (env_is<KS, DRIL_ENV_MOUNTAINCAR>(env.kind)) return mountaincar_step_p(st, a_disc - env.act_start, par, terminated);
-        if (env_is<KS, DRIL_ENV_MOUNTAINCAR_CONTINUOUS>(env.kind))
-            return mountaincar_continuous_step_p(st, env_unscale_action(env, *a_cont), par, terminated);
-        return acrobot_step_p(st, a_disc - env.act_start, par, terminated);
+    constexpr bool P = env_has_params(KS);
+    if (env_is<KS, DRIL_ENV_CARTPOLE>(env.kind)) {
+        constexpr EnvParams D = env_param_default(DRIL_ENV_CARTPOLE);
+        return cartpole_step(st, a_disc - env.act_start, cartpole_coef(P ? par : D.v), terminated);
     }
-    if (env_is<KS, DRIL_ENV_CARTPOLE>(env.kind)) return cartpole_step(st, a_disc - env.act_start, terminated);
-    if (env_is<KS, DRIL_ENV_PENDULUM>(env.kind)) return pendulum_step(st, env_unscale_action(env, *a_cont));
-    if (env_is<KS, DRIL_ENV_MOUNTAINCAR>(env.kind)) return mountaincar_step(st, a_disc - env.act_start, terminated);
-    if (env_is<KS, DRIL_ENV_MOUNTAINCAR_CONTINUOUS>(env.kind))
-        return mountaincar_continuous_step(st, env_unscale_action(env, *a_cont), terminated);
-    if (env_is<KS, DRIL_ENV_ACROBOT>(env.kind)) return acrobot_step(st, a_disc - env.act_start, terminated);
+    if (env_is<KS, DRIL_ENV_PENDULUM>(env.kind)) {
+        constexpr PendulumCoef D = pendulum_default_coef();
+        return pendulum_step(st, env_unscale_action(env, *a_cont), P ? pendulum_coef(par) : D);
+    }
+    if (env_is<KS, DRIL_ENV_MOUNTAINCAR>(env.kind)) {
+        constexpr EnvParams D = env_param_default(DRIL_ENV_MOUNTAINCAR);
+        return mountaincar_step(st, a_disc - env.act_start, P ? par : D.v, terminated);
+    }
+    if (env_is<KS, DRIL_ENV_MOUNTAINCAR_CONTINUOUS>(env.kind)) {
+        constexpr EnvParams D = env_param_default(DRIL_ENV_MOUNTAINCAR_CONTINUOUS);
+        return mountaincar_continuous_step(st, env_unscale_action(env, *a_cont), P ? par : D.v, terminated);
+    }
+    if (env_is<KS, DRIL_ENV_ACROBOT>(env.kind)) {
+        const int idx = a_disc - env.act_start;
+        if (!P) return acrobot_step(st, idx, acrobot_dsdt_default, terminated);
+        const AcrobotCoef C = acrobot_coef(par);
+        return acrobot_step(st, idx, [&C](const float* s, float a, float* ds) { acrobot_dsdt(s, a, C, ds); }, terminated);
+    }
     *life = env.life[n];
     const float r = synthetic_step((uint32_t)(env.gid_offset + n), *life, env.seed, terminated);
     *life += 1;

@@ -262,10 +262,12 @@ __global__ void __launch_bounds__(RT_THREADS, MINB) rollout_tc_kernel(const __gr
             if (r_cand) {
                 // Euler step for BOTH pushes: positions, termination and the reset do not depend on the action
                 const float2 scv = *reinterpret_cast<const float2*>(sSCcur + e * 2);
+                constexpr EnvParams D = env_param_default(DRIL_ENV_CARTPOLE);
+                const CartPoleCoef C = cartpole_coef(D.v);
                 float s0[4] = {s4.x, s4.y, s4.z, s4.w}, s1[4] = {s4.x, s4.y, s4.z, s4.w};
                 bool t0, t1;
-                cartpole_step_sc(s0, 0, scv.x, scv.y, &t0);
-                cartpole_step_sc(s1, 1, scv.x, scv.y, &t1);
+                cartpole_step_sc(s0, 0, scv.x, scv.y, C, &t0);
+                cartpole_step_sc(s1, 1, scv.x, scv.y, C, &t1);
                 *reinterpret_cast<float4*>(sCand + e * 8) = make_float4(s0[0], s0[2], s0[1], s0[3]);     // xn, thn, xd(0), thd(0)
                 *reinterpret_cast<float2*>(sCand + e * 8 + 4) = make_float2(s1[1], s1[3]);              // xd(1), thd(1)
             } else if (r_philox) {

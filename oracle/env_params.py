@@ -4,7 +4,7 @@ batches of oracle/envs.py and oracle/classic_envs.py, restated in NumPy fp32 one
 Parameter k of env n during its episode e (the index the RESET stream used for that episode's start state) is
 lo + (hi - lo) * u, three fp32 roundings, u = u01_f32 of Philox block (gid, e, k // 4, TAG_ENV_PARAMS = 6) word k % 4.
 Every reset draws anew; lo == hi is a fixed value.  The derived coefficients are the fixed fp32 sequences of csrc/env.cuh
-(*_step_p); at the default values they equal the folded constants of the unparametrised batches bit for bit.
+(the step functions and their *_coef); at the default values they equal the folded constants of the unparametrised batches bit for bit.
 
 The *ParamBatch classes subclass the unparametrised batches: without param_ranges they are those batches unchanged.
 """
@@ -185,7 +185,7 @@ class MountainCarContinuousParamBatch(_ParamMixin, MountainCarContinuousBatch):
 
 class AcrobotParamBatch(_ParamMixin, AcrobotBatch):
     """(link_length_1 l1, link_mass_1 m1, link_mass_2 m2, link_com_pos_1 lc1, link_com_pos_2 lc2, link_moi I), I1 = I2 = I,
-    g = 9.8, through the coefficients of `coef` (env.cuh acrobot_coef / acrobot_dsdt_p)"""
+    g = 9.8, through the coefficients of `coef` (env.cuh acrobot_coef / acrobot_dsdt)"""
 
     def __init__(self, n_envs, seed=0, max_steps=500, gid_offset=0, act_start=1, param_ranges=None):
         self.n = n_envs

@@ -223,7 +223,7 @@ def _header_params():
     return out
 
 
-def test_parameter_tables_agree():
+def test_parameter_tables_agree_with_env_defaults():
     from dril_b200 import core
     hdr = _header_params()
     assert set(hdr) == set(core.ENV_KINDS)
@@ -233,8 +233,8 @@ def test_parameter_tables_agree():
     assert re.search(r"#define DRIL_ENV_MAX_PARAMS 8\b", open(os.path.join(ROOT, "include", "dril_b200.h")).read())
     assert max(len(v) for v in hdr.values()) <= 8
     # the defaults and counts in the library
-    api = open(os.path.join(ROOT, "dril.jl_b200", "csrc", "api.cu")).read()
-    m = re.search(r"k_env_param_default\[6\]\[DRIL_ENV_MAX_PARAMS\] = \{(.*?\})\};", api, re.S)
+    env = open(os.path.join(ROOT, "dril.jl_b200", "csrc", "env.cuh")).read()
+    m = re.search(r"k_env_param_default\[6\] = \{(.*?\})\};", env, re.S)
     rows = re.findall(r"\{([^{}]*)\}", m.group(1))
     assert len(rows) == len(core.ENV_KINDS)
     by_id = {v: k for k, v in core.ENV_KINDS.items()}
