@@ -80,6 +80,8 @@ PROTOTYPES = {
     "dril_env_set_observe_params": [P, c_i32],
     "dril_env_obs_dim": [P, C.POINTER(c_i32)],
     "dril_env_set_obs_history": [P, c_i32, c_i32],
+    "dril_env_set_obs_noise": [P, c_i32, P],
+    "dril_env_set_action_delay": [P, P],
     "dril_policy_create": [P, c_i32, c_i32, P, c_i32, c_i32, c_i32, P, P, C.POINTER(P)],
     "dril_policy_destroy": [P],
     "dril_policy_num_params": [P, C.POINTER(c_i64)],

@@ -30,7 +30,7 @@ def _rewrap(env, **over):
                 normalize=env.normalize, gid_offset=env.gid_offset, scaling=env.scaling,
                 obs_shape=env.obs_shape if len(env.obs_shape) > 1 else None, env_params=env.env_param_ranges(),
                 observe_params=env.observes_params(), history_len=env.history_len(),
-                mask_velocities=env.masks_velocities())
+                mask_velocities=env.masks_velocities(), obs_noise=env.obs_noise(), action_delay=env.action_delay())
     args.update(over)
     kind, n = args.pop("kind"), args.pop("n_envs")
     st, steps = env.get_state()

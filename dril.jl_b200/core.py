@@ -36,6 +36,9 @@ def observation_space_with_params(space, kind):
 VELOCITY_FREE = {"cartpole": (0, 2), "pendulum": (0, 1), "mountaincar": (0,), "mountaincar_continuous": (0,),
                  "acrobot": (0, 1, 2, 3)}
 MAX_HISTORY = 4
+MAX_ACTION_DELAY = 4
+# components of each kind's base observation: the rows of an observation-noise array
+BASE_OBS_DIM = {"cartpole": 4, "pendulum": 3, "mountaincar": 2, "mountaincar_continuous": 2, "acrobot": 6}
 
 
 def observation_space_with_history(space, kind, history_len, mask_velocities):
@@ -153,7 +156,7 @@ class CudaBatchedEnv:
 
     def __init__(self, kind, n_envs, max_steps=0, obs_dim=0, act_start=1, seed=None, ctx=None,
                  monitor_window=0, normalize=None, gid_offset=0, obs_shape=None, scaling=False, env_params=None,
-                 observe_params=False, history_len=1, mask_velocities=False):
+                 observe_params=False, history_len=1, mask_velocities=False, obs_noise=None, action_delay=0):
         self.kind = kind.lower()
         assert self.kind in ENV_KINDS, f"unknown env kind {kind}"
         self.ctx = ctx or Context.default()
@@ -228,6 +231,11 @@ class CudaBatchedEnv:
         self._param_ranges = None
         if env_params:
             self.set_env_params(**env_params)
+        self._obs_noise = self._action_delay = None
+        if obs_noise is not None:
+            self.set_obs_noise(obs_noise)
+        if np.any(np.asarray(action_delay) != 0):
+            self.set_action_delay(action_delay)
         if seed is not None:
             self.seed(seed)
             self.reset()
@@ -314,6 +322,46 @@ class CudaBatchedEnv:
     def masks_velocities(self):
         """True if every frame keeps only the non-velocity components (VELOCITY_FREE)."""
         return self._mask_velocities
+
+    # ---- observation noise and action delay ----
+    def set_obs_noise(self, std):
+        """Per-env observation noise (sensor noise).  `std`: a scalar, an (F0,) vector with one deviation per component of the
+        base observation, or an (F0, n_envs) array (F0 = BASE_OBS_DIM[kind]); None turns the noise off.  Component j of every
+        observation gets std[j][n] * z added to its raw value (before Scaling, the velocity mask and the history), z ~ N(0, 1)
+        a pure function of (seed, env, episode, step, j).  Takes effect at the next observation."""
+        if std is None:
+            L.check(self.ctx.lib.dril_env_set_obs_noise(self.h, 0, None))
+            self._obs_noise = None
+            return
+        a = np.asarray(std, np.float32)
+        if a.ndim == 0:
+            a = np.full((BASE_OBS_DIM.get(self.kind, 0), self.n_envs), a, np.float32)
+        elif a.ndim == 1:
+            a = np.repeat(a[:, None], self.n_envs, axis=1)
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        assert a.ndim == 2 and a.shape[1] == self.n_envs, f"obs_noise of shape {a.shape}: need (F0, {self.n_envs})"
+        L.check(self.ctx.lib.dril_env_set_obs_noise(self.h, a.shape[0], L.ptr(a)))
+        self._obs_noise = a.copy()
+
+    def set_action_delay(self, delay):
+        """Per-env action delay (actuation delay): an int or an (n_envs,) array of d in [0, MAX_ACTION_DELAY]; env n applies
+        the action chosen d steps earlier in its episode (the first action after a reset fills its queue).  None turns the
+        delay off.  Restarts every env's queue."""
+        if delay is None:
+            L.check(self.ctx.lib.dril_env_set_action_delay(self.h, None))
+            self._action_delay = None
+            return
+        d = np.ascontiguousarray(np.broadcast_to(np.asarray(delay, np.int32), (self.n_envs,)), dtype=np.int32)
+        L.check(self.ctx.lib.dril_env_set_action_delay(self.h, L.ptr(d)))
+        self._action_delay = d.copy()
+
+    def obs_noise(self):
+        """(F0, n_envs) float32 standard deviations, or None without observation noise."""
+        return None if self._obs_noise is None else self._obs_noise.copy()
+
+    def action_delay(self):
+        """(n_envs,) int32 delays, or 0 without action delay."""
+        return 0 if self._action_delay is None else self._action_delay.copy()
 
     # ---- per-env physical parameters ----
     def observes_params(self):

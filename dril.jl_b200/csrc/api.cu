@@ -102,10 +102,13 @@ static bool tc_eligible(const PolicyDesc& pd) {
 
 // the kind sets the rollout kernels are instantiated for (env.cuh): CartPole, Pendulum and the synthetic env run the ones built
 // for those kinds alone, every other kind the ones built for all kinds, each plain, with per-env parameters (dril_env_set_params),
-// observing its parameters (dril_env_set_observe_params) or with an observation history (dril_env_set_obs_history)
+// observing its parameters (dril_env_set_observe_params) or with an observation history (dril_env_set_obs_history), and the
+// last two with observation noise or action delay (dril_env_set_obs_noise, dril_env_set_action_delay)
 static constexpr unsigned k_kind_sets[] = {
     ENV_KS_CLASSIC, env_param_kind_set(DRIL_ENV_CARTPOLE), env_obs_param_kind_set(DRIL_ENV_CARTPOLE), env_hist_kind_set(DRIL_ENV_CARTPOLE),
-    ENV_KS_ALL, env_param_kind_set(DRIL_ENV_ACROBOT), env_obs_param_kind_set(DRIL_ENV_ACROBOT), env_hist_kind_set(DRIL_ENV_ACROBOT)};
+    ENV_KS_ALL, env_param_kind_set(DRIL_ENV_ACROBOT), env_obs_param_kind_set(DRIL_ENV_ACROBOT), env_hist_kind_set(DRIL_ENV_ACROBOT),
+    env_perturb_kind_set(DRIL_ENV_CARTPOLE), env_hist_perturb_kind_set(DRIL_ENV_CARTPOLE),
+    env_perturb_kind_set(DRIL_ENV_ACROBOT), env_hist_perturb_kind_set(DRIL_ENV_ACROBOT)};
 // f(std::integral_constant<unsigned, KS>) for the entry KS == ks of k_kind_sets (nullptr for a kind set not in the list)
 template <class F, size_t... I>
 static void* ks_pick(unsigned ks, F f, std::index_sequence<I...>) {
@@ -259,12 +262,15 @@ struct dril_env {
     long long* norm_snap_cnt = nullptr;
     unsigned obs_ks = 0;             // ENV_KS_OBS_PARAMS (dril_env_set_observe_params), ENV_KS_HISTORY (dril_env_set_obs_history:
                                      // k > 1 or velocities masked) or 0: the observation layout, as a kind-set bit
-    bool default_params = false;     // parameters held at lo = hi = the defaults only because obs_ks is set
+    bool default_params = false;     // parameters held at lo = hi = the defaults only because obs_ks is set or the env is perturbed
     bool observed = false;           // an observation was made (observe, step, rollout, evaluate): the width is fixed
 };
+// observation noise or action delay on: the ENV_KS_PERTURB kernels
+static bool env_perturbed(const dril_env* e) { return e->d.obs_noise || e->d.act_delay; }
 // the kind set whose kernels run env e (one of k_kind_sets)
 static unsigned env_ks(const dril_env* e) {
     const int kind = e->d.kind;
+    if (env_perturbed(e)) return env_param_kind_set(kind) | e->obs_ks | ENV_KS_PERTURB;
     return e->obs_ks ? env_param_kind_set(kind) | e->obs_ks : e->d.has_params ? env_param_kind_set(kind) : env_kind_set(kind);
 }
 
@@ -1015,7 +1021,7 @@ extern "C" int32_t dril_policy_predict_values(dril_policy* p, const float* obs, 
 // env
 // ---------------------------------------------------------------------------------------
 static int32_t env_alloc_obs_arrays(dril_env* e);
-static int32_t env_hist_refill(dril_env* e);
+static int32_t env_restart(dril_env* e);
 extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, int32_t max_steps, int32_t obs_dim,
                                    int32_t act_start, int64_t gid_offset, const dril_norm_cfg* norm,
                                    int32_t monitor_window, dril_env** out) {
@@ -1103,16 +1109,18 @@ static int32_t env_alloc_obs_arrays(dril_env* e) {
     DRIL_TRY(dmalloc(&e->compat_obs, n * D));
     if (d.hist_len > 1) {
         DRIL_TRY(dmalloc(&d.hist, n * (size_t)(d.hist_len - 1) * d.frame_dim));
-        DRIL_TRY(env_hist_refill(e));
+        DRIL_TRY(env_restart(e));
     }
     return DRIL_OK;
 }
-// every env's observation history restarted from its current frame (no-op without a history store)
-static int32_t env_hist_refill(dril_env* e) {
-    if (!e->d.hist) return DRIL_OK;
+// every env's observation history restarted from its current frame and its action queue restarted (no-op without either)
+static int32_t env_restart(dril_env* e) {
+    if (!e->d.hist && !e->d.act_delay) return DRIL_OK;
     dril_ctx* c = e->ctx;
     Span sp(c, DRIL_K_ENV);
-    env_hist_fill_kernel<<<(unsigned)((e->d.n_envs + 255) / 256), 256, 0, c->stream>>>(e->d);
+    const unsigned grid = (unsigned)((e->d.n_envs + 255) / 256);
+    if (env_perturbed(e)) env_perturb_restart_kernel<<<grid, 256, 0, c->stream>>>(e->d);   // noisy frames, queues
+    else env_hist_fill_kernel<<<grid, 256, 0, c->stream>>>(e->d);
     DRIL_CUDA(cudaGetLastError());
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
     return DRIL_OK;
@@ -1130,7 +1138,7 @@ extern "C" int32_t dril_env_destroy(dril_env* e) {
     void* ps[] = {d.state, d.steps, d.episode, d.life, d.tobs, d.old_obs, d.old_rewards, d.ep_ret, d.ep_len, d.roll_sums,
                   d.roll_eps, d.ret, d.obs_mean, d.obs_var, d.ret_stats, d.counts, d.partials, e->ring.ret, e->ring.len,
                   e->ring.head, e->compat_actions, e->compat_obs, e->roll_moments, e->xr, e->norm_snap, e->norm_snap_cnt,
-                  d.pval, d.plo, d.phi, d.hist};
+                  d.pval, d.plo, d.phi, d.hist, d.obs_noise, d.act_delay, d.act_q};
     for (void* p : ps) if (p) cudaFree(p);
     dril_buffer_destroy(e->compat);
     delete e;
@@ -1157,7 +1165,7 @@ extern "C" int32_t dril_env_reset(dril_env* e) {
         DRIL_CUDA(cudaGetLastError());
     }
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
-    return env_hist_refill(e);
+    return env_restart(e);
 }
 extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const float* lo, const float* hi) {
     DRIL_REQUIRE(e, "NULL argument");
@@ -1169,7 +1177,7 @@ extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const floa
     DRIL_CUDA(cudaSetDevice(c->device));
     const size_t n = (size_t)d.n_envs;
     std::vector<float> dflt;
-    if (!lo && e->obs_ks) {   // observed parameters / history stay: back to lo = hi = the built-in constants
+    if (!lo && (e->obs_ks || env_perturbed(e))) {   // observed parameters / history / perturbation stay: back to lo = hi = the defaults
         dflt.resize(n * np);
         for (int k = 0; k < np; ++k) std::fill(dflt.begin() + (size_t)k * n, dflt.begin() + (size_t)(k + 1) * n, env_param_default(d.kind).v[k]);
         lo = hi = dflt.data();
@@ -1226,9 +1234,15 @@ extern "C" int32_t dril_env_get_params(dril_env* e, int32_t n_params, float* val
     return DRIL_OK;
 }
 
+// An env with an observation layout option, observation noise or action delay runs the parametrised kernels: without ranges it
+// holds lo = hi = the defaults, which it drops again with the last such option.
+static int32_t env_hold_default_params(dril_env* e) {
+    const bool need = e->obs_ks || env_perturbed(e);
+    if ((need && !e->d.has_params) || (!need && e->default_params)) DRIL_TRY(dril_env_set_params(e, env_n_params(e->d.kind), nullptr, nullptr));
+    return DRIL_OK;
+}
 // the observation layout: obs_ks (0, ENV_KS_OBS_PARAMS or ENV_KS_HISTORY), the history's k and frame width, the observation width
-// and the obs-sized arrays.  An env with either option runs the parametrised kernels: without ranges it holds lo = hi = the
-// defaults, which it drops again with the option.
+// and the obs-sized arrays
 static int32_t env_set_obs_layout(dril_env* e, unsigned obs_ks, int hist_len, int frame_dim) {
     EnvDev& d = e->d;
     const int np = env_n_params(d.kind);
@@ -1238,7 +1252,7 @@ static int32_t env_set_obs_layout(dril_env* e, unsigned obs_ks, int hist_len, in
     d.hist_len = hist_len;
     d.frame_dim = frame_dim;
     d.obs_dim = frame_dim * hist_len + (obs_ks == ENV_KS_OBS_PARAMS ? np : 0);
-    if ((obs_ks && !d.has_params) || (!obs_ks && e->default_params)) DRIL_TRY(dril_env_set_params(e, np, nullptr, nullptr));
+    DRIL_TRY(env_hold_default_params(e));
     return env_alloc_obs_arrays(e);
 }
 extern "C" int32_t dril_env_set_observe_params(dril_env* e, int32_t on) {
@@ -1246,6 +1260,7 @@ extern "C" int32_t dril_env_set_observe_params(dril_env* e, int32_t on) {
     EnvDev& d = e->d;
     if (env_n_params(d.kind) == 0) { dril_set_error("env kind %d has no physical parameters to observe", d.kind); return DRIL_ERR_UNSUPPORTED; }
     if (on && e->obs_ks == ENV_KS_HISTORY) { dril_set_error("observe_params cannot be combined with an observation history"); return DRIL_ERR_UNSUPPORTED; }
+    if (on && env_perturbed(e)) { dril_set_error("observe_params cannot be combined with observation noise or action delay"); return DRIL_ERR_UNSUPPORTED; }
     DRIL_REQUIRE(!e->observed, "observe_params can only change before the env's first observation");
     if ((on != 0) == (e->obs_ks == ENV_KS_OBS_PARAMS)) return DRIL_OK;
     return env_set_obs_layout(e, on ? ENV_KS_OBS_PARAMS : 0u, 1, env_base_obs_dim(d.kind));
@@ -1261,6 +1276,61 @@ extern "C" int32_t dril_env_set_obs_history(dril_env* e, int32_t history_len, in
     if (history_len == d.hist_len && frame_dim == d.frame_dim) return DRIL_OK;
     DRIL_REQUIRE(!e->observed, "the observation history can only change before the env's first observation");
     return env_set_obs_layout(e, on ? ENV_KS_HISTORY : 0u, history_len, frame_dim);
+}
+extern "C" int32_t dril_env_set_obs_noise(dril_env* e, int32_t n_comp, const float* std) {
+    DRIL_REQUIRE(e, "NULL argument");
+    EnvDev& d = e->d;
+    if (env_n_params(d.kind) == 0) { dril_set_error("env kind %d has no observation noise", d.kind); return DRIL_ERR_UNSUPPORTED; }
+    if (std && e->obs_ks == ENV_KS_OBS_PARAMS) { dril_set_error("observation noise cannot be combined with observe_params"); return DRIL_ERR_UNSUPPORTED; }
+    const int D0 = env_base_obs_dim(d.kind);
+    const size_t n = (size_t)d.n_envs;
+    if (std) {
+        DRIL_REQUIRE(n_comp == D0, "env kind %d has %d observation components, got %d", d.kind, D0, n_comp);
+        for (size_t i = 0; i < (size_t)D0 * n; ++i)
+            DRIL_REQUIRE(std::isfinite(std[i]) && std[i] >= 0.f, "noise std %g of component %zu, env %zu is not finite and >= 0",
+                         (double)std[i], i / n, i % n);
+    }
+    DRIL_CUDA(cudaSetDevice(e->ctx->device));
+    DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
+    if (!std) {
+        if (d.obs_noise) cudaFree(d.obs_noise);
+        d.obs_noise = nullptr;
+        return env_hold_default_params(e);
+    }
+    if (!d.obs_noise) DRIL_TRY(dmalloc(&d.obs_noise, (size_t)D0 * n));
+    DRIL_CUDA(cudaMemcpy(d.obs_noise, std, (size_t)D0 * n * 4, cudaMemcpyHostToDevice));
+    return env_hold_default_params(e);
+}
+extern "C" int32_t dril_env_set_action_delay(dril_env* e, const int32_t* delay) {
+    DRIL_REQUIRE(e, "NULL argument");
+    EnvDev& d = e->d;
+    if (env_n_params(d.kind) == 0) { dril_set_error("env kind %d has no action delay", d.kind); return DRIL_ERR_UNSUPPORTED; }
+    if (delay && e->obs_ks == ENV_KS_OBS_PARAMS) { dril_set_error("action delay cannot be combined with observe_params"); return DRIL_ERR_UNSUPPORTED; }
+    const size_t n = (size_t)d.n_envs;
+    int max_delay = 0;
+    if (delay) {
+        for (size_t i = 0; i < n; ++i) {
+            DRIL_REQUIRE(delay[i] >= 0 && delay[i] <= DRIL_ENV_MAX_ACTION_DELAY, "delay %d of env %zu outside [0, %d]", delay[i], i,
+                         DRIL_ENV_MAX_ACTION_DELAY);
+            max_delay = std::max(max_delay, (int)delay[i]);
+        }
+    }
+    DRIL_CUDA(cudaSetDevice(e->ctx->device));
+    DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
+    d.max_delay = max_delay;
+    if (!delay) {
+        for (void* p : {(void*)d.act_delay, (void*)d.act_q}) if (p) cudaFree(p);
+        d.act_delay = nullptr; d.act_q = nullptr;
+        return env_hold_default_params(e);
+    }
+    if (!d.act_delay) {
+        DRIL_TRY(dmalloc(&d.act_delay, n));
+        DRIL_TRY(dmalloc(&d.act_q, (size_t)DRIL_ENV_MAX_ACTION_DELAY * n));
+    }
+    std::vector<int32_t> dq(delay, delay + n);   // every queue restarts: the next action fills it
+    for (int32_t& v : dq) v |= ENV_DELAY_RESTART;
+    DRIL_CUDA(cudaMemcpy(d.act_delay, dq.data(), n * 4, cudaMemcpyHostToDevice));
+    return env_hold_default_params(e);
 }
 extern "C" int32_t dril_env_obs_dim(dril_env* e, int32_t* obs_dim) {
     DRIL_REQUIRE(e && obs_dim, "NULL argument");
@@ -1390,7 +1460,7 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
         static const int f_threads = getenv("DRIL_FAST_THREADS") ? atoi(getenv("DRIL_FAST_THREADS")) : 0;
         if (f_threads >= tq && f_threads <= DRIL_THREADS && f_threads % tq == 0) threads = f_threads;
         bool ws = true;
-        const int hist_rows = env_history(ks) ? d.obs_dim - d.frame_dim : 0;
+        const int hist_rows = (env_history(ks) ? d.obs_dim - d.frame_dim : 0) + (d.act_delay ? d.max_delay : 0);   // + action queues
         auto tot = [&](int m4, int th, bool w) { return rollout_fast_smem_layout(a.pd, m4, th, w, hist_rows).total; };
         if (tot(M4, threads, true) > DRIL_SMEM_MAX) ws = false;
         while (M4 > 8 && tot(M4, threads, ws) > DRIL_SMEM_MAX) M4 >>= 1;
@@ -1578,7 +1648,7 @@ extern "C" int32_t dril_env_set_state(dril_env* e, const float* state, const int
     if (state && e->d.state_dim) DRIL_CUDA(cudaMemcpyAsync(e->d.state, state, (size_t)e->d.n_envs * e->d.state_dim * 4, cudaMemcpyHostToDevice, c->stream));
     if (steps) DRIL_CUDA(cudaMemcpyAsync(e->d.steps, steps, (size_t)e->d.n_envs * 4, cudaMemcpyHostToDevice, c->stream));
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
-    return env_hist_refill(e);
+    return env_restart(e);
 }
 extern "C" int32_t dril_env_get_norm_stats(dril_env* e, float* obs_mean, float* obs_var, int64_t* obs_count,
                                            float* ret_mean, float* ret_var, int64_t* ret_count) {
@@ -1621,7 +1691,7 @@ extern "C" int32_t dril_env_set_scaling(dril_env* e, int32_t on, const float* ob
                                         const float* act_high) {
     DRIL_REQUIRE(e, "NULL argument");
     // frames change with the mapping: an observation history restarts from the mapped frame
-    if (!on) { e->d.scaling = 0; return env_hist_refill(e); }
+    if (!on) { e->d.scaling = 0; return env_restart(e); }
     DRIL_REQUIRE(obs_low && obs_high && act_low && act_high, "NULL bounds");
     // ScalingWrapperEnv needs Box observation and action spaces (scalingWrapperEnv.jl:22): of the built-in envs that is Pendulum
     DRIL_REQUIRE(e->d.kind == DRIL_ENV_PENDULUM || e->d.kind == DRIL_ENV_MOUNTAINCAR_CONTINUOUS,
@@ -1637,7 +1707,7 @@ extern "C" int32_t dril_env_set_scaling(dril_env* e, int32_t on, const float* ob
     e->d.sc_act_f = 2.0f / (act_high[0] - act_low[0]);                            // :42-44
     e->d.sc_act_o = act_low[0];
     e->d.scaling = 1;
-    return env_hist_refill(e);
+    return env_restart(e);
 }
 extern "C" int32_t dril_env_get_original(dril_env* e, float* obs_out, float* rewards_out) {
     DRIL_REQUIRE(e, "NULL argument");

@@ -107,6 +107,12 @@ struct EnvDev {
     // their 16-byte alignment, and with it the existing kernels' code.)
     int hist_len, frame_dim;
     float* hist;                // [(hist_len - 1) * frame_dim][n] the older frames of the stack, oldest first
+    // observation noise and action delay (env.cuh, ENV_KS_PERTURB); each null while off.  (32 bytes: 16-byte alignment kept.)
+    float* obs_noise;           // [base obs dim][n] standard deviations
+    int* act_delay;             // [n] delay d | ENV_DELAY_RESTART while the queue waits for its first action
+    float* act_q;               // [DRIL_ENV_MAX_ACTION_DELAY][n] the queued env-space actions, oldest first
+    int max_delay;              // the largest d (rows of the fast kernel's shared-memory queue)
+    int pad_;
 };
 
 struct BufDev {
@@ -129,6 +135,7 @@ struct BufDev {
 #define DRIL_TAG_SHUFFLE 4u
 #define DRIL_TAG_SYN_DYN 5u
 #define DRIL_TAG_ENV_PARAMS 6u
+#define DRIL_TAG_OBS_NOISE 7u
 
 __host__ __device__ __forceinline__ void philox4x32(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                      unsigned long long seed, uint32_t out[4]) {

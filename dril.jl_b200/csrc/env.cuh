@@ -20,14 +20,17 @@
 
 // kind-set bits beyond the kinds: ENV_KS_PARAMS = per-env physical parameters (below); ENV_KS_OBS_PARAMS (only together with
 // ENV_KS_PARAMS) = observations [base observation | the running episode's parameter values in table order]; ENV_KS_HISTORY
-// (only together with ENV_KS_PARAMS) = observations [f_{t-k+1} | ... | f_t], the last k frames (env_frame), k = hist_len
+// (only together with ENV_KS_PARAMS) = observations [f_{t-k+1} | ... | f_t], the last k frames (env_frame), k = hist_len;
+// ENV_KS_PERTURB (only together with ENV_KS_PARAMS, not with ENV_KS_OBS_PARAMS) = observation noise and action delay (below)
 #define ENV_KS_PARAMS (1u << 16)
 #define ENV_KS_OBS_PARAMS (1u << 17)
 #define ENV_KS_HISTORY (1u << 18)
+#define ENV_KS_PERTURB (1u << 19)
 
 __host__ __device__ constexpr bool env_in(unsigned ks, int kind) { return (ks >> kind) & 1u; }
 __host__ __device__ constexpr bool env_obs_params(unsigned ks) { return (ks & ENV_KS_OBS_PARAMS) != 0; }
 __host__ __device__ constexpr bool env_history(unsigned ks) { return (ks & ENV_KS_HISTORY) != 0; }
+__host__ __device__ constexpr bool env_perturb(unsigned ks) { return (ks & ENV_KS_PERTURB) != 0; }
 __host__ __device__ constexpr int env_n_params(int kind) {
     return kind == DRIL_ENV_CARTPOLE || kind == DRIL_ENV_ACROBOT ? 6
          : kind == DRIL_ENV_PENDULUM ? 4
@@ -82,13 +85,76 @@ __device__ __forceinline__ void env_raw_obs_block(int kind, const float* st, int
     }
 }
 
+// ---------------------------------------------------------------------------------------
+// Observation noise and action delay (ENV_KS_PERTURB; dril_b200.h has the rules).  Component j of the base observation of env n
+// in its episode e after s steps of it is o_j + sigma[j][n] z_j, z_j a standard normal of Philox block (gid, e, 2 s + j / 4,
+// DRIL_TAG_OBS_NOISE) word pair (j / 2) % 2 through Box-Muller in fp64 with one rounding to fp32 (like sincos_rn: the fp64 value
+// is far closer to the fp32 result than fp32's rounding steps, so oracle/env_perturb.py reproduces it bit for bit).  The noise is
+// added to the raw observation, before Scaling and the velocity mask.
+// ---------------------------------------------------------------------------------------
+// whose observation a kernel builds: env n, in its episode e (the index of its reset draw), after s steps of that episode
+struct EnvObsAt { long long n; uint32_t e, s; };
+template <unsigned KS>
+__device__ __forceinline__ EnvObsAt env_obs_at(const EnvDev& env, long long n) {
+    if (!env_perturb(KS)) return {};
+    return {n, env.episode[n] - 1u, (uint32_t)env.steps[n]};
+}
+// o[0 .. 3] (raw components 4b .. 4b+3) plus their noise; components beyond the base width and those with sigma 0 are untouched
+__device__ __forceinline__ void env_obs_noise_block(const EnvDev& env, const EnvObsAt& at, int b, float* o) {
+    if (!env.obs_noise) return;
+    const int D0 = env_base_obs_dim(env.kind);
+    uint32_t x[4];
+    philox4x32((uint32_t)(env.gid_offset + at.n), at.e, 2u * at.s + (uint32_t)b, DRIL_TAG_OBS_NOISE, env.seed, x);
+#pragma unroll
+    for (int p = 0; p < 2; ++p) {
+        if (4 * b + 2 * p >= D0) break;
+        const float sg0 = env.obs_noise[(size_t)(4 * b + 2 * p) * env.n_envs + at.n];
+        const float sg1 = 4 * b + 2 * p + 1 < D0 ? env.obs_noise[(size_t)(4 * b + 2 * p + 1) * env.n_envs + at.n] : 0.f;
+        if (sg0 == 0.f && sg1 == 0.f) continue;
+        const double r = sqrt(__dmul_rn(-2.0, log((double)u01_f32_open(x[2 * p]))));
+        double sn, cs;
+        sincos(__dmul_rn(6.283185307179586, (double)u01_f32(x[2 * p + 1])), &sn, &cs);
+        if (sg0 != 0.f) o[2 * p] = __fadd_rn(o[2 * p], __fmul_rn(sg0, (float)__dmul_rn(r, cs)));
+        if (sg1 != 0.f) o[2 * p + 1] = __fadd_rn(o[2 * p + 1], __fmul_rn(sg1, (float)__dmul_rn(r, sn)));
+    }
+}
+// ... out of line for the all-kinds instantiations: inlined, the fp64 draw makes ptxas spill 232 bytes in the all-kinds fast
+// kernel (128 registers); out of line it spills in the CartPole / Pendulum one, so those keep it inline
+__device__ __noinline__ void env_obs_noise_block_call(const EnvDev& env, const EnvObsAt& at, int b, float* o) {
+    env_obs_noise_block(env, at, b, o);
+}
+template <unsigned KS>
+__device__ __forceinline__ void env_obs_noise(const EnvDev& env, const EnvObsAt& at, int b, float* o) {
+    if (env_in(KS, DRIL_ENV_ACROBOT)) env_obs_noise_block_call(env, at, b, o);
+    else env_obs_noise_block(env, at, b, o);
+}
+// the action env n applies this step: `a` (the env-space action it chose, a Discrete index as a float) enters its queue q (rows
+// of stride `stride`, oldest first) and the one chosen d steps earlier leaves it.  *dq = d | ENV_DELAY_RESTART after a restart:
+// the first action then fills the queue.
+#define ENV_DELAY_RESTART 8
+__device__ __forceinline__ float env_delay_action(int* dq, float* q, size_t stride, float a) {
+    const int d = *dq & 7;
+    float out = a;
+    if (*dq & ENV_DELAY_RESTART) {
+        for (int i = 0; i < d; ++i) q[(size_t)i * stride] = a;
+        *dq = d;
+    } else if (d > 0) {
+        out = q[0];
+        for (int i = 0; i + 1 < d; ++i) q[(size_t)i * stride] = q[(size_t)(i + 1) * stride];
+        q[(size_t)(d - 1) * stride] = a;
+    }
+    return out;
+}
+
 // observation block b as the wrappers above the env see it: raw, or mapped to [-1, 1] by ScalingWrapperEnv.observe
 // (scalingWrapperEnv.jl:72-75,94-99: `(x - offset) * scale - 1`, three separate fp32 roundings; Box/Box envs of
 // obs_dim <= 4 only, so block 0).
 // ENV_KS_OBS_PARAMS: components D0 .. D0+P-1 (D0 = env_base_obs_dim, P = env_n_params) are par[0 .. P-1], raw; the blocks
 // straddle the boundary (Acrobot's block 1 is (w1, w2, p0, p1)), and Scaling maps only the D0 base components.
+// ENV_KS_PERTURB: plus the noise of `at`.
 template <unsigned KS>
-__device__ __forceinline__ void env_obs_block(const EnvDev& env, const float* st, int b, float* o, const float* par = nullptr) {
+__device__ __forceinline__ void env_obs_block(const EnvDev& env, const float* st, int b, float* o, const float* par = nullptr,
+                                              const EnvObsAt& at = {}) {
     if (env_obs_params(KS)) {
         const int D0 = env_base_obs_dim(env.kind), P = env_n_params(env.kind);
         if (4 * b < D0) {
@@ -111,6 +177,7 @@ __device__ __forceinline__ void env_obs_block(const EnvDev& env, const float* st
         return;
     }
     env_raw_obs_block<KS>(env.kind, st, b, o);
+    if (env_perturb(KS)) env_obs_noise<KS>(env, at, b, o);
     if (env.scaling && b == 0) {
 #pragma unroll
         for (int j = 0; j < 4; ++j)
@@ -126,10 +193,12 @@ __device__ __forceinline__ void env_obs_block(const EnvDev& env, const float* st
 // ---------------------------------------------------------------------------------------
 #define ENV_MAX_FRAME 6
 // f[0 .. frame_dim-1]: the base observation as the wrappers below Normalize see it (raw, or mapped by Scaling), without its
-// velocity components when frame_dim says so (env_frame_dim); the components beyond frame_dim are unspecified
+// velocity components when frame_dim says so (env_frame_dim); the components beyond frame_dim are unspecified.  ENV_KS_PERTURB:
+// with the noise of `at` (before Scaling and the mask)
 template <unsigned KS>
-__device__ __forceinline__ void env_frame(const EnvDev& env, const float* st, float* f) {
+__device__ __forceinline__ void env_frame(const EnvDev& env, const float* st, float* f, const EnvObsAt& at = {}) {
     env_raw_obs_block<KS>(env.kind, st, 0, f);
+    if (env_perturb(KS)) env_obs_noise<KS>(env, at, 0, f);
     if (env.scaling) {
         const int D0 = env_base_obs_dim(env.kind);
 #pragma unroll
@@ -138,6 +207,11 @@ __device__ __forceinline__ void env_frame(const EnvDev& env, const float* st, fl
     }
     if (env_in(KS, DRIL_ENV_ACROBOT) && env.kind == DRIL_ENV_ACROBOT) {
         f[4] = st[2]; f[5] = st[3];
+        if (env_perturb(KS)) {
+            float w[4] = {f[4], f[5], 0.f, 0.f};
+            env_obs_noise<KS>(env, at, 1, w);
+            f[4] = w[0]; f[5] = w[1];
+        }
     } else if (env.kind == DRIL_ENV_CARTPOLE && env.frame_dim < 4) {
         f[1] = f[2];   // (x, theta)
     }
@@ -203,6 +277,9 @@ __host__ __device__ constexpr unsigned env_obs_param_kind_set(int kind) { return
 // ... and the one with an observation history (an env with history always runs with parameters: lo = hi = the defaults
 // without ranges)
 __host__ __device__ constexpr unsigned env_hist_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_HISTORY; }
+// ... and the ones with observation noise or action delay (parametrised like a history), without and with a history
+__host__ __device__ constexpr unsigned env_perturb_kind_set(int kind) { return env_param_kind_set(kind) | ENV_KS_PERTURB; }
+__host__ __device__ constexpr unsigned env_hist_perturb_kind_set(int kind) { return env_hist_kind_set(kind) | ENV_KS_PERTURB; }
 
 // the defaults of the table (Gymnasium's constants), by kind
 struct EnvParams { float v[DRIL_ENV_MAX_PARAMS]; };

@@ -318,7 +318,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                     float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
                     for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * N + n0 + tid];
-                    env_frame<KS>(env, st, f);
+                    env_frame<KS>(env, st, f, env_obs_at<KS>(env, n0 + tid));
                 }
                 for (int j = 0; j < H; ++j) sRaw[(size_t)j * ld + tid] = v ? env.hist[(size_t)j * N + n0 + tid] : 0.f;
 #pragma unroll
@@ -339,7 +339,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                             env_load_params(env, n0 + tid, par);
                             env_obs_block<KS>(env, st, b, o, par);
                         } else {
-                            env_obs_block<KS>(env, st, b, o);
+                            env_obs_block<KS>(env, st, b, o, nullptr, env_obs_at<KS>(env, n0 + tid));
                         }
                     }
 #pragma unroll
@@ -468,13 +468,19 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                 uint32_t life = 0;
                 float par[DRIL_ENV_MAX_PARAMS];
                 if (env_has_params(KS)) env_load_params(env, n, par);
+                EnvObsAt at = env_obs_at<KS>(env, n);
                 if (env_history(KS)) {                          // the frame the action was chosen on enters the history
                     float f[ENV_MAX_FRAME];
-                    env_frame<KS>(env, st, f);
+                    env_frame<KS>(env, st, f, at);
                     env_hist_push(env.hist + n, (size_t)N, D - env.frame_dim, env.frame_dim, f);
+                }
+                if (env_perturb(KS) && env.act_delay) {         // the action chosen d steps earlier
+                    const float ad = env_delay_action(env.act_delay + n, env.act_q + n, (size_t)N, env.act_dim ? sEnvAct[tid] : (float)a_disc);
+                    if (env.act_dim) sEnvAct[tid] = ad; else a_disc = (int)ad;
                 }
                 r = env_step<KS>(env, st, n, a_disc, sEnvAct + tid, &life, &term, par);
                 steps += 1;
+                at.s = (uint32_t)steps;
                 const bool trunc = steps >= env.max_steps;
                 const bool done = term || trunc;
                 buf.flags[row + n] = (unsigned char)((term ? 1 : 0) | (trunc ? 2 : 0));
@@ -505,7 +511,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                     } else if (env_history(KS)) {             // the stack that ends in the ended episode's final frame
                         const int F = env.frame_dim, H = D - F;
                         float f[ENV_MAX_FRAME];
-                        env_frame<KS>(env, st, f);
+                        env_frame<KS>(env, st, f, at);
                         for (int j = 0; j < H; ++j) env.tobs[(size_t)n * D + j] = env.hist[(size_t)j * N + n];
 #pragma unroll
                         for (int j = 0; j < ENV_MAX_FRAME; ++j) if (j < F) env.tobs[(size_t)n * D + H + j] = f[j];
@@ -513,7 +519,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
 #pragma unroll
                         for (int b = 0; b < env_obs_blocks(KS); ++b) {
                             float o[4];
-                            env_obs_block<KS>(env, st, b, o, par);   // the ended episode's values: drawn anew below
+                            env_obs_block<KS>(env, st, b, o, par, at);   // the ended episode's values: drawn anew below
 #pragma unroll
                             for (int j = 0; j < 4; ++j) if (4 * b + j < D) env.tobs[(size_t)n * D + 4 * b + j] = o[j];
                         }
@@ -525,9 +531,10 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, float* smem, 
                     if (env_has_params(KS)) env_draw_params(env, n, gid, ep, par);
                     if (env_history(KS)) {
                         float f[ENV_MAX_FRAME];
-                        env_frame<KS>(env, st, f);
+                        env_frame<KS>(env, st, f, EnvObsAt{n, ep, 0u});
                         env_hist_fill(env.hist + n, (size_t)N, D - env.frame_dim, env.frame_dim, f);
                     }
+                    if (env_perturb(KS) && env.act_delay) env.act_delay[n] |= ENV_DELAY_RESTART;
                     env.episode[n] = ep + 1;
                     steps = 0;
                 }
@@ -656,7 +663,7 @@ struct RolloutFastSmem {
     size_t w, x, acta, actc, part, stat, hist, total;   // float offsets; total in bytes
 };
 
-// hist_rows: rows of the tile's observation-history store (ENV_KS_HISTORY), 0 otherwise
+// hist_rows: rows of the tile's observation-history store (ENV_KS_HISTORY) and action queues (ENV_KS_PERTURB), 0 otherwise
 __host__ __device__ inline RolloutFastSmem rollout_fast_smem_layout(const PolicyDesc& pd, int M4, int threads, bool weights_smem,
                                                                    int hist_rows = 0) {
     RolloutFastSmem s;
@@ -684,9 +691,11 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
     const PolicyDesc& pd = a.pd;
     const int D = env.obs_dim, Dp = pd.obs_dim_p, M4 = a.M4, NL = pd.n_layers;
     const long long N = env.n_envs;
-    // ENV_KS_HISTORY: the tile's history store in shared memory for the whole rollout, rows [0, H), written back at the end
+    // ENV_KS_HISTORY: the tile's history store in shared memory for the whole rollout, rows [0, H), written back at the end;
+    // ENV_KS_PERTURB with delays: the tile's action queues likewise, rows [H, H + QR)
     const int F = env_history(KS) ? env.frame_dim : 0, H = env_history(KS) ? D - F : 0;
-    const RolloutFastSmem L = rollout_fast_smem_layout(pd, M4, blockDim.x, WS, H);
+    const int QR = env_perturb(KS) && env.act_delay ? env.max_delay : 0;
+    const RolloutFastSmem L = rollout_fast_smem_layout(pd, M4, blockDim.x, WS, H + QR);
     const int ld = L.ld, S = L.slices;
     float* sX = smem + L.x;
     float* sActA = smem + L.acta;
@@ -695,6 +704,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
     float* sMean = smem + L.stat;
     float* sVar = sMean + Dp;
     float* sHist = smem + L.hist;
+    float* sQ = sHist + (size_t)H * L.ld;
     const int tid = threadIdx.x;
     const float* __restrict__ Wbase = WS ? smem : a.pack;
     if (WS) {
@@ -720,6 +730,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
     float ep_ret = 0.f;
     uint32_t episode = 0;
     float eparam[DRIL_ENV_MAX_PARAMS] = {};   // parameter values of the running episode (ENV_KS_PARAMS)
+    int dq = 0;                                // delay | ENV_DELAY_RESTART (ENV_KS_PERTURB)
     if (mine) {
 #pragma unroll
         for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * N + n];
@@ -728,6 +739,10 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         if (env_has_params(KS)) env_load_params(env, n, eparam);
         if (env.monitor) { ep_ret = env.ep_ret[n]; ep_len = env.ep_len[n]; }
         for (int j = 0; j < H; ++j) sHist[(size_t)j * ld + tid] = env.hist[(size_t)j * N + n];
+        if (QR > 0) {
+            dq = env.act_delay[n];
+            for (int j = 0; j < QR; ++j) sQ[(size_t)j * ld + tid] = env.act_q[(size_t)j * N + n];
+        }
     }
     // output-layer split: thread (e = tid % M4, ks = tid / M4) covers k in [ks*Kc, ks*Kc + Kc)
     const LayerDesc& Lao = pd.L[0][NL - 1];
@@ -743,7 +758,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         if (env_history(KS)) {   // older frames straight from sHist, the newest from the registers: no D-wide register array
             if (tid < M4) {
                 float f[ENV_MAX_FRAME] = {};
-                if (mine) env_frame<KS>(env, st, f);
+                if (mine) env_frame<KS>(env, st, f, EnvObsAt{n, episode - 1u, (uint32_t)steps});
                 for (int j = 0; j < H; ++j) {
                     float x = mine ? sHist[(size_t)j * ld + tid] : 0.f;
                     if (mine && norm_obs) x = normalize_obs_val(x, sMean[j], sVar[j], env.eps, env.clip_obs);
@@ -768,7 +783,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             float o[OW] = {};
             if (mine) {
 #pragma unroll
-                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, o + 4 * b, eparam);
+                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, o + 4 * b, eparam, EnvObsAt{n, episode - 1u, (uint32_t)steps});
                 if (norm_obs) {
 #pragma unroll
                     for (int j = 0; j < OW; ++j) if (j < D) o[j] = normalize_obs_val(o[j], sMean[j], sVar[j], env.eps, env.clip_obs);
@@ -919,8 +934,12 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             uint32_t life = 0;
             if (env_history(KS)) {                               // the frame the action was chosen on enters the history
                 float f[ENV_MAX_FRAME];
-                env_frame<KS>(env, st, f);
+                env_frame<KS>(env, st, f, EnvObsAt{n, episode - 1u, (uint32_t)steps});
                 env_hist_push(sHist + tid, (size_t)ld, H, F, f);
+            }
+            if (QR > 0) {                                        // the action chosen d steps earlier
+                const float ad = env_delay_action(&dq, sQ + tid, (size_t)ld, pd.act_kind == DRIL_ACT_DISCRETE ? (float)a_disc : a_cont);
+                if (pd.act_kind == DRIL_ACT_DISCRETE) a_disc = (int)ad; else a_cont = ad;
             }
             r = env_step<KS & ~(1u << DRIL_ENV_SYNTHETIC)>(env, st, n, a_disc, &a_cont, &life, &term, eparam);   // (no synthetic env here)
             steps += 1;
@@ -949,7 +968,7 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             if (trunc && env_history(KS)) {   // the stack ending in the ended episode's final frame, staged like ENV_KS_OBS_PARAMS
                 trunc_i = 1;
                 float f[ENV_MAX_FRAME];
-                env_frame<KS>(env, st, f);
+                env_frame<KS>(env, st, f, EnvObsAt{n, episode - 1u, (uint32_t)steps});
                 for (int j = 0; j < H; ++j) {
                     float x = sHist[(size_t)j * ld + tid];
                     if (norm_obs) x = normalize_obs_val(x, sMean[j], sVar[j], env.eps, env.clip_obs);
@@ -966,7 +985,8 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
             } else if (trunc) {
                 trunc_i = 1;
 #pragma unroll
-                for (int b = 0; b < OW / 4; ++b) env_obs_block<KS>(env, st, b, tobs + 4 * b, eparam);   // before the redraw below
+                for (int b = 0; b < OW / 4; ++b)   // before the redraw below
+                    env_obs_block<KS>(env, st, b, tobs + 4 * b, eparam, EnvObsAt{n, episode - 1u, (uint32_t)steps});
                 if (norm_obs) {
 #pragma unroll
                     for (int j = 0; j < OW; ++j) if (j < D) tobs[j] = normalize_obs_val(tobs[j], sMean[j], sVar[j], env.eps, env.clip_obs);
@@ -981,9 +1001,10 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
                 if (env_has_params(KS)) env_draw_params(env, n, gid, episode, eparam);
                 if (env_history(KS)) {
                     float f[ENV_MAX_FRAME];
-                    env_frame<KS>(env, st, f);
+                    env_frame<KS>(env, st, f, EnvObsAt{n, episode, 0u});
                     env_hist_fill(sHist + tid, (size_t)ld, H, F, f);
                 }
+                if (env_perturb(KS)) dq |= ENV_DELAY_RESTART;
                 episode += 1;
                 steps = 0;
                 if (env.normalize) env.ret[n] = 0.f;             // normalizeWrapperEnv.jl:153-156
@@ -1019,6 +1040,10 @@ __global__ void __launch_bounds__(DRIL_THREADS) rollout_fast_kernel(const __grid
         env.episode[n] = episode;
         if (env.monitor) { env.ep_ret[n] = ep_ret; env.ep_len[n] = ep_len; }
         for (int j = 0; j < H; ++j) env.hist[(size_t)j * N + n] = sHist[(size_t)j * ld + tid];
+        if (QR > 0) {
+            env.act_delay[n] = dq;
+            for (int j = 0; j < QR; ++j) env.act_q[(size_t)j * N + n] = sQ[(size_t)j * ld + tid];
+        }
     }
 }
 
@@ -1032,6 +1057,22 @@ __global__ void env_hist_fill_kernel(EnvDev env) {
     for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * env.n_envs + n];
     float f[ENV_MAX_FRAME];
     env_frame<ENV_KS_ALL>(env, st, f);
+    env_hist_fill(env.hist + n, (size_t)env.n_envs, (env.hist_len - 1) * env.frame_dim, env.frame_dim, f);
+}
+
+// the action queues of every env restarted, and its observation history refilled from its current (noisy) frame
+// (ENV_KS_PERTURB): reset, set_state, Scaling changed, or delays / the history set
+__global__ void env_perturb_restart_kernel(EnvDev env) {
+    constexpr unsigned KS = ENV_KS_ALL | ENV_KS_PARAMS | ENV_KS_PERTURB;
+    long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= env.n_envs) return;
+    if (env.act_delay) env.act_delay[n] |= ENV_DELAY_RESTART;
+    if (!env.hist) return;
+    float st[ENV_MAX_STATE] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int k = 0; k < ENV_MAX_STATE; ++k) if (k < env.state_dim) st[k] = env.state[(size_t)k * env.n_envs + n];
+    float f[ENV_MAX_FRAME];
+    env_frame<KS>(env, st, f, env_obs_at<KS>(env, n));
     env_hist_fill(env.hist + n, (size_t)env.n_envs, (env.hist_len - 1) * env.frame_dim, env.frame_dim, f);
 }
 

@@ -288,6 +288,37 @@ int32_t dril_env_obs_dim(dril_env* env, int32_t* obs_dim);
 #define DRIL_ENV_MAX_HISTORY 4
 int32_t dril_env_set_obs_history(dril_env* env, int32_t history_len, int32_t mask_velocities);
 
+/* Sensor noise and actuation delay, per env; independent of each other.
+ * Observation noise: std = [n_comp][n_envs] standard deviations sigma >= 0 (finite), n_comp = the base observation width
+ * (cartpole 4, pendulum 3, mountaincar(_continuous) 2, acrobot 6).  Component j of env n's observation, in its episode e (the
+ * index of that episode's reset and parameter draws) after s steps of it, is
+ *   o_j + sigma[j][n] * z_j   (fp32: __fadd_rn(o_j, __fmul_rn(sigma, z_j)); sigma == 0 leaves o_j untouched),
+ * z_j = Box-Muller in fp64 with one rounding to fp32 (r cos th for even j, r sin th for odd j) of Philox block
+ * (gid, e, 2 s + j / 4, DRIL_TAG_OBS_NOISE = 7) word pair (j / 2) % 2 (u1 = u01_f32_open, u2 = u01_f32).
+ *   - A sensor: the noise is added to the raw observation, before ScalingWrapperEnv's map, before the velocity mask and
+ *     before the frame enters an observation history (the history holds the noisy frames the policy saw).  Dynamics,
+ *     rewards, termination and dril_env_get_state use the true state.
+ *   - A pure function of (seed, gid, e, s, j): observe() is idempotent, results do not depend on gid_offset sharding, and
+ *     chunked collection equals one-shot collection.  A truncated step's terminal observation (and V(terminal_obs)) carries
+ *     the noise of (e, max_steps), the observation after the reset that of (e', 0).
+ *   - NormalizeWrapperEnv sees the noisy observation, dril_env_get_original returns it; the observation space is unchanged
+ *     and a noisy value may leave it.  std may change at any time and takes effect at the next observation.
+ * Action delay: delay = [n_envs] d in [0, DRIL_ENV_MAX_ACTION_DELAY].  Env n applies the action chosen d steps earlier in the
+ * same episode: every env keeps a FIFO queue of env-space actions, which an action enters as act! receives it (after
+ * ClampAdapter; ScalingWrapperEnv's map applies to the action that leaves it).
+ *   - The queue restarts at every reset (auto-reset, compat act!, dril_env_reset, dril_evaluate's initial reset), at
+ *     dril_env_set_state, at dril_env_set_scaling and whenever delays are set; the first action after a restart fills it, so
+ *     for the first d steps the env applies that action.  Chunked collection, successive rollouts and compat act! continue it.
+ *   - The rollout buffer keeps the chosen action and its log-prob; forced actions are chosen actions and are delayed too.
+ *     Monitor, Normalize and (terminal) observations are unaffected.
+ * std / delay = NULL turns the option off.  With either on the env runs the parametrised kernels (lo = hi = the defaults
+ * without ranges), so CartPole leaves the tensor-core rollout.  The synthetic env, and an env with observe_params (in either
+ * call order): DRIL_ERR_UNSUPPORTED.  A negative or non-finite sigma, n_comp other than the base width, or a delay outside
+ * [0, DRIL_ENV_MAX_ACTION_DELAY]: DRIL_ERR_INVALID. */
+#define DRIL_ENV_MAX_ACTION_DELAY 4
+int32_t dril_env_set_obs_noise(dril_env* env, int32_t n_comp, const float* std);
+int32_t dril_env_set_action_delay(dril_env* env, const int32_t* delay);
+
 /* ---- actor-critic layer + optimiser state: replaces Discrete/ContinuousActorCriticLayer
  *      (layers/) and the Lux TrainState held by Agent (agents/agent_types.jl) ------------ */
 int32_t dril_policy_create(dril_ctx* ctx, int32_t obs_dim, int32_t n_hidden, const int32_t* hidden_dims,

@@ -84,7 +84,7 @@ const VELOCITY_FREE = Dict(:cartpole => [1, 3], :pendulum => [1, 2], :mountainca
 
 """
     CudaBatchedEnv(kind, n_envs; max_steps, act_start, monitor_window, normalize, env_params, observe_params, history_len,
-                   mask_velocities)
+                   mask_velocities, obs_noise, action_delay)
 
 Device-resident replacement of `NormalizeWrapperEnv(MonitorWrapperEnv(MultiThreadedParallelEnv(envs)))`
 for `kind in (:cartpole, :pendulum, :synthetic, :mountaincar, :mountaincar_continuous, :acrobot)`.
@@ -94,6 +94,7 @@ for `kind in (:cartpole, :pendulum, :synthetic, :mountaincar, :mountaincar_conti
 `history_len = k` (1 to 4): every observation is the last k frames `[f_{t-k+1} | ... | f_t]`, oldest first;
 `mask_velocities = true` keeps only each frame's non-velocity components (`VELOCITY_FREE[kind]`); `observation_space` is the
 (scaled) bounds of the kept components tiled k times.  `reset!` restarts the history from the current frame.
+`obs_noise`, `action_delay`: sensor noise and actuation delay, see `set_obs_noise!` and `set_action_delay!`.
 """
 mutable struct CudaBatchedEnv <: AbstractParallelEnv
     ctx::Context
@@ -110,7 +111,8 @@ end
 
 function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_steps = 0, obs_dim = 0, act_start = 1,
         monitor_window = 0, normalize::Union{Nothing, NormCfg} = nothing, gid_offset = 0, scaling::Bool = false,
-        env_params = nothing, observe_params::Bool = false, history_len::Integer = 1, mask_velocities::Bool = false)
+        env_params = nothing, observe_params::Bool = false, history_len::Integer = 1, mask_velocities::Bool = false,
+        obs_noise = nothing, action_delay = 0)
     obs_space, act_space = if kind == :cartpole
         hi = Float32[4.8, Inf32, 0.41887903, Inf32]
         Box(-hi, hi), Discrete(2, act_start)
@@ -160,6 +162,50 @@ function CudaBatchedEnv(kind::Symbol, n_envs::Integer; ctx = default_ctx(), max_
         falses(n_envs), falses(n_envs))
     finalizer(e -> ccall((:dril_env_destroy, LIB), Int32, (Ptr{Cvoid},), e.h), env)
     isnothing(env_params) || isempty(env_params) || set_env_params!(env; env_params...)
+    isnothing(obs_noise) || set_obs_noise!(env, obs_noise)
+    all(iszero, action_delay) || set_action_delay!(env, action_delay)
+    env
+end
+
+# components of each kind's base observation: the rows of an observation-noise array
+const BASE_OBS_DIM = Dict(:cartpole => 4, :pendulum => 3, :mountaincar => 2, :mountaincar_continuous => 2, :acrobot => 6)
+const MAX_ACTION_DELAY = 4
+
+"""
+    set_obs_noise!(env, std)
+
+Per-env observation (sensor) noise: `std` is a number, a vector of `F0 = BASE_OBS_DIM[kind]` deviations (one per component of
+the base observation) or an `F0 x n_envs` matrix; `nothing` turns it off.  Component j of every observation gets
+`std[j, n] * z` added to its raw value (before Scaling, the velocity mask and the history), `z ~ N(0, 1)` a pure function of
+(seed, env, episode, step, j).  Takes effect at the next observation.
+"""
+function set_obs_noise!(env::CudaBatchedEnv, std)
+    if isnothing(std)
+        check(ccall((:dril_env_set_obs_noise, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{Float32}), env.h, 0, C_NULL))
+        return env
+    end
+    F0 = get(BASE_OBS_DIM, env.kind, 0)
+    s = std isa Number ? fill(Float32(std), F0, env.n_envs) : std isa AbstractVector ? repeat(Float32.(std), 1, env.n_envs) : Float32.(std)
+    size(s, 2) == env.n_envs || error("obs_noise of size $(size(s)): need ($F0, $(env.n_envs))")
+    m = Matrix{Float32}(permutedims(s))   # column j = component j: the C layout [n_comp][n_envs]
+    check(ccall((:dril_env_set_obs_noise, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{Float32}), env.h, size(s, 1), m))
+    env
+end
+
+"""
+    set_action_delay!(env, delay)
+
+Per-env action (actuation) delay: a number or a vector of `n_envs` delays d in `0:MAX_ACTION_DELAY`; env n applies the
+action chosen d steps earlier in its episode (the first action after a reset fills its queue); `nothing` turns it off.
+Restarts every env's queue.
+"""
+function set_action_delay!(env::CudaBatchedEnv, delay)
+    if isnothing(delay)
+        check(ccall((:dril_env_set_action_delay, LIB), Int32, (Ptr{Cvoid}, Ptr{Int32}), env.h, C_NULL))
+        return env
+    end
+    d = delay isa Number ? fill(Int32(delay), env.n_envs) : Int32.(collect(delay))
+    check(ccall((:dril_env_set_action_delay, LIB), Int32, (Ptr{Cvoid}, Ptr{Int32}), env.h, d))
     env
 end
 
