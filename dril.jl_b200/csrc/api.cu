@@ -283,6 +283,7 @@ struct dril_policy {
     unsigned char* f2planes_one = nullptr;   // tensor-core path: one partial plane per CTA
     double* sq_part = nullptr;
     unsigned int* ticket = nullptr;
+    unsigned int* stage_ticket = nullptr;   // PermuteTail::ticket
     int loss_M4 = 0, loss_splits = 1;
     bool loss_ws = true;
     long long* step = nullptr;
@@ -832,7 +833,7 @@ extern "C" int32_t dril_policy_destroy(dril_policy* p) {
     }
     void* ps[] = {p->flat, p->pack, p->m, p->v, p->g, p->gpart, p->flat2pack, p->flat2packT, p->flat2g, p->step,
                   p->iter_acc, p->ev_acc, p->mbstats, p->adv_partial, p->stop_flag, p->scratch, p->f2planes, p->f2planes_one, p->sq_part,
-                  p->ticket, p->ft_tiles, p->ft_recs};
+                  p->ticket, p->stage_ticket, p->ft_tiles, p->ft_recs};
     for (void* q : ps) if (q) cudaFree(q);
     for (int i = 0; i < 3; ++i) if (p->ev[i]) cudaEventDestroy(p->ev[i]);
     for (auto& sl : p->slots) {
@@ -1059,7 +1060,9 @@ extern "C" int32_t dril_env_create(dril_ctx* c, int32_t kind, int64_t n_envs, in
     int w = std::max(d.monitor, 1);
     e->ring.window = w;
     DRIL_TRY(dmalloc(&e->ring.ret, (size_t)w)); DRIL_TRY(dmalloc(&e->ring.len, (size_t)w)); DRIL_TRY(dmalloc(&e->ring.head, 1));
+    DRIL_TRY(dmalloc(&e->ring.ticket, 1));
     DRIL_CUDA(cudaMemset(e->ring.ret, 0, w * 4)); DRIL_CUDA(cudaMemset(e->ring.len, 0, w * 4)); DRIL_CUDA(cudaMemset(e->ring.head, 0, 8));
+    DRIL_CUDA(cudaMemset(e->ring.ticket, 0, 4));
     d.normalize = norm ? 1 : 0;
     if (norm) {
         d.training = norm->training; d.norm_obs = norm->norm_obs; d.norm_reward = norm->norm_reward;
@@ -1137,7 +1140,7 @@ extern "C" int32_t dril_env_destroy(dril_env* e) {
     EnvDev& d = e->d;
     void* ps[] = {d.state, d.steps, d.episode, d.life, d.tobs, d.old_obs, d.old_rewards, d.ep_ret, d.ep_len, d.roll_sums,
                   d.roll_eps, d.ret, d.obs_mean, d.obs_var, d.ret_stats, d.counts, d.partials, e->ring.ret, e->ring.len,
-                  e->ring.head, e->compat_actions, e->compat_obs, e->roll_moments, e->xr, e->norm_snap, e->norm_snap_cnt,
+                  e->ring.head, e->ring.ticket, e->compat_actions, e->compat_obs, e->roll_moments, e->xr, e->norm_snap, e->norm_snap_cnt,
                   d.pval, d.plo, d.phi, d.hist, d.obs_noise, d.act_delay, d.act_q};
     for (void* p : ps) if (p) cudaFree(p);
     dril_buffer_destroy(e->compat);
@@ -1584,8 +1587,9 @@ static int32_t launch_rollout(dril_env* e, dril_policy* p, dril_buffer* b, const
 static int32_t launch_monitor_finalize(dril_env* e, dril_buffer* b) {
     if (!e->d.monitor) return DRIL_OK;
     Span sp(e->ctx, DRIL_K_MONITOR);
-    monitor_finalize_kernel<<<1, 1024, 0, e->ctx->stream>>>(e->ring, b->d.flags, b->d.episode_r, b->d.episode_l,
-                                                            b->d.done_count, b->d.T, b->d.N);
+    const unsigned grid = (unsigned)std::min<long long>(b->d.T, e->ctx->sm_count);    // one CTA per row while T <= the SM count
+    monitor_finalize_kernel<<<grid, MON_THREADS, 0, e->ctx->stream>>>(e->ring, b->d.flags, b->d.episode_r, b->d.episode_l,
+                                                                      b->d.done_count, b->d.T, b->d.N);
     DRIL_CUDA(cudaGetLastError());
     return DRIL_OK;
 }
@@ -1969,11 +1973,18 @@ extern "C" int32_t dril_env_zero_returns(dril_env* e) {
     return DRIL_OK;
 }
 
-// ev_acc4 (optional, zeroed by the caller): the explained-variance moments are accumulated in the same pass
-static int32_t gae_async(dril_ctx* c, const BufDev& d, float gamma, float lambda, double* ev_acc4 = nullptr) {
+// ev_acc4 (optional, zeroed by the caller): the explained-variance moments are accumulated in the same pass.
+// recs (optional, stride from ensure_ft_recs): the same pass writes the sample records of the whole buffer.
+static int32_t gae_async(dril_ctx* c, const BufDev& d, float gamma, float lambda, double* ev_acc4 = nullptr, float* recs = nullptr,
+                         int rec_stride = 0) {
+    const GaeRecords rec = {d.obs, reinterpret_cast<const float*>(d.actions), d.logprobs, recs, d.obs_dim, d.act_dim, rec_stride};
+    const int scan_ctas = (int)((d.N + GAE_THREADS - 1) / GAE_THREADS);
+    const long long n_total = d.T * d.N;
+    const int copy_ctas = recs ? (int)std::min<long long>((n_total + GAE_THREADS - 1) / GAE_THREADS, (long long)c->sm_count * 16) : 0;
     Span sp(c, DRIL_K_GAE);
-    gae_kernel<<<(unsigned)((d.N + 255) / 256), 256, 0, c->stream>>>(d.rewards, d.values, d.flags, d.boot, d.last_values,
-                                                                    d.advantages, d.returns, d.T, d.N, gamma, lambda, ev_acc4);
+    gae_kernel<<<(unsigned)(scan_ctas + copy_ctas), GAE_THREADS, 0, c->stream>>>(d.rewards, d.values, d.flags, d.boot, d.last_values,
+                                                                                d.advantages, d.returns, d.T, d.N, gamma, lambda, ev_acc4,
+                                                                                rec, scan_ctas);
     DRIL_CUDA(cudaGetLastError());
     return DRIL_OK;
 }
@@ -2158,10 +2169,11 @@ static int32_t ft_stage_epoch(dril_policy* p, const BufDev& bd, const FeistelKey
 }
 
 // ALL epochs of an update staged by one launch (both tcgen05 paths), which also leaves the per-minibatch advantage moments in
-// p->adv_partial (layout of adv_stats_kernel with `bpm` blocks per minibatch).  *staged = false (nothing launched) when the tile
-// records of all epochs would not fit the memory budget: the caller then stages epoch by epoch.
+// p->adv_partial (layout of adv_stats_kernel with `bpm` blocks per minibatch) and, as `tail` asks, sums them into mbstats and
+// zeroes the iteration accumulators.  *staged = false (nothing launched) when the tile records of all epochs would not fit the
+// memory budget: the caller then stages epoch by epoch.
 static int32_t ft_stage_epochs(dril_policy* p, const BufDev& bd, const FeistelKeys& fks, int ne, long long n_total, long long batch_size, int bpm,
-                               bool* staged) {
+                               const PermuteTail& tail, bool* staged) {
     dril_ctx* c = p->ctx;
     *staged = false;
     const bool ftg = ftg_active(p);
@@ -2179,9 +2191,10 @@ static int32_t ft_stage_epochs(dril_policy* p, const BufDev& bd, const FeistelKe
     Span sp(c, DRIL_K_PERMUTE);
     const dim3 grid(bpm, n_mb, ne);
     if (ftg) ftg_permute_epochs_kernel<<<grid, 256, 0, c->stream>>>(p->ft_recs, p->ft_rec_stride, bd.obs_dim, fks, n_total, batch_size, tpm, p->pd.act_start,
-                                                                   p->pd.act_n, cont, rf, reinterpret_cast<float*>(p->ft_tiles), epoch_tiles, p->adv_partial);
+                                                                   p->pd.act_n, cont, rf, reinterpret_cast<float*>(p->ft_tiles), epoch_tiles, p->adv_partial,
+                                                                   tail);
     else ft_permute_epochs_kernel<<<grid, 256, 0, c->stream>>>(p->ft_recs, p->ft_rec_stride, fks, n_total, batch_size, tpm, p->pd.act_start, p->pd.act_n,
-                                                               p->ft_tiles, epoch_tiles, p->adv_partial);
+                                                               p->ft_tiles, epoch_tiles, p->adv_partial, tail);
     DRIL_CUDA(cudaGetLastError());
     *staged = true;
     return DRIL_OK;
@@ -2333,6 +2346,10 @@ static int32_t ft_persistent_update(dril_policy* p, const BufDev& bd, const Upda
 }
 
 static int32_t ensure_mbstats(dril_policy* p, int n_mb, int blocks_per_mb) {
+    if (!p->stage_ticket) {
+        DRIL_TRY(dmalloc(&p->stage_ticket, 1));
+        DRIL_CUDA(cudaMemset(p->stage_ticket, 0, 4));
+    }
     if (p->mbstats_cap >= n_mb) return DRIL_OK;
     if (p->mbstats) cudaFree(p->mbstats);
     if (p->adv_partial) cudaFree(p->adv_partial);
@@ -2343,9 +2360,10 @@ static int32_t ensure_mbstats(dril_policy* p, int n_mb, int blocks_per_mb) {
     return DRIL_OK;
 }
 
-// extra / n_extra: a second small fp64 array summed over ranks together with the first batch of advantage moments
+// extra / n_extra: a second small fp64 array summed over ranks together with the first batch of advantage moments.
+// recs_packed: the sample records of a tcgen05 update were already written (by the GAE pass)
 static int32_t update_async(dril_policy* p, dril_buffer* b, const dril_ppo_hyper* h, int epochs, int64_t batch_size,
-                            uint64_t shuffle_seed, uint64_t epoch_counter, double* extra = nullptr, int n_extra = 0) {
+                            uint64_t shuffle_seed, uint64_t epoch_counter, bool recs_packed, double* extra = nullptr, int n_extra = 0) {
     dril_ctx* c = p->ctx;
     const long long n_total = b->d.T * b->d.N;
     DRIL_REQUIRE(batch_size >= 1, "batch_size must be positive");
@@ -2356,9 +2374,17 @@ static int32_t update_async(dril_policy* p, dril_buffer* b, const dril_ppo_hyper
     LossLaunch ll;
     DRIL_TRY(plan_loss(p, &ll));
     const int bpm = (int)std::max<long long>(1, std::min<long long>(64, (std::min<long long>(batch_size, n_total) + 2047) / 2048));
-    if (ftg_active(p) || ft_active(p)) DRIL_TRY(ft_pack_records(p, b->d, n_total));
-    DRIL_CUDA(cudaMemsetAsync(p->iter_acc, 0, 12 * 8, c->stream));   // [12],[13] carry beta^t across iterations
-    DRIL_CUDA(cudaMemsetAsync(p->stop_flag, 0, 4, c->stream));
+    if ((ftg_active(p) || ft_active(p)) && !recs_packed) DRIL_TRY(ft_pack_records(p, b->d, n_total));
+    // iter_acc[0 .. 11] and the stop flag are zeroed before the first kernel that uses them: by the first all-epochs permute
+    // launch where there is one, else here ([12],[13] carry beta^t across iterations)
+    bool acc_zeroed = false;
+    auto zero_acc = [&]() -> int32_t {
+        if (acc_zeroed) return DRIL_OK;
+        DRIL_CUDA(cudaMemsetAsync(p->iter_acc, 0, 12 * 8, c->stream));
+        DRIL_CUDA(cudaMemsetAsync(p->stop_flag, 0, 4, c->stream));
+        acc_zeroed = true;
+        return DRIL_OK;
+    };
     // minibatch advantage moments of up to DRIL_MAX_EPOCHS_BATCHED epochs per launch / allreduce
     for (int e0 = 0; e0 < epochs; e0 += DRIL_MAX_EPOCHS_BATCHED) {
         const int ne = std::min(DRIL_MAX_EPOCHS_BATCHED, epochs - e0);
@@ -2368,9 +2394,15 @@ static int32_t update_async(dril_policy* p, dril_buffer* b, const dril_ppo_hyper
         for (int e = ne; e < DRIL_MAX_EPOCHS_BATCHED; ++e) fks.k[e] = fks.k[0];
         // tcgen05 paths: the tile records of all `ne` epochs and the advantage moments come from one launch
         bool staged_all = false;
-        if (ftg_active(p) || ft_active(p)) DRIL_TRY(ft_stage_epochs(p, b->d, fks, ne, n_total, batch_size, bpm, &staged_all));
-        if (hp.normalize_advantage) {
-            if (!staged_all) {
+        if (ftg_active(p) || ft_active(p)) {
+            const PermuteTail tail = {hp.normalize_advantage ? p->mbstats : nullptr, p->stage_ticket, acc_zeroed ? nullptr : p->iter_acc,
+                                      p->stop_flag};
+            DRIL_TRY(ft_stage_epochs(p, b->d, fks, ne, n_total, batch_size, bpm, tail, &staged_all));
+            acc_zeroed = acc_zeroed || staged_all;
+        }
+        DRIL_TRY(zero_acc());
+        if (hp.normalize_advantage && !staged_all) {      // (the all-epochs permute launch finished the moments)
+            {
                 Span sp(c, DRIL_K_ADV_STATS);
                 adv_stats_kernel<<<dim3(bpm, n_mb, ne), 256, 0, c->stream>>>(b->d.advantages, n_total, batch_size, fks, 0, p->adv_partial);
                 DRIL_CUDA(cudaGetLastError());
@@ -2380,6 +2412,8 @@ static int32_t update_async(dril_policy* p, dril_buffer* b, const dril_ppo_hyper
                 adv_stats_finalize_kernel<<<(n_mb * ne * 2 + 127) / 128, 128, 0, c->stream>>>(p->adv_partial, bpm, n_mb * ne, p->mbstats);
                 DRIL_CUDA(cudaGetLastError());
             }
+        }
+        if (hp.normalize_advantage) {
             DRIL_TRY(allreduce_small(c, p->mbstats, n_mb * ne * 2, extra, n_extra));
             n_extra = 0;
         }
@@ -2406,6 +2440,7 @@ static int32_t update_async(dril_policy* p, dril_buffer* b, const dril_ppo_hyper
         }
     }
     p->ft_epoch_tile0 = 0;
+    DRIL_TRY(zero_acc());      // epochs == 0
     if (n_extra) DRIL_TRY(allreduce_small(c, nullptr, 0, extra, n_extra));   // no advantage moments were exchanged
     return DRIL_OK;
 }
@@ -2493,7 +2528,7 @@ extern "C" int32_t dril_ppo_update(dril_policy* p, dril_buffer* b, const dril_pp
     DRIL_CUDA(cudaSetDevice(c->device));
     p->last_lr = h->learning_rate;
     DRIL_CUDA(cudaEventRecord(p->ev[1], c->stream));
-    DRIL_TRY(update_async(p, b, h, epochs, batch_size, shuffle_seed, epoch_counter));
+    DRIL_TRY(update_async(p, b, h, epochs, batch_size, shuffle_seed, epoch_counter, false));
     DRIL_CUDA(cudaEventRecord(p->ev[2], c->stream));
     DRIL_TRY(ev_async(p, b));
     dril_iter_stats s;
@@ -2574,11 +2609,14 @@ extern "C" int32_t dril_ppo_iteration_async(dril_env* e, dril_policy* p, dril_bu
     const bool dp = c->nranks > 1;
     double* ev = dp ? e->xr : p->ev_acc;
     DRIL_CUDA(cudaMemsetAsync(ev, 0, 32, c->stream));
-    DRIL_TRY(gae_async(c, b->d, h->gamma, h->gae_lambda, ev));   // + explained-variance moments (ppo.jl:256)
+    // + explained-variance moments (ppo.jl:256) and, for a tcgen05 update, the sample records
+    const bool recs = ftg_active(p) || ft_active(p);
+    if (recs) DRIL_TRY(ensure_ft_recs(p, b->d, b->d.T * b->d.N));
+    DRIL_TRY(gae_async(c, b->d, h->gamma, h->gae_lambda, ev, recs ? p->ft_recs : nullptr, p->ft_rec_stride));
     DRIL_TRY(launch_monitor_finalize(e, b));
     if (dp) DRIL_TRY(dp_rollout_pack(e));
     DRIL_CUDA(cudaEventRecord(sl.ev[1], c->stream));
-    DRIL_TRY(update_async(p, b, h, epochs, batch_size, shuffle_seed, epoch_counter, ev, dp ? 4 + dp_xr_count(e) : 4));
+    DRIL_TRY(update_async(p, b, h, epochs, batch_size, shuffle_seed, epoch_counter, recs, ev, dp ? 4 + dp_xr_count(e) : 4));
     if (dp) DRIL_TRY(dp_rollout_merge(e));
     DRIL_CUDA(cudaEventRecord(sl.ev[2], c->stream));
     {

@@ -144,13 +144,45 @@ __global__ void __launch_bounds__(256) ft_permute_kernel(const float* __restrict
         ft_permute_slot(recs, stride, fk, n_total, batch_size, per, mb, s - mb * per, identity, act_start, nout, out, valid);
     }
 }
+// What the all-epochs permute kernels (ft_permute_epochs_kernel, ftg_permute_epochs_kernel) do besides the tile records.
+struct PermuteTail {
+    double* mbstats;      // the minibatch advantage moments, summed from the partials by the launch's last block; null: not wanted
+    unsigned* ticket;     // blocks of the running launch that have written their partials (0 between launches)
+    double* iter_acc;     // non-null: the update's first launch zeroes iter_acc[0 .. 11] and *stop_flag (update.cuh ITER_ACC_N)
+    int* stop_flag;
+};
+// Called by every thread after thread 0 wrote this block's partial.  The last block to arrive sums the partials of every
+// minibatch in adv_stats_finalize_kernel's order, so mbstats is the same bit for bit.
+__device__ __forceinline__ void permute_epochs_finish(const PermuteTail& pt, const double* partial) {
+    __shared__ bool last;
+    if (pt.iter_acc && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0) {
+        if (threadIdx.x < 12) pt.iter_acc[threadIdx.x] = 0.0;
+        if (threadIdx.x == 0) *pt.stop_flag = 0;
+    }
+    if (!pt.mbstats) return;
+    if (threadIdx.x == 0) {
+        __threadfence();
+        last = atomicAdd(pt.ticket, 1u) == gridDim.x * gridDim.y * gridDim.z - 1;
+    }
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    const int bpm = gridDim.x, n = gridDim.y * gridDim.z * 2;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const int mb = i >> 1, c = i & 1;
+        double s = 0;
+        for (int b = 0; b < bpm; ++b) s += __ldcg(partial + ((size_t)mb * bpm + b) * 2 + c);
+        pt.mbstats[i] = s;
+    }
+    if (threadIdx.x == 0) *pt.ticket = 0;
+}
 // ALL epochs of an update in one launch, grid (blocks per minibatch, minibatches, epochs): epoch e's records start at tile
 // e * epoch_tiles; the same pass accumulates the minibatch's advantage moments (what adv_stats_kernel computes for the other
-// loss/grad kernels, same partial layout: fixed-order sums => deterministic)
+// loss/grad kernels, same partial layout: fixed-order sums => deterministic) and finishes them (permute_epochs_finish)
 __global__ void __launch_bounds__(256) ft_permute_epochs_kernel(const float* __restrict__ recs, int stride, const __grid_constant__ FeistelKeys fks,
                                                                 long long n_total, long long batch_size, int tiles_per_mb, int act_start,
                                                                 int nout, unsigned char* __restrict__ out, long long epoch_tiles,
-                                                                double* __restrict__ partial) {
+                                                                double* __restrict__ partial, const PermuteTail pt) {
     __shared__ double scratch[32];
     const FeistelKey& fk = fks.k[blockIdx.z];
     const long long per = (long long)tiles_per_mb * FT_TS, mb = blockIdx.y;
@@ -166,6 +198,7 @@ __global__ void __launch_bounds__(256) ft_permute_epochs_kernel(const float* __r
         double* pp = partial + (((size_t)blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 2;
         pp[0] = sm; pp[1] = sq;
     }
+    permute_epochs_finish(pt, partial);
 }
 
 __device__ __forceinline__ uint32_t ft_idesc(int M, int N, int a_mn, int b_mn) {      // kind::f16: F16 x F16 -> F32

@@ -122,7 +122,7 @@ __global__ void __launch_bounds__(256) ftg_permute_kernel(const float* __restric
 __global__ void __launch_bounds__(256) ftg_permute_epochs_kernel(const float* __restrict__ recs, int stride, int D, const __grid_constant__ FeistelKeys fks,
                                                                  long long n_total, long long batch_size, int tiles_per_mb, int act_start, int act_n,
                                                                  int cont, int rec_floats, float* __restrict__ out, long long epoch_tiles,
-                                                                 double* __restrict__ partial) {
+                                                                 double* __restrict__ partial, const PermuteTail pt) {
     __shared__ double scratch[32];
     const FeistelKey& fk = fks.k[blockIdx.z];
     const long long per = (long long)tiles_per_mb * 64, mb = blockIdx.y;
@@ -138,6 +138,7 @@ __global__ void __launch_bounds__(256) ftg_permute_epochs_kernel(const float* __
         double* pp = partial + (((size_t)blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 2;
         pp[0] = sm; pp[1] = sq;
     }
+    permute_epochs_finish(pt, partial);
 }
 
 __device__ __forceinline__ void ftg_st16(uint32_t taddr, const float* r) {
