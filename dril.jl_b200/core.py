@@ -501,6 +501,8 @@ class DevicePolicy:
         L.check(self.ctx.lib.dril_policy_set_opt_state(self.h, L.ptr(m), L.ptr(v), m.size, int(step)))
 
     def seed(self, seed, step_index=0):
+        """Key (64 bits) and counter of the SAMPLE stream.  The counter is 32 bits: step_index is kept mod 2**32, each
+        rollout (or chunk) of T steps advances it by T, and it wraps mod 2**32."""
         L.check(self.ctx.lib.dril_policy_seed(self.h, int(seed), int(step_index)))
 
     def _obs(self, obs):

@@ -340,6 +340,9 @@ int32_t dril_policy_get_params(dril_policy* p, float* flat, int64_t n);
 /* Adam moments + step (the reference never saves them; exposed for checkpointing) */
 int32_t dril_policy_get_opt_state(dril_policy* p, float* m, float* v, int64_t n, int64_t* step);
 int32_t dril_policy_set_opt_state(dril_policy* p, const float* m, const float* v, int64_t n, int64_t step);
+/* Key and counter of the policy's SAMPLE stream: the action of env gid at step t of a rollout is drawn from Philox block
+ * (gid, step_index + t, 0 | j/4, tag 2) under the 64-bit key `seed` (oracle/philox.py).  The sample counter is 32 bits:
+ * step_index is stored mod 2^32, every rollout or chunk of T steps advances it by T, and it wraps mod 2^32. */
 int32_t dril_policy_seed(dril_policy* p, uint64_t seed, uint64_t step_index);
 /* layer(obs, ps, st) -> actions, values, logprobs (layers/layer_forward.jl:3-13,30-39);
  * deterministic=1 gives mode.(ds) (layers/layer_methods.jl:3-26). actions: int64[B] | float[B][act_dim].

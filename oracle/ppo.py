@@ -92,7 +92,8 @@ def gae_timemajor(rewards, values, term, trunc, boot, last_values, gamma, gae_la
 def collect_rollout_timemajor(env, spec, flat, n_steps, policy_seed=0, step0=0, env_gid=None,
                               forced_actions=None):
     """Time-major restatement of trajectory.jl:22-78 (the device layout). Returns a dict of
-    [T,N,...] arrays + boot + last_values. `env` exposes observe()/act() (oracle.envs)."""
+    [T,N,...] arrays + boot + last_values + last_obs; term_obs [T,N,D] holds the terminal observation of
+    every truncated sample (zero elsewhere). `env` exposes observe()/act() (oracle.envs)."""
     N = env.n
     if env_gid is None:
         env_gid = np.arange(N)
@@ -104,7 +105,7 @@ def collect_rollout_timemajor(env, spec, flat, n_steps, policy_seed=0, step0=0, 
         rewards=np.zeros((n_steps, N), dtype=f32), values=np.zeros((n_steps, N), dtype=f32),
         logprobs=np.zeros((n_steps, N), dtype=f32),
         term=np.zeros((n_steps, N), dtype=bool), trunc=np.zeros((n_steps, N), dtype=bool),
-        boot=np.zeros((n_steps, N), dtype=f32),
+        boot=np.zeros((n_steps, N), dtype=f32), term_obs=np.zeros((n_steps, N, D), dtype=f32),
         episode_r=np.zeros((n_steps, N), dtype=f32), episode_l=np.zeros((n_steps, N), dtype=np.int64),
     )
     new_obs = env.observe()                                         # trajectory.jl:32
@@ -128,6 +129,7 @@ def collect_rollout_timemajor(env, spec, flat, n_steps, policy_seed=0, step0=0, 
         if trunc.any() and info.get("terminal_observation") is not None:   # :57-61
             tv = P.predict_values(spec, flat, info["terminal_observation"])
             buf["boot"][t] = np.where(trunc, tv, f32(0))
+            buf["term_obs"][t] = np.where(trunc[:, None], info["terminal_observation"], f32(0))
     buf["last_values"] = P.predict_values(spec, flat, new_obs)            # :65-70
     buf["last_obs"] = new_obs
     return buf

@@ -3,7 +3,8 @@
 It is the high-precision reference the loss/grad kernels are compared with block by block: ``loss64`` evaluates the loss,
 the seven statistics ``DevicePolicy.loss_grad`` returns and the flat gradient in float64 from the float32 inputs;
 ``grad_blocks`` splits a flat gradient into its parameter blocks (ComponentVector order of policy.py) and
-``assert_blocks_close`` compares every block with its own relative bound.
+``assert_blocks_close`` compares every block with its own relative bound.  ``sample_ref64`` is the sampling head (action
+drawn from the Philox stream, its log-probability and the value) in float64, the reference of sampled rollouts.
 """
 import numpy as np
 
@@ -54,6 +55,36 @@ def logp64(spec, flat, out, actions):
     a = np.asarray(actions, dtype=np.float32).reshape(len(out), spec.act_n).astype(np.float64)
     k = spec.act_n
     return -0.5 * (2 * ls.sum() + ((a - out) ** 2 * np.exp(-2 * ls)).sum(1) + k * np.log(2 * np.pi))
+
+
+def sample_ref64(spec, flat, obs, gid, step, seed, actions=None):
+    """float64 reference of the sampling head on observations `obs` [B][D]: sample i is drawn from the Philox SAMPLE stream
+    at (gid[i], step[i], seed), step already reduced mod 2**32.  Returns a dict:
+      out, values   float64 actor outputs (logits or means) and critic values (forward64)
+      actions       Discrete: the first action whose float64 cumulative probability is >= u, the last one if none is
+                    (categorical.jl:44-49); Box: mean64 + exp(log_std) * z, z the fp32 normals of philox.normals
+      margin        Discrete only: min_j |cum64_j - u|, how far u is from flipping the action under rounding of the cumsum
+      logp          logp64 of `actions` (the stored ones) when given"""
+    from . import philox
+    out, v = forward64(spec, flat, obs)
+    gid = np.asarray(gid, dtype=np.int64).reshape(-1)
+    step = np.asarray(step, dtype=np.int64).reshape(-1) & 0xFFFFFFFF
+    r = dict(out=out, values=v)
+    if spec.act_kind == "discrete":
+        z = out - out.max(axis=1, keepdims=True)
+        p = np.exp(z) / np.exp(z).sum(axis=1, keepdims=True)
+        cum = np.cumsum(p, axis=1)
+        u = philox.sample_uniform64(gid, step, seed)
+        ge = cum >= u[:, None]
+        r["actions"] = np.where(ge.any(axis=1), ge.argmax(axis=1), spec.act_n - 1).astype(np.int64) + spec.act_start
+        r["margin"] = np.abs(cum - u[:, None]).min(axis=1)
+    else:
+        ls = np.asarray(flat, dtype=np.float32)[spec.n_params() - spec.act_n:].astype(np.float64)
+        z = philox.normals(gid, step, spec.act_n, seed).astype(np.float64)
+        r["actions"] = out + np.exp(ls) * z
+    if actions is not None:
+        r["logp"] = logp64(spec, flat, out, actions)
+    return r
 
 
 def loss64(spec, flat, obs, actions, adv, ret, old_lp, old_v, cfg):

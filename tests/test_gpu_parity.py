@@ -409,40 +409,6 @@ def test_syn_rollout_kernel_vs_oracle(D, obs_dim, hidden, n, T, per_thread):
     buf.close()
 
 
-def test_fused_rollout_sampling_consistency(D):
-    """Sampling mode: stored logprobs/values equal evaluate_actions on the stored (obs, actions)
-    (test/test_buffers.jl:3-27,166-214) and actions follow the Philox stream."""
-    for kind, n, T in (("cartpole", 500, 40), ("pendulum", 300, 30)):
-        env, oenv, spec = _mk(D, kind, n, 21, 20, True, False)
-        flat = OP.init_params(spec, seed=4)
-        layer = D.ActorCriticLayer(env.observation_space(), env.action_space(), hidden_dims=spec.hidden)
-        alg = D.PPO(n_steps=T)
-        agent = D.Agent(layer, alg, rng=np.random.default_rng(0))
-        agent.set_parameters(flat)
-        agent.device.seed(99, 5)
-        buf = D.RolloutBuffer(env.observation_space(), env.action_space(), alg.gae_lambda, alg.gamma, T, n)
-        D.collect_rollout(buf, agent, alg, env)
-        obs, act = buf.download("obs").reshape(T * n, -1), buf.download("actions").reshape(T * n, -1)
-        v, lp, _ = agent.device.evaluate(obs, act)
-        np.testing.assert_allclose(lp, buf.download("logprobs").reshape(-1), atol=1e-5)
-        np.testing.assert_allclose(v, buf.download("values").reshape(-1), atol=1e-6)
-        gid = np.tile(np.arange(n), T)
-        step = 5 + np.repeat(np.arange(T), n)
-        if kind == "cartpole":
-            probs = OP.softmax(OP.mlp_forward(OP.unflatten(spec, flat)["actor"], obs))
-            u = OPH.sample_uniform64(gid, step, 99)
-            ea = OP.categorical_sample(probs, u, spec.act_start)
-            margin = np.abs(np.cumsum(probs, axis=1) - u[:, None]).min(axis=1)
-            assert ((act[:, 0] == ea) | (margin < 1e-5)).all()
-            assert 0.3 < (act == 1).mean() < 0.7
-        else:
-            mean = OP.mlp_forward(OP.unflatten(spec, flat)["actor"], obs)
-            eps = OPH.normals(gid, step, 1, 99)
-            np.testing.assert_allclose(act, mean + eps, rtol=1e-5, atol=2e-6)
-            assert abs(eps.mean()) < 0.05 and abs(eps.std() - 1) < 0.05
-        buf.close()
-
-
 # ------------------------------------------------------------------------------------------
 # (c) PPO loss + gradients, optimiser, full update
 # ------------------------------------------------------------------------------------------
