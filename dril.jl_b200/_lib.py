@@ -21,6 +21,11 @@ class NormCfg(C.Structure):
                 ("clip_reward", c_f32), ("gamma", c_f32), ("epsilon", c_f32)]
 
 
+class AdrParam(C.Structure):
+    _fields_ = [("index", c_i32), ("init_lo", c_f32), ("init_hi", c_f32), ("limit_lo", c_f32), ("limit_hi", c_f32),
+                ("delta", c_f32)]
+
+
 class PPOHyper(C.Structure):
     _fields_ = [("gamma", c_f32), ("gae_lambda", c_f32), ("clip_range", c_f32), ("clip_range_vf", c_f32),
                 ("ent_coef", c_f32), ("vf_coef", c_f32), ("max_grad_norm", c_f32), ("target_kl", c_f32),
@@ -82,6 +87,8 @@ PROTOTYPES = {
     "dril_env_set_obs_history": [P, c_i32, c_i32],
     "dril_env_set_obs_noise": [P, c_i32, P],
     "dril_env_set_action_delay": [P, P],
+    "dril_env_set_adr": [P, c_i32, P, c_f32, c_i64, c_f32, c_f32],
+    "dril_env_get_adr": [P, P, P, P, P, C.POINTER(c_i64)],
     "dril_policy_create": [P, c_i32, c_i32, P, c_i32, c_i32, c_i32, P, P, C.POINTER(P)],
     "dril_policy_destroy": [P],
     "dril_policy_num_params": [P, C.POINTER(c_i64)],

@@ -24,13 +24,16 @@ BroadcastedParallelEnv = MultiThreadedParallelEnv
 
 def _rewrap(env, **over):
     """The env re-created with `over` switched on: state and step counters are carried over through set_state, which, like
-    dril_env_set_state, restarts an observation history from each env's current frame."""
+    dril_env_set_state, restarts an observation history from each env's current frame.  Automatic domain randomisation is
+    turned on again from its configuration (adr_config): the ranges it reached and its buffers restart at round 0, so wrap
+    before training."""
     args = dict(kind=env.kind, n_envs=env.n_envs, max_steps=env.max_steps, obs_dim=env.obs_dim,
                 act_start=env.act_start, ctx=env.ctx, monitor_window=env.monitor_window,
                 normalize=env.normalize, gid_offset=env.gid_offset, scaling=env.scaling,
                 obs_shape=env.obs_shape if len(env.obs_shape) > 1 else None, env_params=env.env_param_ranges(),
                 observe_params=env.observes_params(), history_len=env.history_len(),
-                mask_velocities=env.masks_velocities(), obs_noise=env.obs_noise(), action_delay=env.action_delay())
+                mask_velocities=env.masks_velocities(), obs_noise=env.obs_noise(), action_delay=env.action_delay(),
+                adr=env.adr_config())
     args.update(over)
     kind, n = args.pop("kind"), args.pop("n_envs")
     st, steps = env.get_state()

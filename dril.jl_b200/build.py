@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdril_b200.so")
 SOURCES = ["api.cu"]
-HEADERS = ["common.cuh", "env.cuh", "mlp.cuh", "mma_tiles.cuh", "rollout.cuh", "rollout_tc.cuh", "rollout_syn.cuh", "rollout_gtc.cuh", "gae.cuh", "update.cuh", "update_tc.cuh", "update_ft.cuh", "update_ftg.cuh",
+HEADERS = ["common.cuh", "env.cuh", "mlp.cuh", "mma_tiles.cuh", "rollout.cuh", "rollout_tc.cuh", "rollout_syn.cuh", "rollout_gtc.cuh", "gae.cuh", "update.cuh", "update_tc.cuh", "update_ft.cuh", "update_ftg.cuh", "adr.cuh",
            os.path.join("..", "..", "include", "dril_b200.h")]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "--cudart", "static"]
 

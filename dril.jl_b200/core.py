@@ -156,7 +156,7 @@ class CudaBatchedEnv:
 
     def __init__(self, kind, n_envs, max_steps=0, obs_dim=0, act_start=1, seed=None, ctx=None,
                  monitor_window=0, normalize=None, gid_offset=0, obs_shape=None, scaling=False, env_params=None,
-                 observe_params=False, history_len=1, mask_velocities=False, obs_noise=None, action_delay=0):
+                 observe_params=False, history_len=1, mask_velocities=False, obs_noise=None, action_delay=0, adr=None):
         self.kind = kind.lower()
         assert self.kind in ENV_KINDS, f"unknown env kind {kind}"
         self.ctx = ctx or Context.default()
@@ -236,6 +236,9 @@ class CudaBatchedEnv:
             self.set_obs_noise(obs_noise)
         if np.any(np.asarray(action_delay) != 0):
             self.set_action_delay(action_delay)
+        self._adr = None
+        if adr is not None:
+            self.set_adr(**adr)
         if seed is not None:
             self.seed(seed)
             self.reset()
@@ -362,6 +365,54 @@ class CudaBatchedEnv:
     def action_delay(self):
         """(n_envs,) int32 delays, or 0 without action delay."""
         return 0 if self._action_delay is None else self._action_delay.copy()
+
+    # ---- automatic domain randomisation ----
+    def set_adr(self, params=None, p_boundary=0.2, buffer_size=64, thresholds=None):
+        """Automatic domain randomisation (include/dril_b200.h has the rules).  `params`: {name: dict(init=(lo, hi),
+        limits=(lo, hi), step=delta)} for the parameters whose ranges ADR moves; None turns ADR off, leaving every env at the
+        ranges it reached.  `thresholds` = (t_low, t_high) in episode-return units: after every collected rollout a boundary
+        whose last `buffer_size` episodes (played by the fraction `p_boundary` of envs pinned to it) average >= t_high moves
+        outwards by its step, <= t_low inwards (never inside the initial range).  Needs a Monitor (monitor_window > 0).
+        adr_state() lists the parameters in the order of `params`.  Calling it again while ADR is on first turns the previous
+        configuration off."""
+        lib = self.ctx.lib
+        if params is None:
+            L.check(lib.dril_env_set_adr(self.h, 0, None, 0.0, 1, 0.0, 1.0))
+            self._adr = None
+            return
+        names = [nm for nm, _ in ENV_PARAMS[self.kind]]
+        unknown = set(params) - set(names)
+        assert not unknown, f"{self.kind} has no parameter(s) {sorted(unknown)}; it has {names}"
+        assert thresholds is not None and len(thresholds) == 2, "thresholds=(t_low, t_high) is required"
+        arr = (L.AdrParam * max(len(params), 1))()
+        for i, (nm, q) in enumerate(params.items()):
+            (il, ih), (ll, lh) = q["init"], q["limits"]
+            arr[i] = L.AdrParam(names.index(nm), il, ih, ll, lh, q["step"])
+        L.check(lib.dril_env_set_adr(self.h, len(params), arr, float(p_boundary), int(buffer_size), float(thresholds[0]),
+                                     float(thresholds[1])))
+        self._adr = dict(params={nm: dict(q) for nm, q in params.items()}, p_boundary=p_boundary, buffer_size=buffer_size,
+                         thresholds=tuple(thresholds))
+
+    def adr_config(self):
+        """The keyword arguments of the last set_adr, or None without ADR."""
+        return None if self._adr is None else dict(self._adr)
+
+    def adr_state(self):
+        """{"ranges": {name: (lo, hi)}, "counts": {name: (low side, high side)}, "means": {name: (low, high)} (the mean return
+        of the episodes each boundary has buffered since its last move, NaN while empty), "round": rollouts since ADR started}"""
+        assert self._adr is not None, "ADR is off"
+        names = list(self._adr["params"])
+        k = len(names)
+        lo, hi = np.empty(k, np.float32), np.empty(k, np.float32)
+        sums, counts = np.empty(2 * k, np.float64), np.empty(2 * k, np.int64)
+        r = L.c_i64(0)
+        L.check(self.ctx.lib.dril_env_get_adr(self.h, L.ptr(lo), L.ptr(hi), L.ptr(sums), L.ptr(counts), C.byref(r)))
+        with np.errstate(invalid="ignore", divide="ignore"):
+            means = np.where(counts > 0, sums / np.maximum(counts, 1), np.nan)
+        return dict(ranges={nm: (float(lo[i]), float(hi[i])) for i, nm in enumerate(names)},
+                    counts={nm: (int(counts[2 * i]), int(counts[2 * i + 1])) for i, nm in enumerate(names)},
+                    means={nm: (float(means[2 * i]), float(means[2 * i + 1])) for i, nm in enumerate(names)},
+                    sums=sums, round=int(r.value))
 
     # ---- per-env physical parameters ----
     def observes_params(self):

@@ -21,6 +21,7 @@
 #include "rollout_tc.cuh"
 #include "rollout_syn.cuh"
 #include "rollout_gtc.cuh"
+#include "adr.cuh"
 
 #define DRIL_SMEM_MAX 232448  // 227 KB opt-in per CTA on sm_100
 #define DRIL_RESULT_SLOTS 4   // iterations that may be enqueued before their results are read
@@ -264,6 +265,12 @@ struct dril_env {
                                      // k > 1 or velocities masked) or 0: the observation layout, as a kind-set bit
     bool default_params = false;     // parameters held at lo = hi = the defaults only because obs_ks is set or the env is perturbed
     bool observed = false;           // an observation was made (observe, step, rollout, evaluate): the width is fixed
+    // automatic domain randomisation (dril_env_set_adr): configuration, device state, attribution words, scan partials
+    bool adr_on = false;
+    AdrCfg adr_cfg;
+    AdrState* adr_state = nullptr;
+    AdrEnv adr_env = {nullptr, nullptr};
+    double* adr_part = nullptr;      // [adr_grid][2 * 2 n]
 };
 // observation noise or action delay on: the ENV_KS_PERTURB kernels
 static bool env_perturbed(const dril_env* e) { return e->d.obs_noise || e->d.act_delay; }
@@ -1100,7 +1107,7 @@ static int32_t env_alloc_obs_arrays(dril_env* e) {
     DRIL_TRY(dmalloc(&d.obs_mean, D)); DRIL_TRY(dmalloc(&d.obs_var, D));
     DRIL_TRY(dmalloc(&d.partials, (size_t)2 * e->max_blocks * (2 * D + 2)));
     DRIL_TRY(dmalloc(&e->roll_moments, (size_t)2 * (D + 1) + 2));     // handed to the kernels only in data-parallel runs
-    DRIL_TRY(dmalloc(&e->xr, (size_t)4 + 3 + 2 * (D + 1) + 2));
+    DRIL_TRY(dmalloc(&e->xr, (size_t)4 + 3 + 2 * (D + 1) + 2 + 2 * ADR_MAX_SLOTS));   // + the ADR tail (adr_roll)
     DRIL_TRY(dmalloc(&e->norm_snap, (size_t)2 * D + 2));
     {
         std::vector<float> ones(D, 1.0f);
@@ -1141,10 +1148,28 @@ extern "C" int32_t dril_env_destroy(dril_env* e) {
     void* ps[] = {d.state, d.steps, d.episode, d.life, d.tobs, d.old_obs, d.old_rewards, d.ep_ret, d.ep_len, d.roll_sums,
                   d.roll_eps, d.ret, d.obs_mean, d.obs_var, d.ret_stats, d.counts, d.partials, e->ring.ret, e->ring.len,
                   e->ring.head, e->ring.ticket, e->compat_actions, e->compat_obs, e->roll_moments, e->xr, e->norm_snap, e->norm_snap_cnt,
-                  d.pval, d.plo, d.phi, d.hist, d.obs_noise, d.act_delay, d.act_q};
+                  d.pval, d.plo, d.phi, d.hist, d.obs_noise, d.act_delay, d.act_q, e->adr_state, e->adr_env.ep_mark,
+                  e->adr_env.run_slot, e->adr_part};
     for (void* p : ps) if (p) cudaFree(p);
     dril_buffer_destroy(e->compat);
     delete e;
+    return DRIL_OK;
+}
+// the current round's ranges of the ADR parameters rewritten from the device state (adr_write_kernel's modes)
+static int32_t adr_rewrite(dril_env* e, int mode) {
+    dril_ctx* c = e->ctx;
+    AdrState st;
+    DRIL_CUDA(cudaMemcpyAsync(&st, e->adr_state, sizeof(st), cudaMemcpyDeviceToHost, c->stream));
+    DRIL_CUDA(cudaStreamSynchronize(c->stream));
+    AdrRanges r;
+    memcpy(r.lo, st.lo, sizeof(r.lo)); memcpy(r.hi, st.hi, sizeof(r.hi));
+    {
+        Span sp(c, DRIL_K_ENV);
+        adr_write_kernel<<<(unsigned)((e->d.n_envs + ADR_THREADS - 1) / ADR_THREADS), ADR_THREADS, 0, c->stream>>>(
+            e->adr_cfg, r, e->d, e->adr_env, st.round, mode);
+        DRIL_CUDA(cudaGetLastError());
+    }
+    DRIL_CUDA(cudaStreamSynchronize(c->stream));
     return DRIL_OK;
 }
 extern "C" int32_t dril_env_seed(dril_env* e, uint64_t seed) {
@@ -1154,6 +1179,8 @@ extern "C" int32_t dril_env_seed(dril_env* e, uint64_t seed) {
     DRIL_CUDA(cudaMemsetAsync(e->d.episode, 0, (size_t)e->d.n_envs * 4, e->ctx->stream));
     DRIL_CUDA(cudaMemsetAsync(e->d.life, 0, (size_t)e->d.n_envs * 4, e->ctx->stream));
     DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
+    // the boundary envs of the current round are a function of the seed: pins and attribution restart under the new one
+    if (e->adr_on) DRIL_TRY(adr_rewrite(e, ADR_WRITE_RESEED));
     return DRIL_OK;
 }
 extern "C" int32_t dril_env_reset(dril_env* e) {
@@ -1170,8 +1197,13 @@ extern "C" int32_t dril_env_reset(dril_env* e) {
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
     return env_restart(e);
 }
+static int32_t env_set_params(dril_env* e, int32_t n_params, const float* lo, const float* hi);
 extern "C" int32_t dril_env_set_params(dril_env* e, int32_t n_params, const float* lo, const float* hi) {
     DRIL_REQUIRE(e, "NULL argument");
+    DRIL_REQUIRE(!e->adr_on, "the parameter ranges belong to automatic domain randomisation while it is on (dril_env_set_adr)");
+    return env_set_params(e, n_params, lo, hi);
+}
+static int32_t env_set_params(dril_env* e, int32_t n_params, const float* lo, const float* hi) {
     EnvDev& d = e->d;
     const int np = env_n_params(d.kind);
     DRIL_REQUIRE(np > 0, "env kind %d has no physical parameters", d.kind);
@@ -1240,8 +1272,8 @@ extern "C" int32_t dril_env_get_params(dril_env* e, int32_t n_params, float* val
 // An env with an observation layout option, observation noise or action delay runs the parametrised kernels: without ranges it
 // holds lo = hi = the defaults, which it drops again with the last such option.
 static int32_t env_hold_default_params(dril_env* e) {
-    const bool need = e->obs_ks || env_perturbed(e);
-    if ((need && !e->d.has_params) || (!need && e->default_params)) DRIL_TRY(dril_env_set_params(e, env_n_params(e->d.kind), nullptr, nullptr));
+    const bool need = e->obs_ks || env_perturbed(e) || e->adr_on;
+    if ((need && !e->d.has_params) || (!need && e->default_params)) DRIL_TRY(env_set_params(e, env_n_params(e->d.kind), nullptr, nullptr));
     return DRIL_OK;
 }
 // the observation layout: obs_ks (0, ENV_KS_OBS_PARAMS or ENV_KS_HISTORY), the history's k and frame width, the observation width
@@ -1334,6 +1366,112 @@ extern "C" int32_t dril_env_set_action_delay(dril_env* e, const int32_t* delay) 
     for (int32_t& v : dq) v |= ENV_DELAY_RESTART;
     DRIL_CUDA(cudaMemcpy(d.act_delay, dq.data(), n * 4, cudaMemcpyHostToDevice));
     return env_hold_default_params(e);
+}
+extern "C" int32_t dril_env_set_adr(dril_env* e, int32_t n, const dril_adr_param* params, float p_boundary, int64_t buffer_size,
+                                    float t_low, float t_high) {
+    DRIL_REQUIRE(e, "NULL argument");
+    EnvDev& d = e->d;
+    const int np = env_n_params(d.kind);
+    if (np == 0) { dril_set_error("env kind %d has no parameters to randomise", d.kind); return DRIL_ERR_UNSUPPORTED; }
+    dril_ctx* c = e->ctx;
+    DRIL_CUDA(cudaSetDevice(c->device));
+    DRIL_CUDA(cudaStreamSynchronize(c->stream));
+    const size_t N = (size_t)d.n_envs;
+    const unsigned grid = (unsigned)((N + ADR_THREADS - 1) / ADR_THREADS);
+    if (!params) {   // off: every env at [lo_j, hi_j], no pins; the ranges stay the env's
+        if (!e->adr_on) return DRIL_OK;
+        DRIL_TRY(adr_rewrite(e, ADR_WRITE_OFF));
+        e->adr_on = false;
+        return DRIL_OK;
+    }
+    DRIL_REQUIRE(d.monitor, "automatic domain randomisation measures the Monitor's episode returns: the env needs a MonitorWrapperEnv");
+    DRIL_REQUIRE(n >= 1 && n <= np, "env kind %d has %d parameters, got %d under ADR", d.kind, np, n);
+    DRIL_REQUIRE(std::isfinite(p_boundary) && p_boundary >= 0.f && p_boundary <= 1.f, "p_boundary %g outside [0, 1]", (double)p_boundary);
+    DRIL_REQUIRE(buffer_size >= 1, "buffer_size %lld < 1", (long long)buffer_size);
+    DRIL_REQUIRE(std::isfinite(t_low) && std::isfinite(t_high) && t_low < t_high, "thresholds (%g, %g): need finite t_low < t_high",
+                 (double)t_low, (double)t_high);
+    AdrCfg cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.n = n; cfg.p_boundary = p_boundary; cfg.m = buffer_size; cfg.t_low = t_low; cfg.t_high = t_high;
+    for (int i = 0; i < n; ++i) {
+        const dril_adr_param& q = params[i];
+        DRIL_REQUIRE(q.index >= 0 && q.index < np, "ADR parameter %d: index %d outside [0, %d)", i, q.index, np);
+        for (int j = 0; j < i; ++j) DRIL_REQUIRE(params[j].index != q.index, "parameter %d is under ADR twice", q.index);
+        DRIL_REQUIRE(std::isfinite(q.init_lo) && std::isfinite(q.init_hi) && std::isfinite(q.limit_lo) && std::isfinite(q.limit_hi) &&
+                     std::isfinite(q.delta), "ADR parameter %d: values must be finite", q.index);
+        DRIL_REQUIRE(q.limit_lo <= q.init_lo && q.init_lo <= q.init_hi && q.init_hi <= q.limit_hi,
+                     "ADR parameter %d: need limit_lo <= init_lo <= init_hi <= limit_hi", q.index);
+        const bool pos = k_env_param_positive[d.kind][q.index] != 0;
+        DRIL_REQUIRE(pos ? q.limit_lo > 0.f : q.limit_lo >= 0.f, "ADR parameter %d: limit_lo %g must be %s 0", q.index,
+                     (double)q.limit_lo, pos ? ">" : ">=");
+        DRIL_REQUIRE(q.delta > 0.f, "ADR parameter %d: delta %g must be > 0", q.index, (double)q.delta);
+        cfg.idx[i] = q.index;
+        cfg.init_lo[i] = q.init_lo; cfg.init_hi[i] = q.init_hi; cfg.limit_lo[i] = q.limit_lo; cfg.limit_hi[i] = q.limit_hi;
+        cfg.delta[i] = q.delta;
+    }
+    // the ranges outside J stay (the defaults without ranges; a reconfiguration first unpins the previous J); J starts at the
+    // initial ranges
+    if (e->adr_on) {
+        DRIL_TRY(adr_rewrite(e, ADR_WRITE_OFF));
+        e->adr_on = false;
+    }
+    std::vector<float> lo(N * np), hi(N * np);
+    if (d.has_params) {
+        DRIL_CUDA(cudaMemcpy(lo.data(), d.plo, N * np * 4, cudaMemcpyDeviceToHost));
+        DRIL_CUDA(cudaMemcpy(hi.data(), d.phi, N * np * 4, cudaMemcpyDeviceToHost));
+    } else {
+        for (int k = 0; k < np; ++k) {
+            std::fill(lo.begin() + (size_t)k * N, lo.begin() + (size_t)(k + 1) * N, env_param_default(d.kind).v[k]);
+            std::fill(hi.begin() + (size_t)k * N, hi.begin() + (size_t)(k + 1) * N, env_param_default(d.kind).v[k]);
+        }
+    }
+    AdrRanges r0;
+    memset(&r0, 0, sizeof(r0));
+    for (int i = 0; i < n; ++i) {
+        std::fill(lo.begin() + (size_t)cfg.idx[i] * N, lo.begin() + (size_t)(cfg.idx[i] + 1) * N, cfg.init_lo[i]);
+        std::fill(hi.begin() + (size_t)cfg.idx[i] * N, hi.begin() + (size_t)(cfg.idx[i] + 1) * N, cfg.init_hi[i]);
+        r0.lo[i] = cfg.init_lo[i]; r0.hi[i] = cfg.init_hi[i];
+    }
+    DRIL_TRY(env_set_params(e, np, lo.data(), hi.data()));
+    if (!e->adr_state) {
+        DRIL_TRY(dmalloc(&e->adr_state, 1));
+        DRIL_TRY(dmalloc(&e->adr_env.ep_mark, N));
+        DRIL_TRY(dmalloc(&e->adr_env.run_slot, N));
+        DRIL_TRY(dmalloc(&e->adr_part, (size_t)grid * 2 * ADR_MAX_SLOTS));
+    }
+    AdrState st;
+    memset(&st, 0, sizeof(st));
+    memcpy(st.lo, r0.lo, sizeof(st.lo)); memcpy(st.hi, r0.hi, sizeof(st.hi));
+    DRIL_CUDA(cudaMemcpy(e->adr_state, &st, sizeof(st), cudaMemcpyHostToDevice));
+    e->adr_cfg = cfg;
+    e->adr_on = true;
+    {   // round 0 with its boundary envs, the running episodes redrawn from it, the attribution words started
+        Span sp(c, DRIL_K_ENV);
+        adr_write_kernel<<<grid, ADR_THREADS, 0, c->stream>>>(cfg, r0, d, e->adr_env, 0, ADR_WRITE_ON);
+        env_params_draw_kernel<<<grid, ADR_THREADS, 0, c->stream>>>(d);
+        DRIL_CUDA(cudaGetLastError());
+    }
+    DRIL_CUDA(cudaStreamSynchronize(c->stream));
+    return DRIL_OK;
+}
+extern "C" int32_t dril_env_get_adr(dril_env* e, float* lo, float* hi, double* sums, int64_t* counts, int64_t* round) {
+    DRIL_REQUIRE(e, "NULL argument");
+    DRIL_REQUIRE(e->adr_on, "the env has no automatic domain randomisation");
+    DRIL_CUDA(cudaSetDevice(e->ctx->device));
+    AdrState st;
+    DRIL_CUDA(cudaMemcpyAsync(&st, e->adr_state, sizeof(st), cudaMemcpyDeviceToHost, e->ctx->stream));
+    DRIL_CUDA(cudaStreamSynchronize(e->ctx->stream));
+    const int n = e->adr_cfg.n;
+    for (int i = 0; i < n; ++i) {
+        if (lo) lo[i] = st.lo[i];
+        if (hi) hi[i] = st.hi[i];
+    }
+    for (int s = 0; s < 2 * n; ++s) {
+        if (sums) sums[s] = st.sum[s];
+        if (counts) counts[s] = st.cnt[s];
+    }
+    if (round) *round = st.round;
+    return DRIL_OK;
 }
 extern "C" int32_t dril_env_obs_dim(dril_env* e, int32_t* obs_dim) {
     DRIL_REQUIRE(e && obs_dim, "NULL argument");
@@ -1771,7 +1909,29 @@ static int32_t check_compat(dril_env* e, dril_policy* p, dril_buffer* b) {
 static bool dp_norm_active(const dril_env* e) {
     return e->ctx->nranks > 1 && e->d.normalize && e->d.training && (e->d.norm_obs || e->d.norm_reward);
 }
-static int dp_xr_count(const dril_env* e) { return 3 + 2 * (e->d.obs_dim + 1) + 2; }
+static int dp_xr_count(const dril_env* e) { return 3 + 2 * (e->d.obs_dim + 1) + 2 + (e->adr_on ? 4 * e->adr_cfg.n : 0); }
+// the rollout's ADR sums and counts [2 * 2 n]: the tail of the small exchange, so data-parallel runs sum it with the rest
+static double* adr_roll(const dril_env* e) { return e->xr + 4 + 3 + 2 * (e->d.obs_dim + 1) + 2; }
+static unsigned adr_grid(const dril_env* e) { return (unsigned)((e->d.n_envs + ADR_THREADS - 1) / ADR_THREADS); }
+// ADR after a collected rollout in b: attribution (before the exchange of the rollout's sums) ...
+static int32_t adr_scan(dril_env* e, dril_buffer* b) {
+    if (!e->adr_on) return DRIL_OK;
+    dril_ctx* c = e->ctx;
+    Span sp(c, DRIL_K_ENV);
+    adr_scan_kernel<<<adr_grid(e), ADR_THREADS, 0, c->stream>>>(e->adr_cfg, e->adr_state, e->d, e->adr_env, b->d.flags, b->d.episode_r,
+                                                                 b->d.T, e->adr_part, adr_roll(e));
+    DRIL_CUDA(cudaGetLastError());
+    return DRIL_OK;
+}
+// ... and the update with the next round's ranges (after it)
+static int32_t adr_update(dril_env* e) {
+    if (!e->adr_on) return DRIL_OK;
+    dril_ctx* c = e->ctx;
+    Span sp(c, DRIL_K_ENV);
+    adr_update_kernel<<<adr_grid(e), ADR_THREADS, 0, c->stream>>>(e->adr_cfg, e->adr_state, e->d, adr_roll(e));
+    DRIL_CUDA(cudaGetLastError());
+    return DRIL_OK;
+}
 static int32_t dp_rollout_begin(dril_env* e) {
     dril_ctx* c = e->ctx;
     e->d.roll_moments = nullptr;
@@ -1824,12 +1984,14 @@ extern "C" int32_t dril_rollout_collect(dril_env* e, dril_policy* p, dril_buffer
     DRIL_CUDA(cudaEventRecord(p->ev[0], c->stream));
     DRIL_TRY(rollout_async(e, p, b, forced_dev));
     DRIL_CUDA(cudaEventRecord(p->ev[1], c->stream));
+    DRIL_TRY(adr_scan(e, b));
     if (c->nranks > 1) {
         DRIL_TRY(dp_rollout_pack(e));
         DRIL_TRY(allreduce_small(c, nullptr, 0, e->xr + 4, dp_xr_count(e)));
         DRIL_TRY(dp_rollout_merge(e));
     }
     DRIL_TRY(launch_monitor_finalize(e, b));
+    DRIL_TRY(adr_update(e));
     unsigned long long eps = 0;
     DRIL_CUDA(cudaMemcpyAsync(&eps, e->d.roll_eps, 8, cudaMemcpyDeviceToHost, c->stream));
     DRIL_CUDA(cudaStreamSynchronize(c->stream));
@@ -1887,6 +2049,11 @@ extern "C" int32_t dril_rollout_collect_steps(dril_env* e, dril_policy* p, dril_
     p->step_index += (uint32_t)t_count;
     if (t_count > 0 && t_begin + t_count == b->d.T) {
         DRIL_TRY(launch_monitor_finalize(e, b));
+        if (e->adr_on) {
+            DRIL_TRY(adr_scan(e, b));
+            DRIL_TRY(allreduce_small(c, nullptr, 0, adr_roll(e), 4 * e->adr_cfg.n));
+            DRIL_TRY(adr_update(e));
+        }
         unsigned long long eps = 0;
         DRIL_CUDA(cudaMemcpyAsync(&eps, e->d.roll_eps, 8, cudaMemcpyDeviceToHost, c->stream));
         DRIL_CUDA(cudaStreamSynchronize(c->stream));
@@ -2614,10 +2781,12 @@ extern "C" int32_t dril_ppo_iteration_async(dril_env* e, dril_policy* p, dril_bu
     if (recs) DRIL_TRY(ensure_ft_recs(p, b->d, b->d.T * b->d.N));
     DRIL_TRY(gae_async(c, b->d, h->gamma, h->gae_lambda, ev, recs ? p->ft_recs : nullptr, p->ft_rec_stride));
     DRIL_TRY(launch_monitor_finalize(e, b));
+    DRIL_TRY(adr_scan(e, b));
     if (dp) DRIL_TRY(dp_rollout_pack(e));
     DRIL_CUDA(cudaEventRecord(sl.ev[1], c->stream));
     DRIL_TRY(update_async(p, b, h, epochs, batch_size, shuffle_seed, epoch_counter, recs, ev, dp ? 4 + dp_xr_count(e) : 4));
     if (dp) DRIL_TRY(dp_rollout_merge(e));
+    DRIL_TRY(adr_update(e));
     DRIL_CUDA(cudaEventRecord(sl.ev[2], c->stream));
     {
         IterRecordSrc src;

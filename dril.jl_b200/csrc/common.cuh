@@ -136,6 +136,7 @@ struct BufDev {
 #define DRIL_TAG_SYN_DYN 5u
 #define DRIL_TAG_ENV_PARAMS 6u
 #define DRIL_TAG_OBS_NOISE 7u
+#define DRIL_TAG_ADR 8u
 
 __host__ __device__ __forceinline__ void philox4x32(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                      unsigned long long seed, uint32_t out[4]) {

@@ -319,6 +319,53 @@ int32_t dril_env_set_obs_history(dril_env* env, int32_t history_len, int32_t mas
 int32_t dril_env_set_obs_noise(dril_env* env, int32_t n_comp, const float* std);
 int32_t dril_env_set_action_delay(dril_env* env, const int32_t* delay);
 
+/* Automatic domain randomisation (ADR; OpenAI et al., "Solving Rubik's Cube with a Robot Hand", 2019): parameter ranges that
+ * grow where the policy does well at their boundaries and shrink where it does badly, updated on the device after every
+ * collected rollout.
+ * Configuration: a set J of n parameters (table order above, distinct indices), each with an initial range
+ * [init_lo, init_hi], limits limit_lo <= init_lo <= init_hi <= limit_hi (finite; limit_lo obeys the sign rule of
+ * dril_env_set_params) and a step delta > 0; a boundary probability p_boundary in [0, 1], a buffer size m >= 1 and thresholds
+ * t_low < t_high in episode-return units.  The state (lo_j, hi_j, a fp64 return sum and an int64 count per slot, the round r)
+ * is global: identical for every env and, in data-parallel runs, on every rank.
+ *   - Slots: 2 n boundary slots, 2 i + 0 the low and 2 i + 1 the high side of the i-th ADR parameter.
+ *   - Assignment in round r: env gid is a boundary env when u01_f32(w0) < p_boundary, w = Philox block (gid, r mod 2^32, 0,
+ *     DRIL_TAG_ADR = 8); its slot is w1 mod 2 n.  A pure function of (seed, gid, r): sharding does not change it.
+ *   - Ranges of round r: every env has [lo_j, hi_j] for j in J, except that a boundary env of slot (j, side) has parameter j
+ *     pinned, lo = hi = (side ? hi_j : lo_j).  Parameters outside J keep what dril_env_set_params gave them (the defaults
+ *     without ranges).  New ranges take effect at each env's next reset; running episodes are not redrawn.
+ *   - Attribution: episodes that END inside a collected rollout (dril_rollout_collect, dril_ppo_iteration_async, the last
+ *     chunk of dril_rollout_collect_steps) count, with their Monitor return (episode_r: raw rewards, below Normalize), for
+ *     the slot in force when their parameters were drawn.  Per env, ep_mark holds the reset counter at the end of the previous
+ *     round and run_slot the slot of the episode running then: env n's k-th of d dones in the rollout ends episode
+ *     episode[n] - 1 - d + k, which belongs to the round's slot if >= ep_mark[n], else to run_slot[n].  Host reset!, compat
+ *     act! and dril_evaluate between rollouts keep this exact (their resets draw from the current round's ranges); episodes
+ *     that end outside a rollout are not counted.  A reset between the chunks of one chunked rollout is not supported.
+ *     dril_env_seed rewrites the current round's boundary envs under the new seed and restarts the attribution: episodes
+ *     running at that moment are not counted, every later one counts for the round in force.
+ *   - Update after round r (after the data-parallel merge, so on the global sums): the rollout's sums and counts are added;
+ *     every slot with count >= m takes mean = sum / count (fp64) and, from the state before this update, widens its side if
+ *     mean >= t_high (lo_j = max(limit_lo, lo_j - delta) | hi_j = min(limit_hi, hi_j + delta)) or narrows it if mean <= t_low,
+ *     never inside the initial range (lo_j = min(init_lo, lo_j + delta) | hi_j = max(init_hi, hi_j - delta)), fp32 add / sub
+ *     rounded to nearest; its sum and count restart from 0.  Then r += 1 and round r + 1's ranges are written.
+ * dril_env_set_adr: params == NULL turns ADR off and leaves every env at [lo_j, hi_j] without pins.  Turning it on validates;
+ * turning it on again first turns the previous configuration off (so a parameter that leaves J keeps [lo_j, hi_j]).  Either
+ * sets r = 0, the ranges to the initial ones, clears the accumulators, writes round 0's ranges and redraws the
+ * running episodes from them (like dril_env_set_params).  ADR needs a MonitorWrapperEnv and a valid configuration, else
+ * DRIL_ERR_INVALID; the synthetic env: DRIL_ERR_UNSUPPORTED.  While it is on, dril_env_set_params is DRIL_ERR_INVALID.  An env
+ * with ADR has parameters (lo = hi = the defaults outside J), so CartPole leaves the tensor-core rollout; ADR combines with
+ * observe_params, history, noise and delay.  Nothing is read back to the host, so pipelined iterations keep their depth.
+ * dril_env_get_adr: lo, hi float[n]; sums double[2 n], counts int64[2 n] (the accumulators since each slot's last decision);
+ * round; any may be NULL.  DRIL_ERR_INVALID without ADR. */
+typedef struct {
+    int32_t index;                   /* table index of the parameter */
+    float init_lo, init_hi;
+    float limit_lo, limit_hi;
+    float delta;
+} dril_adr_param;
+int32_t dril_env_set_adr(dril_env* env, int32_t n, const dril_adr_param* params, float p_boundary, int64_t buffer_size,
+                         float t_low, float t_high);
+int32_t dril_env_get_adr(dril_env* env, float* lo, float* hi, double* sums, int64_t* counts, int64_t* round);
+
 /* ---- actor-critic layer + optimiser state: replaces Discrete/ContinuousActorCriticLayer
  *      (layers/) and the Lux TrainState held by Agent (agents/agent_types.jl) ------------ */
 int32_t dril_policy_create(dril_ctx* ctx, int32_t obs_dim, int32_t n_hidden, const int32_t* hidden_dims,

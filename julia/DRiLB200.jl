@@ -209,6 +209,56 @@ function set_action_delay!(env::CudaBatchedEnv, delay)
     env
 end
 
+# dril_adr_param
+struct AdrParam
+    index::Int32
+    init_lo::Float32
+    init_hi::Float32
+    limit_lo::Float32
+    limit_hi::Float32
+    delta::Float32
+end
+
+"""
+    set_adr!(env, params; thresholds, p_boundary = 0.2, buffer_size = 64)
+    set_adr!(env, nothing)
+
+Automatic domain randomisation (include/dril_b200.h has the rules): `params = [:length => (init = (0.5, 0.5),
+limits = (0.1, 2.0), step = 0.05), ...]` (any iterable of `name => (init, limits, step)` pairs: its iteration order is the
+order of `adr_state`; a `Dict` iterates in no fixed order), `thresholds = (t_low, t_high)` in episode-return units (required).
+After every collected rollout a boundary whose last `buffer_size` episodes average `>= t_high` moves outwards by its step,
+`<= t_low` inwards (never inside the initial range).  `nothing` turns ADR off and leaves every env at the ranges it reached.
+Needs a Monitor.
+"""
+function set_adr!(env::CudaBatchedEnv, ::Nothing)
+    check(ccall((:dril_env_set_adr, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{AdrParam}, Float32, Int64, Float32, Float32),
+        env.h, 0, C_NULL, 0, 1, 0, 1))
+    env
+end
+function set_adr!(env::CudaBatchedEnv, params; thresholds, p_boundary = 0.2, buffer_size = 64)
+    names = [first(p) for p in ENV_PARAMS[env.kind]]
+    ps = [AdrParam(findfirst(==(k), names) - 1, q.init[1], q.init[2], q.limits[1], q.limits[2], q.step) for (k, q) in params]
+    check(ccall((:dril_env_set_adr, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{AdrParam}, Float32, Int64, Float32, Float32),
+        env.h, length(ps), ps, p_boundary, buffer_size, thresholds[1], thresholds[2]))
+    env
+end
+
+"""
+    adr_state(env, n) -> (lo, hi, sums, counts, round)
+
+The ADR state of an env with `n` parameters under ADR (in the iteration order of the `params` given to `set_adr!`): the ranges, the per-slot return
+sums and episode counts buffered since each slot's last decision (slot `2i - 1` the low and `2i` the high side of parameter i),
+and the number of rounds so far.
+"""
+function adr_state(env::CudaBatchedEnv, n::Integer)
+    lo, hi = zeros(Float32, n), zeros(Float32, n)
+    sums, counts = zeros(Float64, 2n), zeros(Int64, 2n)
+    r = Ref{Int64}(0)
+    check(ccall((:dril_env_get_adr, LIB), Int32, (Ptr{Cvoid}, Ptr{Float32}, Ptr{Float32}, Ptr{Float64}, Ptr{Int64}, Ref{Int64}),
+        env.h, lo, hi, sums, counts, r))
+    (lo, hi, sums, counts, r[])
+end
+
 """
     set_env_params!(env; length = (0.25, 1.0), masspole = 0.2, ...)
 
